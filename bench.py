@@ -169,8 +169,7 @@ def cpu_arm(cfg: dict, n_points: int, steps: int, warmup: int, sample_queries: i
     os.environ["OMP_NUM_THREADS"] = str(os.cpu_count() or 1)   # torchrun exports 1 to its workers
     from oracle import oracle as O
 
-    O.build()
-    O.set_num_threads(os.cpu_count() or 1)
+    O.set_num_threads(os.cpu_count() or 1)   # liboracle.so comes from build(): the benchmark compiles nothing in the tree
     x = _cpu_cloud(cfg, n_points)
     t0 = time.perf_counter()
     tree = O.KdTree(x, leaf=8)
@@ -307,6 +306,27 @@ def roofline_block(t, wl, cfg, cs, nq, n_points, n_nodes, kern_ms_per_step, ms_p
 # --------------------------------------------------------------------------------------------------
 # GPU arm
 # --------------------------------------------------------------------------------------------------
+DUMP_BYTES = 60_000_000   # array bytes of --dump-outputs: with the .npy headers, under 64 MB
+
+
+def dump_outputs(path, qid, idx, dist, rank, world):
+    """Write the rows one search step returned (query ids, neighbour indices, distances) as DIR/<name>.npy, for comparing
+    two builds output for output.  Rows are taken in query-id order, so the files do not depend on the order the engine
+    emits rows in; when all rows exceed DUMP_BYTES (over all ranks), a fixed seeded sample of them is written.  Ids and
+    indices are stored as float64, which holds every int32 exactly.  With several ranks each writes its own files."""
+    import torch
+
+    n, k = int(idx.shape[0]), int(idx.shape[1])
+    m = min(n, DUMP_BYTES // ((8 + 8 * k + 4 * k) * world))
+    pick = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, m, replace=False))).to(qid.device)
+    rows = torch.argsort(qid.long())[pick]
+    suffix = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("query_ids", qid[rows].double()), ("neighbour_indices", idx[rows].double()),
+                    ("neighbour_distances", dist[rows].float())):
+        np.save(os.path.join(path, f"{name}{suffix}.npy"), a.cpu().numpy())
+
+
 def run_gpu(args):
     # ONE JSON line on stdout: whatever libraries print there (NCCL announces its version on stdout when a communicator
     # is created) goes to stderr; the line itself is written to the saved descriptor at the end
@@ -431,6 +451,8 @@ def run_gpu(args):
     ms_per_step = elapsed_ms / args.steps
     value = total_queries / (ms_per_step * 1e-3)
     sm_mhz = sampler.sm_mhz_so_far() if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, q_r, i_r, d_r, rank, world)   # before any later search reuses the buffers
 
     # ---- in-bench correctness: sampled rows against the exact GPU brute force, at every N ----
     if partition:
@@ -690,7 +712,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-single", action="store_true", help="N > 1 strong scaling: skip the single-GPU run of the same workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's results (a seeded sample, <= 64 MB) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU search's results; it does not apply to --impl reference")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     if args.impl == "reference":

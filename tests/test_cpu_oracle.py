@@ -226,10 +226,10 @@ def test_option_keys_match_header():
     assert sorted(TrueKNN._OPTS.values()) == sorted(keys.values())
 
 
-def test_stats_struct_layout_matches_header():
+def test_stats_struct_layout_matches_header(tmp_path):
     src = "#include <stdio.h>\n#include \"trueknn.h\"\nint main(){printf(\"%zu %zu %zu\", sizeof(tknn_stats), " \
           "__builtin_offsetof(tknn_stats, round_ms), __builtin_offsetof(tknn_stats, h2d_bytes));return 0;}"
-    exe = "/tmp/tknn_layout"
+    exe = str(tmp_path / "tknn_layout")
     subprocess.run(["/usr/bin/gcc", "-x", "c", "-", "-I", os.path.join(ROOT, "include"), "-o", exe], input=src, text=True,
                    check=True)
     size, off_round, off_h2d = (int(v) for v in subprocess.run([exe], capture_output=True, text=True).stdout.split())
@@ -237,11 +237,11 @@ def test_stats_struct_layout_matches_header():
     assert off_round == _lib.Stats.round_ms.offset and off_h2d == _lib.Stats.h2d_bytes.offset
 
 
-def test_dist_stats_struct_layout_matches_header():
+def test_dist_stats_struct_layout_matches_header(tmp_path):
     src = "#include <stdio.h>\n#include \"trueknn.h\"\nint main(){printf(\"%zu %zu %zu %zu\", sizeof(tknn_dist_stats), " \
           "__builtin_offsetof(tknn_dist_stats, h2d_ms), __builtin_offsetof(tknn_dist_stats, search_total_ms), " \
           "__builtin_offsetof(tknn_dist_stats, bytes_sent_search));return 0;}"
-    exe = "/tmp/tknn_dist_layout"
+    exe = str(tmp_path / "tknn_dist_layout")
     subprocess.run(["/usr/bin/gcc", "-x", "c", "-", "-I", os.path.join(ROOT, "include"), "-o", exe], input=src, text=True,
                    check=True)
     size, o1, o2, o3 = (int(v) for v in subprocess.run([exe], capture_output=True, text=True).stdout.split())
