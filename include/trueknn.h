@@ -185,8 +185,25 @@ TKNN_API int tknn_query(tknn_ctx* ctx, const float* queries, uint64_t nq, int di
                         int32_t* idx_out, float* dist_out);
 
 /* Fixed-radius neighbour count per point (closed ball, self excluded) on the same traversal
- * (SURVEY.md §8f rank 4: the DBSCAN core-point test).  count_out: n entries, build order. */
+ * (SURVEY.md §8f rank 4: the DBSCAN core-point test; tknn_dbscan below clusters with it).  count_out: n entries,
+ * build order. */
 TKNN_API int tknn_range_count(tknn_ctx* ctx, float radius, uint32_t* count_out);
+
+/* Exact DBSCAN over the built cloud (SURVEY.md §8f rank 4; the reference README's RT-DBSCAN).  p is in q's eps-ball iff
+ * d2(q, p) <= fl(eps * eps) with the d2 rule above (closed ball, as tknn_range_count); q is a CORE point iff its ball
+ * holds at least min_pts points, q itself and coincident duplicates included (scikit-learn's min_samples, i.e.
+ * range_count(eps)[q] >= min_pts - 1).  Clusters are the connected components of the core points under "within eps",
+ * numbered 0 .. C-1 in ascending order of their smallest core index; a non-core point with a core point in its ball
+ * takes the lowest cluster id among those core points (border); every other point is noise (-1).  The result is
+ * deterministic and equals sklearn.cluster.DBSCAN(eps, min_samples=min_pts) wherever no pair distance lies within
+ * rounding of eps.  eps = +inf and min_pts > n are legal; eps NaN or < 0, min_pts < 1 or a NULL label_out: TKNN_EINVAL;
+ * before a build or on a point-partitioned context: TKNN_ESTATE.
+ * label_out: n entries, build order, cluster id or -1 (noise); core_out (may be NULL): n bytes, 1 = core point;
+ * *n_clusters_out (may be NULL): number of clusters.  Host or device arrays.
+ * Statistics: rounds = 4 phases (core test, link, labelling, border) in round_ms / round_queries, the traversal kernel of
+ * each in kernel_ms (0 for the labelling), search_ms = the whole call on the device, k = min_pts, radii = eps. */
+TKNN_API int tknn_dbscan(tknn_ctx* ctx, float eps, int min_pts, int32_t* label_out, uint8_t* core_out,
+                         uint64_t* n_clusters_out);
 
 /* Start-radius estimator alone (replaces samples/s01-trueknn/Util/random_sample.py:5-32). */
 TKNN_API int tknn_estimate_start_radius(tknn_ctx* ctx, int k, float* radius_out);

@@ -62,6 +62,8 @@ struct tknn_ctx {
   int file_order_chunks = 0;  // same for tknn_search (file-order rows): slices by original index (1 = off; 0 = auto: 5 with
                               // distances, 2 indices-only; k > 24: 2 and 1 — the sweeps of profiles/r2_e2e_mailbox.txt, r2_e2e_cfg3.txt)
   DevBuf chunk_queue;
+  // tknn_dbscan scratch (grow-only): union-find parents, per-root smallest original index and cluster id per position
+  DevBuf db_parent, db_min_idx, db_pos_label, db_bits, db_core_stage;
   // Mailbox: 16 words of mapped pinned host memory that a one-thread kernel fills (fetch_words): the small read-backs of a
   // search or build (unresolved count, radius, leaf count, flags) then never queue behind a bulk device->host copy on the
   // copy engine, and never pass through pageable staging.
@@ -94,7 +96,8 @@ inline unsigned blocks_for(uint64_t n, int threads) { return (unsigned)((n + thr
 
 // scalars layout (uint32 words unless noted)
 enum { SC_GROUP_COUNTER = 0, SC_TOTAL = 1, SC_ERROR = 2, SC_QBAD = 3 /* non-finite query coordinate */, SC_BOUNDS = 4 /* 7 words */, SC_SCENE = 12 /* 6 floats */,
-       SC_COUNTERS = 20 /* 8 x u64, 8-byte aligned */, SC_DUPLEAF = 40, SC_QUANTILE = 41 /* 2 floats: r, r * r */, SC_WORDS = 48 };
+       SC_COUNTERS = 20 /* 8 x u64, 8-byte aligned */, SC_DUPLEAF = 40, SC_QUANTILE = 41 /* 2 floats: r, r * r */,
+       SC_DBSCAN = 43 /* core points, other points */, SC_WORDS = 48 };
 
 #define TK_CUDA(c, expr)                                                                            \
   do {                                                                                              \

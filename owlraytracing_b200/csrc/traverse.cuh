@@ -22,11 +22,18 @@
 // is strict (`>`), ties are resolved on the full (d2, index) key, self is excluded by index.
 #pragma once
 #include "common.cuh"
+#include "dbscan.cuh"
 
 namespace tknn {
 namespace trav {
 
-enum Mode { MODE_KNN = 0, MODE_RANGE_COUNT = 1 };
+// MODE_DBSCAN_*: the three traversal passes of tknn_dbscan (dbscan.cuh has the pipeline around them).  All three use the
+// closed eps-ball of MODE_RANGE_COUNT, the query's own point included.
+//   CORE    every position; a lane stops wanting nodes (bound = -1) once its ball holds min_pts (= P.k) points; one
+//           "is core" ballot word per group of 32 positions (P.unresolved, the core bitset).
+//   LINK    the core queue; every core point of the ball is united with the query in the union-find (P.uf_parent).
+//   BORDER  the non-core queue; the lowest cluster id (P.pos_label) among the core points of the ball, or -1.
+enum Mode { MODE_KNN = 0, MODE_RANGE_COUNT = 1, MODE_DBSCAN_CORE = 2, MODE_DBSCAN_LINK = 3, MODE_DBSCAN_BORDER = 4 };
 
 struct Params {
   const Node* nodes;
@@ -60,6 +67,13 @@ struct Params {
   unsigned long long* counters;  // [0] node visits x active lanes, [1] point tests x active lanes, [2] inserts,
                                  // [3] warp node loads, [4] warp leaf loads, [5] warp point loads,
                                  // [6] pre-filter violations (must stay 0)
+  // MODE_DBSCAN_LINK / _BORDER
+  const uint32_t* core_words;    // the core bitset over positions, n_core_words words
+  uint32_t n_core_words;
+  int* uf_parent;                // LINK: union-find parents over positions
+  const int32_t* pos_label;      // BORDER: cluster id of every core position
+  int32_t* label_out;            // BORDER: label per original index (-1 = noise)
+  uint8_t* core_out;             // BORDER: 0 per original index (may be nullptr)
 };
 
 // ---- bounded 4-ary max-heap of u64 keys in shared memory, slot s of lane l at H[s * 32 + l] ----
@@ -396,6 +410,11 @@ __device__ __forceinline__ uint32_t filter4(const float* sx, int j0, float2 qx, 
 #ifndef TKNN_WORST_REG
 #define TKNN_WORST_REG 2
 #endif
+// MODE_DBSCAN_LINK: 1 = a core query unites only the core points of its ball at LOWER positions (every edge joins two core
+// queries, so each is still united once); 0 = every core point of the ball (each edge twice).
+#ifndef TKNN_DBSCAN_HALF_EDGES
+#define TKNN_DBSCAN_HALF_EDGES 1
+#endif
 
 // VARIANT: 0 = exact filter, 1 = conservative pre-filter (audited option), 2 = exact filter + index-aware
 // tie pruning (chosen by the host when the build found leaves of coincident points).
@@ -449,7 +468,7 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
     float r2 = round_r2;
     if (valid && P.query_r2) r2 = fminf(r2, P.query_r2[qpos]);
     float bound = valid ? r2 : -1.0f;  // d2 >= 0 > -1: an idle lane never wants anything
-    int cnt = 0;
+    int cnt = 0;                       // MODE_DBSCAN_BORDER: 1 + the lowest cluster id of a core point in the ball so far, 0: none
     int widx = 0x7fffffff;             // index of the list's worst entry once it is full (TKNN_WORST_REG)
     if (MODE == MODE_KNN) H[0] = 0;    // sentinel of this lane's k-list
     // group-local origin and this lane's pre-filter constants
@@ -579,12 +598,14 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
             }
             __syncwarp();
             if (COUNT) { c_tests += valid ? lcount : 0; c_wleaves += 1; c_wpts += lcount; }
-            if (MODE == MODE_RANGE_COUNT) {
+            if (MODE == MODE_RANGE_COUNT || MODE == MODE_DBSCAN_CORE) {
               // every point within the radius, the query's own point included: it lies at distance 0 in the one
               // leaf that holds it and is taken off again at emit time
               const float2 qx2 = make_float2(q.x, q.x), qy2 = make_float2(q.y, q.y), qz2 = make_float2(q.z, q.z);
 #pragma unroll 1
               for (int j0 = 0; j0 < lcount; j0 += 4) cnt += __popc(filter4<NS>(soa, j0, qx2, qy2, qz2, bound));
+              // decided: a core point wants nothing more, and the group's walk ends once every lane is decided
+              if (MODE == MODE_DBSCAN_CORE && cnt >= k) bound = -1.0f;
             } else {
               // filter: full chunks of 8 with compile-time bit positions, then the remainder in chunks of 4
               int j0 = 0;
@@ -621,6 +642,31 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
 #pragma unroll 1
                 for (; j0 < lcount; j0 += 4)  // tail in chunks of 4, NaN-padded past the last point
                   mask_a |= filter4<NS>(soa, j0, qx2, qy2, qz2, bound) << j0;
+              }
+            }
+            if (MODE == MODE_DBSCAN_LINK || MODE == MODE_DBSCAN_BORDER) {
+              // the survivors that are core points: the leaf's core bits come with one bitset load (<= 32 consecutive positions)
+              uint32_t m = mask_a & dbscan::bits_at(P.core_words, P.n_core_words, (uint32_t)start);
+              if (MODE == MODE_DBSCAN_LINK) {
+#if TKNN_DBSCAN_HALF_EDGES
+                // both ends of an edge are core queries: only the end at the higher position unites it
+                const int64_t below = (int64_t)qpos - (int64_t)(uint32_t)start;  // leaf slots at positions < qpos
+                m &= below >= 32 ? FULL_MASK : (below <= 0 ? 0u : (1u << below) - 1u);
+#endif
+                while (m) {
+                  const int j = __ffs(m) - 1;
+                  m &= m - 1u;
+                  const int hooked = dbscan::uf_unite(P.uf_parent, (int)qpos, start + j);
+                  if (COUNT) c_ins += hooked;
+                }
+              } else {
+                while (m) {
+                  const int j = __ffs(m) - 1;
+                  m &= m - 1u;
+                  const int id1 = __ldg(&P.pos_label[(uint32_t)start + j]) + 1;
+                  cnt = (cnt == 0 || id1 < cnt) ? id1 : cnt;
+                  if (COUNT) c_ins += 1;
+                }
               }
             }
           }
@@ -684,6 +730,16 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
     // ---- emit ----
     if (MODE == MODE_RANGE_COUNT) {
       if (valid) P.count_out[row_id] = (uint32_t)(cnt - (self >= 0 ? 1 : 0));
+    } else if (MODE == MODE_DBSCAN_CORE) {
+      const unsigned core = __ballot_sync(FULL_MASK, valid && cnt >= k);
+      if (lane == 0) P.unresolved[group] = core;  // groups are positions 32 g .. 32 g + 31 (no queue)
+    } else if (MODE == MODE_DBSCAN_LINK) {
+      // nothing to emit: the unions are the result
+    } else if (MODE == MODE_DBSCAN_BORDER) {
+      if (valid) {
+        P.label_out[row_id] = cnt - 1;  // -1: noise
+        if (P.core_out) P.core_out[row_id] = 0;
+      }
     } else {
       const bool resolved = valid && cnt == k;
       const bool emit = valid && (resolved || P.final_round);

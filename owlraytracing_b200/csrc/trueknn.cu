@@ -121,8 +121,12 @@ int launch_traverse(tknn_ctx* c, const trav::Params& P) {
   const int variant = MODE != trav::MODE_KNN ? 0 : (ties ? 2 : (c->approx_filter ? 1 : 0));
   const bool hp = MODE == trav::MODE_KNN && k > trav::LIST_MAX_K;
 #define TK_PICK(CNT, VAR) (hp ? trav::traverse_kernel<MODE, CNT, VAR, true> : trav::traverse_kernel<MODE, CNT, VAR, false>)
-  if (c->counters) kern = variant == 2 ? TK_PICK(true, 2) : variant == 1 ? TK_PICK(true, 1) : TK_PICK(true, 0);
-  else kern = variant == 2 ? TK_PICK(false, 2) : variant == 1 ? TK_PICK(false, 1) : TK_PICK(false, 0);
+  if constexpr (MODE >= trav::MODE_DBSCAN_CORE) {  // the DBSCAN passes: exact filter, no k-list (one variant each)
+    kern = c->counters ? trav::traverse_kernel<MODE, true, 0, false> : trav::traverse_kernel<MODE, false, 0, false>;
+  } else {
+    if (c->counters) kern = variant == 2 ? TK_PICK(true, 2) : variant == 1 ? TK_PICK(true, 1) : TK_PICK(true, 0);
+    else kern = variant == 2 ? TK_PICK(false, 2) : variant == 1 ? TK_PICK(false, 1) : TK_PICK(false, 0);
+  }
 #undef TK_PICK
   cudaFuncAttributes fa;
   TK_CUDA(c, cudaFuncGetAttributes(&fa, kern));
@@ -805,7 +809,7 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->b_keys_b, &c->b_vals_a, &c->b_vals_b, &c->b_sort_tmp, &c->b_delta, &c->b_ballots, &c->b_leaf_key,
                     &c->b_child_info, &c->b_parent_leaf, &c->b_parent_node, &c->b_arrive, &c->q_stage, &c->q_keys_a, &c->q_keys_b,
                     &c->q_vals_a, &c->q_vals_b, &c->q_sort_tmp, &c->q_pts, &c->q_sid_stage, &c->q_sid_sorted, &c->q_rad_stage,
-                    &c->q_r2_sorted})
+                    &c->q_r2_sorted, &c->db_parent, &c->db_min_idx, &c->db_pos_label, &c->db_bits, &c->db_core_stage})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -1322,6 +1326,147 @@ int tknn_range_count(tknn_ctx* c, float radius, uint32_t* count_out) {
   c->stats.rounds = 1;
   c->stats.kernel_launches = 1;
   c->stats.start_radius = c->stats.final_radius = radius;
+  TK_TRY(collect_counters(c));
+  TK_TRY(read_error_flag(c));
+  return TKNN_OK;
+}
+
+// Four phases, all on the device (dbscan.cuh): core test + queue split, link, labelling, border.  The only host read-back is
+// the queue sizes and C at the end: the link and border passes take their query counts from the device.
+int tknn_dbscan(tknn_ctx* c, float eps, int min_pts, int32_t* label_out, uint8_t* core_out, uint64_t* n_clusters_out) {
+  TK_TRY(check_ctx(c));
+  if (c->n == 0) return fail(c, TKNN_ESTATE, "tknn_dbscan before tknn_build");
+  if (c->ids_in_w) return fail(c, TKNN_ESTATE, "this BVH carries caller-chosen point ids (point-partitioned build)");
+  if (!(eps >= 0.0f)) return fail(c, TKNN_EINVAL, "eps must be >= 0");
+  if (min_pts < 1) return fail(c, TKNN_EINVAL, "min_pts = %d must be >= 1", min_pts);
+  if (!label_out) return fail(c, TKNN_EINVAL, "null label array");
+  if (c->n > (uint64_t)INT32_MAX) return fail(c, TKNN_EINVAL, "tknn_dbscan supports at most 2^31 - 1 points");
+  ScopedDevice sd(c->device);
+  reset_search_stats(c);
+  const uint64_t n = c->n;
+  const uint32_t n_groups = (uint32_t)((n + 31) / 32);
+  cudaStream_t st = c->stream;
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  const bool label_dev = is_device_ptr(label_out), core_dev = core_out && is_device_ptr(core_out);
+  TK_TRY(ensure(c, c->unresolved, sizeof(uint32_t) * (size_t)(n_groups + 1)));
+  TK_TRY(ensure(c, c->offsets, sizeof(uint32_t) * (size_t)(n_groups + 1)));
+  TK_TRY(ensure(c, c->queue_a, sizeof(uint32_t) * n));
+  TK_TRY(ensure(c, c->queue_b, sizeof(uint32_t) * n));
+  TK_TRY(ensure(c, c->db_parent, sizeof(int) * n));
+  TK_TRY(ensure(c, c->db_min_idx, sizeof(int) * n));
+  TK_TRY(ensure(c, c->db_pos_label, sizeof(int32_t) * n));
+  TK_TRY(ensure(c, c->db_bits, sizeof(uint32_t) * (size_t)n_groups));
+  if (!label_dev) TK_TRY(ensure(c, c->stage_idx, sizeof(int32_t) * n));
+  if (core_out && !core_dev) TK_TRY(ensure(c, c->db_core_stage, n));
+  int32_t* d_label = label_dev ? label_out : c->stage_idx.as<int32_t>();
+  uint8_t* d_core = core_out ? (core_dev ? core_out : c->db_core_stage.as<uint8_t>()) : nullptr;
+  uint32_t* core_words = c->unresolved.as<uint32_t>();
+  uint32_t* core_q = c->queue_a.as<uint32_t>();
+  uint32_t* other_q = c->queue_b.as<uint32_t>();
+  int* parent = c->db_parent.as<int>();
+  int* min_idx = c->db_min_idx.as<int>();
+  int32_t* pos_label = c->db_pos_label.as<int32_t>();
+  uint32_t* cluster_bits = c->db_bits.as<uint32_t>();
+  int launches = 0;
+  for (size_t i = c->round_ev.size(); i < 16; ++i) {
+    cudaEvent_t e;
+    TK_CUDA(c, cudaEventCreate(&e));
+    c->round_ev.push_back(e);
+  }
+  cudaEvent_t* ev = c->round_ev.data();  // phase r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its traversal kernel
+
+  trav::Params P;
+  std::memset(&P, 0, sizeof(P));
+  P.nodes = c->nodes.as<Node>();
+  P.node_min_idx = c->node_min_idx.as<int2>();
+  P.pts = c->pts.as<float4>();
+  P.queries = c->pts.as<float4>();
+  P.r2 = eps * eps;
+  P.k = min_pts;
+  P.final_round = 1;
+  P.error = sc + SC_ERROR;
+  P.group_counter = sc + SC_GROUP_COUNTER;
+  P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
+  P.core_words = core_words;
+  P.n_core_words = n_groups;
+  const unsigned blocks = blocks_for(n, dbscan::THREADS);
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
+  TK_CUDA(c, cudaEventRecord(c->ev[0], st));
+
+  // 1. core test over every position, then the core / non-core queues
+  TK_CUDA(c, cudaEventRecord(ev[0], st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), st));
+  P.n_active = n;
+  P.n_groups = n_groups;
+  P.unresolved = core_words;
+  TK_CUDA(c, cudaEventRecord(ev[2], st));
+  TK_TRY(launch_traverse<trav::MODE_DBSCAN_CORE>(c, P));
+  TK_CUDA(c, cudaEventRecord(ev[3], st));
+  TK_TRY(popc_scan(c, core_words, n_groups, c->offsets.as<uint32_t>(), &launches));
+  dbscan::split_queues_kernel<<<blocks, dbscan::THREADS, 0, st>>>(core_words, c->offsets.as<uint32_t>(), n, core_q, other_q, parent,
+                                                                  min_idx, sc + SC_DBSCAN);
+  TK_CUDA(c, cudaGetLastError());
+  TK_CUDA(c, cudaEventRecord(ev[1], st));
+  P.unresolved = nullptr;
+
+  // 2. link: the core queue, its length read on the device
+  TK_CUDA(c, cudaEventRecord(ev[4], st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), st));
+  P.queue = core_q;
+  P.n_active_dev = sc + SC_DBSCAN;
+  P.uf_parent = parent;
+  TK_CUDA(c, cudaEventRecord(ev[6], st));
+  TK_TRY(launch_traverse<trav::MODE_DBSCAN_LINK>(c, P));
+  TK_CUDA(c, cudaEventRecord(ev[7], st));
+  TK_CUDA(c, cudaEventRecord(ev[5], st));
+
+  // 3. labelling: roots, the smallest original index per cluster, dense ids from a popc scan of one bit per cluster
+  TK_CUDA(c, cudaEventRecord(ev[8], st));
+  TK_CUDA(c, cudaEventRecord(ev[10], st));  // no traversal kernel in this phase
+  TK_CUDA(c, cudaEventRecord(ev[11], st));
+  TK_CUDA(c, cudaMemsetAsync(cluster_bits, 0, sizeof(uint32_t) * (size_t)n_groups, st));
+  dbscan::flatten_kernel<<<blocks, dbscan::THREADS, 0, st>>>(core_words, P.pts, n, parent, min_idx);
+  dbscan::mark_kernel<<<blocks, dbscan::THREADS, 0, st>>>(core_words, n, parent, min_idx, cluster_bits);
+  TK_CUDA(c, cudaGetLastError());
+  TK_TRY(popc_scan(c, cluster_bits, n_groups, c->offsets.as<uint32_t>(), &launches));  // C -> sc[SC_TOTAL]
+  dbscan::label_core_kernel<<<blocks, dbscan::THREADS, 0, st>>>(core_words, P.pts, n, parent, min_idx, cluster_bits,
+                                                                c->offsets.as<uint32_t>(), pos_label, d_label, d_core);
+  TK_CUDA(c, cudaGetLastError());
+  TK_CUDA(c, cudaEventRecord(ev[9], st));
+
+  // 4. border: the non-core queue
+  TK_CUDA(c, cudaEventRecord(ev[12], st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), st));
+  P.queue = other_q;
+  P.n_active_dev = sc + SC_DBSCAN + 1;
+  P.uf_parent = nullptr;
+  P.pos_label = pos_label;
+  P.label_out = d_label;
+  P.core_out = d_core;
+  TK_CUDA(c, cudaEventRecord(ev[14], st));
+  TK_TRY(launch_traverse<trav::MODE_DBSCAN_BORDER>(c, P));
+  TK_CUDA(c, cudaEventRecord(ev[15], st));
+  TK_CUDA(c, cudaEventRecord(ev[13], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
+  launches += 3 /* traversals */ + 4 /* split, flatten, mark, label */;
+
+  if (!label_dev) TK_CUDA(c, cudaMemcpyAsync(label_out, d_label, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, st));
+  if (core_out && !core_dev) TK_CUDA(c, cudaMemcpyAsync(core_out, d_core, n, cudaMemcpyDeviceToHost, st));
+  c->stats.d2h_bytes = (label_dev ? 0 : sizeof(int32_t) * n) + (core_out && !core_dev ? n : 0);
+  uint32_t rb[3] = {0, 0, 0};  // core points, other points, clusters
+  TK_TRY(fetch_words(c, sc + SC_DBSCAN, 2, sc + SC_TOTAL, 1, rb));  // synchronises the stream
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
+  c->stats.n_queries = n;
+  c->stats.k = min_pts;
+  c->stats.rounds = 4;
+  c->stats.start_radius = c->stats.final_radius = eps;
+  c->stats.round_queries[0] = n;
+  c->stats.round_queries[1] = c->stats.round_queries[2] = rb[0];
+  c->stats.round_queries[3] = rb[1];
+  c->stats.kernel_launches = (uint32_t)(launches + c->mailbox_launches + (c->mailbox_h ? 1 : 0));  // + the error-flag fetch
+  TK_TRY(finish_round_stats(c));
+  if (n_clusters_out) *n_clusters_out = rb[2];
   TK_TRY(collect_counters(c));
   TK_TRY(read_error_flag(c));
   return TKNN_OK;

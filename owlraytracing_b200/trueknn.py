@@ -45,7 +45,8 @@ def _check_dtype(a, np_dtype, name):
     if _is_tensor(a):
         import torch
 
-        want = {np.float32: torch.float32, np.int32: torch.int32, np.uint32: torch.int32, np.uint64: torch.int64}[np_dtype]
+        want = {np.float32: torch.float32, np.int32: torch.int32, np.uint32: torch.int32, np.uint64: torch.int64,
+                np.uint8: torch.uint8}[np_dtype]
         if a.dtype != want and not (np_dtype is np.uint32 and a.dtype == torch.uint32):
             raise TypeError(f"{name}: expected {want}, got {a.dtype}")
     elif a.dtype != np_dtype:
@@ -228,7 +229,7 @@ class TrueKNN:
         return idx, dist
 
     def range_count(self, radius: float):
-        """Neighbours within the closed ball of `radius` for every point (DBSCAN core-point test)."""
+        """Neighbours within the closed ball of `radius` for every point (DBSCAN core-point test; see dbscan())."""
         if _is_tensor(self._like):
             import torch
 
@@ -237,6 +238,31 @@ class TrueKNN:
             out = np.empty((self.n,), np.uint32)
         self._check(self._L.tknn_range_count(self._h, C.c_float(radius), _ptr(out)))
         return out
+
+    def dbscan(self, eps: float, min_pts: int, with_core: bool = True, out=None):
+        """Exact DBSCAN of the built cloud (closed eps-ball, min_pts counts the point itself: scikit-learn's min_samples).
+
+        Returns (labels [n] int32: cluster id in 0 .. C-1 or -1 for noise, core [n] uint8: 1 = core point (None when
+        with_core is False), C).  Clusters are numbered in ascending order of their smallest core index; a border point
+        takes the lowest id among the clusters of the core points in its ball.  numpy outputs for numpy input, CUDA
+        tensors for CUDA tensor input; out = (labels, core) supplies the arrays (core may be None)."""
+        if out is not None:
+            labels, core = out
+        elif _is_tensor(self._like):
+            import torch
+
+            labels = torch.empty((self.n,), dtype=torch.int32, device=self._like.device)
+            core = torch.empty((self.n,), dtype=torch.uint8, device=self._like.device) if with_core else None
+            self._settle_outputs(labels)
+        else:
+            labels = np.empty((self.n,), np.int32)
+            core = np.empty((self.n,), np.uint8) if with_core else None
+        _check_dtype(labels, np.int32, "labels")
+        if core is not None:
+            _check_dtype(core, np.uint8, "core")
+        c = C.c_uint64(0)
+        self._check(self._L.tknn_dbscan(self._h, C.c_float(eps), int(min_pts), _ptr(labels), _ptr(core), C.byref(c)))
+        return labels, core, int(c.value)
 
     def estimate_start_radius(self, k: int) -> float:
         r = C.c_float(0)

@@ -1,8 +1,10 @@
 // trueknn_cli.cpp — the sample's command line over libtrueknn (C++ host side of the drop-in).
 //
 //   trueknn <file> <n> <dim> <start radius> <k> <output file> [--neighbours <path> [--binary]] [--device <d>] [--json]
-//           [--gpus <N> | --devices <a,b,...>] [--mode shard|partition]
+//           [--gpus <N> | --devices <a,b,...>] [--mode shard|partition] [--dbscan <eps> <min_pts> [--labels <path> [--binary]]]
 //
+// --dbscan runs exact DBSCAN (tknn_dbscan) instead of the kNN search after the build; k and the start radius are still
+// required and are ignored.  --labels writes `point,label` lines (label -1 = noise), or raw int32 labels with --binary.
 // --gpus N (devices 0..N-1) or --devices (an explicit list; naming one device several times runs that many ranks on
 // it) drives all devices from this one process through tknn_create_multi: the device-list form of the reference's
 // owlContextCreate(ids, n) (owl/include/owl/owl_host.h:360; the sample itself passes one device, hostCode.cpp:141).
@@ -28,7 +30,10 @@
 
 int main(int ac, char** av) {
   std::vector<std::string> pos;
-  std::string neigh_path, mode = "shard";
+  std::string neigh_path, labels_path, mode = "shard";
+  bool dbscan = false;
+  float db_eps = 0.f;
+  int db_min_pts = 0;
   std::vector<int> devices;
   int device = 0;
   bool json = false, binary = false;
@@ -44,13 +49,20 @@ int main(int ac, char** av) {
       }
     }
     else if (a == "--mode") { if (++i < ac) mode = av[i]; }
+    else if (a == "--dbscan") {
+      dbscan = true;
+      if (i + 2 < ac) { db_eps = (float)std::atof(av[i + 1]); db_min_pts = std::atoi(av[i + 2]); }
+      i += 2;
+    }
+    else if (a == "--labels") { if (++i < ac) labels_path = av[i]; }
     else if (a == "--json") json = true;
     else if (a == "--binary") binary = true;  // --neighbours as raw arrays: <path>.idx.i32 / <path>.dist.f32
     else pos.push_back(a);
   }
-  if (pos.size() != 6 || (mode != "shard" && mode != "partition")) {
+  if (pos.size() != 6 || (mode != "shard" && mode != "partition") || (dbscan && !devices.empty())) {
     std::fprintf(stderr, "usage: %s <file> <n> <dim> <start radius> <k> <output file> [--neighbours <path>] [--device <d>] [--json]\n"
-                         "          [--gpus <N> | --devices <a,b,...>] [--mode shard|partition]\n", av[0]);
+                         "          [--gpus <N> | --devices <a,b,...>] [--mode shard|partition]\n"
+                         "          [--dbscan <eps> <min_pts> [--labels <path> [--binary]]]   (one GPU)\n", av[0]);
     return 64;
   }
   const std::string path = pos[0], outfile = pos[5];
@@ -132,6 +144,46 @@ int main(int ac, char** av) {
   if (rc != TKNN_OK) { std::fprintf(stderr, "tknn_build: %s\n", tknn_last_error(ctx)); tknn_destroy(ctx); return 71; }
   const double build_s = std::chrono::duration<double>(t1 - t0).count();
   std::cout << "Build time: " << build_s << '\n';
+
+  if (dbscan) {
+    std::vector<int32_t> labels((size_t)np);
+    uint64_t n_clusters = 0;
+    auto d0 = std::chrono::steady_clock::now();
+    rc = tknn_dbscan(ctx, db_eps, db_min_pts, labels.data(), nullptr, &n_clusters);
+    auto d1 = std::chrono::steady_clock::now();
+    if (rc != TKNN_OK) { std::fprintf(stderr, "tknn_dbscan: %s\n", tknn_last_error(ctx)); tknn_destroy(ctx); return 72; }
+    const double db_s = std::chrono::duration<double>(d1 - d0).count();
+    tknn_stats st;
+    tknn_get_stats(ctx, &st);
+    static const char* phase[4] = {"core test", "link", "labelling", "border"};
+    for (int i = 0; i < 4; ++i)
+      std::cout << "Phase: " << phase[i] << " Queries = " << st.round_queries[i] << " Time: " << st.round_ms[i] / 1000.0 << " seconds\n";
+    uint64_t noise = 0;
+    for (int32_t l : labels) noise += l < 0;
+    std::cout << "Clusters: " << n_clusters << " Noise points: " << noise << '\n';
+    std::cout << "DBSCAN time: " << db_s << " seconds." << std::endl;
+    const double tot = build_s + db_s;
+    std::cout << "Total time: " << tot << '\n';
+    std::ofstream out(outfile, std::ios::app);
+    if (!out.is_open()) { std::perror("Error open"); tknn_destroy(ctx); return 73; }
+    out << tot << std::endl;
+    if (!labels_path.empty()) {
+      FILE* f = std::fopen(labels_path.c_str(), binary ? "wb" : "w");
+      bool ok = f != nullptr;
+      if (ok && binary) ok = std::fwrite(labels.data(), sizeof(int32_t), labels.size(), f) == labels.size();
+      for (size_t i = 0; ok && !binary && i < labels.size(); ++i) ok = std::fprintf(f, "%zu,%d\n", i, labels[i]) > 0;
+      if (f && std::fclose(f) != 0) ok = false;
+      if (!ok) { std::perror("Error open"); tknn_destroy(ctx); return 73; }
+    }
+    if (json) {
+      std::printf("{\"n\": %llu, \"eps\": %.9g, \"min_pts\": %d, \"clusters\": %llu, \"noise\": %llu, \"build_ms\": %.4f, "
+                  "\"dbscan_ms\": %.4f, \"points_per_s\": %.1f}\n",
+                  (unsigned long long)np, db_eps, db_min_pts, (unsigned long long)n_clusters, (unsigned long long)noise, st.build_ms,
+                  st.search_ms, st.search_ms > 0 ? np / (st.search_ms * 1e-3) : 0.0);
+    }
+    tknn_destroy(ctx);
+    return 0;
+  }
 
   std::vector<int32_t> idx((size_t)np * k);
   std::vector<float> dist((size_t)np * k);
