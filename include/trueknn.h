@@ -205,6 +205,28 @@ TKNN_API int tknn_range_count(tknn_ctx* ctx, float radius, uint32_t* count_out);
 TKNN_API int tknn_dbscan(tknn_ctx* ctx, float eps, int min_pts, int32_t* label_out, uint8_t* core_out,
                          uint64_t* n_clusters_out);
 
+/* Exact fixed-radius neighbour lists (scipy's cKDTree.query_ball_point, scikit-learn's radius_neighbors).  The row of
+ * query q holds every data point p with index(p) != self(q) and d2(q, p) <= fl(radius * radius), the d2 rule and closed
+ * ball of tknn_range_count, sorted ascending by (d2, index): coincident duplicates are neighbours at distance 0, ties
+ * are ordered by index.  So in the all-points form row q has range_count(radius)[q] entries, and a row of length >= k
+ * starts with row q of tknn_search(k), bit for bit.
+ * Output, CSR: offsets_out[0 .. nq] (u64, offsets_out[0] = 0); idx_out[offsets[q] .. offsets[q + 1]) = data indices;
+ * dist_out the same entries' sqrtf(d2), or d2 while TKNN_OPT_SQUARED_DIST is set (may be NULL: indices only).
+ * Sizing: idx_out == NULL asks for the size (offsets_out and *total_out are filled, TKNN_OK); capacity < total fills
+ * offsets_out and *total_out, writes no entries and returns TKNN_EINVAL; otherwise all rows are written.
+ * tknn_radius_search: every built point is a query, rows in build order, self = the point itself.
+ * tknn_radius_query: nq query rows (dim, stride and self_ids as tknn_query; self_ids may be NULL, -1 = no exclusion),
+ * rows in query order.  Host or device arrays.  radius = +inf is legal; radius NaN or < 0 or a NULL offsets_out:
+ * TKNN_EINVAL; before a build or on a point-partitioned context: TKNN_ESTATE.
+ * Statistics: rounds = 3 phases (count + scans, fill, order) in round_ms, their traversal kernels in kernel_ms (the
+ * order phase: all of its kernels), round_queries = {queries, queries filled, rows sorted by the long-row radix sort},
+ * search_ms = the whole call on the device. */
+TKNN_API int tknn_radius_search(tknn_ctx* ctx, float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out,
+                                uint64_t capacity, uint64_t* total_out);
+TKNN_API int tknn_radius_query(tknn_ctx* ctx, const float* queries, uint64_t nq, int dim, int stride_floats,
+                               const int32_t* self_ids, float radius, uint64_t* offsets_out, int32_t* idx_out,
+                               float* dist_out, uint64_t capacity, uint64_t* total_out);
+
 /* Start-radius estimator alone (replaces samples/s01-trueknn/Util/random_sample.py:5-32). */
 TKNN_API int tknn_estimate_start_radius(tknn_ctx* ctx, int k, float* radius_out);
 
@@ -367,6 +389,11 @@ TKNN_API int tknn_generate_uniform(tknn_ctx* ctx, uint64_t seed, uint64_t first,
  * hostCode.cpp:312-319), or raw arrays (path + ".idx.i32" / ".dist.f32") when binary != 0. */
 TKNN_API int tknn_read_points(const char* path, uint64_t n, int dim, float* xyz_out, uint64_t n_cap, uint64_t* n_out);
 TKNN_API int tknn_write_neighbours(const char* path, const int32_t* idx, const float* dist, uint64_t n, int k, int binary);
+/* tknn_write_neighbour_lists: the CSR rows of tknn_radius_search / _query (host arrays; dist may be NULL).  Text: one
+ * `query,neighbourIndex,distance` line per entry (no distance column without dist); binary: path.off.u64 (nq + 1
+ * offsets), path.idx.i32 and path.dist.f32 (raw little-endian arrays). */
+TKNN_API int tknn_write_neighbour_lists(const char* path, const uint64_t* offsets, const int32_t* idx, const float* dist,
+                                        uint64_t nq, int binary);
 
 /* Device properties the roofline needs: SM count, L2 bytes, and a measured L2 / HBM read
  * bandwidth (GB/s) from a short read loop over an L2-resident / HBM-sized buffer. */

@@ -98,6 +98,7 @@ EXPORTS = [
     "tknn_partition_owned", "tknn_partition_search", "tknn_partition_verify", "tknn_create_multi", "tknn_multi_destroy",
     "tknn_multi_set_option", "tknn_multi_build", "tknn_multi_search", "tknn_multi_ranks", "tknn_multi_ctx",
     "tknn_multi_last_error", "tknn_multi_get_times", "tknn_measure_smem_bandwidth", "tknn_key_layout", "tknn_dbscan",
+    "tknn_radius_search", "tknn_radius_query", "tknn_write_neighbour_lists",
 ]
 
 _lib = None
@@ -130,6 +131,9 @@ def load() -> C.CDLL:
     L.tknn_query.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, vp, C.c_int, f32, vp, vp]
     L.tknn_range_count.argtypes = [vp, f32, vp]
     L.tknn_dbscan.argtypes = [vp, f32, C.c_int, vp, vp, C.POINTER(u64)]
+    L.tknn_radius_search.argtypes = [vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
+    L.tknn_radius_query.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
+    L.tknn_write_neighbour_lists.argtypes = [C.c_char_p, vp, vp, vp, u64, C.c_int]
     L.tknn_estimate_start_radius.argtypes = [vp, C.c_int, C.POINTER(f32)]
     L.tknn_brute_force.argtypes = [vp, vp, u64, C.c_int, vp, vp]
     L.tknn_merge_topk.argtypes = [vp, vp, vp, C.c_int, u64, C.c_int, vp, vp]

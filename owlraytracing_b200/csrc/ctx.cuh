@@ -64,6 +64,10 @@ struct tknn_ctx {
   DevBuf chunk_queue;
   // tknn_dbscan scratch (grow-only): union-find parents, per-root smallest original index and cluster id per position
   DevBuf db_parent, db_min_idx, db_pos_label, db_bits, db_core_stage;
+  // tknn_radius_search / _query scratch (grow-only): counts and u64 offsets by position and by row, scan block sums, the
+  // mailbox words, self positions, the unsorted rows, the long-row list and the long-row sort buffers (radius.cuh)
+  DevBuf rl_cnt_pos, rl_cnt_row, rl_off_pos, rl_off_row, rl_sums, rl_stats, rl_pos_of, rl_self_pos, rl_keys, rl_long_pos,
+      rl_long_len, rl_boff, rl_ka, rl_kb, rl_kc, rl_va, rl_vb, rl_vc, rl_row_of, rl_sort_tmp;
   // Mailbox: 16 words of mapped pinned host memory that a one-thread kernel fills (fetch_words): the small read-backs of a
   // search or build (unresolved count, radius, leaf count, flags) then never queue behind a bulk device->host copy on the
   // copy engine, and never pass through pageable staging.

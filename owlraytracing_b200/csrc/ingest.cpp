@@ -171,4 +171,54 @@ TKNN_API int tknn_write_neighbours(const char* path, const int32_t* idx, const f
   return ok ? TKNN_OK : TKNN_EINVAL;
 }
 
+// The CSR rows of tknn_radius_search / _query: `query,neighbourIndex,distance` lines (`query,neighbourIndex` without dist),
+// or raw arrays when binary != 0 (path + ".off.u64" / ".idx.i32" / ".dist.f32").
+TKNN_API int tknn_write_neighbour_lists(const char* path, const uint64_t* offsets, const int32_t* idx, const float* dist,
+                                        uint64_t nq, int binary) {
+  if (!path || !offsets) return TKNN_EINVAL;
+  const uint64_t total = offsets[nq];
+  if (total && !idx) return TKNN_EINVAL;
+  if (binary) {
+    const std::string po = std::string(path) + ".off.u64", pi = std::string(path) + ".idx.i32",
+                      pd = std::string(path) + ".dist.f32";
+    FILE* fo = fopen(po.c_str(), "wb");
+    FILE* fi = fopen(pi.c_str(), "wb");
+    FILE* fd = dist ? fopen(pd.c_str(), "wb") : nullptr;
+    bool ok = fo && fi && (!dist || fd) && fwrite(offsets, sizeof(uint64_t), (size_t)nq + 1, fo) == (size_t)nq + 1 &&
+              fwrite(idx, sizeof(int32_t), (size_t)total, fi) == (size_t)total &&
+              (!dist || fwrite(dist, sizeof(float), (size_t)total, fd) == (size_t)total);
+    if (fo) fclose(fo);
+    if (fi) fclose(fi);
+    if (fd) fclose(fd);
+    return ok ? TKNN_OK : TKNN_EINVAL;
+  }
+  unsigned nt = std::max(1u, std::thread::hardware_concurrency());
+  nt = (unsigned)std::min<uint64_t>(nt, std::max<uint64_t>(1, total / 65536));
+  std::vector<std::string> parts(nt);
+  std::vector<std::thread> th;
+  for (unsigned t = 0; t < nt; ++t)
+    th.emplace_back([&, t]() {
+      // rows split so that every thread writes about the same number of entries
+      const uint64_t lo = total * t / nt, hi = total * (t + 1) / nt;
+      const uint64_t a = (uint64_t)(std::upper_bound(offsets, offsets + nq + 1, lo) - offsets) - 1;
+      const uint64_t b = t + 1 == nt ? nq : (uint64_t)(std::upper_bound(offsets, offsets + nq + 1, hi) - offsets) - 1;
+      std::string& s = parts[t];
+      s.reserve((size_t)(offsets[b] - offsets[a]) * 28);
+      char buf[96];
+      for (uint64_t q = (t == 0 ? 0 : a); q < b; ++q)
+        for (uint64_t e = offsets[q]; e < offsets[q + 1]; ++e) {
+          const int m = dist ? snprintf(buf, sizeof(buf), "%llu,%d,%.9g\n", (unsigned long long)q, idx[e], (double)dist[e])
+                             : snprintf(buf, sizeof(buf), "%llu,%d\n", (unsigned long long)q, idx[e]);
+          s.append(buf, (size_t)m);
+        }
+    });
+  for (auto& x : th) x.join();
+  FILE* f = fopen(path, "w");
+  if (!f) return TKNN_EINVAL;
+  bool ok = true;
+  for (auto& s : parts) ok = ok && fwrite(s.data(), 1, s.size(), f) == s.size();
+  fclose(f);
+  return ok ? TKNN_OK : TKNN_EINVAL;
+}
+
 }  // extern "C"

@@ -33,7 +33,14 @@ namespace trav {
 //           "is core" ballot word per group of 32 positions (P.unresolved, the core bitset).
 //   LINK    the core queue; every core point of the ball is united with the query in the union-find (P.uf_parent).
 //   BORDER  the non-core queue; the lowest cluster id (P.pos_label) among the core points of the ball, or -1.
-enum Mode { MODE_KNN = 0, MODE_RANGE_COUNT = 1, MODE_DBSCAN_CORE = 2, MODE_DBSCAN_LINK = 3, MODE_DBSCAN_BORDER = 4 };
+// MODE_RANGE_LIST_*: the two traversal passes of tknn_radius_search / tknn_radius_query (radius.cuh has the pipeline).
+// Both take the exact closed ball and drop the excluded point by POSITION (P.self_pos, or the query's own position when
+// self_is_row): one bit of the leaf mask, which is "index != self" because positions and indices are a bijection.
+//   COUNT   every query position; the ball's size minus self, written by position (P.count_out) and by row (P.count_row).
+//   FILL    every query position; each member as the key make_key(d2, index) at the lane's cursor, which starts at
+//           P.list_off[position] in P.list_keys (unsorted; the order pass sorts every row).
+enum Mode { MODE_KNN = 0, MODE_RANGE_COUNT = 1, MODE_DBSCAN_CORE = 2, MODE_DBSCAN_LINK = 3, MODE_DBSCAN_BORDER = 4,
+            MODE_RANGE_LIST_COUNT = 5, MODE_RANGE_LIST = 6 };
 
 struct Params {
   const Node* nodes;
@@ -74,6 +81,18 @@ struct Params {
   const int32_t* pos_label;      // BORDER: cluster id of every core position
   int32_t* label_out;            // BORDER: label per original index (-1 = noise)
   uint8_t* core_out;             // BORDER: 0 per original index (may be nullptr)
+  // MODE_RANGE_LIST_COUNT / _LIST
+  const int32_t* self_pos;       // per query position: the data position to exclude or -1; nullptr => see self_is_row
+  uint32_t* count_row;           // LIST_COUNT: ball size per output row (count_out: per query position)
+  const uint64_t* list_off;      // LIST: first key slot of every query position
+  uint64_t* list_keys;           // LIST: the unsorted rows, in position order
+};
+
+// per-lane state of the MODE_RANGE_LIST_* passes (an empty object in the other modes)
+template <bool LIST> struct ListLane {};
+template <> struct ListLane<true> {
+  int64_t spos = -1;    // position of the excluded data point (-1: none)
+  uint64_t cursor = 0;  // MODE_RANGE_LIST: next key slot of the lane's row
 };
 
 // ---- bounded 4-ary max-heap of u64 keys in shared memory, slot s of lane l at H[s * 32 + l] ----
@@ -471,6 +490,11 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
     int cnt = 0;                       // MODE_DBSCAN_BORDER: 1 + the lowest cluster id of a core point in the ball so far, 0: none
     int widx = 0x7fffffff;             // index of the list's worst entry once it is full (TKNN_WORST_REG)
     if (MODE == MODE_KNN) H[0] = 0;    // sentinel of this lane's k-list
+    ListLane<MODE == MODE_RANGE_LIST_COUNT || MODE == MODE_RANGE_LIST> rl;  // empty in every other mode
+    if constexpr (MODE == MODE_RANGE_LIST_COUNT || MODE == MODE_RANGE_LIST) {
+      if (valid) rl.spos = P.self_pos ? (int64_t)P.self_pos[qpos] : (P.self_is_row ? (int64_t)qpos : -1);
+      if (MODE == MODE_RANGE_LIST && valid) rl.cursor = P.list_off[qpos];
+    }
     // group-local origin and this lane's pre-filter constants
     float ax, ay, az, qq;
     {
@@ -644,6 +668,22 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
                   mask_a |= filter4<NS>(soa, j0, qx2, qy2, qz2, bound) << j0;
               }
             }
+            if constexpr (MODE == MODE_RANGE_LIST_COUNT || MODE == MODE_RANGE_LIST) {
+              // the excluded point is one slot of this leaf at most
+              const int64_t rel = rl.spos - (int64_t)(uint32_t)start;
+              uint32_t m = mask_a & ((rel >= 0 && rel < 32) ? ~(1u << rel) : FULL_MASK);
+              if (MODE == MODE_RANGE_LIST_COUNT) {
+                cnt += __popc(m);
+              } else {
+                while (m) {  // the distance of the filter, recomputed with the chain of try_insert (bit-identical)
+                  const int j = __ffs(m) - 1;
+                  m &= m - 1u;
+                  const float4 p = stage[j];
+                  P.list_keys[rl.cursor++] = make_key(dist2(q.x, q.y, q.z, p.x, p.y, p.z), __float_as_int(p.w));
+                  if (COUNT) c_ins += 1;
+                }
+              }
+            }
             if (MODE == MODE_DBSCAN_LINK || MODE == MODE_DBSCAN_BORDER) {
               // the survivors that are core points: the leaf's core bits come with one bitset load (<= 32 consecutive positions)
               uint32_t m = mask_a & dbscan::bits_at(P.core_words, P.n_core_words, (uint32_t)start);
@@ -733,6 +773,13 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
     } else if (MODE == MODE_DBSCAN_CORE) {
       const unsigned core = __ballot_sync(FULL_MASK, valid && cnt >= k);
       if (lane == 0) P.unresolved[group] = core;  // groups are positions 32 g .. 32 g + 31 (no queue)
+    } else if (MODE == MODE_RANGE_LIST_COUNT) {
+      if (valid) {
+        P.count_out[qpos] = (uint32_t)cnt;
+        P.count_row[row_id] = (uint32_t)cnt;
+      }
+    } else if (MODE == MODE_RANGE_LIST) {
+      // nothing to emit: the keys are written
     } else if (MODE == MODE_DBSCAN_LINK) {
       // nothing to emit: the unions are the result
     } else if (MODE == MODE_DBSCAN_BORDER) {

@@ -20,6 +20,7 @@
 #include "ctx.cuh"
 #include "lbvh.cuh"
 #include "radix_sort.cuh"
+#include "radius.cuh"
 #include "traverse.cuh"
 
 using namespace tknn;
@@ -809,7 +810,10 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->b_keys_b, &c->b_vals_a, &c->b_vals_b, &c->b_sort_tmp, &c->b_delta, &c->b_ballots, &c->b_leaf_key,
                     &c->b_child_info, &c->b_parent_leaf, &c->b_parent_node, &c->b_arrive, &c->q_stage, &c->q_keys_a, &c->q_keys_b,
                     &c->q_vals_a, &c->q_vals_b, &c->q_sort_tmp, &c->q_pts, &c->q_sid_stage, &c->q_sid_sorted, &c->q_rad_stage,
-                    &c->q_r2_sorted, &c->db_parent, &c->db_min_idx, &c->db_pos_label, &c->db_bits, &c->db_core_stage})
+                    &c->q_r2_sorted, &c->db_parent, &c->db_min_idx, &c->db_pos_label, &c->db_bits, &c->db_core_stage,
+                    &c->rl_cnt_pos, &c->rl_cnt_row, &c->rl_off_pos, &c->rl_off_row, &c->rl_sums, &c->rl_stats, &c->rl_pos_of,
+                    &c->rl_self_pos, &c->rl_keys, &c->rl_long_pos, &c->rl_long_len, &c->rl_boff, &c->rl_ka, &c->rl_kb,
+                    &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -1140,6 +1144,79 @@ int tknn_estimate_start_radius(tknn_ctx* c, int k, float* radius_out) {
   return TKNN_OK;
 }
 
+}  // extern "C"
+
+namespace {
+// The query staging of tknn_query and tknn_radius_query: host inputs are copied to the device, the queries are sorted on
+// the DATA's space-filling curve so that groups of 32 are spatially coherent, and gathered into c->q_pts (x, y, z, query
+// row bits); self ids and radius caps follow into that order.  Sets SC_ERROR / SC_QBAD (a non-finite query coordinate).
+int stage_queries(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats, const int32_t* self_ids,
+                  const float* init_radius2, const int32_t** sid_sorted_out, const float** r2_sorted_out, int* launches) {
+  cudaStream_t st = c->stream;
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  DevBuf &q_stage = c->q_stage, &keys_a = c->q_keys_a, &keys_b = c->q_keys_b, &vals_a = c->q_vals_a, &vals_b = c->q_vals_b,
+         &sort_tmp = c->q_sort_tmp, &qpts = c->q_pts, &sid_stage = c->q_sid_stage, &sid_sorted = c->q_sid_sorted,
+         &rad_stage = c->q_rad_stage, &r2_sorted = c->q_r2_sorted;
+  *sid_sorted_out = nullptr;
+  *r2_sorted_out = nullptr;
+  const float* d_q = queries;
+  if (!is_device_ptr(queries)) {
+    const size_t bytes = (size_t)nq * stride_floats * sizeof(float);
+    TK_TRY(ensure(c, q_stage, bytes));
+    TK_CUDA(c, cudaMemcpyAsync(q_stage.p, queries, bytes, cudaMemcpyHostToDevice, st));
+    d_q = q_stage.as<float>();
+  }
+  const int32_t* d_sid = self_ids;
+  if (self_ids && !is_device_ptr(self_ids)) {
+    TK_TRY(ensure(c, sid_stage, nq * sizeof(int32_t)));
+    TK_CUDA(c, cudaMemcpyAsync(sid_stage.p, self_ids, nq * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    d_sid = sid_stage.as<int32_t>();
+  }
+  const float* d_rad = init_radius2;
+  if (init_radius2 && !is_device_ptr(init_radius2)) {
+    TK_TRY(ensure(c, rad_stage, nq * sizeof(float)));
+    TK_CUDA(c, cudaMemcpyAsync(rad_stage.p, init_radius2, nq * sizeof(float), cudaMemcpyHostToDevice, st));
+    d_rad = rad_stage.as<float>();
+  }
+  // Morton-sort the queries on the DATA's grid so that groups of 32 are spatially coherent
+  TK_TRY(ensure(c, keys_a, nq * sizeof(uint64_t)));
+  TK_TRY(ensure(c, keys_b, nq * sizeof(uint64_t)));
+  TK_TRY(ensure(c, vals_a, nq * sizeof(uint32_t)));
+  TK_TRY(ensure(c, vals_b, nq * sizeof(uint32_t)));
+  TK_TRY(ensure(c, sort_tmp, rsort::temp_words(nq) * sizeof(uint32_t)));
+  TK_TRY(ensure(c, qpts, nq * sizeof(float4)));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), st));
+  const int qbits = c->built_morton_bits;
+  lbvh::morton_kernel<<<blocks_for(nq, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_q, nq, dim, stride_floats, sc + SC_BOUNDS, qbits,
+                                                                              c->built_curve, 0, keys_a.as<uint64_t>(), vals_a.as<uint32_t>());
+  ++*launches;
+  bool q_in_b = false;
+  *launches += rsort::sort_pairs(keys_a.as<uint64_t>(), vals_a.as<uint32_t>(), keys_b.as<uint64_t>(), vals_b.as<uint32_t>(), nq,
+                                sort_tmp.as<uint32_t>(), c->sm_count, st, (3 * qbits + 7) / 8, &q_in_b);
+  const uint32_t* qorder = q_in_b ? vals_b.as<uint32_t>() : vals_a.as<uint32_t>();
+  lbvh::gather_points_kernel<<<blocks_for(nq, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_q, dim, stride_floats,
+                                                                                    qorder, nullptr, 0, nq, 0, qpts.as<float4>(), sc + SC_QBAD);
+  TK_CUDA(c, cudaGetLastError());
+  ++*launches;
+  if (d_sid) {
+    TK_TRY(ensure(c, sid_sorted, nq * sizeof(int32_t)));
+    brute::gather_i32_kernel<<<blocks_for(nq, 256), 256, 0, st>>>(d_sid, qorder, nq, sid_sorted.as<int32_t>());
+    *sid_sorted_out = sid_sorted.as<int32_t>();
+    ++*launches;
+  }
+  if (d_rad) {
+    TK_TRY(ensure(c, r2_sorted, nq * sizeof(float)));
+    brute::gather_r2_kernel<<<blocks_for(nq, 256), 256, 0, st>>>(d_rad, qorder, nq, r2_sorted.as<float>());
+    *r2_sorted_out = r2_sorted.as<float>();
+    ++*launches;
+  }
+  return TKNN_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
 int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats, const int32_t* self_ids,
                const float* init_radius2, int k, float start_radius, int32_t* idx_out, float* dist_out) {
   TK_TRY(check_ctx(c));
@@ -1175,60 +1252,10 @@ int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stri
     return fail(c, e_ == cudaErrorMemoryAllocation ? TKNN_ENOMEM : TKNN_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_)); } } while (0)
 
   TK_BC(cudaEventRecord(c->ev[0], st));
-  const float* d_q = queries;
-  if (!is_device_ptr(queries)) {
-    const size_t bytes = (size_t)nq * stride_floats * sizeof(float);
-    TK_B(ensure(c, q_stage, bytes));
-    TK_BC(cudaMemcpyAsync(q_stage.p, queries, bytes, cudaMemcpyHostToDevice, st));
-    d_q = q_stage.as<float>();
-  }
-  const int32_t* d_sid = self_ids;
-  if (self_ids && !is_device_ptr(self_ids)) {
-    TK_B(ensure(c, sid_stage, nq * sizeof(int32_t)));
-    TK_BC(cudaMemcpyAsync(sid_stage.p, self_ids, nq * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    d_sid = sid_stage.as<int32_t>();
-  }
-  const float* d_rad = init_radius2;
-  if (init_radius2 && !is_device_ptr(init_radius2)) {
-    TK_B(ensure(c, rad_stage, nq * sizeof(float)));
-    TK_BC(cudaMemcpyAsync(rad_stage.p, init_radius2, nq * sizeof(float), cudaMemcpyHostToDevice, st));
-    d_rad = rad_stage.as<float>();
-  }
-  // Morton-sort the queries on the DATA's grid so that groups of 32 are spatially coherent
-  TK_B(ensure(c, keys_a, nq * sizeof(uint64_t)));
-  TK_B(ensure(c, keys_b, nq * sizeof(uint64_t)));
-  TK_B(ensure(c, vals_a, nq * sizeof(uint32_t)));
-  TK_B(ensure(c, vals_b, nq * sizeof(uint32_t)));
-  TK_B(ensure(c, sort_tmp, rsort::temp_words(nq) * sizeof(uint32_t)));
-  TK_B(ensure(c, qpts, nq * sizeof(float4)));
   int launches = 0;
-  TK_BC(cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), st));
-  const int qbits = c->built_morton_bits;
-  lbvh::morton_kernel<<<blocks_for(nq, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_q, nq, dim, stride_floats, sc + SC_BOUNDS, qbits,
-                                                                              c->built_curve, 0, keys_a.as<uint64_t>(), vals_a.as<uint32_t>());
-  ++launches;
-  bool q_in_b = false;
-  launches += rsort::sort_pairs(keys_a.as<uint64_t>(), vals_a.as<uint32_t>(), keys_b.as<uint64_t>(), vals_b.as<uint32_t>(), nq,
-                                sort_tmp.as<uint32_t>(), c->sm_count, st, (3 * qbits + 7) / 8, &q_in_b);
-  const uint32_t* qorder = q_in_b ? vals_b.as<uint32_t>() : vals_a.as<uint32_t>();
-  lbvh::gather_points_kernel<<<blocks_for(nq, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_q, dim, stride_floats,
-                                                                                    qorder, nullptr, 0, nq, 0, qpts.as<float4>(), sc + SC_QBAD);
-  TK_BC(cudaGetLastError());
-  ++launches;
   const int32_t* d_sid_sorted = nullptr;
   const float* d_r2_sorted = nullptr;
-  if (d_sid) {
-    TK_B(ensure(c, sid_sorted, nq * sizeof(int32_t)));
-    brute::gather_i32_kernel<<<blocks_for(nq, 256), 256, 0, st>>>(d_sid, qorder, nq, sid_sorted.as<int32_t>());
-    d_sid_sorted = sid_sorted.as<int32_t>();
-    ++launches;
-  }
-  if (d_rad) {
-    TK_B(ensure(c, r2_sorted, nq * sizeof(float)));
-    brute::gather_r2_kernel<<<blocks_for(nq, 256), 256, 0, st>>>(d_rad, qorder, nq, r2_sorted.as<float>());
-    d_r2_sorted = r2_sorted.as<float>();
-    ++launches;
-  }
+  TK_B(stage_queries(c, queries, nq, dim, stride_floats, self_ids, init_radius2, &d_sid_sorted, &d_r2_sorted, &launches));
 
   const bool idx_dev = is_device_ptr(idx_out), dist_dev = is_device_ptr(dist_out);
   int32_t* d_idx = idx_out;
@@ -1470,6 +1497,311 @@ int tknn_dbscan(tknn_ctx* c, float eps, int min_pts, int32_t* label_out, uint8_t
   TK_TRY(collect_counters(c));
   TK_TRY(read_error_flag(c));
   return TKNN_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+// Long rows are radix-sorted in batches of at most this many entries (40 B of device scratch per entry).
+constexpr uint64_t RADIUS_LONG_BATCH = 1ull << 26;
+
+// exclusive u64 scan of counts[0 .. m) into off[0 .. m] (off[m] = total, also written to *total)
+int scan_counts(tknn_ctx* c, const uint32_t* counts, uint64_t m, uint64_t* off, uint64_t* total, int* launches) {
+  const uint64_t nb = std::max<uint64_t>(1, (m + radius::SCAN_CHUNK - 1) / radius::SCAN_CHUNK);
+  TK_TRY(ensure(c, c->rl_sums, sizeof(uint64_t) * nb));
+  uint64_t* sums = c->rl_sums.as<uint64_t>();
+  radius::scan_reduce_kernel<<<(unsigned)nb, radius::THREADS, 0, c->stream>>>(counts, m, sums);
+  radius::scan_sums_kernel<<<1, radius::THREADS, 0, c->stream>>>(sums, nb, total);
+  radius::scan_apply_kernel<<<(unsigned)nb, radius::THREADS, 0, c->stream>>>(counts, m, sums, total, off);
+  TK_CUDA(c, cudaGetLastError());
+  *launches += 3;
+  return TKNN_OK;
+}
+
+// The pipeline of radius.cuh over nq staged query positions (qpts: x, y, z, output row bits).  self_sorted: the excluded
+// data index per position (query form) or nullptr with self_is_row (all-points form: the point itself).  The caller has
+// recorded c->ev[0] and cleared SC_ERROR / SC_QBAD; launches counts its own kernels so far.
+int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* self_sorted, int self_is_row, float radius,
+                uint64_t* offsets_out, int32_t* idx_out, float* dist_out, uint64_t capacity, uint64_t* total_out,
+                int launches) {
+  cudaStream_t st = c->stream;
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  const uint64_t n = c->n;
+  const bool fill_rows = idx_out != nullptr;
+  const bool off_dev = is_device_ptr(offsets_out);
+  auto cleanup = [&]() {
+    if (c->keep_scratch) return;
+    for (DevBuf* b : {&c->rl_cnt_pos, &c->rl_cnt_row, &c->rl_off_pos, &c->rl_off_row, &c->rl_sums, &c->rl_stats, &c->rl_pos_of,
+                      &c->rl_self_pos, &c->rl_keys, &c->rl_long_pos, &c->rl_long_len, &c->rl_boff, &c->rl_ka, &c->rl_kb,
+                      &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp})
+      release(*b);
+  };
+#define TK_R(expr) do { int rc_ = (expr); if (rc_ != TKNN_OK) { cleanup(); return rc_; } } while (0)
+#define TK_RC(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { cudaGetLastError(); cleanup(); \
+    return fail(c, e_ == cudaErrorMemoryAllocation ? TKNN_ENOMEM : TKNN_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_)); } } while (0)
+  for (size_t i = c->round_ev.size(); i < 12; ++i) {
+    cudaEvent_t e;
+    TK_RC(cudaEventCreate(&e));
+    c->round_ev.push_back(e);
+  }
+  cudaEvent_t* ev = c->round_ev.data();  // phase r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its kernels
+
+  TK_R(ensure(c, c->rl_cnt_pos, sizeof(uint32_t) * nq));
+  TK_R(ensure(c, c->rl_cnt_row, sizeof(uint32_t) * nq));
+  TK_R(ensure(c, c->rl_off_pos, sizeof(uint64_t) * (nq + 1)));
+  if (!off_dev) TK_R(ensure(c, c->rl_off_row, sizeof(uint64_t) * (nq + 1)));
+  TK_R(ensure(c, c->rl_stats, sizeof(uint64_t) * 4));
+  TK_R(ensure(c, c->rl_long_pos, sizeof(uint32_t) * nq));
+  TK_R(ensure(c, c->rl_long_len, sizeof(uint32_t) * nq));
+  uint32_t* cnt_pos = c->rl_cnt_pos.as<uint32_t>();
+  uint32_t* cnt_row = c->rl_cnt_row.as<uint32_t>();
+  uint64_t* off_pos = c->rl_off_pos.as<uint64_t>();
+  uint64_t* off_row = off_dev ? offsets_out : c->rl_off_row.as<uint64_t>();
+  uint64_t* rstats = c->rl_stats.as<uint64_t>();  // row total, position total, long rows, long-row entries
+  uint32_t* long_pos = c->rl_long_pos.as<uint32_t>();
+  const int32_t* self_pos = nullptr;
+  if (self_sorted) {
+    TK_R(ensure(c, c->rl_pos_of, sizeof(int32_t) * n));
+    TK_R(ensure(c, c->rl_self_pos, sizeof(int32_t) * nq));
+    self_pos = c->rl_self_pos.as<int32_t>();
+  }
+
+  trav::Params P;
+  std::memset(&P, 0, sizeof(P));
+  P.nodes = c->nodes.as<Node>();
+  P.node_min_idx = c->node_min_idx.as<int2>();
+  P.pts = c->pts.as<float4>();
+  P.queries = qpts;
+  P.n_active = nq;
+  P.n_groups = (uint32_t)((nq + 31) / 32);
+  P.r2 = radius * radius;
+  P.k = 0;
+  P.self_is_row = self_is_row;
+  P.self_pos = self_pos;
+  P.final_round = 1;
+  P.squared = c->squared;
+  P.error = sc + SC_ERROR;
+  P.group_counter = sc + SC_GROUP_COUNTER;
+  P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
+  TK_RC(cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
+
+  // 1. count (minus self, by position and by row), both scans, the long-row list; one read-back
+  TK_RC(cudaEventRecord(ev[0], st));
+  if (self_sorted) {
+    radius::inverse_kernel<<<blocks_for(n, 256), 256, 0, st>>>(P.pts, n, c->rl_pos_of.as<int32_t>());
+    radius::self_pos_kernel<<<blocks_for(nq, 256), 256, 0, st>>>(self_sorted, nq, c->rl_pos_of.as<int32_t>(), n,
+                                                                 c->rl_self_pos.as<int32_t>());
+    TK_RC(cudaGetLastError());
+    launches += 2;
+  }
+  TK_RC(cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), st));
+  P.count_out = cnt_pos;
+  P.count_row = cnt_row;
+  TK_RC(cudaEventRecord(ev[2], st));
+  TK_R(launch_traverse<trav::MODE_RANGE_LIST_COUNT>(c, P));
+  TK_RC(cudaEventRecord(ev[3], st));
+  TK_R(scan_counts(c, cnt_row, nq, off_row, rstats, &launches));
+  TK_R(scan_counts(c, cnt_pos, nq, off_pos, rstats + 1, &launches));
+  TK_RC(cudaMemsetAsync(rstats + 2, 0, 2 * sizeof(uint64_t), st));
+  radius::long_rows_kernel<<<blocks_for(nq, 256), 256, 0, st>>>(cnt_pos, nq, long_pos, c->rl_long_len.as<uint32_t>(),
+                                                                 reinterpret_cast<unsigned long long*>(rstats + 2));
+  TK_RC(cudaGetLastError());
+  launches += 2;  // the traversal, long_rows_kernel
+  TK_RC(cudaEventRecord(ev[1], st));
+  uint64_t rb[4] = {0, 0, 0, 0};
+  TK_R(fetch_words(c, reinterpret_cast<const uint32_t*>(rstats), 8, nullptr, 0, reinterpret_cast<uint32_t*>(rb)));
+  const uint64_t total = rb[0], n_long = rb[2];
+  if (rb[1] != total) { cleanup(); return fail(c, TKNN_ECUDA, "internal: row and position totals differ"); }
+  if (total_out) *total_out = total;
+  if (!off_dev) {
+    TK_RC(cudaMemcpyAsync(offsets_out, off_row, sizeof(uint64_t) * (nq + 1), cudaMemcpyDeviceToHost, st));
+    c->stats.d2h_bytes += sizeof(uint64_t) * (nq + 1);
+  }
+  const bool write_rows = fill_rows && capacity >= total;
+
+  // 2. fill: the unsorted rows in position order
+  TK_RC(cudaEventRecord(ev[4], st));
+  TK_RC(cudaEventRecord(ev[6], st));
+  const bool idx_dev = write_rows && is_device_ptr(idx_out), dist_dev = write_rows && dist_out && is_device_ptr(dist_out);
+  int32_t* d_idx = idx_out;
+  float* d_dist = dist_out;
+  if (write_rows && total) {
+    TK_R(ensure(c, c->rl_keys, sizeof(uint64_t) * total));
+    if (!idx_dev) { TK_R(ensure(c, c->stage_idx, sizeof(int32_t) * total)); d_idx = c->stage_idx.as<int32_t>(); }
+    if (dist_out && !dist_dev) { TK_R(ensure(c, c->stage_dist, sizeof(float) * total)); d_dist = c->stage_dist.as<float>(); }
+    TK_RC(cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), st));
+    P.list_off = off_pos;
+    P.list_keys = c->rl_keys.as<uint64_t>();
+    TK_R(launch_traverse<trav::MODE_RANGE_LIST>(c, P));
+    ++launches;
+  }
+  TK_RC(cudaEventRecord(ev[7], st));
+  TK_RC(cudaEventRecord(ev[5], st));
+
+  // 3. order: short rows one warp each in shared memory, long rows by the radix sort in batches
+  TK_RC(cudaEventRecord(ev[8], st));
+  TK_RC(cudaEventRecord(ev[10], st));
+  if (write_rows && total) {
+    const uint64_t* keys = c->rl_keys.as<uint64_t>();
+    radius::sort_rows_warp_kernel<<<blocks_for(nq, radius::SORT_WARPS), radius::SORT_WARPS * 32, 0, st>>>(
+        keys, off_pos, cnt_pos, qpts, nq, off_row, c->squared, d_idx, d_dist);
+    TK_RC(cudaGetLastError());
+    ++launches;
+    if (n_long) {
+      // the long rows in position order (the list was appended in any order), their lengths and global prefix
+      std::vector<uint32_t> hpos(n_long), hlen(n_long), lp(n_long);
+      std::vector<uint64_t> order(n_long), boff(n_long + 1);
+      TK_RC(cudaMemcpyAsync(hpos.data(), long_pos, sizeof(uint32_t) * n_long, cudaMemcpyDeviceToHost, st));
+      TK_RC(cudaMemcpyAsync(hlen.data(), c->rl_long_len.p, sizeof(uint32_t) * n_long, cudaMemcpyDeviceToHost, st));
+      TK_RC(cudaStreamSynchronize(st));
+      for (uint64_t r = 0; r < n_long; ++r) order[r] = r;
+      std::sort(order.begin(), order.end(), [&](uint64_t a, uint64_t b) { return hpos[a] < hpos[b]; });
+      boff[0] = 0;
+      for (uint64_t r = 0; r < n_long; ++r) {
+        lp[r] = hpos[order[r]];
+        const uint64_t len = hlen[order[r]];
+        if (len > rsort::MAX_N) { cleanup(); return fail(c, TKNN_EINVAL, "a row of %llu entries exceeds the sort's limit",
+                                                         (unsigned long long)len); }
+        boff[r + 1] = boff[r] + len;
+      }
+      TK_R(ensure(c, c->rl_boff, sizeof(uint64_t) * (n_long + 1)));
+      TK_RC(cudaMemcpyAsync(long_pos, lp.data(), sizeof(uint32_t) * n_long, cudaMemcpyHostToDevice, st));
+      TK_RC(cudaMemcpyAsync(c->rl_boff.p, boff.data(), sizeof(uint64_t) * (n_long + 1), cudaMemcpyHostToDevice, st));
+      uint64_t batch_max = 0;  // entries of the largest batch
+      std::vector<uint64_t> firsts;
+      for (uint64_t r = 0; r < n_long;) {
+        uint64_t e = r + 1;
+        while (e < n_long && boff[e + 1] - boff[r] <= RADIUS_LONG_BATCH) ++e;
+        firsts.push_back(r);
+        batch_max = std::max(batch_max, boff[e] - boff[r]);
+        r = e;
+      }
+      firsts.push_back(n_long);
+      TK_R(ensure(c, c->rl_ka, sizeof(uint64_t) * batch_max));
+      TK_R(ensure(c, c->rl_kb, sizeof(uint64_t) * batch_max));
+      TK_R(ensure(c, c->rl_kc, sizeof(uint64_t) * batch_max));
+      TK_R(ensure(c, c->rl_va, sizeof(uint32_t) * batch_max));
+      TK_R(ensure(c, c->rl_vb, sizeof(uint32_t) * batch_max));
+      TK_R(ensure(c, c->rl_vc, sizeof(uint32_t) * batch_max));
+      TK_R(ensure(c, c->rl_row_of, sizeof(uint32_t) * batch_max));
+      TK_R(ensure(c, c->rl_sort_tmp, sizeof(uint32_t) * rsort::temp_words(batch_max)));
+      uint64_t *ka = c->rl_ka.as<uint64_t>(), *kb = c->rl_kb.as<uint64_t>(), *kc = c->rl_kc.as<uint64_t>();
+      uint32_t *va = c->rl_va.as<uint32_t>(), *vb = c->rl_vb.as<uint32_t>(), *vc = c->rl_vc.as<uint32_t>();
+      uint32_t* row_of = c->rl_row_of.as<uint32_t>();
+      const uint64_t* d_boff = c->rl_boff.as<uint64_t>();
+      for (size_t b = 0; b + 1 < firsts.size(); ++b) {
+        const uint32_t first = (uint32_t)firsts[b], rows = (uint32_t)(firsts[b + 1] - firsts[b]);
+        const uint64_t e = boff[firsts[b + 1]] - boff[first];
+        radius::long_gather_kernel<<<rows, radius::THREADS, 0, st>>>(keys, off_pos, long_pos, d_boff, first, ka, va, row_of);
+        // by key (all 64 bits: 8 passes, so the result is back in ka / va) ...
+        bool in_b = false;
+        launches += 1 + rsort::sort_pairs(ka, va, kb, vb, e, c->rl_sort_tmp.as<uint32_t>(), c->sm_count, st, rsort::PASSES, &in_b);
+        if (in_b) { cleanup(); return fail(c, TKNN_ECUDA, "internal: odd key-sort pass count"); }
+        // ... then stably by the row's rank in the batch
+        radius::long_rowkey_kernel<<<blocks_for(e, 256), 256, 0, st>>>(va, row_of, e, kb, vb);
+        const int row_bits = rows > 1 ? 32 - __builtin_clz(rows - 1) : 1;
+        launches += 1 + rsort::sort_pairs(kb, vb, kc, vc, e, c->rl_sort_tmp.as<uint32_t>(), c->sm_count, st,
+                                          (row_bits + 7) / 8, &in_b);
+        radius::long_emit_kernel<<<blocks_for(e, 256), 256, 0, st>>>(ka, in_b ? kc : kb, in_b ? vc : vb, e, long_pos, d_boff,
+                                                                     first, qpts, off_row, c->squared, d_idx, d_dist);
+        TK_RC(cudaGetLastError());
+        ++launches;
+      }
+    }
+  }
+  TK_RC(cudaEventRecord(ev[11], st));
+  TK_RC(cudaEventRecord(ev[9], st));
+  TK_RC(cudaEventRecord(c->ev[2], st));
+  if (write_rows && total) {
+    if (!idx_dev) {
+      TK_RC(cudaMemcpyAsync(idx_out, d_idx, sizeof(int32_t) * total, cudaMemcpyDeviceToHost, st));
+      c->stats.d2h_bytes += sizeof(int32_t) * total;
+    }
+    if (dist_out && !dist_dev) {
+      TK_RC(cudaMemcpyAsync(dist_out, d_dist, sizeof(float) * total, cudaMemcpyDeviceToHost, st));
+      c->stats.d2h_bytes += sizeof(float) * total;
+    }
+  }
+  TK_RC(cudaStreamSynchronize(st));
+  cleanup();
+#undef TK_R
+#undef TK_RC
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
+  c->stats.n_queries = nq;
+  c->stats.rounds = 3;
+  c->stats.start_radius = c->stats.final_radius = radius;
+  c->stats.round_queries[0] = nq;
+  c->stats.round_queries[1] = write_rows ? nq : 0;
+  c->stats.round_queries[2] = write_rows ? n_long : 0;
+  c->stats.kernel_launches = (uint32_t)(launches + c->mailbox_launches + (c->mailbox_h ? 1 : 0));  // + the error-flag fetch
+  TK_TRY(finish_round_stats(c));
+  TK_TRY(collect_counters(c));
+  TK_TRY(read_error_flag(c));
+  if (fill_rows && !write_rows)
+    return fail(c, TKNN_EINVAL, "capacity %llu < %llu entries", (unsigned long long)capacity, (unsigned long long)total);
+  return TKNN_OK;
+}
+
+// checks shared by both forms; nq = 0 (query form) writes offsets_out[0] = 0 and a zero total
+int radius_args(tknn_ctx* c, const char* what, float radius, uint64_t* offsets_out) {
+  TK_TRY(check_ctx(c));
+  if (c->n == 0) return fail(c, TKNN_ESTATE, "%s before tknn_build", what);
+  if (c->ids_in_w) return fail(c, TKNN_ESTATE, "this BVH carries caller-chosen point ids (point-partitioned build)");
+  if (!(radius >= 0.0f)) return fail(c, TKNN_EINVAL, "radius must be >= 0");
+  if (!offsets_out) return fail(c, TKNN_EINVAL, "null offsets array");
+  if (c->n > (uint64_t)INT32_MAX) return fail(c, TKNN_EINVAL, "%s supports at most 2^31 - 1 points", what);
+  return TKNN_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tknn_radius_search(tknn_ctx* c, float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out,
+                       uint64_t capacity, uint64_t* total_out) {
+  TK_TRY(radius_args(c, "tknn_radius_search", radius, offsets_out));
+  ScopedDevice sd(c->device);
+  reset_search_stats(c);
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  TK_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), c->stream));
+  return radius_core(c, c->pts.as<float4>(), c->n, nullptr, 1, radius, offsets_out, idx_out, dist_out, capacity, total_out, 0);
+}
+
+int tknn_radius_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats, const int32_t* self_ids,
+                      float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out, uint64_t capacity,
+                      uint64_t* total_out) {
+  TK_TRY(radius_args(c, "tknn_radius_query", radius, offsets_out));
+  if (!queries && nq) return fail(c, TKNN_EINVAL, "null query array");
+  if (dim != 2 && dim != 3) return fail(c, TKNN_EINVAL, "dim = %d (must be 2 or 3)", dim);
+  if (stride_floats < dim) return fail(c, TKNN_EINVAL, "stride %d < dim %d", stride_floats, dim);
+  if (nq > rsort::MAX_N) return fail(c, TKNN_EINVAL, "too many queries");
+  ScopedDevice sd(c->device);
+  reset_search_stats(c);
+  if (nq == 0) {
+    if (total_out) *total_out = 0;
+    if (is_device_ptr(offsets_out)) {
+      TK_CUDA(c, cudaMemsetAsync(offsets_out, 0, sizeof(uint64_t), c->stream));
+      TK_CUDA(c, cudaStreamSynchronize(c->stream));
+    } else {
+      offsets_out[0] = 0;
+    }
+    return TKNN_OK;
+  }
+  TK_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  int launches = 0;
+  const int32_t* d_sid_sorted = nullptr;
+  const float* d_r2_sorted = nullptr;
+  int rc = stage_queries(c, queries, nq, dim, stride_floats, self_ids, nullptr, &d_sid_sorted, &d_r2_sorted, &launches);
+  if (rc == TKNN_OK)
+    rc = radius_core(c, c->q_pts.as<float4>(), nq, d_sid_sorted, 0, radius, offsets_out, idx_out, dist_out, capacity,
+                     total_out, launches);
+  if (!c->keep_scratch)
+    for (DevBuf* b : {&c->q_stage, &c->q_keys_a, &c->q_keys_b, &c->q_vals_a, &c->q_vals_b, &c->q_sort_tmp, &c->q_pts,
+                      &c->q_sid_stage, &c->q_sid_sorted})
+      release(*b);
+  return rc;
 }
 
 int tknn_brute_force(tknn_ctx* c, const int32_t* query_ids, uint64_t nq, int k, int32_t* idx_out, float* dist_out) {

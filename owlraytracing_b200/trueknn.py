@@ -264,6 +264,82 @@ class TrueKNN:
         self._check(self._L.tknn_dbscan(self._h, C.c_float(eps), int(min_pts), _ptr(labels), _ptr(core), C.byref(c)))
         return labels, core, int(c.value)
 
+    def radius_search(self, radius: float, indices_only: bool = False, out=None):
+        """Exact fixed-radius neighbour lists of every built point (closed ball, the point itself excluded).
+
+        Returns CSR (offsets [n + 1] int64, idx [total] int32, dist [total] float32 or None when indices_only): row q is
+        idx[offsets[q]:offsets[q + 1]], sorted by (distance, index), rows in build order; dist is d2 while squared_dist
+        is set.  numpy outputs for numpy input, CUDA tensors for CUDA tensor input, so that
+        torch.sparse_csr_tensor(offsets, idx, dist) works directly.  Without `out` a size call comes first;
+        out = (offsets, idx, dist) (dist may be None) makes one call and raises TrueKNNError naming the total needed
+        when idx is too short."""
+        def call(off, idx, dist, cap, total):
+            return self._L.tknn_radius_search(self._h, C.c_float(radius), _ptr(off), _ptr(idx), _ptr(dist), cap,
+                                              C.byref(total))
+
+        return self._radius_lists(self._like, self.n, indices_only, out, call)
+
+    def radius_query(self, queries, radius: float, self_ids=None, dim: int | None = None, indices_only: bool = False,
+                     out=None):
+        """Exact fixed-radius neighbour lists of a separate query set (rows in query order); self_ids (optional, -1 =
+        none) names the data index each query excludes.  Returns (offsets, idx, dist) as radius_search()."""
+        if not _is_tensor(queries):
+            queries = np.ascontiguousarray(queries, dtype=np.float32)
+        _check_dtype(queries, np.float32, "queries")
+        nq, stride = int(queries.shape[0]), int(queries.shape[1])
+        if dim is None:
+            dim = min(stride, 3)
+        if self_ids is not None and not _is_tensor(self_ids):
+            self_ids = np.ascontiguousarray(self_ids, dtype=np.int32)
+        if self_ids is not None:
+            _check_dtype(self_ids, np.int32, "self_ids")
+        q_ptr, sid_ptr = self._in(queries), self._in(self_ids)
+
+        def call(off, idx, dist, cap, total):
+            return self._L.tknn_radius_query(self._h, q_ptr, nq, int(dim), stride, sid_ptr, C.c_float(radius), _ptr(off),
+                                             _ptr(idx), _ptr(dist), cap, C.byref(total))
+
+        return self._radius_lists(queries, nq, indices_only, out, call)
+
+    def _radius_lists(self, like, nq: int, indices_only: bool, out, call):
+        def empty(m, dtype):
+            if _is_tensor(like):
+                import torch
+
+                t = torch.empty((m,), dtype={np.int64: torch.int64, np.int32: torch.int32, np.float32: torch.float32}[dtype],
+                                device=like.device)
+                self._settle_outputs(t)
+                return t
+            return np.empty((m,), dtype)
+
+        total = C.c_uint64(0)
+        if out is not None:
+            offsets, idx, dist = out
+            _check_dtype(idx, np.int32, "idx")
+            if dist is not None:
+                _check_dtype(dist, np.float32, "dist")
+            if _is_tensor(offsets):
+                _check_dtype(offsets, np.uint64, "offsets")
+            elif offsets.dtype not in (np.int64, np.uint64):
+                raise TypeError(f"offsets: expected int64, got {offsets.dtype}")
+            if int(offsets.shape[0]) < nq + 1:
+                raise ValueError(f"offsets holds {int(offsets.shape[0])} entries, {nq + 1} needed")
+            cap = int(idx.shape[0]) if dist is None else min(int(idx.shape[0]), int(dist.shape[0]))
+            rc = call(offsets, idx, dist, cap, total)
+            if rc == _lib.EINVAL and total.value > cap:
+                raise TrueKNNError(rc, f"the neighbour lists hold {total.value} entries, out has room for {cap}")
+            self._check(rc)
+            t = int(total.value)
+            return offsets, idx[:t], dist[:t] if dist is not None else None
+        offsets = empty(nq + 1, np.int64)
+        self._check(call(offsets, None, None, 0, total))
+        t = int(total.value)
+        idx = empty(t, np.int32)
+        dist = None if indices_only else empty(t, np.float32)
+        if t:
+            self._check(call(offsets, idx, dist, t, total))
+        return offsets, idx, dist
+
     def estimate_start_radius(self, k: int) -> float:
         r = C.c_float(0)
         self._check(self._L.tknn_estimate_start_radius(self._h, int(k), C.byref(r)))
@@ -595,6 +671,21 @@ def write_neighbours(path: str, idx: np.ndarray, dist: np.ndarray, binary: bool 
                                  idx.shape[1], 1 if binary else 0)
     if rc != _lib.OK:
         raise OSError(f"tknn_write_neighbours({path!r}) failed")
+
+
+def write_neighbour_lists(path: str, offsets: np.ndarray, idx: np.ndarray, dist: np.ndarray | None, binary: bool = False):
+    """The CSR rows of radius_search / radius_query: `query,neighbourIndex,distance` lines, or path.off.u64,
+    path.idx.i32 and path.dist.f32 when binary (tknn_write_neighbour_lists)."""
+    L = _lib.load()
+    offsets = np.ascontiguousarray(offsets).view(np.uint64) if np.asarray(offsets).dtype == np.int64 else \
+        np.ascontiguousarray(offsets, dtype=np.uint64)
+    idx = np.ascontiguousarray(idx, dtype=np.int32)
+    dist = None if dist is None else np.ascontiguousarray(dist, dtype=np.float32)
+    rc = L.tknn_write_neighbour_lists(path.encode(), C.c_void_p(offsets.ctypes.data), C.c_void_p(idx.ctypes.data),
+                                      None if dist is None else C.c_void_p(dist.ctypes.data), offsets.shape[0] - 1,
+                                      1 if binary else 0)
+    if rc != _lib.OK:
+        raise OSError(f"tknn_write_neighbour_lists({path!r}) failed")
 
 
 def run_sample(argv: list[str], device: int = 0, neighbours_path: str | None = None) -> dict:

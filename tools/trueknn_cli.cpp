@@ -2,7 +2,11 @@
 //
 //   trueknn <file> <n> <dim> <start radius> <k> <output file> [--neighbours <path> [--binary]] [--device <d>] [--json]
 //           [--gpus <N> | --devices <a,b,...>] [--mode shard|partition] [--dbscan <eps> <min_pts> [--labels <path> [--binary]]]
+//           [--radius-search <r> [--neighbours <path> [--binary]]]
 //
+// --radius-search runs the exact fixed-radius neighbour lists (tknn_radius_search) instead of the kNN search after the
+// build; k and the start radius are still required and are ignored.  --neighbours then writes one
+// `query,neighbourIndex,distance` line per entry, or <path>.off.u64 / .idx.i32 / .dist.f32 with --binary.
 // --dbscan runs exact DBSCAN (tknn_dbscan) instead of the kNN search after the build; k and the start radius are still
 // required and are ignored.  --labels writes `point,label` lines (label -1 = noise), or raw int32 labels with --binary.
 // --gpus N (devices 0..N-1) or --devices (an explicit list; naming one device several times runs that many ranks on
@@ -31,7 +35,8 @@
 int main(int ac, char** av) {
   std::vector<std::string> pos;
   std::string neigh_path, labels_path, mode = "shard";
-  bool dbscan = false;
+  bool dbscan = false, radius_search = false;
+  float rs_radius = 0.f;
   float db_eps = 0.f;
   int db_min_pts = 0;
   std::vector<int> devices;
@@ -54,15 +59,18 @@ int main(int ac, char** av) {
       if (i + 2 < ac) { db_eps = (float)std::atof(av[i + 1]); db_min_pts = std::atoi(av[i + 2]); }
       i += 2;
     }
+    else if (a == "--radius-search") { radius_search = true; if (++i < ac) rs_radius = (float)std::atof(av[i]); }
     else if (a == "--labels") { if (++i < ac) labels_path = av[i]; }
     else if (a == "--json") json = true;
     else if (a == "--binary") binary = true;  // --neighbours as raw arrays: <path>.idx.i32 / <path>.dist.f32
     else pos.push_back(a);
   }
-  if (pos.size() != 6 || (mode != "shard" && mode != "partition") || (dbscan && !devices.empty())) {
+  if (pos.size() != 6 || (mode != "shard" && mode != "partition") || ((dbscan || radius_search) && !devices.empty()) ||
+      (dbscan && radius_search)) {
     std::fprintf(stderr, "usage: %s <file> <n> <dim> <start radius> <k> <output file> [--neighbours <path>] [--device <d>] [--json]\n"
                          "          [--gpus <N> | --devices <a,b,...>] [--mode shard|partition]\n"
-                         "          [--dbscan <eps> <min_pts> [--labels <path> [--binary]]]   (one GPU)\n", av[0]);
+                         "          [--dbscan <eps> <min_pts> [--labels <path> [--binary]]]   (one GPU)\n"
+                         "          [--radius-search <r> [--neighbours <path> [--binary]]]   (one GPU)\n", av[0]);
     return 64;
   }
   const std::string path = pos[0], outfile = pos[5];
@@ -180,6 +188,47 @@ int main(int ac, char** av) {
                   "\"dbscan_ms\": %.4f, \"points_per_s\": %.1f}\n",
                   (unsigned long long)np, db_eps, db_min_pts, (unsigned long long)n_clusters, (unsigned long long)noise, st.build_ms,
                   st.search_ms, st.search_ms > 0 ? np / (st.search_ms * 1e-3) : 0.0);
+    }
+    tknn_destroy(ctx);
+    return 0;
+  }
+
+  if (radius_search) {
+    std::vector<uint64_t> offsets((size_t)np + 1);
+    uint64_t total = 0;
+    auto s0 = std::chrono::steady_clock::now();
+    rc = tknn_radius_search(ctx, rs_radius, offsets.data(), nullptr, nullptr, 0, &total);  // size query
+    std::vector<int32_t> ridx;
+    std::vector<float> rdist;
+    if (rc == TKNN_OK) {
+      ridx.resize((size_t)total);
+      rdist.resize((size_t)total);
+      rc = tknn_radius_search(ctx, rs_radius, offsets.data(), ridx.data(), rdist.data(), total, &total);
+    }
+    auto s1 = std::chrono::steady_clock::now();
+    if (rc != TKNN_OK) { std::fprintf(stderr, "tknn_radius_search: %s\n", tknn_last_error(ctx)); tknn_destroy(ctx); return 72; }
+    const double rs_s = std::chrono::duration<double>(s1 - s0).count();
+    tknn_stats st;
+    tknn_get_stats(ctx, &st);
+    static const char* phase[3] = {"count", "fill", "order"};
+    for (int i = 0; i < 3; ++i)
+      std::cout << "Phase: " << phase[i] << " Queries = " << st.round_queries[i] << " Time: " << st.round_ms[i] / 1000.0 << " seconds\n";
+    std::cout << "Neighbours: " << total << '\n';
+    std::cout << "Radius search time: " << rs_s << " seconds." << std::endl;
+    const double tot = build_s + rs_s;
+    std::cout << "Total time: " << tot << '\n';
+    std::ofstream out(outfile, std::ios::app);
+    if (!out.is_open()) { std::perror("Error open"); tknn_destroy(ctx); return 73; }
+    out << tot << std::endl;
+    if (!neigh_path.empty() &&
+        tknn_write_neighbour_lists(neigh_path.c_str(), offsets.data(), ridx.data(), rdist.data(), np, binary ? 1 : 0) != TKNN_OK) {
+      std::perror("Error open");
+      tknn_destroy(ctx);
+      return 73;
+    }
+    if (json) {
+      std::printf("{\"n\": %llu, \"radius\": %.9g, \"neighbours\": %llu, \"build_ms\": %.4f, \"radius_ms\": %.4f}\n",
+                  (unsigned long long)np, rs_radius, (unsigned long long)total, st.build_ms, st.search_ms);
     }
     tknn_destroy(ctx);
     return 0;
