@@ -156,6 +156,20 @@ TKNN_API int tknn_set_option(tknn_ctx* ctx, int key, int64_t value);
  * xyz: n rows of `stride_floats` floats (>= dim); dim 2 => z = 0 (hostCode.cpp:114-118), dim 3. */
 TKNN_API int tknn_build(tknn_ctx* ctx, const float* xyz, uint64_t n, int dim, int stride_floats);
 
+/* Segmented build: a batch of independent point clouds in one BVH (torch_cluster's `batch`).  Segment s is the points
+ * with indices in [seg_offsets[s], seg_offsets[s + 1]); seg_offsets holds n_segments + 1 entries, host or device, that
+ * start at 0, never decrease and end at n (empty segments are legal); anything else, or n_segments outside
+ * [1, 2^31 - 1]: TKNN_EINVAL.  n_segments = 1 is tknn_build, bit for bit.  A later tknn_build clears the segments.
+ * After a segmented build:
+ *   tknn_search / tknn_estimate_start_radius: row q holds the k points p of q's segment with index(p) != q and the
+ *     smallest (d2, index), i.e. tknn_search run on q's segment alone with indices shifted by seg_offsets[s].  A row
+ *     whose segment has at most k points ends in -1 / FLT_MAX.  k <= min(n - 1, TKNN_MAX_K) stays the global check.
+ *   tknn_range_count / tknn_radius_search: only points of q's own segment are in its ball; nothing else changes.
+ *   tknn_search_shard, tknn_query, tknn_radius_query, tknn_dbscan, tknn_brute_force, tknn_partition_search and
+ *     tknn_partition_verify: TKNN_ESTATE (segmented builds do not support them yet). */
+TKNN_API int tknn_build_segments(tknn_ctx* ctx, const float* xyz, uint64_t n, int dim, int stride_floats,
+                                 const uint64_t* seg_offsets, uint64_t n_segments);
+
 /* Replaces the whole round loop (hostCode.cpp:285-340: owlLaunch2D + host termination scan +
  * radius *= 2 + 2x owlGroupRefitAccel) and the raygen / intersection programs
  * (deviceCode.cu:62-152).  All n points are the queries (samples/s01-trueknn/README.md:2).

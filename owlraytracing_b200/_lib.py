@@ -98,7 +98,7 @@ EXPORTS = [
     "tknn_partition_owned", "tknn_partition_search", "tknn_partition_verify", "tknn_create_multi", "tknn_multi_destroy",
     "tknn_multi_set_option", "tknn_multi_build", "tknn_multi_search", "tknn_multi_ranks", "tknn_multi_ctx",
     "tknn_multi_last_error", "tknn_multi_get_times", "tknn_measure_smem_bandwidth", "tknn_key_layout", "tknn_dbscan",
-    "tknn_radius_search", "tknn_radius_query", "tknn_write_neighbour_lists",
+    "tknn_radius_search", "tknn_radius_query", "tknn_write_neighbour_lists", "tknn_build_segments",
 ]
 
 _lib = None
@@ -123,6 +123,7 @@ def load() -> C.CDLL:
     L.tknn_set_stream.argtypes = [vp, vp]
     L.tknn_set_option.argtypes = [vp, C.c_int, C.c_int64]
     L.tknn_build.argtypes = [vp, vp, u64, C.c_int, C.c_int]
+    L.tknn_build_segments.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64]
     L.tknn_search.argtypes = [vp, C.c_int, f32, vp, vp]
     L.tknn_search_shard.argtypes = [vp, C.c_int, f32, C.c_int, C.c_int, vp, vp, vp, C.POINTER(u64)]
     L.tknn_key_layout.argtypes = [u64, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]

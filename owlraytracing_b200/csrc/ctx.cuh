@@ -68,6 +68,12 @@ struct tknn_ctx {
   // mailbox words, self positions, the unsorted rows, the long-row list and the long-row sort buffers (radius.cuh)
   DevBuf rl_cnt_pos, rl_cnt_row, rl_off_pos, rl_off_row, rl_sums, rl_stats, rl_pos_of, rl_self_pos, rl_keys, rl_long_pos,
       rl_long_len, rl_boff, rl_ka, rl_kb, rl_kc, rl_va, rl_vb, rl_vc, rl_row_of, rl_sort_tmp;
+  // segmented build (tknn_build_segments with n_segments > 1; a later tknn_build clears it): the offsets (u64,
+  // n_segments + 1), the segment of every position (u32; positions and indices of a segment share its offsets) and per
+  // node the segment ranges of its two children (int4: lo0, hi0, lo1, hi1)
+  bool segmented = false;
+  uint64_t n_segments = 0;
+  DevBuf seg_off, seg_of, node_seg;
   // Mailbox: 16 words of mapped pinned host memory that a one-thread kernel fills (fetch_words): the small read-backs of a
   // search or build (unresolved count, radius, leaf count, flags) then never queue behind a bulk device->host copy on the
   // copy engine, and never pass through pageable staging.
@@ -123,7 +129,9 @@ enum { SC_GROUP_COUNTER = 0, SC_TOTAL = 1, SC_ERROR = 2, SC_QBAD = 3 /* non-fini
 
 // LBVH over n rows of `stride` floats on the DEVICE or HOST.  ids_in_w: rows are (x, y, z, id bits) and the id of
 // every point is taken from its 4th float instead of its row number (requires stride >= 4, dim 3).
-int build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int stride, bool ids_in_w);
+// seg_offsets (device, n_segments + 1 validated offsets, n_segments > 1) or nullptr: an unsegmented build.
+int build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int stride, bool ids_in_w,
+               const uint64_t* seg_offsets = nullptr, uint64_t n_segments = 0, uint64_t max_segment = 0);
 
 // all-points search over sorted positions [q_begin, q_begin + nq); row_mode as in trav::Params
 int search_range(tknn_ctx* c, int k, float start_radius, uint64_t q_begin, uint64_t nq, int row_mode, int32_t* qid_out,

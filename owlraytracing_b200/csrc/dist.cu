@@ -1251,15 +1251,17 @@ uint64_t tknn_partition_owned(const tknn_ctx* c) { return (c && c->dist && c->di
 
 int tknn_partition_search(tknn_ctx* c, int k, float start_radius, int32_t* gid_out, int32_t* idx_out, float* dist_out,
                           uint64_t capacity, uint64_t* n_out) {
+  if (c && c->segmented) return fail(c, TKNN_ESTATE, "tknn_partition_search: segmented builds (tknn_build_segments) do not support it yet");
   return partition_search(c, k, start_radius, gid_out, idx_out, dist_out, capacity, n_out);
 }
 
 int tknn_partition_verify(tknn_ctx* c, int k, int samples, const int32_t* gid, const int32_t* idx, const float* dist, uint64_t n_rows,
                           uint64_t* n_checked, uint64_t* n_bad) {
+  if (c && c->segmented) return fail(c, TKNN_ESTATE, "tknn_partition_verify: segmented builds (tknn_build_segments) do not support it yet");
   return partition_verify(c, k, samples, gid, idx, dist, n_rows, n_checked, n_bad);
 }
 
-// called by tknn_build (trueknn.cu): a plain build replaces whatever a partitioned build left in the context
+// called by tknn_build and tknn_build_segments (trueknn.cu): a plain build replaces whatever a partitioned build left in the context
 void tknn_internal_dist_invalidate(tknn_ctx* c) {
   if (c && c->dist) c->dist->partition_built = false;
 }

@@ -348,13 +348,9 @@ __device__ __forceinline__ int karras_delta(const uint64_t* __restrict__ key, in
   return x ? __clzll((long long)x) : 64 + __clz((uint32_t)i ^ (uint32_t)j);
 }
 
-static __global__ void __launch_bounds__(THREADS) karras_kernel(const uint64_t* __restrict__ leaf_key,
-                                                         const uint32_t* __restrict__ leaf_start, uint32_t n_leaves,
-                                                         int4* __restrict__ child_info, int32_t* __restrict__ parent_leaf,
-                                                         int32_t* __restrict__ parent_node) {
-  const int64_t i = (int64_t)blockIdx.x * THREADS + threadIdx.x;
-  const int64_t m = n_leaves;
-  if (i >= m - 1) return;
+// the leaf range [lo, hi] of internal node i and its split: child 0 covers leaves lo .. gamma, child 1 gamma + 1 .. hi
+__device__ __forceinline__ void karras_range(const uint64_t* __restrict__ leaf_key, int64_t m, int64_t i, int64_t& lo,
+                                             int64_t& hi, int64_t& gamma) {
   const int d = (karras_delta(leaf_key, m, i, i + 1) - karras_delta(leaf_key, m, i, i - 1)) >= 0 ? 1 : -1;
   const int dmin = karras_delta(leaf_key, m, i, i - d);
   int64_t lmax = 2;
@@ -369,8 +365,20 @@ static __global__ void __launch_bounds__(THREADS) karras_kernel(const uint64_t* 
     t = (t + 1) >> 1;
     if (karras_delta(leaf_key, m, i, i + (s + t) * d) > dnode) s += t;
   } while (t > 1);
-  const int64_t gamma = i + s * d + (d < 0 ? -1 : 0);
-  const int64_t lo = i < j ? i : j, hi = i < j ? j : i;
+  gamma = i + s * d + (d < 0 ? -1 : 0);
+  lo = i < j ? i : j;
+  hi = i < j ? j : i;
+}
+
+static __global__ void __launch_bounds__(THREADS) karras_kernel(const uint64_t* __restrict__ leaf_key,
+                                                         const uint32_t* __restrict__ leaf_start, uint32_t n_leaves,
+                                                         int4* __restrict__ child_info, int32_t* __restrict__ parent_leaf,
+                                                         int32_t* __restrict__ parent_node) {
+  const int64_t i = (int64_t)blockIdx.x * THREADS + threadIdx.x;
+  const int64_t m = n_leaves;
+  if (i >= m - 1) return;
+  int64_t lo, hi, gamma;
+  karras_range(leaf_key, m, i, lo, hi, gamma);
   int4 info;
   if (lo == gamma) {
     info.x = (int)leaf_start[gamma];
@@ -392,6 +400,50 @@ static __global__ void __launch_bounds__(THREADS) karras_kernel(const uint64_t* 
   }
   child_info[i] = info;
   if (i == 0) parent_node[0] = -1;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Segmented builds (tknn_build_segments).  Segment s is the points with indices in [off[s], off[s + 1]).  Its id sits in
+// the top bits of the sort key, above the curve code, so the sort keeps the segments contiguous and in order: the sorted
+// positions of segment s are [off[s], off[s + 1]) as well, and seg_of serves both numberings.
+// ------------------------------------------------------------------------------------------------
+// seg_of[i] = the segment of index i (the last s with off[s] <= i: an empty segment never wins); keys[i] |= seg << shift
+static __global__ void __launch_bounds__(THREADS) segment_key_kernel(const uint64_t* __restrict__ off, uint64_t n_segments,
+                                                                     uint64_t n, int shift, uint64_t* __restrict__ keys,
+                                                                     uint32_t* __restrict__ seg_of) {
+  const uint64_t i = (uint64_t)blockIdx.x * THREADS + threadIdx.x;
+  if (i >= n) return;
+  uint64_t lo = 0, hi = n_segments;  // off[lo] <= i < off[hi]
+  while (hi - lo > 1) {
+    const uint64_t mid = (lo + hi) >> 1;
+    if (__ldg(&off[mid]) <= i) lo = mid; else hi = mid;
+  }
+  seg_of[i] = (uint32_t)lo;
+  keys[i] |= lo << shift;
+}
+
+// a leaf boundary at the start of every non-empty segment: no leaf holds points of two segments
+static __global__ void __launch_bounds__(THREADS) segment_cut_kernel(const uint64_t* __restrict__ off, uint64_t n_segments,
+                                                                     uint64_t n, uint32_t* __restrict__ ballots) {
+  const uint64_t s = (uint64_t)blockIdx.x * THREADS + threadIdx.x;
+  if (s >= n_segments) return;
+  const uint64_t b = off[s];
+  if (b < n && b < off[s + 1]) atomicOr(&ballots[b >> 5], 1u << (b & 31));
+}
+
+// node_seg[i] = the segment ranges of node i's children: (first, last segment under child 0, the same for child 1).  With
+// the segment prefix and the cut above, a node lies inside one segment or is a union of whole segments.
+static __global__ void __launch_bounds__(THREADS) node_segments_kernel(const uint64_t* __restrict__ leaf_key,
+                                                                       const uint32_t* __restrict__ leaf_start, uint32_t n_leaves,
+                                                                       const uint32_t* __restrict__ seg_of,
+                                                                       int4* __restrict__ node_seg) {
+  const int64_t i = (int64_t)blockIdx.x * THREADS + threadIdx.x;
+  const int64_t m = n_leaves;
+  if (i >= m - 1) return;
+  int64_t lo, hi, gamma;
+  karras_range(leaf_key, m, i, lo, hi, gamma);
+  const uint32_t p0 = leaf_start[lo], p1 = leaf_start[gamma + 1], p2 = leaf_start[hi + 1];
+  node_seg[i] = make_int4((int)seg_of[p0], (int)seg_of[p1 - 1], (int)seg_of[p1], (int)seg_of[p2 - 1]);
 }
 
 // ------------------------------------------------------------------------------------------------

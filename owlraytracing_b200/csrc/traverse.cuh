@@ -86,7 +86,38 @@ struct Params {
   uint32_t* count_row;           // LIST_COUNT: ball size per output row (count_out: per query position)
   const uint64_t* list_off;      // LIST: first key slot of every query position
   uint64_t* list_keys;           // LIST: the unsorted rows, in position order
+  // segmented builds (the SEG kernels; queries are built positions)
+  const uint32_t* seg_of;        // segment of every position
+  const uint64_t* seg_off;       // segment offsets, n_segments + 1
+  const int4* node_seg;          // per node: first / last segment under child 0, the same under child 1
 };
+
+// ---- segmented builds -----------------------------------------------------------------------------
+// A lane searches only its query's segment.  At every node visit a child whose segment range does not hold the lane's
+// segment gets box distance NaN for that lane: NaN fails every `<=`, `<` and `==` the walk makes, so the lane never wants
+// it, even in an unbounded round (+inf would pass `<= +inf`).  Leaves never straddle segments, so a leaf staged for other
+// lanes is foreign to this lane as a whole and its filter mask is cleared.  A row whose segment has at most k points is
+// resolved once it holds all the other points of its segment (need = size - 1), so it does not wait for the radius to
+// pass the scene diagonal.  SegLane is empty in the other kernels.
+template <bool SEG> struct SegLane {};
+template <> struct SegLane<true> {
+  int seg = -1;  // the lane's segment
+};
+
+__device__ __forceinline__ void seg_lane_init(SegLane<true>& sl, const Params& P, uint64_t qpos) { sl.seg = (int)__ldg(&P.seg_of[qpos]); }
+
+// MODE_KNN: min(k, segment size - 1) entries resolve the row (read at emit: nothing more stays live during the walk)
+__device__ __forceinline__ int seg_need(const Params& P, int seg, int k) {
+  const uint64_t size = __ldg(&P.seg_off[seg + 1]) - __ldg(&P.seg_off[seg]);
+  return (uint64_t)k < size ? k : (int)(size - 1);
+}
+
+__device__ __forceinline__ void seg_cull(const Params& P, int node, int seg, float& d0, float& d1) {
+  const int4 r = __ldg(&P.node_seg[node]);
+  const float qnan = __int_as_float(0x7fc00000);
+  if (seg < r.x || seg > r.y) d0 = qnan;
+  if (seg < r.z || seg > r.w) d1 = qnan;
+}
 
 // per-lane state of the MODE_RANGE_LIST_* passes (an empty object in the other modes)
 template <bool LIST> struct ListLane {};
@@ -441,7 +472,8 @@ __device__ __forceinline__ uint32_t filter4(const float* sx, int j0, float2 qx, 
 // Launch bounds: the list kernels are capped at 48 registers (5 blocks of 8 warps = 40 resident warps; uncapped, the
 // unified leaf section compiles to 64 and loses a fifth of them); the heap kernels (12 resident warps: shared memory)
 // and the counting variants (diagnostics) take what they need.
-template <int MODE, bool COUNT, int VARIANT, bool HEAP>
+// SEG: segmented build (MODE_KNN, MODE_RANGE_COUNT, MODE_RANGE_LIST_*): the per-lane segment cull above.
+template <int MODE, bool COUNT, int VARIANT, bool HEAP, bool SEG = false>
 static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_kernel(const Params P) {
   constexpr bool APPROX = VARIANT == 1;
   constexpr bool TIES = VARIANT == 2 && MODE == MODE_KNN;
@@ -495,6 +527,10 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
       if (valid) rl.spos = P.self_pos ? (int64_t)P.self_pos[qpos] : (P.self_is_row ? (int64_t)qpos : -1);
       if (MODE == MODE_RANGE_LIST && valid) rl.cursor = P.list_off[qpos];
     }
+    SegLane<SEG> sl;
+    if constexpr (SEG) {
+      if (valid) seg_lane_init(sl, P, qpos);
+    }
     // group-local origin and this lane's pre-filter constants
     float ax, ay, az, qq;
     {
@@ -539,7 +575,8 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
       const float4* np = reinterpret_cast<const float4*>(P.nodes + node);
       const float4 na = __ldg(np), nb = __ldg(np + 1), nc = __ldg(np + 2), nd = __ldg(np + 3);
       const float2 d01 = box_dist2_x2(q.x, q.y, q.z, na, nb, nc);
-      const float d0 = d01.x, d1 = d01.y;
+      float d0 = d01.x, d1 = d01.y;
+      if constexpr (SEG) seg_cull(P, node, sl.seg, d0, d1);
       if (COUNT) { c_nodes += valid ? 1 : 0; c_wnodes += 1; }
       const int ref0 = __float_as_int(nd.x), cnt0 = __float_as_int(nd.z);
       const int ref1 = __float_as_int(nd.y), cnt1 = __float_as_int(nd.w);
@@ -599,11 +636,16 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
 #pragma unroll 1
             for (int j0 = 0; j0 < cnt1; j0 += 4) mask_b |= filter4<NS>(soa + MAX_LEAF, j0, qx2, qy2, qz2, bound) << j0;
 #endif
+            if constexpr (SEG) {  // a leaf of another segment: nothing in it is this lane's
+              if (isnan(d0)) mask_a = 0;
+              if (isnan(d1)) mask_b = 0;
+            }
           } else {
             const bool second = (c == 1) != swap;  // false: child 0, true: child 1
             if (!leaf_wanted(second)) continue;
             const int lcount = second ? cnt1 : cnt0;
             const int start = second ? ref1 : ref0;
+            const bool own = !SEG || !isnan(second ? d1 : d0);  // SEG: the leaf holds this lane's segment
             float cx = 0.f, cy = 0.f, cz = 0.f;
             if (APPROX && MODE == MODE_KNN) {  // the group origin = lane 0's query (re-broadcast: saves 3 registers)
               cx = __shfl_sync(FULL_MASK, q.x, 0); cy = __shfl_sync(FULL_MASK, q.y, 0); cz = __shfl_sync(FULL_MASK, q.z, 0);
@@ -626,8 +668,10 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
               // every point within the radius, the query's own point included: it lies at distance 0 in the one
               // leaf that holds it and is taken off again at emit time
               const float2 qx2 = make_float2(q.x, q.x), qy2 = make_float2(q.y, q.y), qz2 = make_float2(q.z, q.z);
+              if (own) {
 #pragma unroll 1
-              for (int j0 = 0; j0 < lcount; j0 += 4) cnt += __popc(filter4<NS>(soa, j0, qx2, qy2, qz2, bound));
+                for (int j0 = 0; j0 < lcount; j0 += 4) cnt += __popc(filter4<NS>(soa, j0, qx2, qy2, qz2, bound));
+              }
               // decided: a core point wants nothing more, and the group's walk ends once every lane is decided
               if (MODE == MODE_DBSCAN_CORE && cnt >= k) bound = -1.0f;
             } else {
@@ -667,6 +711,7 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
                 for (; j0 < lcount; j0 += 4)  // tail in chunks of 4, NaN-padded past the last point
                   mask_a |= filter4<NS>(soa, j0, qx2, qy2, qz2, bound) << j0;
               }
+              if (!own) mask_a = 0;
             }
             if constexpr (MODE == MODE_RANGE_LIST_COUNT || MODE == MODE_RANGE_LIST) {
               // the excluded point is one slot of this leaf at most
@@ -788,7 +833,11 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
         if (P.core_out) P.core_out[row_id] = 0;
       }
     } else {
-      const bool resolved = valid && cnt == k;
+      int need = k;
+      if constexpr (SEG) {
+        if (valid && cnt < k) need = seg_need(P, sl.seg, k);
+      }
+      const bool resolved = valid && cnt == need;
       const bool emit = valid && (resolved || P.final_round);
       const unsigned un = __ballot_sync(FULL_MASK, valid && !resolved);
       if (lane == 0 && P.unresolved) P.unresolved[group] = un;
@@ -834,7 +883,7 @@ constexpr int SPARSE_CHUNK = TKNN_SPARSE_CHUNK;  // leaf points fetched per step
 // + 3 slots of padding in front: list_insert prefetches up to three slots below the sentinel
 __host__ __device__ inline size_t sparse_smem(int k) { return ((size_t)(k + 1) * SPARSE_THREADS + 3 * 32) * sizeof(uint64_t); }
 
-template <bool COUNT>
+template <bool COUNT, bool SEG = false>
 static __global__ void __launch_bounds__(SPARSE_THREADS) traverse_sparse_kernel(const Params P) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -859,6 +908,10 @@ static __global__ void __launch_bounds__(SPARSE_THREADS) traverse_sparse_kernel(
   if (valid && P.query_r2) r2 = fminf(r2, P.query_r2[qpos]);
   float bound = r2;
   int cnt = 0;
+  SegLane<SEG> sl;
+  if constexpr (SEG) {
+    if (valid) seg_lane_init(sl, P, qpos);
+  }
 
   if (valid) {
     int sp = 0;
@@ -867,7 +920,8 @@ static __global__ void __launch_bounds__(SPARSE_THREADS) traverse_sparse_kernel(
       const float4* np = reinterpret_cast<const float4*>(P.nodes + node);
       const float4 na = __ldg(np), nb = __ldg(np + 1), nc = __ldg(np + 2), nd = __ldg(np + 3);
       const float2 d01 = box_dist2_x2(q.x, q.y, q.z, na, nb, nc);
-      const float d0 = d01.x, d1 = d01.y;
+      float d0 = d01.x, d1 = d01.y;
+      if constexpr (SEG) seg_cull(P, node, sl.seg, d0, d1);
       if (COUNT) c_nodes += 1;
       const int ref0 = __float_as_int(nd.x), cnt0 = __float_as_int(nd.z);
       const int ref1 = __float_as_int(nd.y), cnt1 = __float_as_int(nd.w);
@@ -928,7 +982,11 @@ static __global__ void __launch_bounds__(SPARSE_THREADS) traverse_sparse_kernel(
     }
   }
 
-  const bool resolved = valid && cnt == k;
+  int need = k;
+  if constexpr (SEG) {
+    if (valid && cnt < k) need = seg_need(P, sl.seg, k);
+  }
+  const bool resolved = valid && cnt == need;
   const unsigned un = __ballot_sync(FULL_MASK, valid && !resolved);
   if (lane == 0 && P.unresolved && (gi >> 5) < P.n_groups) P.unresolved[gi >> 5] = un;  // P.n_groups: the launch's capacity
   if (valid && (resolved || P.final_round)) {
@@ -998,7 +1056,7 @@ __device__ __forceinline__ void team_list_insert(uint64_t* L, int& cnt, int k, u
   cnt = n_new;
 }
 
-template <bool COUNT, int T>
+template <bool COUNT, int T, bool SEG = false>
 static __global__ void __launch_bounds__(WQ_WARPS * 32) traverse_warp_kernel(const Params P) {
   extern __shared__ __align__(16) unsigned char smem[];
   constexpr int TEAMS = 32 / T;                 // queries per warp
@@ -1021,6 +1079,8 @@ static __global__ void __launch_bounds__(WQ_WARPS * 32) traverse_warp_kernel(con
   int cnt = 0;
   uint64_t worst = ~0ull;  // L[k - 1] once the list is full
   unsigned long long c_nodes = 0, c_tests = 0, c_ins = 0;
+  SegLane<SEG> sl;
+  if constexpr (SEG) seg_lane_init(sl, P, qpos);
 
   int sp = 0;
   int node = 0;
@@ -1028,7 +1088,8 @@ static __global__ void __launch_bounds__(WQ_WARPS * 32) traverse_warp_kernel(con
     const float4* np = reinterpret_cast<const float4*>(P.nodes + node);
     const float4 na = __ldg(np), nb = __ldg(np + 1), nc = __ldg(np + 2), nd = __ldg(np + 3);
     const float2 d01 = box_dist2_x2(q.x, q.y, q.z, na, nb, nc);
-    const float d0 = d01.x, d1 = d01.y;
+    float d0 = d01.x, d1 = d01.y;
+    if constexpr (SEG) seg_cull(P, node, sl.seg, d0, d1);
     if (COUNT) c_nodes += 1;
     const int ref0 = __float_as_int(nd.x), cnt0 = __float_as_int(nd.z);
     const int ref1 = __float_as_int(nd.y), cnt1 = __float_as_int(nd.w);
@@ -1100,7 +1161,11 @@ static __global__ void __launch_bounds__(WQ_WARPS * 32) traverse_warp_kernel(con
     }
   }
 
-  const bool resolved = cnt == k;
+  int need = k;
+  if constexpr (SEG) {
+    if (cnt < k) need = seg_need(P, sl.seg, k);
+  }
+  const bool resolved = cnt == need;
   if (!resolved && P.unresolved && tl == 0) atomicOr(&P.unresolved[gi >> 5], 1u << (unsigned)(gi & 31));
   if (resolved || P.final_round) {
     const uint64_t row = P.row_mode == 0 ? (uint64_t)(uint32_t)row_id : (P.row_mode == 1 ? qpos - P.q_begin : gi);
@@ -1143,10 +1208,27 @@ static __global__ void __launch_bounds__(256) sample_queue_kernel(uint64_t group
 // square (the round's r2, the same fp32 product the host forms).  Radix select over the bit patterns (non-negative
 // floats order like unsigned ints): four 8-bit passes of one block.  A degenerate sample (the quantile is 0: duplicate
 // clusters) falls back to the largest finite positive value, or +inf (one unbounded round) when there is none.
+// quantile_pm >= 0 (segmented builds): rows that came back unfilled (k-th distance FLT_MAX: their segment has at most k
+// points) are left out, and the position is quantile_pm per mille of the filled rows; +inf when no row is filled.
 static __global__ void __launch_bounds__(1024) radius_quantile_kernel(const float* __restrict__ dist, uint32_t m, int k, uint32_t pos,
-                                                                      float* __restrict__ out) {
+                                                                      float* __restrict__ out, int quantile_pm = -1) {
   __shared__ uint32_t s_hist[256];
-  __shared__ uint32_t s_prefix, s_want, s_maxpos;
+  __shared__ uint32_t s_prefix, s_want, s_maxpos, s_filled;
+  constexpr uint32_t UNFILLED = 0x7f7fffffu;  // FLT_MAX
+  const bool skip = quantile_pm >= 0;
+  if (skip) {
+    if (threadIdx.x == 0) s_filled = 0;
+    __syncthreads();
+    uint32_t f = 0;
+    for (uint32_t i = threadIdx.x; i < m; i += 1024) f += __float_as_uint(dist[(uint64_t)i * k + (k - 1)]) != UNFILLED;
+    atomicAdd(&s_filled, f);
+    __syncthreads();
+    if (s_filled == 0) {
+      if (threadIdx.x == 0) { out[0] = INFINITY; out[1] = INFINITY; }
+      return;
+    }
+    pos = (uint32_t)((double)(s_filled - 1) * quantile_pm / 1000.0);
+  }
   uint32_t prefix = 0, mask = 0, want = pos;
   if (threadIdx.x == 0) s_maxpos = 0;
   for (int shift = 24; shift >= 0; shift -= 8) {
@@ -1154,6 +1236,7 @@ static __global__ void __launch_bounds__(1024) radius_quantile_kernel(const floa
     __syncthreads();
     for (uint32_t i = threadIdx.x; i < m; i += 1024) {
       const uint32_t u = __float_as_uint(dist[(uint64_t)i * k + (k - 1)]);
+      if (skip && u == UNFILLED) continue;
       if ((u & mask) == prefix) atomicAdd(&s_hist[(u >> shift) & 255u], 1u);
       if (shift == 24 && u > 0u && u < 0x7f800000u) atomicMax(&s_maxpos, u);
     }

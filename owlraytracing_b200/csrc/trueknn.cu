@@ -122,13 +122,30 @@ int launch_traverse(tknn_ctx* c, const trav::Params& P) {
   const int variant = MODE != trav::MODE_KNN ? 0 : (ties ? 2 : (c->approx_filter ? 1 : 0));
   const bool hp = MODE == trav::MODE_KNN && k > trav::LIST_MAX_K;
 #define TK_PICK(CNT, VAR) (hp ? trav::traverse_kernel<MODE, CNT, VAR, true> : trav::traverse_kernel<MODE, CNT, VAR, false>)
-  if constexpr (MODE >= trav::MODE_DBSCAN_CORE) {  // the DBSCAN passes: exact filter, no k-list (one variant each)
-    kern = c->counters ? trav::traverse_kernel<MODE, true, 0, false> : trav::traverse_kernel<MODE, false, 0, false>;
-  } else {
-    if (c->counters) kern = variant == 2 ? TK_PICK(true, 2) : variant == 1 ? TK_PICK(true, 1) : TK_PICK(true, 0);
-    else kern = variant == 2 ? TK_PICK(false, 2) : variant == 1 ? TK_PICK(false, 1) : TK_PICK(false, 0);
+#define TK_PICK_SEG(CNT, VAR) \
+  (hp ? trav::traverse_kernel<MODE, CNT, VAR, true, true> : trav::traverse_kernel<MODE, CNT, VAR, false, true>)
+  constexpr bool seg_mode = MODE == trav::MODE_KNN || MODE == trav::MODE_RANGE_COUNT || MODE == trav::MODE_RANGE_LIST_COUNT ||
+                            MODE == trav::MODE_RANGE_LIST;
+  if constexpr (seg_mode) {  // segmented build: the kernels with the per-lane segment cull
+    if (c->segmented) {
+      if constexpr (MODE == trav::MODE_KNN) {
+        if (c->counters) kern = variant == 2 ? TK_PICK_SEG(true, 2) : variant == 1 ? TK_PICK_SEG(true, 1) : TK_PICK_SEG(true, 0);
+        else kern = variant == 2 ? TK_PICK_SEG(false, 2) : variant == 1 ? TK_PICK_SEG(false, 1) : TK_PICK_SEG(false, 0);
+      } else {
+        kern = c->counters ? trav::traverse_kernel<MODE, true, 0, false, true> : trav::traverse_kernel<MODE, false, 0, false, true>;
+      }
+    }
+  }
+  if (!kern) {
+    if constexpr (MODE >= trav::MODE_DBSCAN_CORE) {  // the DBSCAN passes: exact filter, no k-list (one variant each)
+      kern = c->counters ? trav::traverse_kernel<MODE, true, 0, false> : trav::traverse_kernel<MODE, false, 0, false>;
+    } else {
+      if (c->counters) kern = variant == 2 ? TK_PICK(true, 2) : variant == 1 ? TK_PICK(true, 1) : TK_PICK(true, 0);
+      else kern = variant == 2 ? TK_PICK(false, 2) : variant == 1 ? TK_PICK(false, 1) : TK_PICK(false, 0);
+    }
   }
 #undef TK_PICK
+#undef TK_PICK_SEG
   cudaFuncAttributes fa;
   TK_CUDA(c, cudaFuncGetAttributes(&fa, kern));
   const int regs_alloc = ((fa.numRegs + 7) / 8) * 8;  // registers are allocated in units of 8 per thread
@@ -175,15 +192,11 @@ int launch_traverse_sparse(tknn_ctx* c, const trav::Params& P) {
   const size_t smem = trav::sparse_smem(P.k);
   if (smem > 200 * 1024) return TKNN_EINVAL;  // caller falls back to the cooperative kernel
   const unsigned grid = (unsigned)((P.n_active + trav::SPARSE_THREADS - 1) / trav::SPARSE_THREADS);
-  if (c->counters) {
-    auto kern = trav::traverse_sparse_kernel<true>;
-    TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, trav::SPARSE_THREADS, smem, c->stream>>>(P);
-  } else {
-    auto kern = trav::traverse_sparse_kernel<false>;
-    TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, trav::SPARSE_THREADS, smem, c->stream>>>(P);
-  }
+  void (*kern)(const trav::Params) =
+      c->segmented ? (c->counters ? trav::traverse_sparse_kernel<true, true> : trav::traverse_sparse_kernel<false, true>)
+                   : (c->counters ? trav::traverse_sparse_kernel<true> : trav::traverse_sparse_kernel<false>);
+  TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<grid, trav::SPARSE_THREADS, smem, c->stream>>>(P);
   TK_CUDA(c, cudaGetLastError());
   return TKNN_OK;
 }
@@ -197,15 +210,11 @@ int launch_traverse_team(tknn_ctx* c, const trav::Params& P) {
   const unsigned grid = (unsigned)((P.n_active + per_block - 1) / per_block);
   if (P.unresolved)  // the kernel ORs bits into the ballot words
     TK_CUDA(c, cudaMemsetAsync(P.unresolved, 0, sizeof(uint32_t) * (size_t)P.n_groups, c->stream));
-  if (c->counters) {
-    auto kern = trav::traverse_warp_kernel<true, T>;
-    TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, trav::WQ_WARPS * 32, smem, c->stream>>>(P);
-  } else {
-    auto kern = trav::traverse_warp_kernel<false, T>;
-    TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, trav::WQ_WARPS * 32, smem, c->stream>>>(P);
-  }
+  void (*kern)(const trav::Params) =
+      c->segmented ? (c->counters ? trav::traverse_warp_kernel<true, T, true> : trav::traverse_warp_kernel<false, T, true>)
+                   : (c->counters ? trav::traverse_warp_kernel<true, T> : trav::traverse_warp_kernel<false, T>);
+  TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<grid, trav::WQ_WARPS * 32, smem, c->stream>>>(P);
   TK_CUDA(c, cudaGetLastError());
   return TKNN_OK;
 }
@@ -221,6 +230,14 @@ int launch_traverse_sparse_round(tknn_ctx* c, const trav::Params& P) {
     case 16: return launch_traverse_team<16>(c, P);
     default: return launch_traverse_team<8>(c, P);
   }
+}
+
+// the segment arrays of a segmented build (read by the SEG kernels only)
+void set_segments(const tknn_ctx* c, trav::Params& P) {
+  if (!c->segmented) return;
+  P.seg_of = c->seg_of.as<uint32_t>();
+  P.seg_off = c->seg_off.as<uint64_t>();
+  P.node_seg = c->node_seg.as<int4>();
 }
 
 // One round = one traversal launch over the active queries; unresolved ones are compacted (order preserved) into the
@@ -276,6 +293,7 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
     P.unresolved = last ? nullptr : c->unresolved.as<uint32_t>();
     P.group_counter = sc + SC_GROUP_COUNTER;
     P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
+    set_segments(c, P);
   };
   auto round_events = [&](int r) -> int {
     while ((int)c->round_ev.size() < 4 * (r + 1)) {
@@ -432,8 +450,10 @@ int estimate_radius_device(tknn_ctx* c, const float4* queries, uint64_t q_begin,
   c->counters = saved;
   TK_TRY(rc);
   const uint32_t pos = (uint32_t)((double)(m - 1) * std::min(1000, std::max(0, c->radius_quantile)) / 1000.0);
+  // a segmented build leaves the rows of segments with at most k points unfilled: the quantile ignores them
   trav::radius_quantile_kernel<<<1, 1024, 0, c->stream>>>(dd, (uint32_t)m, k, pos,
-                                                          reinterpret_cast<float*>(c->scalars.as<uint32_t>() + SC_QUANTILE));
+                                                          reinterpret_cast<float*>(c->scalars.as<uint32_t>() + SC_QUANTILE),
+                                                          c->segmented ? std::min(1000, std::max(0, c->radius_quantile)) : -1);
   TK_CUDA(c, cudaGetLastError());
   if (launches) *launches += 2;
   return TKNN_OK;
@@ -476,6 +496,30 @@ void choose_key_layout(const tknn_ctx* c, uint64_t n, int* mbits, int* idx_bits)
   key_layout(n, c->morton_bits, c->sort_mode, mbits, idx_bits);
 }
 
+// Key layout of a segmented build: the segment id (*seg_bits = ceil(log2 n_segments) bits) above the curve code, and the
+// code sized for the LARGEST segment, not for n (65 536 clouds of 64 points need few bits per axis).  Packed keys (code
+// above the index) while the code keeps that segment's point spacing plus three bits per axis; else (code, index) pairs
+// with the code cut to fit beside the segment id.
+void segment_key_layout(const tknn_ctx* c, uint64_t n, uint64_t n_segments, uint64_t max_segment, int* mbits, int* idx_bits,
+                        int* seg_bits) {
+  int sb = 0, lg = 0, ls = 0;
+  while (((uint64_t)1 << sb) < n_segments) ++sb;
+  while (((uint64_t)1 << lg) < n) ++lg;
+  const uint64_t ms = std::max<uint64_t>(2, max_segment);
+  while (((uint64_t)1 << ls) < ms) ++ls;
+  const int ib = std::max(1, lg), spacing = (ls + 2) / 3, fit = (64 - ib - sb) / 3;
+  int want = 0, want_idx = 0;
+  key_layout(ms, c->morton_bits, c->sort_mode, &want, &want_idx);
+  *seg_bits = sb;
+  if (c->sort_mode == 0 && (c->morton_bits > 0 ? c->morton_bits <= fit : fit >= spacing + 3)) {
+    *mbits = std::min(want, fit);
+    *idx_bits = ib;
+    return;
+  }
+  *mbits = std::min(c->morton_bits > 0 ? c->morton_bits : auto_morton_bits(ms), (64 - sb) / 3);
+  *idx_bits = 0;
+}
+
 // Hilbert levels of the key kernel (lbvh.cuh: morton_kernel): two levels below the one where a cell holds one point
 int hilbert_levels(uint64_t n, int bits, int forced = 0) {
   if (forced > 0) return std::max(2, std::min(bits, forced));
@@ -485,6 +529,12 @@ int hilbert_levels(uint64_t n, int bits, int forced = 0) {
 }
 
 int check_ctx(tknn_ctx* c) { return c ? TKNN_OK : TKNN_EINVAL; }
+
+// the calls that do not restrict their neighbours to a segment yet refuse a segmented build rather than ignore it
+int refuse_segmented(tknn_ctx* c, const char* what) {
+  if (c->segmented) return fail(c, TKNN_ESTATE, "%s: segmented builds (tknn_build_segments) do not support it yet", what);
+  return TKNN_OK;
+}
 
 // out[0 .. na) = a[0 .. na), out[na .. na + nb) = b[0 .. nb): the mailbox writer (ctx.cuh)
 static __global__ void mailbox_kernel(const uint32_t* __restrict__ a, int na, const uint32_t* __restrict__ b, int nb,
@@ -813,7 +863,7 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->q_r2_sorted, &c->db_parent, &c->db_min_idx, &c->db_pos_label, &c->db_bits, &c->db_core_stage,
                     &c->rl_cnt_pos, &c->rl_cnt_row, &c->rl_off_pos, &c->rl_off_row, &c->rl_sums, &c->rl_stats, &c->rl_pos_of,
                     &c->rl_self_pos, &c->rl_keys, &c->rl_long_pos, &c->rl_long_len, &c->rl_boff, &c->rl_ka, &c->rl_kb,
-                    &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp})
+                    &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp, &c->seg_off, &c->seg_of, &c->node_seg})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -909,9 +959,42 @@ int tknn_build(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int stride_fl
   return build_core(c, xyz, n, dim, stride_floats, false);
 }
 
+int tknn_build_segments(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int stride_floats, const uint64_t* seg_offsets,
+                        uint64_t n_segments) {
+  TK_TRY(check_ctx(c));
+  if (!seg_offsets) return fail(c, TKNN_EINVAL, "null segment offsets");
+  if (n_segments < 1 || n_segments > (uint64_t)INT32_MAX)
+    return fail(c, TKNN_EINVAL, "n_segments = %llu outside [1, 2^31 - 1]", (unsigned long long)n_segments);
+  ScopedDevice sd(c->device);
+  std::vector<uint64_t> off(n_segments + 1);
+  if (is_device_ptr(seg_offsets)) {
+    TK_CUDA(c, cudaMemcpyAsync(off.data(), seg_offsets, off.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
+    TK_CUDA(c, cudaStreamSynchronize(c->stream));
+  } else {
+    std::memcpy(off.data(), seg_offsets, off.size() * sizeof(uint64_t));
+  }
+  if (off[0] != 0) return fail(c, TKNN_EINVAL, "segment offsets must start at 0");
+  if (off[n_segments] != n) return fail(c, TKNN_EINVAL, "segment offsets must end at n = %llu", (unsigned long long)n);
+  uint64_t max_segment = 0;
+  for (uint64_t s = 0; s < n_segments; ++s) {
+    if (off[s + 1] < off[s]) return fail(c, TKNN_EINVAL, "segment offsets decrease at segment %llu", (unsigned long long)s);
+    max_segment = std::max(max_segment, off[s + 1] - off[s]);
+  }
+  if (n_segments == 1) return tknn_build(c, xyz, n, dim, stride_floats);  // one segment: an ordinary build
+  tknn_internal_dist_invalidate(c);
+  c->n = 0;  // the offsets of the previous build are overwritten: it is gone whatever happens below
+  c->n_leaves = 0;
+  c->segmented = false;
+  TK_TRY(ensure(c, c->seg_off, off.size() * sizeof(uint64_t)));
+  TK_CUDA(c, cudaMemcpyAsync(c->seg_off.p, off.data(), off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, c->stream));
+  TK_CUDA(c, cudaStreamSynchronize(c->stream));
+  return build_core(c, xyz, n, dim, stride_floats, false, c->seg_off.as<uint64_t>(), n_segments, max_segment);
+}
+
 }  // extern "C"
 
-int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int stride_floats, bool ids_in_w) {
+int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int stride_floats, bool ids_in_w,
+                           const uint64_t* seg_offsets, uint64_t n_segments, uint64_t max_segment) {
   TK_TRY(check_ctx(c));
   if (!xyz) return fail(c, TKNN_EINVAL, "null point array");
   if (ids_in_w && (dim != 3 || stride_floats < 4)) return fail(c, TKNN_EINVAL, "ids in w need dim 3 and stride >= 4");
@@ -924,6 +1007,8 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
   cudaStream_t st = c->stream;
   c->n = 0;
   c->n_leaves = 0;
+  c->segmented = false;
+  const bool seg = seg_offsets != nullptr;
   tknn_stats& S = c->stats;
   std::memset(&S, 0, sizeof(S));
   c->mailbox_launches = 0;
@@ -953,6 +1038,7 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
     if (rc0 == TKNN_OK) rc0 = ensure(c, c->offsets, (nw0 + 1) * sizeof(uint32_t));
     if (rc0 == TKNN_OK) rc0 = ensure(c, c->block_sums, sizeof(uint32_t) * (size_t)(nw0 / lbvh::SCAN_CHUNK + 2));
     if (rc0 == TKNN_OK) rc0 = ensure(c, c->pts, n * sizeof(float4));
+    if (rc0 == TKNN_OK && seg) rc0 = ensure(c, c->seg_of, n * sizeof(uint32_t));
     if (rc0 != TKNN_OK) { cleanup(); return rc0; }
   }
 #define TK_B(expr) do { int rc_ = (expr); if (rc_ != TKNN_OK) { cleanup(); return rc_; } } while (0)
@@ -986,12 +1072,20 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
   TK_B(ensure(c, keys_b, n * sizeof(uint64_t)));
   TK_B(ensure(c, vals_a, n * sizeof(uint32_t)));
   TK_B(ensure(c, vals_b, n * sizeof(uint32_t)));
-  int mbits = 0, idx_bits = 0;
-  choose_key_layout(c, n, &mbits, &idx_bits);
+  int mbits = 0, idx_bits = 0, seg_bits = 0;
+  if (seg) segment_key_layout(c, n, n_segments, max_segment, &mbits, &idx_bits, &seg_bits);
+  else choose_key_layout(c, n, &mbits, &idx_bits);
+  const uint64_t curve_n = seg ? std::max<uint64_t>(2, max_segment) : n;  // the curve resolves the largest segment
   lbvh::morton_kernel<<<blocks_for(n, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_xyz, n, dim, stride_floats, sc + SC_BOUNDS, mbits,
-                                                                             c->curve ? hilbert_levels(n, mbits, c->curve_levels) : 0, idx_bits,
+                                                                             c->curve ? hilbert_levels(curve_n, mbits, c->curve_levels) : 0, idx_bits,
                                                                              keys_a.as<uint64_t>(), vals_a.as<uint32_t>());
   ++launches;
+  if (seg) {  // the segment id above the code
+    lbvh::segment_key_kernel<<<blocks_for(n, lbvh::THREADS), lbvh::THREADS, 0, st>>>(seg_offsets, n_segments, n, 3 * mbits + idx_bits,
+                                                                                    keys_a.as<uint64_t>(), c->seg_of.as<uint32_t>());
+    ++launches;
+  }
+  const int sort_passes = (3 * mbits + seg_bits + 7) / 8;
   TK_BC(cudaEventRecord(c->ev[3], st));
 
   // ---- onesweep radix sort ----
@@ -999,10 +1093,10 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
   bool sorted_in_b = false;
   if (idx_bits > 0)
     launches += rsort::sort_keys(keys_a.as<uint64_t>(), keys_b.as<uint64_t>(), n, sort_tmp.as<uint32_t>(), c->sm_count, st, idx_bits,
-                                 (3 * mbits + 7) / 8, &sorted_in_b);
+                                 sort_passes, &sorted_in_b);
   else
     launches += rsort::sort_pairs(keys_a.as<uint64_t>(), vals_a.as<uint32_t>(), keys_b.as<uint64_t>(), vals_b.as<uint32_t>(), n,
-                                  sort_tmp.as<uint32_t>(), c->sm_count, st, (3 * mbits + 7) / 8, &sorted_in_b);
+                                  sort_tmp.as<uint32_t>(), c->sm_count, st, sort_passes, &sorted_in_b);
   const uint64_t* skeys = sorted_in_b ? keys_b.as<uint64_t>() : keys_a.as<uint64_t>();
   const uint32_t* svals = idx_bits > 0 ? nullptr : (sorted_in_b ? vals_b.as<uint32_t>() : vals_a.as<uint32_t>());
   TK_BC(cudaGetLastError());
@@ -1016,6 +1110,11 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
   lbvh::leaf_flag_kernel<<<blocks_for(nw * 32, lbvh::THREADS), lbvh::THREADS, 0, st>>>(
       skeys, n, c->leaf_size, c->leaf_policy, force_split, ballots.as<uint32_t>());
   launches += 1;
+  if (seg) {
+    lbvh::segment_cut_kernel<<<blocks_for(n_segments, lbvh::THREADS), lbvh::THREADS, 0, st>>>(seg_offsets, n_segments, n,
+                                                                                              ballots.as<uint32_t>());
+    launches += 1;
+  }
   TK_B(popc_scan(c, ballots.as<uint32_t>(), nw, c->offsets.as<uint32_t>(), &launches));
   uint32_t mb[2] = {0, 0};
   TK_B(fetch_words(c, sc + SC_TOTAL, 1, sc + SC_BOUNDS + 6, 1, mb));  // the leaf count sizes every later launch
@@ -1047,6 +1146,12 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
       leaf_key.as<uint64_t>(), c->leaf_start.as<uint32_t>(), m, child_info.as<int4>(), parent_leaf.as<int32_t>(),
       parent_node.as<int32_t>());
   ++launches;
+  if (seg) {
+    TK_B(ensure(c, c->node_seg, (size_t)(m - 1) * sizeof(int4)));
+    lbvh::node_segments_kernel<<<blocks_for(m - 1, lbvh::THREADS), lbvh::THREADS, 0, st>>>(
+        leaf_key.as<uint64_t>(), c->leaf_start.as<uint32_t>(), m, c->seg_of.as<uint32_t>(), c->node_seg.as<int4>());
+    ++launches;
+  }
   TK_BC(cudaEventRecord(c->ev[6], st));
 
   // ---- bottom-up refit ----
@@ -1078,12 +1183,14 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
   S.n_nodes = m - 1;
   c->built_morton_bits = mbits;
   c->built_idx_bits = idx_bits;
-  c->built_curve = c->curve ? hilbert_levels(n, mbits, c->curve_levels) : 0;
+  c->built_curve = c->curve ? hilbert_levels(curve_n, mbits, c->curve_levels) : 0;
   c->has_dup_leaves = dupleaf != 0;
   S.build_launches = (uint32_t)(launches + c->mailbox_launches);
   c->n = n;
   c->n_leaves = m;
   c->ids_in_w = ids_in_w;
+  c->segmented = seg;
+  c->n_segments = seg ? n_segments : 1;
   return TKNN_OK;
 }
 
@@ -1115,6 +1222,7 @@ int tknn_search_shard(tknn_ctx* c, int k, float start_radius, int shard, int n_s
   TK_TRY(check_ctx(c));
   if (n_shards < 1 || shard < 0 || shard >= n_shards) return fail(c, TKNN_EINVAL, "shard %d of %d", shard, n_shards);
   if (!n_out) return fail(c, TKNN_EINVAL, "null n_out");
+  TK_TRY(refuse_segmented(c, "tknn_search_shard"));
   ScopedDevice sd(c->device);
   const uint64_t groups = (c->n + 31) / 32;
   const uint64_t g0 = groups * (uint64_t)shard / (uint64_t)n_shards, g1 = groups * (uint64_t)(shard + 1) / (uint64_t)n_shards;
@@ -1221,6 +1329,7 @@ int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stri
                const float* init_radius2, int k, float start_radius, int32_t* idx_out, float* dist_out) {
   TK_TRY(check_ctx(c));
   if (c->n == 0) return fail(c, TKNN_ESTATE, "tknn_query before tknn_build");
+  TK_TRY(refuse_segmented(c, "tknn_query"));
   if (!queries && nq) return fail(c, TKNN_EINVAL, "null query array");
   if (dim != 2 && dim != 3) return fail(c, TKNN_EINVAL, "dim = %d (must be 2 or 3)", dim);
   if (stride_floats < dim) return fail(c, TKNN_EINVAL, "stride %d < dim %d", stride_floats, dim);
@@ -1338,6 +1447,7 @@ int tknn_range_count(tknn_ctx* c, float radius, uint32_t* count_out) {
   P.count_out = d_out;
   P.group_counter = sc + SC_GROUP_COUNTER;
   P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
+  set_segments(c, P);
   TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), c->stream));
   TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), c->stream));
   TK_CUDA(c, cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), c->stream));
@@ -1364,6 +1474,7 @@ int tknn_dbscan(tknn_ctx* c, float eps, int min_pts, int32_t* label_out, uint8_t
   TK_TRY(check_ctx(c));
   if (c->n == 0) return fail(c, TKNN_ESTATE, "tknn_dbscan before tknn_build");
   if (c->ids_in_w) return fail(c, TKNN_ESTATE, "this BVH carries caller-chosen point ids (point-partitioned build)");
+  TK_TRY(refuse_segmented(c, "tknn_dbscan"));
   if (!(eps >= 0.0f)) return fail(c, TKNN_EINVAL, "eps must be >= 0");
   if (min_pts < 1) return fail(c, TKNN_EINVAL, "min_pts = %d must be >= 1", min_pts);
   if (!label_out) return fail(c, TKNN_EINVAL, "null label array");
@@ -1584,6 +1695,7 @@ int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* sel
   P.error = sc + SC_ERROR;
   P.group_counter = sc + SC_GROUP_COUNTER;
   P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
+  set_segments(c, P);
   TK_RC(cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
 
   // 1. count (minus self, by position and by row), both scans, the long-row list; one read-back
@@ -1773,6 +1885,7 @@ int tknn_radius_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, i
                       float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out, uint64_t capacity,
                       uint64_t* total_out) {
   TK_TRY(radius_args(c, "tknn_radius_query", radius, offsets_out));
+  TK_TRY(refuse_segmented(c, "tknn_radius_query"));
   if (!queries && nq) return fail(c, TKNN_EINVAL, "null query array");
   if (dim != 2 && dim != 3) return fail(c, TKNN_EINVAL, "dim = %d (must be 2 or 3)", dim);
   if (stride_floats < dim) return fail(c, TKNN_EINVAL, "stride %d < dim %d", stride_floats, dim);
@@ -1807,6 +1920,7 @@ int tknn_radius_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, i
 int tknn_brute_force(tknn_ctx* c, const int32_t* query_ids, uint64_t nq, int k, int32_t* idx_out, float* dist_out) {
   TK_TRY(check_ctx(c));
   if (c->n == 0) return fail(c, TKNN_ESTATE, "tknn_brute_force before tknn_build");
+  TK_TRY(refuse_segmented(c, "tknn_brute_force"));
   if (k < 1 || k > TKNN_MAX_K || (uint64_t)k > c->n - 1) return fail(c, TKNN_EINVAL, "k = %d invalid for n = %llu", k,
                                                                      (unsigned long long)c->n);
   if (nq == 0) return TKNN_OK;

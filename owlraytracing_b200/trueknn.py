@@ -157,8 +157,13 @@ class TrueKNN:
             torch.cuda.current_stream(t.device).synchronize()
 
     # ---- the path ----
-    def build(self, points, dim: int | None = None):
-        """Build the LBVH over `points` ([n, 2|3] float32; extra columns are skipped through the stride)."""
+    def build(self, points, dim: int | None = None, batch=None):
+        """Build the LBVH over `points` ([n, 2|3] float32; extra columns are skipped through the stride).
+
+        batch (optional, torch_cluster's convention): one non-decreasing, non-negative integer cloud id per point, numpy
+        or a CUDA tensor.  Each cloud then is searched on its own: search(), estimate_start_radius(), range_count() and
+        radius_search() only find neighbours in the point's own cloud (tknn_build_segments); search_shard(), query(),
+        radius_query(), dbscan() and brute_force() raise TrueKNNError (TKNN_ESTATE) on such a build."""
         if not _is_tensor(points):
             points = np.ascontiguousarray(points, dtype=np.float32)
         _check_dtype(points, np.float32, "points")
@@ -167,7 +172,12 @@ class TrueKNN:
         stride = int(points.shape[1])
         if dim is None:
             dim = min(stride, 3)
-        self._check(self._L.tknn_build(self._h, self._in(points), int(points.shape[0]), int(dim), stride))
+        if batch is None:
+            self._check(self._L.tknn_build(self._h, self._in(points), int(points.shape[0]), int(dim), stride))
+        else:
+            offsets = batch_to_offsets(batch, int(points.shape[0]))
+            self._check(self._L.tknn_build_segments(self._h, self._in(points), int(points.shape[0]), int(dim), stride,
+                                                    self._in(offsets), int(offsets.shape[0]) - 1))
         self.n = int(points.shape[0])
         self._like = points
         return self
@@ -601,6 +611,91 @@ class MultiTrueKNN:
 # The sample's command line (hostCode.cpp:66-73) as a function.
 # ------------------------------------------------------------------------------------------------
 _FLOAT_RE = re.compile(r"[+-]?(?:\d+\.?\d*|\.\d+)(?:[eE][+-]?\d+)?")
+
+
+def batch_to_offsets(batch, n: int):
+    """Cloud ids per point (torch_cluster's `batch`: non-decreasing, non-negative integers) -> the n_clouds + 1 segment
+    offsets of tknn_build_segments, by bincount + cumsum on the batch's own device: uint64 numpy for numpy input, an
+    int64 tensor for a tensor.  Cloud c is the points [offsets[c], offsets[c + 1]); ids that no point carries are empty
+    clouds.  Raises ValueError for a batch that is not 1-D of length n, not integer, negative or decreasing."""
+    if _is_tensor(batch):
+        import torch
+
+        if batch.dim() != 1 or int(batch.shape[0]) != n:
+            raise ValueError(f"batch must be 1-D with one entry per point ({n})")
+        if batch.dtype.is_floating_point or batch.dtype == torch.bool:
+            raise ValueError(f"batch must hold integer cloud ids, got {batch.dtype}")
+        b = batch.to(torch.int64)
+        if n == 0:
+            return torch.zeros((1,), dtype=torch.int64, device=b.device)
+        if bool((b[0] < 0).item()) or (n > 1 and bool((b[1:] < b[:-1]).any().item())):
+            raise ValueError("batch must be non-negative and non-decreasing (the points of a cloud are contiguous)")
+        counts = torch.bincount(b, minlength=int(b[-1].item()) + 1)
+        return torch.cat([torch.zeros((1,), dtype=torch.int64, device=b.device), torch.cumsum(counts, 0)]).contiguous()
+    b = np.asarray(batch)
+    if b.ndim != 1 or b.shape[0] != n:
+        raise ValueError(f"batch must be 1-D with one entry per point ({n})")
+    if not np.issubdtype(b.dtype, np.integer):
+        raise ValueError(f"batch must hold integer cloud ids, got {b.dtype}")
+    b = b.astype(np.int64)
+    if n == 0:
+        return np.zeros(1, np.uint64)
+    if b[0] < 0 or (n > 1 and bool((b[1:] < b[:-1]).any())):
+        raise ValueError("batch must be non-negative and non-decreasing (the points of a cloud are contiguous)")
+    counts = np.bincount(b, minlength=int(b[-1]) + 1)
+    return np.concatenate([[0], np.cumsum(counts)]).astype(np.uint64)
+
+
+def _edge_index(centre, neighbour, like):
+    """[2, E] int64 in torch_cluster's source_to_target flow: row 0 the neighbour, row 1 the centre."""
+    if _is_tensor(like):
+        import torch
+
+        return torch.stack([neighbour.to(torch.int64), centre.to(torch.int64)])
+    return np.stack([neighbour.astype(np.int64), centre.astype(np.int64)])
+
+
+def knn_graph(x, k: int, batch=None, device: int | None = None):
+    """torch_cluster.knn_graph(x, k, batch) on the GPU, exact: the k nearest points of every point inside its own cloud.
+
+    Returns edge_index [2, E] int64 (row 0 the neighbour, row 1 the centre), edges ordered by centre and then by
+    (distance, index); a cloud of at most k points gives each of its points fewer than k edges.  Differences from
+    torch_cluster: no `loop` option (a point is never its own neighbour) and no truncation of any kind.  numpy in, numpy
+    out; a CUDA tensor in, a tensor on its device out (device: the CUDA device for numpy input, default 0)."""
+    dev = x.device.index if _is_tensor(x) else (device or 0)
+    with TrueKNN(dev) as t:
+        idx, _ = t.build(x, batch=batch).search(int(k), indices_only=True)
+    n = int(idx.shape[0])
+    if _is_tensor(idx):
+        import torch
+
+        centre = torch.arange(n, device=idx.device).repeat_interleave(int(k))
+        flat = idx.reshape(-1)
+        keep = flat >= 0
+        return _edge_index(centre[keep], flat[keep], idx)
+    centre = np.repeat(np.arange(n), int(k))
+    flat = idx.reshape(-1)
+    keep = flat >= 0
+    return _edge_index(centre[keep], flat[keep], idx)
+
+
+def radius_graph(x, r: float, batch=None, device: int | None = None):
+    """torch_cluster.radius_graph(x, r, batch) on the GPU, exact: every pair within the closed ball of radius r inside one
+    cloud.  Returns edge_index [2, E] int64 (row 0 the neighbour, row 1 the centre), edges ordered by centre and then by
+    (distance, index).  Differences from torch_cluster: no `loop` option (a point is never its own neighbour) and no
+    max_num_neighbors truncation: every neighbour in the ball is returned."""
+    dev = x.device.index if _is_tensor(x) else (device or 0)
+    with TrueKNN(dev) as t:
+        offsets, idx, _ = t.build(x, batch=batch).radius_search(float(r), indices_only=True)
+    n = int(offsets.shape[0]) - 1
+    if _is_tensor(idx):
+        import torch
+
+        counts = (offsets[1:] - offsets[:-1]).to(torch.int64)
+        centre = torch.arange(n, device=idx.device).repeat_interleave(counts)
+        return _edge_index(centre, idx, idx)
+    counts = np.diff(offsets.astype(np.int64))
+    return _edge_index(np.repeat(np.arange(n), counts), idx, idx)
 
 
 def read_points(path: str, n: int, dim: int) -> np.ndarray:
