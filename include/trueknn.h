@@ -165,8 +165,10 @@ TKNN_API int tknn_build(tknn_ctx* ctx, const float* xyz, uint64_t n, int dim, in
  *     smallest (d2, index), i.e. tknn_search run on q's segment alone with indices shifted by seg_offsets[s].  A row
  *     whose segment has at most k points ends in -1 / FLT_MAX.  k <= min(n - 1, TKNN_MAX_K) stays the global check.
  *   tknn_range_count / tknn_radius_search: only points of q's own segment are in its ball; nothing else changes.
- *   tknn_search_shard, tknn_query, tknn_radius_query, tknn_dbscan, tknn_brute_force, tknn_partition_search and
- *     tknn_partition_verify: TKNN_ESTATE (segmented builds do not support them yet). */
+ *   tknn_query / tknn_radius_query: TKNN_ESTATE; a separate query set takes tknn_query_segments /
+ *     tknn_radius_query_segments, which give each query segment the data segment of the same number.
+ *   tknn_search_shard, tknn_dbscan, tknn_brute_force, tknn_partition_search and tknn_partition_verify: TKNN_ESTATE
+ *     (segmented builds do not support them yet). */
 TKNN_API int tknn_build_segments(tknn_ctx* ctx, const float* xyz, uint64_t n, int dim, int stride_floats,
                                  const uint64_t* seg_offsets, uint64_t n_segments);
 
@@ -240,6 +242,30 @@ TKNN_API int tknn_radius_search(tknn_ctx* ctx, float radius, uint64_t* offsets_o
 TKNN_API int tknn_radius_query(tknn_ctx* ctx, const float* queries, uint64_t nq, int dim, int stride_floats,
                                const int32_t* self_ids, float radius, uint64_t* offsets_out, int32_t* idx_out,
                                float* dist_out, uint64_t capacity, uint64_t* total_out);
+
+/* Segmented query sets (torch_cluster's knn(x, y, k, batch_x, batch_y) and radius(x, y, r, batch_x, batch_y)): query
+ * segment s is rows [q_seg_offsets[s], q_seg_offsets[s + 1]) and searches data segment s of the last build only.
+ * q_seg_offsets: n_segments + 1 entries, host or device, that start at 0, never decrease and end at nq (empty query
+ * segments are legal); n_segments must equal the segment count of the last build (1 after tknn_build).  NULL, a count
+ * mismatch or malformed offsets: TKNN_EINVAL.  Before a build or on a point-partitioned context: TKNN_ESTATE.
+ *   tknn_query_segments: row j of segment s holds the k points p with index(p) in [off[s], off[s + 1]),
+ *     index(p) != self_ids[j] and d2 <= init_radius2[j] (when given) with the smallest (d2, index), i.e. tknn_query run
+ *     on data segment s alone with indices shifted by off[s].  A self id of -1 or outside data segment s excludes
+ *     nothing.  A row with fewer eligible points (an empty data segment included) ends in -1 / FLT_MAX.  The argument
+ *     checks are those of tknn_query (1 <= k <= min(n, TKNN_MAX_K) globally).
+ *   tknn_radius_query_segments: row j of segment s holds every p of data segment s with index(p) != self_ids[j] and
+ *     d2 <= fl(radius * radius), sorted by (d2, index); output, sizing, capacity, statistics and errors as
+ *     tknn_radius_query.
+ * After a segmented build with the built points as queries, self_ids = 0 .. n - 1 and the build's offsets, the two
+ * calls equal tknn_search and tknn_radius_search bit for bit; on a plain build with n_segments = 1 they are tknn_query
+ * and tknn_radius_query. */
+TKNN_API int tknn_query_segments(tknn_ctx* ctx, const float* queries, uint64_t nq, int dim, int stride_floats,
+                                 const uint64_t* q_seg_offsets, uint64_t n_segments, const int32_t* self_ids,
+                                 const float* init_radius2, int k, float start_radius, int32_t* idx_out, float* dist_out);
+TKNN_API int tknn_radius_query_segments(tknn_ctx* ctx, const float* queries, uint64_t nq, int dim, int stride_floats,
+                                        const uint64_t* q_seg_offsets, uint64_t n_segments, const int32_t* self_ids,
+                                        float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out,
+                                        uint64_t capacity, uint64_t* total_out);
 
 /* Start-radius estimator alone (replaces samples/s01-trueknn/Util/random_sample.py:5-32). */
 TKNN_API int tknn_estimate_start_radius(tknn_ctx* ctx, int k, float* radius_out);

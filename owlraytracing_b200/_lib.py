@@ -99,6 +99,7 @@ EXPORTS = [
     "tknn_multi_set_option", "tknn_multi_build", "tknn_multi_search", "tknn_multi_ranks", "tknn_multi_ctx",
     "tknn_multi_last_error", "tknn_multi_get_times", "tknn_measure_smem_bandwidth", "tknn_key_layout", "tknn_dbscan",
     "tknn_radius_search", "tknn_radius_query", "tknn_write_neighbour_lists", "tknn_build_segments",
+    "tknn_query_segments", "tknn_radius_query_segments",
 ]
 
 _lib = None
@@ -134,6 +135,9 @@ def load() -> C.CDLL:
     L.tknn_dbscan.argtypes = [vp, f32, C.c_int, vp, vp, C.POINTER(u64)]
     L.tknn_radius_search.argtypes = [vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_radius_query.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
+    L.tknn_query_segments.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, vp, vp, C.c_int, f32, vp, vp]
+    L.tknn_radius_query_segments.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, vp, f32, vp, vp, vp, u64,
+                                             C.POINTER(u64)]
     L.tknn_write_neighbour_lists.argtypes = [C.c_char_p, vp, vp, vp, u64, C.c_int]
     L.tknn_estimate_start_radius.argtypes = [vp, C.c_int, C.POINTER(f32)]
     L.tknn_brute_force.argtypes = [vp, vp, u64, C.c_int, vp, vp]

@@ -43,6 +43,9 @@ struct tknn_ctx {
   // tknn_query scratch (grow-only; the reference has no analogue — it only queries its own points)
   DevBuf q_stage, q_keys_a, q_keys_b, q_vals_a, q_vals_b, q_sort_tmp, q_pts, q_sid_stage, q_sid_sorted, q_rad_stage,
       q_r2_sorted;
+  // query sets of a segmented build (tknn_query_segments / tknn_radius_query_segments): the uploaded host offsets (u64,
+  // n_segments + 1), the segment of every query row and of every sorted query position (u32)
+  DevBuf q_seg_off, q_seg_row, q_seg_sorted;
   int keep_scratch = 1;
   int sparse_divisor = 8;
   int warp_round_max = 49152;  // rounds with at most this many active queries run one warp per query (0 = never)

@@ -86,9 +86,9 @@ struct Params {
   uint32_t* count_row;           // LIST_COUNT: ball size per output row (count_out: per query position)
   const uint64_t* list_off;      // LIST: first key slot of every query position
   uint64_t* list_keys;           // LIST: the unsorted rows, in position order
-  // segmented builds (the SEG kernels; queries are built positions)
-  const uint32_t* seg_of;        // segment of every position
-  const uint64_t* seg_off;       // segment offsets, n_segments + 1
+  // segmented builds (the SEG kernels)
+  const uint32_t* seg_of;        // segment of every query position (built positions, or a staged query set's sorted rows)
+  const uint64_t* seg_off;       // data segment offsets, n_segments + 1
   const int4* node_seg;          // per node: first / last segment under child 0, the same under child 1
 };
 
@@ -96,9 +96,9 @@ struct Params {
 // A lane searches only its query's segment.  At every node visit a child whose segment range does not hold the lane's
 // segment gets box distance NaN for that lane: NaN fails every `<=`, `<` and `==` the walk makes, so the lane never wants
 // it, even in an unbounded round (+inf would pass `<= +inf`).  Leaves never straddle segments, so a leaf staged for other
-// lanes is foreign to this lane as a whole and its filter mask is cleared.  A row whose segment has at most k points is
-// resolved once it holds all the other points of its segment (need = size - 1), so it does not wait for the radius to
-// pass the scene diagonal.  SegLane is empty in the other kernels.
+// lanes is foreign to this lane as a whole and its filter mask is cleared.  A row whose data segment has too few eligible
+// points is resolved once it holds all of them (need = segment size minus the query's self id when that lies inside the
+// segment), so it does not wait for the radius to pass the scene diagonal.  SegLane is empty in the other kernels.
 template <bool SEG> struct SegLane {};
 template <> struct SegLane<true> {
   int seg = -1;  // the lane's segment
@@ -106,10 +106,12 @@ template <> struct SegLane<true> {
 
 __device__ __forceinline__ void seg_lane_init(SegLane<true>& sl, const Params& P, uint64_t qpos) { sl.seg = (int)__ldg(&P.seg_of[qpos]); }
 
-// MODE_KNN: min(k, segment size - 1) entries resolve the row (read at emit: nothing more stays live during the walk)
-__device__ __forceinline__ int seg_need(const Params& P, int seg, int k) {
-  const uint64_t size = __ldg(&P.seg_off[seg + 1]) - __ldg(&P.seg_off[seg]);
-  return (uint64_t)k < size ? k : (int)(size - 1);
+// MODE_KNN: min(k, size - [self in the segment]) entries resolve the row (read at emit: nothing more stays live during
+// the walk).  A built point is always in its own segment (size - 1); an empty data segment needs 0.
+__device__ __forceinline__ int seg_need(const Params& P, int seg, int k, int self) {
+  const uint64_t lo = __ldg(&P.seg_off[seg]), size = __ldg(&P.seg_off[seg + 1]) - lo;
+  const uint64_t eligible = size - (self >= 0 && (uint64_t)self - lo < size ? 1 : 0);
+  return (uint64_t)k < eligible ? k : (int)eligible;
 }
 
 __device__ __forceinline__ void seg_cull(const Params& P, int node, int seg, float& d0, float& d1) {
@@ -835,7 +837,7 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
     } else {
       int need = k;
       if constexpr (SEG) {
-        if (valid && cnt < k) need = seg_need(P, sl.seg, k);
+        if (valid && cnt < k) need = seg_need(P, sl.seg, k, self);
       }
       const bool resolved = valid && cnt == need;
       const bool emit = valid && (resolved || P.final_round);
@@ -984,7 +986,7 @@ static __global__ void __launch_bounds__(SPARSE_THREADS) traverse_sparse_kernel(
 
   int need = k;
   if constexpr (SEG) {
-    if (valid && cnt < k) need = seg_need(P, sl.seg, k);
+    if (valid && cnt < k) need = seg_need(P, sl.seg, k, self);
   }
   const bool resolved = valid && cnt == need;
   const unsigned un = __ballot_sync(FULL_MASK, valid && !resolved);
@@ -1163,7 +1165,7 @@ static __global__ void __launch_bounds__(WQ_WARPS * 32) traverse_warp_kernel(con
 
   int need = k;
   if constexpr (SEG) {
-    if (cnt < k) need = seg_need(P, sl.seg, k);
+    if (cnt < k) need = seg_need(P, sl.seg, k, self);
   }
   const bool resolved = cnt == need;
   if (!resolved && P.unresolved && tl == 0) atomicOr(&P.unresolved[gi >> 5], 1u << (unsigned)(gi & 31));

@@ -94,6 +94,7 @@ struct Job {
   const float4* queries = nullptr;
   const int32_t* self_ids = nullptr;
   const float* query_r2 = nullptr;
+  const uint32_t* seg_of = nullptr;       // segmented build: the segment of every query position
   const uint32_t* first_queue = nullptr;  // optional explicit queue for round 1
   uint64_t n_queries = 0;                 // queries in round 1
   uint64_t q_begin = 0;
@@ -232,10 +233,11 @@ int launch_traverse_sparse_round(tknn_ctx* c, const trav::Params& P) {
   }
 }
 
-// the segment arrays of a segmented build (read by the SEG kernels only)
-void set_segments(const tknn_ctx* c, trav::Params& P) {
+// the segment arrays of a segmented build (read by the SEG kernels only).  seg_of: the segment of every query position,
+// c->seg_of when the queries are the built points, the sorted query segments of a staged query set otherwise.
+void set_segments(const tknn_ctx* c, trav::Params& P, const uint32_t* seg_of) {
   if (!c->segmented) return;
-  P.seg_of = c->seg_of.as<uint32_t>();
+  P.seg_of = seg_of;
   P.seg_off = c->seg_off.as<uint64_t>();
   P.node_seg = c->node_seg.as<int4>();
 }
@@ -293,7 +295,7 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
     P.unresolved = last ? nullptr : c->unresolved.as<uint32_t>();
     P.group_counter = sc + SC_GROUP_COUNTER;
     P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
-    set_segments(c, P);
+    set_segments(c, P, job.seg_of);
   };
   auto round_events = [&](int r) -> int {
     while ((int)c->round_ev.size() < 4 * (r + 1)) {
@@ -418,7 +420,7 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
 // one-block radix select leaves {r, r * r} at sc[SC_QUANTILE].  Nothing is copied and nothing waits: round 1 reads r2
 // from there (Job::r_dev).
 int estimate_radius_device(tknn_ctx* c, const float4* queries, uint64_t q_begin, uint64_t nq, const int32_t* self_ids,
-                           int self_is_row, int k, int* launches) {
+                           int self_is_row, const uint32_t* seg_of, int k, int* launches) {
   // sample_groups runs of 32 consecutive sorted positions: neighbouring queries walk nearly the same nodes and leaves
   const uint64_t groups = (nq + 31) / 32;
   const uint64_t sg = std::min<uint64_t>((uint64_t)std::max(1, c->sample_groups), groups);
@@ -432,6 +434,7 @@ int estimate_radius_device(tknn_ctx* c, const float4* queries, uint64_t q_begin,
   Job job;
   job.queries = queries;
   job.self_ids = self_ids;
+  job.seg_of = seg_of;
   job.first_queue = dq;
   job.n_queries = m;
   job.q_begin = q_begin;
@@ -654,7 +657,8 @@ int tknn::host::search_range(tknn_ctx* c, int k, float start_radius, uint64_t q_
   int launches = 0;
   float r0 = start_radius;
   const bool estimated = nq > 0 && !(r0 > 0.0f);
-  if (estimated) TK_TRY(estimate_radius_device(c, c->pts.as<float4>(), q_begin, nq, nullptr, 1, k, &launches));
+  if (estimated)
+    TK_TRY(estimate_radius_device(c, c->pts.as<float4>(), q_begin, nq, nullptr, 1, c->seg_of.as<uint32_t>(), k, &launches));
   TK_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   c->stats.start_radius = r0;
 
@@ -664,6 +668,7 @@ int tknn::host::search_range(tknn_ctx* c, int k, float start_radius, uint64_t q_
     job.r_host = &c->stats.start_radius;
   }
   job.queries = c->pts.as<float4>();
+  job.seg_of = c->seg_of.as<uint32_t>();
   job.n_queries = nq;
   job.q_begin = q_begin;
   job.self_is_row = 1;
@@ -863,7 +868,8 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->q_r2_sorted, &c->db_parent, &c->db_min_idx, &c->db_pos_label, &c->db_bits, &c->db_core_stage,
                     &c->rl_cnt_pos, &c->rl_cnt_row, &c->rl_off_pos, &c->rl_off_row, &c->rl_sums, &c->rl_stats, &c->rl_pos_of,
                     &c->rl_self_pos, &c->rl_keys, &c->rl_long_pos, &c->rl_long_len, &c->rl_boff, &c->rl_ka, &c->rl_kb,
-                    &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp, &c->seg_off, &c->seg_of, &c->node_seg})
+                    &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp, &c->seg_off, &c->seg_of, &c->node_seg,
+                    &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -1245,7 +1251,7 @@ int tknn_estimate_start_radius(tknn_ctx* c, int k, float* radius_out) {
                                                                      (unsigned long long)c->n);
   ScopedDevice sd(c->device);
   int launches = 0;
-  TK_TRY(estimate_radius_device(c, c->pts.as<float4>(), 0, c->n, nullptr, 1, k, &launches));
+  TK_TRY(estimate_radius_device(c, c->pts.as<float4>(), 0, c->n, nullptr, 1, c->seg_of.as<uint32_t>(), k, &launches));
   uint32_t rb = 0;
   TK_TRY(fetch_words(c, c->scalars.as<uint32_t>() + SC_QUANTILE, 1, nullptr, 0, &rb));
   std::memcpy(radius_out, &rb, sizeof(float));
@@ -1255,11 +1261,36 @@ int tknn_estimate_start_radius(tknn_ctx* c, int k, float* radius_out) {
 }  // extern "C"
 
 namespace {
+// Query offsets of the _segments calls (host or device): n_segments + 1 entries that start at 0, never decrease and end at
+// nq, with n_segments the segment count of the last build.  Device offsets cost one small read-back.
+int check_query_offsets(tknn_ctx* c, const char* what, const uint64_t* q_seg_offsets, uint64_t n_segments, uint64_t nq) {
+  if (!q_seg_offsets) return fail(c, TKNN_EINVAL, "%s: null query segment offsets", what);
+  if (n_segments != c->n_segments)
+    return fail(c, TKNN_EINVAL, "%s: n_segments = %llu, the last build has %llu", what, (unsigned long long)n_segments,
+                (unsigned long long)c->n_segments);
+  std::vector<uint64_t> off(n_segments + 1);
+  if (is_device_ptr(q_seg_offsets)) {
+    TK_CUDA(c, cudaMemcpyAsync(off.data(), q_seg_offsets, off.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
+    TK_CUDA(c, cudaStreamSynchronize(c->stream));
+  } else {
+    std::memcpy(off.data(), q_seg_offsets, off.size() * sizeof(uint64_t));
+  }
+  if (off[0] != 0) return fail(c, TKNN_EINVAL, "%s: query segment offsets must start at 0", what);
+  if (off[n_segments] != nq) return fail(c, TKNN_EINVAL, "%s: query segment offsets must end at nq = %llu", what, (unsigned long long)nq);
+  for (uint64_t s = 0; s < n_segments; ++s)
+    if (off[s + 1] < off[s]) return fail(c, TKNN_EINVAL, "%s: query segment offsets decrease at segment %llu", what, (unsigned long long)s);
+  return TKNN_OK;
+}
+
 // The query staging of tknn_query and tknn_radius_query: host inputs are copied to the device, the queries are sorted on
 // the DATA's space-filling curve so that groups of 32 are spatially coherent, and gathered into c->q_pts (x, y, z, query
 // row bits); self ids and radius caps follow into that order.  Sets SC_ERROR / SC_QBAD (a non-finite query coordinate).
+// q_seg_offsets (validated, host or device; segmented builds only): the query segment id goes above the curve code as in
+// the build, so each segment's queries stay contiguous in the sorted order, and *seg_sorted_out receives the segment of
+// every sorted position.
 int stage_queries(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats, const int32_t* self_ids,
-                  const float* init_radius2, const int32_t** sid_sorted_out, const float** r2_sorted_out, int* launches) {
+                  const float* init_radius2, const int32_t** sid_sorted_out, const float** r2_sorted_out, int* launches,
+                  const uint64_t* q_seg_offsets = nullptr, uint64_t n_segments = 0, const uint32_t** seg_sorted_out = nullptr) {
   cudaStream_t st = c->stream;
   uint32_t* sc = c->scalars.as<uint32_t>();
   DevBuf &q_stage = c->q_stage, &keys_a = c->q_keys_a, &keys_b = c->q_keys_b, &vals_a = c->q_vals_a, &vals_b = c->q_vals_b,
@@ -1267,6 +1298,7 @@ int stage_queries(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int s
          &rad_stage = c->q_rad_stage, &r2_sorted = c->q_r2_sorted;
   *sid_sorted_out = nullptr;
   *r2_sorted_out = nullptr;
+  if (seg_sorted_out) *seg_sorted_out = nullptr;
   const float* d_q = queries;
   if (!is_device_ptr(queries)) {
     const size_t bytes = (size_t)nq * stride_floats * sizeof(float);
@@ -1286,6 +1318,17 @@ int stage_queries(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int s
     TK_CUDA(c, cudaMemcpyAsync(rad_stage.p, init_radius2, nq * sizeof(float), cudaMemcpyHostToDevice, st));
     d_rad = rad_stage.as<float>();
   }
+  const bool seg = q_seg_offsets != nullptr;
+  const uint64_t* d_qoff = q_seg_offsets;
+  if (seg) {
+    TK_TRY(ensure(c, c->q_seg_row, nq * sizeof(uint32_t)));
+    TK_TRY(ensure(c, c->q_seg_sorted, nq * sizeof(uint32_t)));
+    if (!is_device_ptr(q_seg_offsets)) {
+      TK_TRY(ensure(c, c->q_seg_off, (n_segments + 1) * sizeof(uint64_t)));
+      TK_CUDA(c, cudaMemcpyAsync(c->q_seg_off.p, q_seg_offsets, (n_segments + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+      d_qoff = c->q_seg_off.as<uint64_t>();
+    }
+  }
   // Morton-sort the queries on the DATA's grid so that groups of 32 are spatially coherent
   TK_TRY(ensure(c, keys_a, nq * sizeof(uint64_t)));
   TK_TRY(ensure(c, keys_b, nq * sizeof(uint64_t)));
@@ -1298,9 +1341,16 @@ int stage_queries(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int s
   lbvh::morton_kernel<<<blocks_for(nq, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_q, nq, dim, stride_floats, sc + SC_BOUNDS, qbits,
                                                                               c->built_curve, 0, keys_a.as<uint64_t>(), vals_a.as<uint32_t>());
   ++*launches;
+  int seg_bits = 0;
+  if (seg) {  // the segment id above the code (3 * qbits + seg_bits <= 64: the build's key layout fits it too)
+    while (((uint64_t)1 << seg_bits) < n_segments) ++seg_bits;
+    lbvh::segment_key_kernel<<<blocks_for(nq, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_qoff, n_segments, nq, 3 * qbits,
+                                                                                     keys_a.as<uint64_t>(), c->q_seg_row.as<uint32_t>());
+    ++*launches;
+  }
   bool q_in_b = false;
   *launches += rsort::sort_pairs(keys_a.as<uint64_t>(), vals_a.as<uint32_t>(), keys_b.as<uint64_t>(), vals_b.as<uint32_t>(), nq,
-                                sort_tmp.as<uint32_t>(), c->sm_count, st, (3 * qbits + 7) / 8, &q_in_b);
+                                sort_tmp.as<uint32_t>(), c->sm_count, st, (3 * qbits + seg_bits + 7) / 8, &q_in_b);
   const uint32_t* qorder = q_in_b ? vals_b.as<uint32_t>() : vals_a.as<uint32_t>();
   lbvh::gather_points_kernel<<<blocks_for(nq, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_q, dim, stride_floats,
                                                                                     qorder, nullptr, 0, nq, 0, qpts.as<float4>(), sc + SC_QBAD);
@@ -1318,18 +1368,22 @@ int stage_queries(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int s
     *r2_sorted_out = r2_sorted.as<float>();
     ++*launches;
   }
+  if (seg) {  // segment ids are < 2^31: the i32 gather moves them unchanged
+    brute::gather_i32_kernel<<<blocks_for(nq, 256), 256, 0, st>>>(c->q_seg_row.as<int32_t>(), qorder, nq,
+                                                                  c->q_seg_sorted.as<int32_t>());
+    *seg_sorted_out = c->q_seg_sorted.as<uint32_t>();
+    ++*launches;
+  }
   return TKNN_OK;
 }
 
-}  // namespace
 
-extern "C" {
-
-int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats, const int32_t* self_ids,
+// tknn_query and tknn_query_segments after their state checks.  segments: the call carries query segment offsets, which
+// are validated here; on a segmented build they restrict query segment s to data segment s, on a plain build (one
+// segment) the call is tknn_query.
+int query_core(tknn_ctx* c, const char* what, const float* queries, uint64_t nq, int dim, int stride_floats,
+               bool segments, const uint64_t* q_seg_offsets, uint64_t n_segments, const int32_t* self_ids,
                const float* init_radius2, int k, float start_radius, int32_t* idx_out, float* dist_out) {
-  TK_TRY(check_ctx(c));
-  if (c->n == 0) return fail(c, TKNN_ESTATE, "tknn_query before tknn_build");
-  TK_TRY(refuse_segmented(c, "tknn_query"));
   if (!queries && nq) return fail(c, TKNN_EINVAL, "null query array");
   if (dim != 2 && dim != 3) return fail(c, TKNN_EINVAL, "dim = %d (must be 2 or 3)", dim);
   if (stride_floats < dim) return fail(c, TKNN_EINVAL, "stride %d < dim %d", stride_floats, dim);
@@ -1338,11 +1392,13 @@ int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stri
   if (nq > rsort::MAX_N) return fail(c, TKNN_EINVAL, "too many queries");
   if (nq && (!idx_out || !dist_out)) return fail(c, TKNN_EINVAL, "null output array");
   if (std::isnan(start_radius)) return fail(c, TKNN_EINVAL, "start_radius is NaN");
+  ScopedDevice sd(c->device);
+  if (segments) TK_TRY(check_query_offsets(c, what, q_seg_offsets, n_segments, nq));
+  if (!c->segmented) q_seg_offsets = nullptr;
   reset_search_stats(c);
   c->stats.n_queries = nq;
   c->stats.k = k;
   if (nq == 0) return TKNN_OK;
-  ScopedDevice sd(c->device);
   cudaStream_t st = c->stream;
   uint32_t* sc = c->scalars.as<uint32_t>();
 
@@ -1353,7 +1409,7 @@ int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stri
   auto cleanup = [&]() {
     if (c->keep_scratch) return;
     for (DevBuf* b : {&q_stage, &keys_a, &keys_b, &vals_a, &vals_b, &sort_tmp, &qpts, &sid_stage, &sid_sorted, &rad_stage,
-                      &r2_sorted})
+                      &r2_sorted, &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted})
       release(*b);
   };
 #define TK_B(expr) do { int rc_ = (expr); if (rc_ != TKNN_OK) { cleanup(); return rc_; } } while (0)
@@ -1364,7 +1420,9 @@ int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stri
   int launches = 0;
   const int32_t* d_sid_sorted = nullptr;
   const float* d_r2_sorted = nullptr;
-  TK_B(stage_queries(c, queries, nq, dim, stride_floats, self_ids, init_radius2, &d_sid_sorted, &d_r2_sorted, &launches));
+  const uint32_t* d_seg_sorted = nullptr;
+  TK_B(stage_queries(c, queries, nq, dim, stride_floats, self_ids, init_radius2, &d_sid_sorted, &d_r2_sorted, &launches,
+                     q_seg_offsets, n_segments, &d_seg_sorted));
 
   const bool idx_dev = is_device_ptr(idx_out), dist_dev = is_device_ptr(dist_out);
   int32_t* d_idx = idx_out;
@@ -1380,7 +1438,7 @@ int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stri
   bool estimated = false;
   if (!(r0 > 0.0f)) {
     if (init_radius2 || may_underfill) r0 = INFINITY;
-    else { TK_B(estimate_radius_device(c, qpts.as<float4>(), 0, nq, d_sid_sorted, 0, k, &launches)); estimated = true; }
+    else { TK_B(estimate_radius_device(c, qpts.as<float4>(), 0, nq, d_sid_sorted, 0, d_seg_sorted, k, &launches)); estimated = true; }
   }
   TK_BC(cudaEventRecord(c->ev[1], st));
   c->stats.start_radius = r0;
@@ -1392,6 +1450,7 @@ int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stri
   job.queries = qpts.as<float4>();
   job.self_ids = d_sid_sorted;
   job.query_r2 = d_r2_sorted;
+  job.seg_of = d_seg_sorted;
   job.n_queries = nq;
   job.q_begin = 0;
   job.self_is_row = 0;
@@ -1417,6 +1476,29 @@ int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stri
   TK_TRY(collect_counters(c));
   TK_TRY(read_error_flag(c));
   return TKNN_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tknn_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats, const int32_t* self_ids,
+               const float* init_radius2, int k, float start_radius, int32_t* idx_out, float* dist_out) {
+  TK_TRY(check_ctx(c));
+  if (c->n == 0) return fail(c, TKNN_ESTATE, "tknn_query before tknn_build");
+  TK_TRY(refuse_segmented(c, "tknn_query"));
+  return query_core(c, "tknn_query", queries, nq, dim, stride_floats, false, nullptr, 0, self_ids, init_radius2, k,
+                    start_radius, idx_out, dist_out);
+}
+
+int tknn_query_segments(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats,
+                        const uint64_t* q_seg_offsets, uint64_t n_segments, const int32_t* self_ids,
+                        const float* init_radius2, int k, float start_radius, int32_t* idx_out, float* dist_out) {
+  TK_TRY(check_ctx(c));
+  if (c->n == 0) return fail(c, TKNN_ESTATE, "tknn_query_segments before tknn_build");
+  if (c->ids_in_w) return fail(c, TKNN_ESTATE, "this BVH carries caller-chosen point ids (point-partitioned build)");
+  return query_core(c, "tknn_query_segments", queries, nq, dim, stride_floats, true, q_seg_offsets, n_segments, self_ids,
+                    init_radius2, k, start_radius, idx_out, dist_out);
 }
 
 int tknn_range_count(tknn_ctx* c, float radius, uint32_t* count_out) {
@@ -1447,7 +1529,7 @@ int tknn_range_count(tknn_ctx* c, float radius, uint32_t* count_out) {
   P.count_out = d_out;
   P.group_counter = sc + SC_GROUP_COUNTER;
   P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
-  set_segments(c, P);
+  set_segments(c, P, c->seg_of.as<uint32_t>());
   TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), c->stream));
   TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), c->stream));
   TK_CUDA(c, cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), c->stream));
@@ -1631,11 +1713,12 @@ int scan_counts(tknn_ctx* c, const uint32_t* counts, uint64_t m, uint64_t* off, 
 }
 
 // The pipeline of radius.cuh over nq staged query positions (qpts: x, y, z, output row bits).  self_sorted: the excluded
-// data index per position (query form) or nullptr with self_is_row (all-points form: the point itself).  The caller has
-// recorded c->ev[0] and cleared SC_ERROR / SC_QBAD; launches counts its own kernels so far.
-int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* self_sorted, int self_is_row, float radius,
-                uint64_t* offsets_out, int32_t* idx_out, float* dist_out, uint64_t capacity, uint64_t* total_out,
-                int launches) {
+// data index per position (query form) or nullptr with self_is_row (all-points form: the point itself).  seg_of: the
+// segment of every position on a segmented build (set_segments).  The caller has recorded c->ev[0] and cleared
+// SC_ERROR / SC_QBAD; launches counts its own kernels so far.
+int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* self_sorted, int self_is_row,
+                const uint32_t* seg_of, float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out,
+                uint64_t capacity, uint64_t* total_out, int launches) {
   cudaStream_t st = c->stream;
   uint32_t* sc = c->scalars.as<uint32_t>();
   const uint64_t n = c->n;
@@ -1695,7 +1778,7 @@ int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* sel
   P.error = sc + SC_ERROR;
   P.group_counter = sc + SC_GROUP_COUNTER;
   P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
-  set_segments(c, P);
+  set_segments(c, P, seg_of);
   TK_RC(cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
 
   // 1. count (minus self, by position and by row), both scans, the long-row list; one read-back
@@ -1866,31 +1949,18 @@ int radius_args(tknn_ctx* c, const char* what, float radius, uint64_t* offsets_o
   return TKNN_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-int tknn_radius_search(tknn_ctx* c, float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out,
-                       uint64_t capacity, uint64_t* total_out) {
-  TK_TRY(radius_args(c, "tknn_radius_search", radius, offsets_out));
-  ScopedDevice sd(c->device);
-  reset_search_stats(c);
-  uint32_t* sc = c->scalars.as<uint32_t>();
-  TK_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
-  TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), c->stream));
-  return radius_core(c, c->pts.as<float4>(), c->n, nullptr, 1, radius, offsets_out, idx_out, dist_out, capacity, total_out, 0);
-}
-
-int tknn_radius_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats, const int32_t* self_ids,
+// tknn_radius_query and tknn_radius_query_segments after radius_args; segments as in query_core
+int radius_query_core(tknn_ctx* c, const char* what, const float* queries, uint64_t nq, int dim, int stride_floats,
+                      bool segments, const uint64_t* q_seg_offsets, uint64_t n_segments, const int32_t* self_ids,
                       float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out, uint64_t capacity,
                       uint64_t* total_out) {
-  TK_TRY(radius_args(c, "tknn_radius_query", radius, offsets_out));
-  TK_TRY(refuse_segmented(c, "tknn_radius_query"));
   if (!queries && nq) return fail(c, TKNN_EINVAL, "null query array");
   if (dim != 2 && dim != 3) return fail(c, TKNN_EINVAL, "dim = %d (must be 2 or 3)", dim);
   if (stride_floats < dim) return fail(c, TKNN_EINVAL, "stride %d < dim %d", stride_floats, dim);
   if (nq > rsort::MAX_N) return fail(c, TKNN_EINVAL, "too many queries");
   ScopedDevice sd(c->device);
+  if (segments) TK_TRY(check_query_offsets(c, what, q_seg_offsets, n_segments, nq));
+  if (!c->segmented) q_seg_offsets = nullptr;
   reset_search_stats(c);
   if (nq == 0) {
     if (total_out) *total_out = 0;
@@ -1906,15 +1976,51 @@ int tknn_radius_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, i
   int launches = 0;
   const int32_t* d_sid_sorted = nullptr;
   const float* d_r2_sorted = nullptr;
-  int rc = stage_queries(c, queries, nq, dim, stride_floats, self_ids, nullptr, &d_sid_sorted, &d_r2_sorted, &launches);
+  const uint32_t* d_seg_sorted = nullptr;
+  int rc = stage_queries(c, queries, nq, dim, stride_floats, self_ids, nullptr, &d_sid_sorted, &d_r2_sorted, &launches,
+                         q_seg_offsets, n_segments, &d_seg_sorted);
   if (rc == TKNN_OK)
-    rc = radius_core(c, c->q_pts.as<float4>(), nq, d_sid_sorted, 0, radius, offsets_out, idx_out, dist_out, capacity,
-                     total_out, launches);
+    rc = radius_core(c, c->q_pts.as<float4>(), nq, d_sid_sorted, 0, d_seg_sorted, radius, offsets_out, idx_out, dist_out,
+                     capacity, total_out, launches);
   if (!c->keep_scratch)
     for (DevBuf* b : {&c->q_stage, &c->q_keys_a, &c->q_keys_b, &c->q_vals_a, &c->q_vals_b, &c->q_sort_tmp, &c->q_pts,
-                      &c->q_sid_stage, &c->q_sid_sorted})
+                      &c->q_sid_stage, &c->q_sid_sorted, &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted})
       release(*b);
   return rc;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tknn_radius_search(tknn_ctx* c, float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out,
+                       uint64_t capacity, uint64_t* total_out) {
+  TK_TRY(radius_args(c, "tknn_radius_search", radius, offsets_out));
+  ScopedDevice sd(c->device);
+  reset_search_stats(c);
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  TK_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), c->stream));
+  return radius_core(c, c->pts.as<float4>(), c->n, nullptr, 1, c->seg_of.as<uint32_t>(), radius, offsets_out, idx_out,
+                     dist_out, capacity, total_out, 0);
+}
+
+int tknn_radius_query(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats, const int32_t* self_ids,
+                      float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out, uint64_t capacity,
+                      uint64_t* total_out) {
+  TK_TRY(radius_args(c, "tknn_radius_query", radius, offsets_out));
+  TK_TRY(refuse_segmented(c, "tknn_radius_query"));
+  return radius_query_core(c, "tknn_radius_query", queries, nq, dim, stride_floats, false, nullptr, 0, self_ids, radius,
+                           offsets_out, idx_out, dist_out, capacity, total_out);
+}
+
+int tknn_radius_query_segments(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int stride_floats,
+                               const uint64_t* q_seg_offsets, uint64_t n_segments, const int32_t* self_ids, float radius,
+                               uint64_t* offsets_out, int32_t* idx_out, float* dist_out, uint64_t capacity,
+                               uint64_t* total_out) {
+  TK_TRY(radius_args(c, "tknn_radius_query_segments", radius, offsets_out));
+  return radius_query_core(c, "tknn_radius_query_segments", queries, nq, dim, stride_floats, true, q_seg_offsets,
+                           n_segments, self_ids, radius, offsets_out, idx_out, dist_out, capacity, total_out);
 }
 
 int tknn_brute_force(tknn_ctx* c, const int32_t* query_ids, uint64_t nq, int k, int32_t* idx_out, float* dist_out) {

@@ -67,6 +67,7 @@ class TrueKNN:
         self.device = int(device)
         self._own_stream = True  # until set_stream() hands over a caller stream
         self.n = 0
+        self.n_segments = 1  # clouds of the last build (batch_size of query(batch=...) / radius_query(batch=...))
         self._like = None
         for k, v in options.items():
             self.set_option(k, v)
@@ -157,13 +158,15 @@ class TrueKNN:
             torch.cuda.current_stream(t.device).synchronize()
 
     # ---- the path ----
-    def build(self, points, dim: int | None = None, batch=None):
+    def build(self, points, dim: int | None = None, batch=None, batch_size: int | None = None):
         """Build the LBVH over `points` ([n, 2|3] float32; extra columns are skipped through the stride).
 
         batch (optional, torch_cluster's convention): one non-decreasing, non-negative integer cloud id per point, numpy
         or a CUDA tensor.  Each cloud then is searched on its own: search(), estimate_start_radius(), range_count() and
-        radius_search() only find neighbours in the point's own cloud (tknn_build_segments); search_shard(), query(),
-        radius_query(), dbscan() and brute_force() raise TrueKNNError (TKNN_ESTATE) on such a build."""
+        radius_search() only find neighbours in the point's own cloud (tknn_build_segments).  batch_size (optional, with
+        batch): the number of clouds, for trailing clouds without points.  A separate query set of a batch takes
+        query(..., batch=) / radius_query(..., batch=); without a batch they, search_shard(), dbscan() and brute_force()
+        raise TrueKNNError (TKNN_ESTATE) on such a build."""
         if not _is_tensor(points):
             points = np.ascontiguousarray(points, dtype=np.float32)
         _check_dtype(points, np.float32, "points")
@@ -173,11 +176,15 @@ class TrueKNN:
         if dim is None:
             dim = min(stride, 3)
         if batch is None:
+            if batch_size is not None:
+                raise ValueError("batch_size needs a batch")
             self._check(self._L.tknn_build(self._h, self._in(points), int(points.shape[0]), int(dim), stride))
+            self.n_segments = 1
         else:
-            offsets = batch_to_offsets(batch, int(points.shape[0]))
+            offsets = batch_to_offsets(batch, int(points.shape[0]), batch_size)
             self._check(self._L.tknn_build_segments(self._h, self._in(points), int(points.shape[0]), int(dim), stride,
                                                     self._in(offsets), int(offsets.shape[0]) - 1))
+            self.n_segments = int(offsets.shape[0]) - 1
         self.n = int(points.shape[0])
         self._like = points
         return self
@@ -219,9 +226,12 @@ class TrueKNN:
         m = int(m.value)
         return qid[:m], idx[:m], dist[:m]
 
-    def query(self, queries, k: int, self_ids=None, init_radius2=None, start_radius: float = 0.0, dim: int | None = None):
+    def query(self, queries, k: int, self_ids=None, init_radius2=None, start_radius: float = 0.0, dim: int | None = None,
+              batch=None):
         """kNN of a separate query set against the built BVH; rows follow the query order.
-        init_radius2: optional per-query cap on the squared distance (closed; negative = none)."""
+        init_radius2: optional per-query cap on the squared distance (closed; negative = none).
+        batch (after build(batch=...)): the cloud id of every query, as build()'s; the queries of cloud c search the points
+        of cloud c only (tknn_query_segments), and a query whose cloud has too few points ends in -1 / FLT_MAX."""
         if not _is_tensor(queries):
             queries = np.ascontiguousarray(queries, dtype=np.float32)
         _check_dtype(queries, np.float32, "queries")
@@ -234,8 +244,14 @@ class TrueKNN:
             init_radius2 = np.ascontiguousarray(init_radius2, dtype=np.float32)
         idx = self._out(queries, nq, k, np.int32)
         dist = self._out(queries, nq, k, np.float32)
-        self._check(self._L.tknn_query(self._h, self._in(queries), nq, int(dim), stride, self._in(self_ids), self._in(init_radius2), int(k),
-                                       C.c_float(start_radius), _ptr(idx), _ptr(dist)))
+        if batch is None:
+            self._check(self._L.tknn_query(self._h, self._in(queries), nq, int(dim), stride, self._in(self_ids), self._in(init_radius2), int(k),
+                                           C.c_float(start_radius), _ptr(idx), _ptr(dist)))
+        else:
+            offsets = batch_to_offsets(batch, nq, self.n_segments)
+            self._check(self._L.tknn_query_segments(self._h, self._in(queries), nq, int(dim), stride, self._in(offsets),
+                                                    int(offsets.shape[0]) - 1, self._in(self_ids), self._in(init_radius2),
+                                                    int(k), C.c_float(start_radius), _ptr(idx), _ptr(dist)))
         return idx, dist
 
     def range_count(self, radius: float):
@@ -290,9 +306,11 @@ class TrueKNN:
         return self._radius_lists(self._like, self.n, indices_only, out, call)
 
     def radius_query(self, queries, radius: float, self_ids=None, dim: int | None = None, indices_only: bool = False,
-                     out=None):
+                     out=None, batch=None):
         """Exact fixed-radius neighbour lists of a separate query set (rows in query order); self_ids (optional, -1 =
-        none) names the data index each query excludes.  Returns (offsets, idx, dist) as radius_search()."""
+        none) names the data index each query excludes.  Returns (offsets, idx, dist) as radius_search().
+        batch (after build(batch=...)): the cloud id of every query; the ball of a query holds points of its own cloud
+        only (tknn_radius_query_segments)."""
         if not _is_tensor(queries):
             queries = np.ascontiguousarray(queries, dtype=np.float32)
         _check_dtype(queries, np.float32, "queries")
@@ -304,8 +322,15 @@ class TrueKNN:
         if self_ids is not None:
             _check_dtype(self_ids, np.int32, "self_ids")
         q_ptr, sid_ptr = self._in(queries), self._in(self_ids)
+        if batch is not None:
+            q_off = batch_to_offsets(batch, nq, self.n_segments)
+            off_ptr, n_seg = self._in(q_off), int(q_off.shape[0]) - 1
 
         def call(off, idx, dist, cap, total):
+            if batch is not None:
+                return self._L.tknn_radius_query_segments(self._h, q_ptr, nq, int(dim), stride, off_ptr, n_seg, sid_ptr,
+                                                          C.c_float(radius), _ptr(off), _ptr(idx), _ptr(dist), cap,
+                                                          C.byref(total))
             return self._L.tknn_radius_query(self._h, q_ptr, nq, int(dim), stride, sid_ptr, C.c_float(radius), _ptr(off),
                                              _ptr(idx), _ptr(dist), cap, C.byref(total))
 
@@ -416,6 +441,7 @@ class TrueKNN:
         self._check(self._L.tknn_build_replicated(self._h, self._in(local_points), int(local_points.shape[0]), int(first),
                                                   int(n_total), int(dim), stride))
         self.n = int(n_total)
+        self.n_segments = 1
         self._like = local_points
         return self
 
@@ -430,6 +456,7 @@ class TrueKNN:
         self._check(self._L.tknn_partition_build(self._h, self._in(local_points), int(local_points.shape[0]), int(first_index),
                                                  int(dim), stride))
         self.n = int(self._L.tknn_partition_owned(self._h))
+        self.n_segments = 1
         self._like = local_points
         return self
 
@@ -613,11 +640,14 @@ class MultiTrueKNN:
 _FLOAT_RE = re.compile(r"[+-]?(?:\d+\.?\d*|\.\d+)(?:[eE][+-]?\d+)?")
 
 
-def batch_to_offsets(batch, n: int):
+def batch_to_offsets(batch, n: int, batch_size: int | None = None):
     """Cloud ids per point (torch_cluster's `batch`: non-decreasing, non-negative integers) -> the n_clouds + 1 segment
     offsets of tknn_build_segments, by bincount + cumsum on the batch's own device: uint64 numpy for numpy input, an
     int64 tensor for a tensor.  Cloud c is the points [offsets[c], offsets[c + 1]); ids that no point carries are empty
-    clouds.  Raises ValueError for a batch that is not 1-D of length n, not integer, negative or decreasing."""
+    clouds.  batch_size (optional): n_clouds, padding with trailing empty clouds.  Raises ValueError for a batch that is
+    not 1-D of length n, not integer, negative or decreasing, for a batch_size below 1 and for an id >= batch_size."""
+    if batch_size is not None and int(batch_size) < 1:
+        raise ValueError(f"batch_size = {batch_size} must be >= 1")
     if _is_tensor(batch):
         import torch
 
@@ -627,10 +657,13 @@ def batch_to_offsets(batch, n: int):
             raise ValueError(f"batch must hold integer cloud ids, got {batch.dtype}")
         b = batch.to(torch.int64)
         if n == 0:
-            return torch.zeros((1,), dtype=torch.int64, device=b.device)
+            return torch.zeros((1 if batch_size is None else int(batch_size) + 1,), dtype=torch.int64, device=b.device)
         if bool((b[0] < 0).item()) or (n > 1 and bool((b[1:] < b[:-1]).any().item())):
             raise ValueError("batch must be non-negative and non-decreasing (the points of a cloud are contiguous)")
-        counts = torch.bincount(b, minlength=int(b[-1].item()) + 1)
+        last = int(b[-1].item())
+        if batch_size is not None and last >= int(batch_size):
+            raise ValueError(f"batch holds cloud id {last} >= batch_size = {batch_size}")
+        counts = torch.bincount(b, minlength=last + 1 if batch_size is None else int(batch_size))
         return torch.cat([torch.zeros((1,), dtype=torch.int64, device=b.device), torch.cumsum(counts, 0)]).contiguous()
     b = np.asarray(batch)
     if b.ndim != 1 or b.shape[0] != n:
@@ -639,10 +672,12 @@ def batch_to_offsets(batch, n: int):
         raise ValueError(f"batch must hold integer cloud ids, got {b.dtype}")
     b = b.astype(np.int64)
     if n == 0:
-        return np.zeros(1, np.uint64)
+        return np.zeros(1 if batch_size is None else int(batch_size) + 1, np.uint64)
     if b[0] < 0 or (n > 1 and bool((b[1:] < b[:-1]).any())):
         raise ValueError("batch must be non-negative and non-decreasing (the points of a cloud are contiguous)")
-    counts = np.bincount(b, minlength=int(b[-1]) + 1)
+    if batch_size is not None and int(b[-1]) >= int(batch_size):
+        raise ValueError(f"batch holds cloud id {int(b[-1])} >= batch_size = {batch_size}")
+    counts = np.bincount(b, minlength=int(b[-1]) + 1 if batch_size is None else int(batch_size))
     return np.concatenate([[0], np.cumsum(counts)]).astype(np.uint64)
 
 
@@ -696,6 +731,96 @@ def radius_graph(x, r: float, batch=None, device: int | None = None):
         return _edge_index(centre, idx, idx)
     counts = np.diff(offsets.astype(np.int64))
     return _edge_index(np.repeat(np.arange(n), counts), idx, idx)
+
+
+def _bipartite_setup(x, y, batch_x, batch_y):
+    """(batch_x, batch_y, batch_size) of knn() / radius(): both batches None (one cloud) or both filled in, a missing one
+    with zeros; batch_size = max(batch_x.max(), batch_y.max()) + 1."""
+    if batch_x is None and batch_y is None:
+        return None, None, None
+
+    def zeros_like_rows(a):
+        if _is_tensor(a):
+            import torch
+
+            return torch.zeros((int(a.shape[0]),), dtype=torch.int64, device=a.device)
+        return np.zeros(int(a.shape[0]), np.int64)
+
+    batch_x = zeros_like_rows(x) if batch_x is None else batch_x
+    batch_y = zeros_like_rows(y) if batch_y is None else batch_y
+    top = max(int(b.max().item()) if _is_tensor(b) else int(np.max(b)) for b in (batch_x, batch_y))
+    return batch_x, batch_y, top + 1
+
+
+def _empty_edges(like):
+    if _is_tensor(like):
+        import torch
+
+        return torch.zeros((2, 0), dtype=torch.int64, device=like.device)
+    return np.zeros((2, 0), np.int64)
+
+
+def knn(x, y, k: int, batch_x=None, batch_y=None, device: int | None = None):
+    """torch_cluster.knn(x, y, k, batch_x, batch_y) on the GPU, exact: for every point of y, the k nearest points of x in
+    the same cloud (tknn_query_segments).  Returns [2, E] int64 with row 0 the index into y (the query) and row 1 the
+    index into x, torch_cluster's orientation for this call; edges are ordered by query and then by (distance, index).
+    batch_size = max(batch_x.max(), batch_y.max()) + 1; a cloud present in only one of x and y gives no edges.  k is
+    clamped to len(x); an empty x or y gives [2, 0].  A point of y is not excluded from its own neighbours: there is no
+    self exclusion, as in torch_cluster.  numpy in, numpy out; a CUDA tensor in, a tensor on its device out (device:
+    the CUDA device for numpy input, default 0)."""
+    if int(x.shape[0]) == 0 or int(y.shape[0]) == 0:
+        return _empty_edges(x)
+    batch_x, batch_y, batch_size = _bipartite_setup(x, y, batch_x, batch_y)
+    k = min(int(k), int(x.shape[0]))
+    dev = x.device.index if _is_tensor(x) else (device or 0)
+    with TrueKNN(dev) as t:
+        t.build(x, batch=batch_x, batch_size=batch_size)
+        idx, _ = t.query(y, k, batch=batch_y)
+    m = int(idx.shape[0])
+    if _is_tensor(idx):
+        import torch
+
+        query = torch.arange(m, device=idx.device).repeat_interleave(k)
+        flat = idx.reshape(-1)
+        keep = flat >= 0
+        return _edge_index(flat[keep], query[keep], idx)
+    query = np.repeat(np.arange(m), k)
+    flat = idx.reshape(-1)
+    keep = flat >= 0
+    return _edge_index(flat[keep], query[keep], idx)
+
+
+def radius(x, y, r: float, batch_x=None, batch_y=None, max_num_neighbors: int | None = None, device: int | None = None):
+    """torch_cluster.radius(x, y, r, batch_x, batch_y) on the GPU, exact: for every point of y, the points of x in the same
+    cloud within the closed ball of radius r (tknn_radius_query_segments).  Returns [2, E] int64 with row 0 the index
+    into y (the query) and row 1 the index into x; edges are ordered by query and then by (distance, index).  Batches,
+    empty inputs and the missing self exclusion as knn().  max_num_neighbors=None returns the whole ball; an integer m
+    keeps the first m entries of each sorted row, i.e. the m nearest.  This differs from torch_cluster, whose default
+    is 32 and whose CUDA kernel keeps an unspecified m of the ball."""
+    if int(x.shape[0]) == 0 or int(y.shape[0]) == 0:
+        return _empty_edges(x)
+    batch_x, batch_y, batch_size = _bipartite_setup(x, y, batch_x, batch_y)
+    dev = x.device.index if _is_tensor(x) else (device or 0)
+    with TrueKNN(dev) as t:
+        t.build(x, batch=batch_x, batch_size=batch_size)
+        offsets, idx, _ = t.radius_query(y, float(r), indices_only=True, batch=batch_y)
+    m = int(offsets.shape[0]) - 1
+    if _is_tensor(idx):
+        import torch
+
+        off = offsets.to(torch.int64)
+        counts = off[1:] - off[:-1]
+        query = torch.arange(m, device=idx.device).repeat_interleave(counts)
+        if max_num_neighbors is not None:
+            keep = torch.arange(int(idx.shape[0]), device=idx.device) - off[query] < int(max_num_neighbors)
+            idx, query = idx[keep], query[keep]
+        return _edge_index(idx, query, idx)
+    off = offsets.astype(np.int64)
+    query = np.repeat(np.arange(m), np.diff(off))
+    if max_num_neighbors is not None:
+        keep = np.arange(idx.shape[0]) - off[query] < int(max_num_neighbors)
+        idx, query = idx[keep], query[keep]
+    return _edge_index(idx, query, idx)
 
 
 def read_points(path: str, n: int, dim: int) -> np.ndarray:
