@@ -20,7 +20,8 @@ ERROR_NAMES = {0: "TKNN_OK", 1: "TKNN_EINVAL", 2: "TKNN_ENOMEM", 3: "TKNN_ECUDA"
 
 (OPT_LEAF_SIZE, OPT_COUNTERS, OPT_LEAF_POLICY, OPT_SAMPLE_GROUPS, OPT_BLOCKS_PER_SM, OPT_SQUARED_DIST, OPT_RADIUS_QUANTILE,
  OPT_KEEP_SCRATCH, OPT_SPARSE_DIVISOR, OPT_APPROX_FILTER, OPT_OUTPUT_CHUNKS, OPT_FILE_ORDER_CHUNKS, OPT_MORTON_BITS,
- OPT_TIE_PRUNING, OPT_WARP_ROUND_MAX, OPT_CURVE, OPT_SPECULATIVE_MAX, OPT_SPARSE_TEAM, OPT_SORT_MODE) = (1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17, 18, 19)
+ OPT_TIE_PRUNING, OPT_WARP_ROUND_MAX, OPT_CURVE, OPT_SPECULATIVE_MAX, OPT_SPARSE_TEAM, OPT_SORT_MODE, OPT_GRID,
+ OPT_GRID_LEVEL) = (1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17, 18, 19, 20, 21)
 
 
 class Stats(C.Structure):
@@ -58,6 +59,13 @@ class Stats(C.Structure):
         ("filter_violations", C.c_uint64),
         ("h2d_bytes", C.c_uint64),
         ("d2h_bytes", C.c_uint64),
+        ("grid_level", C.c_int32),
+        ("grid_selected", C.c_int32),
+        ("grid_max_cell", C.c_uint32),
+        ("grid_split_cells", C.c_uint32),
+        ("grid_ms", C.c_float),
+        ("grid_reserved", C.c_uint32),
+        ("grid_deferred", C.c_uint64),
     ]
 
     def as_dict(self) -> dict:

@@ -77,6 +77,13 @@ struct tknn_ctx {
   bool segmented = false;
   uint64_t n_segments = 0;
   DevBuf seg_off, seg_of, node_seg;
+  // cell grid over the sorted points (grid.cuh): runs per level-L cell and the table's frame; made by a plain build when
+  // the cloud qualifies, and then round 1 of a dense kNN search with k <= 24 walks it instead of the LBVH
+  int grid_mode = 0;        // TKNN_OPT_GRID: 0 = auto (occupancy decides), 1 = off, 2 = whenever the table is valid
+  int grid_level = 0;       // TKNN_OPT_GRID_LEVEL: 0 = auto (floor(log2 n / 3)), else forced (1..8)
+  bool grid_on = false;     // the current build's table serves dense kNN rounds
+  int built_grid_level = 0;
+  DevBuf grid_cells, grid_frame;
   // Mailbox: 16 words of mapped pinned host memory that a one-thread kernel fills (fetch_words): the small read-backs of a
   // search or build (unresolved count, radius, leaf count, flags) then never queue behind a bulk device->host copy on the
   // copy engine, and never pass through pageable staging.
@@ -84,7 +91,7 @@ struct tknn_ctx {
   uint32_t* mailbox_d = nullptr;
   int mailbox_launches = 0;  // mailbox kernels since the counter was last folded into a launch count
   std::vector<cudaEvent_t> chunk_ev;
-  cudaEvent_t ev[8] = {};
+  cudaEvent_t ev[10] = {};
   std::vector<cudaEvent_t> round_ev;
   tknn_stats stats;
   tknn::dist::State* dist = nullptr;  // multi-GPU state (dist.cu), nullptr until tknn_comm_init
@@ -110,7 +117,8 @@ inline unsigned blocks_for(uint64_t n, int threads) { return (unsigned)((n + thr
 // scalars layout (uint32 words unless noted)
 enum { SC_GROUP_COUNTER = 0, SC_TOTAL = 1, SC_ERROR = 2, SC_QBAD = 3 /* non-finite query coordinate */, SC_BOUNDS = 4 /* 7 words */, SC_SCENE = 12 /* 6 floats */,
        SC_COUNTERS = 20 /* 8 x u64, 8-byte aligned */, SC_DUPLEAF = 40, SC_QUANTILE = 41 /* 2 floats: r, r * r */,
-       SC_DBSCAN = 43 /* core points, other points */, SC_WORDS = 48 };
+       SC_DBSCAN = 43 /* core points, other points */,
+       SC_GRID = 45 /* largest cell, cells split into several runs */, SC_WORDS = 48 };
 
 #define TK_CUDA(c, expr)                                                                            \
   do {                                                                                              \

@@ -104,6 +104,26 @@ __device__ __forceinline__ void hilbert_transpose(uint32_t& x0, uint32_t& x1, ui
   x0 ^= t; x1 ^= t; x2 ^= t;
 }
 
+// The key's quantisation: the cubic frame over the scene bounds (origin = the box's low corner, 2^21 cells along the
+// longest axis) and a coordinate's 21-bit cell.  The grid table (grid.cuh) reuses both, so a point's level-L cell there is
+// exactly the one the top 3 L bits of its sort key name.  Every step is monotone in v (RN subtract and multiply, clamps,
+// truncation), which grid.cuh relies on too.
+struct KeyFrame {
+  float lx, ly, lz, scale;
+};
+__device__ __forceinline__ KeyFrame key_frame(const uint32_t* __restrict__ bounds) {
+  KeyFrame f;
+  f.lx = ordered_to_float(bounds[0]); f.ly = ordered_to_float(bounds[1]); f.lz = ordered_to_float(bounds[2]);
+  const float ex = ordered_to_float(bounds[3]) - f.lx, ey = ordered_to_float(bounds[4]) - f.ly,
+              ez = ordered_to_float(bounds[5]) - f.lz;
+  const float ext = fmaxf(fmaxf(ex, ey), fmaxf(ez, FLT_MIN));
+  f.scale = 2097152.0f / ext;  // 2^21 cells along the longest axis
+  return f;
+}
+__device__ __forceinline__ uint32_t quantise21(float v, float lo, float scale) {
+  return (uint32_t)fminf(fmaxf(__fmul_rn(__fsub_rn(v, lo), scale), 0.0f), 2097151.0f);
+}
+
 // curve: 0 = Morton (Z-order); h > 0 = Hilbert order on the top h bits per axis, Morton order below.  The curve only
 // has to keep consecutive points together down to the level where a cell holds about one point (log2(n) / 3 bits per
 // axis); the builder asks for two levels more.  Below that the digits stay plain Morton digits — each still names one
@@ -115,17 +135,13 @@ static __global__ void __launch_bounds__(THREADS) morton_kernel(const float* __r
                                                          uint32_t* __restrict__ vals) {
   const uint64_t i = (uint64_t)blockIdx.x * THREADS + threadIdx.x;
   if (i >= n) return;
-  const float lx = ordered_to_float(bounds[0]), ly = ordered_to_float(bounds[1]), lz = ordered_to_float(bounds[2]);
-  const float ex = ordered_to_float(bounds[3]) - lx, ey = ordered_to_float(bounds[4]) - ly,
-              ez = ordered_to_float(bounds[5]) - lz;
-  const float ext = fmaxf(fmaxf(ex, ey), fmaxf(ez, FLT_MIN));
-  const float scale = 2097152.0f / ext;  // 2^21 cells along the longest axis
+  const KeyFrame f = key_frame(bounds);
   const float* p = xyz + i * (uint64_t)stride;
   const float x = p[0], y = p[1], z = dim > 2 ? p[2] : 0.0f;
   const int drop = 21 - bits;  // keep the top `bits` bits of each 21-bit coordinate
-  uint32_t cx = (uint32_t)fminf(fmaxf((x - lx) * scale, 0.0f), 2097151.0f) >> drop;
-  uint32_t cy = (uint32_t)fminf(fmaxf((y - ly) * scale, 0.0f), 2097151.0f) >> drop;
-  uint32_t cz = (uint32_t)fminf(fmaxf((z - lz) * scale, 0.0f), 2097151.0f) >> drop;
+  uint32_t cx = quantise21(x, f.lx, f.scale) >> drop;
+  uint32_t cy = quantise21(y, f.ly, f.scale) >> drop;
+  uint32_t cz = quantise21(z, f.lz, f.scale) >> drop;
   if (curve > 0) {
     const int h = curve < bits ? curve : bits, low = bits - h;
     uint32_t hx = cx >> low, hy = cy >> low, hz = cz >> low;

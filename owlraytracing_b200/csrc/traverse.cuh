@@ -462,6 +462,18 @@ __device__ __forceinline__ uint32_t filter4(const float* sx, int j0, float2 qx, 
 #ifndef TKNN_WORST_REG
 #define TKNN_WORST_REG 2
 #endif
+
+// The insert rule of the ascending list with TKNN_WORST_REG 2, for a candidate that passed `d <= bound` and is not self:
+// the key beats the worst entry unless the list is full and it TIES the bound's distance with a higher index.  The bound
+// becomes the new tail's distance once the list is full.  (The LBVH kernel and the grid kernel, grid.cuh.)
+template <int S, bool COUNT>
+__device__ __forceinline__ void list_take(uint64_t* H, int& cnt, int k, float& bound, float d, int pid, unsigned long long& c_ins) {
+  if (cnt < k || d < bound || pid < key_idx(kl_worst<S>(H, k, false))) {
+    const uint64_t tail = list_insert<S>(H, cnt, k, make_key(d, pid));
+    if (cnt == k) bound = key_d2(tail);
+    if (COUNT) c_ins += 1;
+  }
+}
 // MODE_DBSCAN_LINK: 1 = a core query unites only the core points of its ball at LOWER positions (every edge joins two core
 // queries, so each is still united once); 0 = every core point of the ball (each edge twice).
 #ifndef TKNN_DBSCAN_HALF_EDGES
@@ -550,12 +562,7 @@ static __global__ void __launch_bounds__(256, (HEAP || COUNT) ? 1 : 5) traverse_
       if (pid != self && d <= bound) {
         const uint64_t key = make_key(d, pid);
         if (!HEAP && TKNN_WORST_REG == 2) {
-          // d <= bound holds: the key beats the worst entry unless it TIES its distance with a higher index
-          if (cnt < k || d < bound || pid < key_idx(kl_worst<S>(H, k, heap))) {
-            const uint64_t tail = list_insert<S>(H, cnt, k, key);
-            if (cnt == k) bound = key_d2(tail);
-            if (COUNT) c_ins += 1;
-          }
+          list_take<S, COUNT>(H, cnt, k, bound, d, pid, c_ins);
         } else if (!HEAP && TKNN_WORST_REG) {
           // (d, pid) < (bound, widx): the worst entry's key lives in registers (bound = its d2)
           if (cnt < k || d < bound || pid < widx) {

@@ -18,6 +18,7 @@
 #include "brute.cuh"
 #include "common.cuh"
 #include "ctx.cuh"
+#include "grid.cuh"
 #include "lbvh.cuh"
 #include "radix_sort.cuh"
 #include "radius.cuh"
@@ -111,7 +112,41 @@ struct Job {
   int32_t* qid_out = nullptr;
   bool record_stats = true;
   bool force_sparse = false;  // thread-per-query kernel from round 1 (the start-radius sample)
+  bool grid = false;          // the queries are the built points: a dense round 1 may walk the cell grid (grid.cuh)
 };
+
+// block shape of a persistent traversal kernel: the warps-per-block that keeps the most warps resident per SM
+// (227 KB shared memory, 64 K registers, 64 warps, 32 blocks); false when not even one warp fits
+bool pick_shape(size_t per_warp, int num_regs, int* warps_out, int* bps_out) {
+  const int regs_alloc = ((num_regs + 7) / 8) * 8;  // registers are allocated in units of 8 per thread
+  const size_t sm_smem = 227 * 1024;
+  int warps = 0, bps = 1, best = 0;
+  for (int w = 8; w >= 1; --w) {
+    const size_t need_b = per_warp * w + 1024;  // + per-block reservation
+    if (need_b > sm_smem) continue;
+    int b = (int)std::min<size_t>(sm_smem / need_b, (size_t)(64 / w));
+    // registers: each of the 4 SM sub-partitions owns 16 K of them and the warps of successive blocks go to
+    // the sub-partitions round-robin, so a block fits only while no sub-partition overflows (ncu: at 48
+    // registers 224-thread blocks were limited to 5 per SM and 192-thread blocks to 6, not 6 and 7)
+    {
+      const int per_smsp = 16384 / (regs_alloc * 32);
+      int load[4] = {0, 0, 0, 0}, next = 0, fit = 0;
+      for (; fit < b; ++fit) {
+        int trial[4] = {load[0], load[1], load[2], load[3]};
+        for (int i = 0; i < w; ++i) ++trial[(next + i) & 3];
+        if (std::max(std::max(trial[0], trial[1]), std::max(trial[2], trial[3])) > per_smsp) break;
+        for (int i = 0; i < 4; ++i) load[i] = trial[i];
+        next = (next + w) & 3;
+      }
+      b = fit;
+    }
+    b = std::min(b, 32);
+    if (b * w > best) { best = b * w; warps = w; bps = b; }
+  }
+  *warps_out = warps;
+  *bps_out = bps;
+  return warps >= 1;
+}
 
 template <int MODE>
 int launch_traverse(tknn_ctx* c, const trav::Params& P) {
@@ -149,34 +184,9 @@ int launch_traverse(tknn_ctx* c, const trav::Params& P) {
 #undef TK_PICK_SEG
   cudaFuncAttributes fa;
   TK_CUDA(c, cudaFuncGetAttributes(&fa, kern));
-  const int regs_alloc = ((fa.numRegs + 7) / 8) * 8;  // registers are allocated in units of 8 per thread
-  // block shape: the warps-per-block that keeps the most warps resident per SM
-  // (227 KB shared memory, 64 K registers, 64 warps, 32 blocks)
-  const size_t sm_smem = 227 * 1024;
-  int warps = 0, bps = 1, best = 0;
-  for (int w = 8; w >= 1; --w) {
-    const size_t need_b = per_warp * w + 1024;  // + per-block reservation
-    if (need_b > sm_smem) continue;
-    int b = (int)std::min<size_t>(sm_smem / need_b, (size_t)(64 / w));
-    // registers: each of the 4 SM sub-partitions owns 16 K of them and the warps of successive blocks go to
-    // the sub-partitions round-robin, so a block fits only while no sub-partition overflows (ncu: at 48
-    // registers 224-thread blocks were limited to 5 per SM and 192-thread blocks to 6, not 6 and 7)
-    {
-      const int per_smsp = 16384 / (regs_alloc * 32);
-      int load[4] = {0, 0, 0, 0}, next = 0, fit = 0;
-      for (; fit < b; ++fit) {
-        int trial[4] = {load[0], load[1], load[2], load[3]};
-        for (int i = 0; i < w; ++i) ++trial[(next + i) & 3];
-        if (std::max(std::max(trial[0], trial[1]), std::max(trial[2], trial[3])) > per_smsp) break;
-        for (int i = 0; i < 4; ++i) load[i] = trial[i];
-        next = (next + w) & 3;
-      }
-      b = fit;
-    }
-    b = std::min(b, 32);
-    if (b * w > best) { best = b * w; warps = w; bps = b; }
-  }
-  if (warps < 1) return fail(c, TKNN_EINVAL, "k = %d needs %zu B of shared memory per warp", k, per_warp);
+  int warps = 0, bps = 1;
+  if (!pick_shape(per_warp, fa.numRegs, &warps, &bps))
+    return fail(c, TKNN_EINVAL, "k = %d needs %zu B of shared memory per warp", k, per_warp);
   const size_t smem = per_warp * warps;
   if (c->blocks_per_sm > 0) bps = c->blocks_per_sm;
   uint64_t grid = (uint64_t)c->sm_count * bps;
@@ -184,6 +194,30 @@ int launch_traverse(tknn_ctx* c, const trav::Params& P) {
   if (grid > need) grid = std::max<uint64_t>(1, need);
   TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<(unsigned)grid, warps * 32, smem, c->stream>>>(P);
+  TK_CUDA(c, cudaGetLastError());
+  return TKNN_OK;
+}
+
+// dense kNN round (k <= 24, not final) on the cell grid of the current build (grid.cuh)
+int launch_grid(tknn_ctx* c, const trav::Params& P) {
+  void (*kern)(const trav::Params, const grid::GridParams) = c->counters ? grid::grid_knn_kernel<true> : grid::grid_knn_kernel<false>;
+  const size_t per_warp = grid::smem_per_warp(P.k);
+  cudaFuncAttributes fa;
+  TK_CUDA(c, cudaFuncGetAttributes(&fa, kern));
+  int warps = 0, bps = 1;
+  if (!pick_shape(per_warp, fa.numRegs, &warps, &bps))
+    return fail(c, TKNN_EINVAL, "k = %d needs %zu B of shared memory per warp", P.k, per_warp);
+  const size_t smem = per_warp * warps;
+  if (c->blocks_per_sm > 0) bps = c->blocks_per_sm;
+  uint64_t grid = (uint64_t)c->sm_count * bps;
+  const uint64_t need = ((uint64_t)P.n_groups + warps - 1) / warps;
+  if (grid > need) grid = std::max<uint64_t>(1, need);
+  grid::GridParams G;
+  G.cells = c->grid_cells.as<uint2>();
+  G.frame = c->grid_frame.as<float>();
+  G.level = c->built_grid_level;
+  TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<(unsigned)grid, warps * 32, smem, c->stream>>>(P, G);
   TK_CUDA(c, cudaGetLastError());
   return TKNN_OK;
 }
@@ -339,8 +373,11 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
     // (cfg3, 51 725 leftover queries: 3.6 ms on the thread-per-query kernel, profiles/r2_ab_opts.jsonl)
     const bool tiny = c->warp_round_max > 0 &&
                       active <= (uint64_t)c->warp_round_max * (job.k > trav::LIST_MAX_K ? 4u : 1u);
+    // the cell grid: round 1 only (its groups are 32 consecutive sorted queries, or a regular slice of them), never final
+    const bool on_grid = job.grid && c->grid_on && round == 0 && !last && job.k <= trav::LIST_MAX_K;
     if (tiny) TK_TRY(launch_traverse_warp(c, P));
     else if (sparse) TK_TRY(launch_traverse_sparse_round(c, P));
+    else if (on_grid) TK_TRY(launch_grid(c, P));
     else TK_TRY(launch_traverse<trav::MODE_KNN>(c, P));
     if (timed) TK_CUDA(c, cudaEventRecord(c->round_ev[4 * round + 3], c->stream));
     ++launches;
@@ -587,6 +624,7 @@ int collect_counters(tknn_ctx* c) {
   c->stats.warp_leaf_visits = h[4];
   c->stats.warp_point_loads = h[5];
   c->stats.filter_violations = h[6];
+  c->stats.grid_deferred = h[7];
   return TKNN_OK;
 }
 
@@ -611,6 +649,7 @@ void reset_search_stats(tknn_ctx* c) {
   s.kernel_launches = 0;
   s.nodes_visited = s.points_tested = s.heap_inserts = 0;
   s.warp_node_visits = s.warp_leaf_visits = s.warp_point_loads = s.filter_violations = 0;
+  s.grid_deferred = 0;
   s.d2h_bytes = 0;
   c->mailbox_launches = 0;
 }
@@ -679,6 +718,7 @@ int tknn::host::search_range(tknn_ctx* c, int k, float start_radius, uint64_t q_
   job.idx_out = d_idx;
   job.dist_out = d_dist;
   job.qid_out = d_qid;
+  job.grid = true;
 
   // Compact rows (row_mode 1) are in Morton order, so a contiguous slice of the queries yields a
   // contiguous, FINAL slice of the output: with host outputs the shard is searched in chunks and each
@@ -869,7 +909,7 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->rl_cnt_pos, &c->rl_cnt_row, &c->rl_off_pos, &c->rl_off_row, &c->rl_sums, &c->rl_stats, &c->rl_pos_of,
                     &c->rl_self_pos, &c->rl_keys, &c->rl_long_pos, &c->rl_long_len, &c->rl_boff, &c->rl_ka, &c->rl_kb,
                     &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp, &c->seg_off, &c->seg_of, &c->node_seg,
-                    &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted})
+                    &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted, &c->grid_cells, &c->grid_frame})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -952,6 +992,14 @@ int tknn_set_option(tknn_ctx* c, int key, int64_t value) {
       if (value < 0 || value > (int64_t)1 << 30) return fail(c, TKNN_EINVAL, "warp round maximum outside [0, 2^30]");
       c->warp_round_max = (int)value;
       return TKNN_OK;
+    case TKNN_OPT_GRID:
+      if (value < 0 || value > 2) return fail(c, TKNN_EINVAL, "grid must be 0 (auto), 1 (off) or 2 (whenever the table is valid)");
+      c->grid_mode = (int)value;
+      return TKNN_OK;
+    case TKNN_OPT_GRID_LEVEL:
+      if (value < 0 || value > grid::MAX_LEVEL) return fail(c, TKNN_EINVAL, "grid level outside [0 (auto), %d]", grid::MAX_LEVEL);
+      c->grid_level = (int)value;
+      return TKNN_OK;
     case TKNN_OPT_RADIUS_QUANTILE:
       if (value < 0 || value > 1000) return fail(c, TKNN_EINVAL, "radius quantile outside [0, 1000] per mille");
       c->radius_quantile = (int)value;
@@ -999,6 +1047,43 @@ int tknn_build_segments(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int 
 
 }  // extern "C"
 
+// Level of the cell table: floor(log2(n) / 3), i.e. one to eight points per cell on a uniform cloud, at most the key's code
+// bits per axis (a level-L cell must be a prefix of the key) and grid::MAX_LEVEL.  TKNN_OPT_GRID_LEVEL forces it.
+static int grid_level_for(uint64_t n, int mbits, int forced) {
+  int lg = 0;
+  while (((uint64_t)2 << lg) <= n) ++lg;  // floor(log2 n)
+  return std::max(1, std::min(std::min(forced > 0 ? forced : lg / 3, mbits), grid::MAX_LEVEL));
+}
+
+// The cell table of the current build (c->pts sorted, the scene bounds at SC_BOUNDS) and the decision to use it: every cell
+// one contiguous run, and (auto) no cell fuller than grid::SELECT_MAX_CELL.
+static int build_grid(tknn_ctx* c, uint64_t n, int mbits, int* launches) {
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  cudaStream_t st = c->stream;
+  const int L = grid_level_for(n, mbits, c->grid_level);
+  const uint64_t n_cells = 1ull << (3 * L);
+  TK_TRY(ensure(c, c->grid_cells, n_cells * sizeof(uint2)));
+  TK_TRY(ensure(c, c->grid_frame, grid::frame_words(L) * sizeof(float)));
+  TK_CUDA(c, cudaMemsetAsync(c->grid_cells.p, 0xff, n_cells * sizeof(uint2), st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_GRID, 0, 2 * sizeof(uint32_t), st));
+  grid::fill_kernel<<<blocks_for(n, 256), 256, 0, st>>>(c->pts.as<float4>(), n, sc + SC_BOUNDS, L, c->grid_cells.as<uint2>(),
+                                                         sc + SC_GRID + 1);
+  grid::frame_kernel<<<blocks_for(3 * ((1ull << L) + 1), 256), 256, 0, st>>>(sc + SC_BOUNDS, L, c->grid_frame.as<float>());
+  grid::occupancy_kernel<<<(unsigned)std::min<uint64_t>(blocks_for(n_cells, 256), (uint64_t)c->sm_count * 8), 256, 0, st>>>(
+      c->grid_cells.as<uint2>(), n_cells, sc + SC_GRID);
+  TK_CUDA(c, cudaGetLastError());
+  *launches += 3;
+  uint32_t h[2] = {0, 0};
+  TK_TRY(fetch_words(c, sc + SC_GRID, 2, nullptr, 0, h));
+  c->stats.grid_level = L;
+  c->stats.grid_max_cell = h[0];
+  c->stats.grid_split_cells = h[1];
+  c->built_grid_level = L;
+  c->grid_on = h[1] == 0 && (c->grid_mode == 2 || h[0] <= grid::SELECT_MAX_CELL);
+  c->stats.grid_selected = c->grid_on ? 1 : 0;
+  return TKNN_OK;
+}
+
 int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int stride_floats, bool ids_in_w,
                            const uint64_t* seg_offsets, uint64_t n_segments, uint64_t max_segment) {
   TK_TRY(check_ctx(c));
@@ -1014,6 +1099,7 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
   c->n = 0;
   c->n_leaves = 0;
   c->segmented = false;
+  c->grid_on = false;
   const bool seg = seg_offsets != nullptr;
   tknn_stats& S = c->stats;
   std::memset(&S, 0, sizeof(S));
@@ -1176,6 +1262,11 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
 #undef TK_B
 #undef TK_BC
 
+  // ---- cell grid: plain builds without coincident-point leaves (those take the tie-pruning LBVH kernel) ----
+  TK_CUDA(c, cudaEventRecord(c->ev[8], st));
+  if (!seg && dupleaf == 0 && c->grid_mode != 1) TK_TRY(build_grid(c, n, mbits, &launches));
+  TK_CUDA(c, cudaEventRecord(c->ev[9], st));
+
   TK_CUDA(c, cudaEventElapsedTime(&S.h2d_ms, c->ev[0], c->ev[1]));
   TK_CUDA(c, cudaEventElapsedTime(&S.bounds_ms, c->ev[1], c->ev[2]));
   TK_CUDA(c, cudaEventElapsedTime(&S.morton_ms, c->ev[2], c->ev[3]));
@@ -1183,7 +1274,9 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
   TK_CUDA(c, cudaEventElapsedTime(&S.leaves_ms, c->ev[4], c->ev[5]));
   TK_CUDA(c, cudaEventElapsedTime(&S.hierarchy_ms, c->ev[5], c->ev[6]));
   TK_CUDA(c, cudaEventElapsedTime(&S.refit_ms, c->ev[6], c->ev[7]));
+  TK_CUDA(c, cudaEventElapsedTime(&S.grid_ms, c->ev[8], c->ev[9]));
   TK_CUDA(c, cudaEventElapsedTime(&S.build_ms, c->ev[1], c->ev[7]));
+  S.build_ms += S.grid_ms;
   S.n_points = n;
   S.n_leaves = m;
   S.n_nodes = m - 1;

@@ -103,6 +103,7 @@ class TrueKNN:
         "file_order_chunks": _lib.OPT_FILE_ORDER_CHUNKS, "morton_bits": _lib.OPT_MORTON_BITS,
         "tie_pruning": _lib.OPT_TIE_PRUNING, "warp_round_max": _lib.OPT_WARP_ROUND_MAX, "curve": _lib.OPT_CURVE,
         "speculative_max": _lib.OPT_SPECULATIVE_MAX, "sparse_team": _lib.OPT_SPARSE_TEAM, "sort_mode": _lib.OPT_SORT_MODE,
+        "grid": _lib.OPT_GRID, "grid_level": _lib.OPT_GRID_LEVEL,
     }
 
     def set_option(self, name: str, value: int):
