@@ -188,10 +188,12 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
     H[0] = 0;  // sentinel of this lane's k-list
 
     // ---- the group's cell range ----
-    // A point p with dist2(q, p) <= bound has RN(dx * dx) <= bound (the fma chain only adds non-negative terms), so
-    // |q - p| <= sqrt(bound) (1 + 2u) per axis (u = 2^-24).  s = fma(sqrtf(bound), 1.0001, |q| 2^-18) exceeds that by more
-    // than the rounding of q -/+ s (<= u (|q| + s)), so p lies in [RN(q - s), RN(q + s)], and the monotone cell function
-    // maps it into the range.  bound = +inf gives the whole grid (and the cap below).
+    // A point p with dist2(q, p) <= bound has RN(dx * dx) <= bound (the fma chain only adds non-negative terms).  Rounding
+    // errs by at most u = 2^-24 relative, or by 2^-150 absolute where dx * dx is subnormal, so dx^2 <= bound (1 + 2u) + 2^-150
+    // and |q - p| <= sqrt(bound) (1 + 2u) + 2^-75 per axis.  s = fma(sqrtf(bound), 1.0001, fma(|q|, 2^-18, 2^-74)) exceeds
+    // that by more than the rounding of q -/+ s (<= u (|q| + s)), so p lies in [RN(q - s), RN(q + s)], and the monotone cell
+    // function maps it into the range.  Without the 2^-74 term a bound that is subnormal or 0 (a tiny cloud, a tiny start
+    // radius) would miss points whose d2 underflows to it.  bound = +inf gives the whole grid (and the cap below).
     bool defer = false;
     {
       const float sb = valid ? sqrtf(bound) : 0.0f;
@@ -202,7 +204,7 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
         const float qa = a == 0 ? q.x : (a == 1 ? q.y : q.z);
         const float org = __ldg(&G.frame[a]);
         const uint32_t top = __ldg(reinterpret_cast<const uint32_t*>(G.frame) + 4 + a);
-        const float s = __fmaf_rn(sb, 1.0001f, fabsf(qa) * 0x1p-18f);
+        const float s = __fmaf_rn(sb, 1.0001f, __fmaf_rn(fabsf(qa), 0x1p-18f, 0x1p-74f));
         const uint32_t l = cell_of(__fsub_rn(qa, s), org, scale, sh);
         const uint32_t h = min(cell_of(__fadd_rn(qa, s), org, scale, sh), top);
         const uint32_t glo = __reduce_min_sync(FULL_MASK, valid ? l : 0xffffffffu);
