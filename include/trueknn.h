@@ -182,6 +182,7 @@ TKNN_API int tknn_build(tknn_ctx* ctx, const float* xyz, uint64_t n, int dim, in
  *   tknn_range_count / tknn_radius_search: only points of q's own segment are in its ball; nothing else changes.
  *   tknn_query / tknn_radius_query: TKNN_ESTATE; a separate query set takes tknn_query_segments /
  *     tknn_radius_query_segments, which give each query segment the data segment of the same number.
+ *   tknn_fps: samples every segment on its own (sample_offsets give each segment its count).
  *   tknn_search_shard, tknn_dbscan, tknn_brute_force, tknn_partition_search and tknn_partition_verify: TKNN_ESTATE
  *     (segmented builds do not support them yet). */
 TKNN_API int tknn_build_segments(tknn_ctx* ctx, const float* xyz, uint64_t n, int dim, int stride_floats,
@@ -281,6 +282,31 @@ TKNN_API int tknn_radius_query_segments(tknn_ctx* ctx, const float* queries, uin
                                         const uint64_t* q_seg_offsets, uint64_t n_segments, const int32_t* self_ids,
                                         float radius, uint64_t* offsets_out, int32_t* idx_out, float* dist_out,
                                         uint64_t capacity, uint64_t* total_out);
+
+/* Exact farthest point sampling of the last build (torch_cluster's fps), plain (one segment) or segmented; segment s is
+ * the points with indices [off[s], off[s + 1]).  Per segment, with a sample count m_s and a start index start_s in it:
+ * D(p) is the minimum over the samples selected so far in p's segment of d2(c, p) (the d2 rule above; +inf before the
+ * first sample).  Sample 0 is start_s; sample i + 1 is the point of the segment that maximises D(p), ties to the LOWEST
+ * index (torch.argmax's first occurrence), i.e. the largest u64 key (bits(D) << 32) | (0xFFFFFFFF - index), which orders
+ * +inf correctly too.  When every point of a segment has D = 0 (duplicates, m_s above its distinct locations) the rule
+ * picks the segment's lowest index again, so samples may repeat; for distinct points and m_s = n_s they are a
+ * permutation of the segment.  The result depends only on the points, the offsets, the counts and the starts (not on
+ * leaf size, curve, sort mode, grid option or stream) and is identical from call to call.
+ * sample_offsets: n_segments + 1 u64 entries, host or device, starting at 0, non-decreasing, with m_s =
+ * sample_offsets[s+1] - sample_offsets[s] <= the segment's point count; n_segments must equal the build's segment count
+ * (1 after tknn_build).  start_ids (may be NULL: the first point of every segment, off[s]): n_segments global indices,
+ * each inside its segment wherever m_s > 0.  idx_out: sample_offsets[n_segments] entries, idx_out[soff[s] + i] = the
+ * i-th sample of segment s as a global index; dist_out (may be NULL): sqrtf(D(sample i)) when it was selected (the
+ * coverage radius after i samples, non-increasing in i), d2 while TKNN_OPT_SQUARED_DIST is set, FLT_MAX for sample 0.
+ * Host or device arrays.  Errors: malformed offsets, a count above its segment, a start outside its segment, a NULL
+ * idx_out or n > 2^31 - 1: TKNN_EINVAL; before a build, on a point-partitioned context or a BVH with caller-chosen ids:
+ * TKNN_ESTATE; a device without cooperative launch when a segment is above the block tier's capacity: TKNN_ECUDA.
+ * Statistics: rounds = 2 tiers (segments of at most 14 336 points: one CTA each; larger ones: one cooperative kernel,
+ * leaf-culled) in round_ms / kernel_ms, round_queries = the samples of each tier, n_queries = all samples, search_ms =
+ * the whole call on the device.  TKNN_OPT_COUNTERS: nodes_visited = leaf box tests of the grid tier, warp_leaf_visits
+ * = leaves whose points were updated, points_tested = point distance updates. */
+TKNN_API int tknn_fps(tknn_ctx* ctx, const uint64_t* sample_offsets, uint64_t n_segments, const int32_t* start_ids,
+                      int32_t* idx_out, float* dist_out);
 
 /* Start-radius estimator alone (replaces samples/s01-trueknn/Util/random_sample.py:5-32). */
 TKNN_API int tknn_estimate_start_radius(tknn_ctx* ctx, int k, float* radius_out);

@@ -77,6 +77,11 @@ struct tknn_ctx {
   bool segmented = false;
   uint64_t n_segments = 0;
   DevBuf seg_off, seg_of, node_seg;
+  std::vector<uint64_t> seg_off_host;  // the same offsets on the host (tknn_fps sizes its tiers from them)
+  // tknn_fps scratch (grow-only, fps.cuh): the segments of each tier, the tier of every segment, leaf flags, the grid
+  // tier's compact leaf records (box, first position, key), D by position, position by index and the key slots
+  DevBuf fps_segs, fps_slot_of_seg, fps_words, fps_leaf_lo, fps_leaf_hi, fps_leaf_first, fps_leaf_key, fps_D, fps_pos_of,
+      fps_best;
   // cell grid over the sorted points (grid.cuh): runs per level-L cell and the table's frame; made by a plain build when
   // the cloud qualifies, and then round 1 of a dense kNN search with k <= 24 walks it instead of the LBVH
   int grid_mode = 0;        // TKNN_OPT_GRID: 0 = auto (occupancy decides), 1 = off, 2 = whenever the table is valid

@@ -18,6 +18,7 @@
 #include "brute.cuh"
 #include "common.cuh"
 #include "ctx.cuh"
+#include "fps.cuh"
 #include "grid.cuh"
 #include "lbvh.cuh"
 #include "radix_sort.cuh"
@@ -909,7 +910,9 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->rl_cnt_pos, &c->rl_cnt_row, &c->rl_off_pos, &c->rl_off_row, &c->rl_sums, &c->rl_stats, &c->rl_pos_of,
                     &c->rl_self_pos, &c->rl_keys, &c->rl_long_pos, &c->rl_long_len, &c->rl_boff, &c->rl_ka, &c->rl_kb,
                     &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp, &c->seg_off, &c->seg_of, &c->node_seg,
-                    &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted, &c->grid_cells, &c->grid_frame})
+                    &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted, &c->grid_cells, &c->grid_frame, &c->fps_segs,
+                    &c->fps_slot_of_seg, &c->fps_words, &c->fps_leaf_lo, &c->fps_leaf_hi, &c->fps_leaf_first,
+                    &c->fps_leaf_key, &c->fps_D, &c->fps_pos_of, &c->fps_best})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -1042,6 +1045,7 @@ int tknn_build_segments(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int 
   TK_TRY(ensure(c, c->seg_off, off.size() * sizeof(uint64_t)));
   TK_CUDA(c, cudaMemcpyAsync(c->seg_off.p, off.data(), off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, c->stream));
   TK_CUDA(c, cudaStreamSynchronize(c->stream));
+  c->seg_off_host = std::move(off);
   return build_core(c, xyz, n, dim, stride_floats, false, c->seg_off.as<uint64_t>(), n_segments, max_segment);
 }
 
@@ -1782,6 +1786,197 @@ int tknn_dbscan(tknn_ctx* c, float eps, int min_pts, int32_t* label_out, uint8_t
   if (n_clusters_out) *n_clusters_out = rb[2];
   TK_TRY(collect_counters(c));
   TK_TRY(read_error_flag(c));
+  return TKNN_OK;
+}
+
+// Farthest point sampling (fps.cuh).  The host reads the offsets, counts and starts (host copies, or one read-back of each
+// for device arrays), splits the segments into the block tier (at most fps::BLOCK_CAP points) and the grid tier, and runs
+// both on the stream, one after the other.
+int tknn_fps(tknn_ctx* c, const uint64_t* sample_offsets, uint64_t n_segments, const int32_t* start_ids, int32_t* idx_out,
+             float* dist_out) {
+  TK_TRY(check_ctx(c));
+  if (c->n == 0) return fail(c, TKNN_ESTATE, "tknn_fps before tknn_build");
+  if (c->ids_in_w) return fail(c, TKNN_ESTATE, "this BVH carries caller-chosen point ids (point-partitioned build)");
+  if (!sample_offsets) return fail(c, TKNN_EINVAL, "tknn_fps: null sample offsets");
+  if (!idx_out) return fail(c, TKNN_EINVAL, "tknn_fps: null idx_out");
+  if (c->n > (uint64_t)INT32_MAX) return fail(c, TKNN_EINVAL, "tknn_fps supports at most 2^31 - 1 points");
+  if (n_segments != c->n_segments)
+    return fail(c, TKNN_EINVAL, "tknn_fps: n_segments = %llu, the last build has %llu", (unsigned long long)n_segments,
+                (unsigned long long)c->n_segments);
+  ScopedDevice sd(c->device);
+  cudaStream_t st = c->stream;
+  const uint64_t S = n_segments;
+  const std::vector<uint64_t> off = c->segmented ? c->seg_off_host : std::vector<uint64_t>{0, c->n};
+  std::vector<uint64_t> soff(S + 1);
+  std::vector<int32_t> starts(S);
+  if (is_device_ptr(sample_offsets))
+    TK_CUDA(c, cudaMemcpyAsync(soff.data(), sample_offsets, soff.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+  else
+    std::memcpy(soff.data(), sample_offsets, soff.size() * sizeof(uint64_t));
+  if (start_ids && is_device_ptr(start_ids))
+    TK_CUDA(c, cudaMemcpyAsync(starts.data(), start_ids, starts.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  else if (start_ids)
+    std::memcpy(starts.data(), start_ids, starts.size() * sizeof(int32_t));
+  TK_CUDA(c, cudaStreamSynchronize(st));
+  if (soff[0] != 0) return fail(c, TKNN_EINVAL, "tknn_fps: sample offsets must start at 0");
+  std::vector<fps::Seg> small, large;
+  std::vector<uint32_t> slot_of_seg;
+  uint32_t small_max = 0, large_max_m = 0;
+  uint64_t small_samples = 0, large_samples = 0;
+  for (uint64_t s = 0; s < S; ++s) {
+    if (soff[s + 1] < soff[s]) return fail(c, TKNN_EINVAL, "tknn_fps: sample offsets decrease at segment %llu", (unsigned long long)s);
+    const uint64_t ns = off[s + 1] - off[s], m = soff[s + 1] - soff[s];
+    if (m > ns)
+      return fail(c, TKNN_EINVAL, "tknn_fps: %llu samples of segment %llu, which has %llu points", (unsigned long long)m,
+                  (unsigned long long)s, (unsigned long long)ns);
+    if (!start_ids) starts[s] = (int32_t)off[s];
+    if (m > 0 && (starts[s] < 0 || (uint64_t)starts[s] < off[s] || (uint64_t)starts[s] >= off[s + 1]))
+      return fail(c, TKNN_EINVAL, "tknn_fps: start %d outside segment %llu = [%llu, %llu)", starts[s], (unsigned long long)s,
+                  (unsigned long long)off[s], (unsigned long long)off[s + 1]);
+  }
+  for (uint64_t s = 0; s < S; ++s) {
+    const uint64_t ns = off[s + 1] - off[s], m = soff[s + 1] - soff[s];
+    if (m == 0) continue;
+    const fps::Seg sg = {(uint32_t)off[s], (uint32_t)ns, (uint32_t)soff[s], (uint32_t)m, (uint32_t)starts[s], 0, 0, 0};
+    if (ns <= (uint64_t)fps::BLOCK_CAP) {
+      small.push_back(sg);
+      small_max = std::max(small_max, (uint32_t)ns);
+      small_samples += m;
+    } else {
+      if (slot_of_seg.empty()) slot_of_seg.assign(S, fps::NO_SLOT);
+      slot_of_seg[s] = (uint32_t)large.size();
+      large.push_back(sg);
+      large_max_m = std::max(large_max_m, (uint32_t)m);
+      large_samples += m;
+    }
+  }
+  const uint64_t total = soff[S];
+  if (!large.empty()) {
+    int coop = 0;
+    TK_CUDA(c, cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, c->device));
+    if (!coop) return fail(c, TKNN_ECUDA, "tknn_fps: the device does not support cooperative launches (needed by clouds above %d points)",
+                           fps::BLOCK_CAP);
+  }
+
+  reset_search_stats(c);
+  const bool idx_dev = is_device_ptr(idx_out), dist_dev = dist_out && is_device_ptr(dist_out);
+  if (!idx_dev) TK_TRY(ensure(c, c->stage_idx, sizeof(int32_t) * std::max<uint64_t>(total, 1)));
+  if (dist_out && !dist_dev) TK_TRY(ensure(c, c->stage_dist, sizeof(float) * std::max<uint64_t>(total, 1)));
+  int32_t* d_idx = idx_dev ? idx_out : c->stage_idx.as<int32_t>();
+  float* d_dist = dist_out ? (dist_dev ? dist_out : c->stage_dist.as<float>()) : nullptr;
+  TK_TRY(ensure(c, c->fps_segs, sizeof(fps::Seg) * (small.size() + large.size())));
+  fps::Seg* d_small = c->fps_segs.as<fps::Seg>();
+  fps::Seg* d_large = d_small + small.size();
+  if (!small.empty())
+    TK_CUDA(c, cudaMemcpyAsync(d_small, small.data(), sizeof(fps::Seg) * small.size(), cudaMemcpyHostToDevice, st));
+  if (!large.empty())
+    TK_CUDA(c, cudaMemcpyAsync(d_large, large.data(), sizeof(fps::Seg) * large.size(), cudaMemcpyHostToDevice, st));
+  for (size_t i = c->round_ev.size(); i < 8; ++i) {
+    cudaEvent_t e;
+    TK_CUDA(c, cudaEventCreate(&e));
+    c->round_ev.push_back(e);
+  }
+  cudaEvent_t* ev = c->round_ev.data();  // tier r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its sampling kernel
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  unsigned long long* counters = reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS);
+  int launches = 0;
+  TK_CUDA(c, cudaMemsetAsync(counters, 0, 8 * sizeof(unsigned long long), st));
+  TK_CUDA(c, cudaEventRecord(c->ev[0], st));
+
+  // block tier: one CTA per segment, sized for the largest one (about BLOCK_TARGET_PER points per thread)
+  TK_CUDA(c, cudaEventRecord(ev[0], st));
+  TK_CUDA(c, cudaEventRecord(ev[2], st));
+  if (!small.empty()) {
+    const uint32_t per = (small_max + fps::BLOCK_TARGET_PER - 1) / fps::BLOCK_TARGET_PER;
+    const unsigned threads = std::min(1024u, std::max(32u, (per + 31u) / 32u * 32u));
+    const size_t smem = sizeof(float4) * small_max + 2 * WARP * (sizeof(uint64_t) + sizeof(uint32_t));
+    TK_CUDA(c, cudaFuncSetAttribute(fps::fps_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fps::fps_block_kernel<<<(unsigned)small.size(), threads, smem, st>>>(c->pts.as<float4>(), d_small, small_max, d_idx, d_dist,
+                                                                         c->squared);
+    TK_CUDA(c, cudaGetLastError());
+    ++launches;
+  }
+  TK_CUDA(c, cudaEventRecord(ev[3], st));
+  TK_CUDA(c, cudaEventRecord(ev[1], st));
+
+  // grid tier: compact leaf records of the large segments, then the cooperative kernel
+  TK_CUDA(c, cudaEventRecord(ev[4], st));
+  if (large.empty()) {
+    TK_CUDA(c, cudaEventRecord(ev[6], st));
+    TK_CUDA(c, cudaEventRecord(ev[7], st));
+  } else {
+    const uint32_t nl = c->n_leaves, n_words = (nl + 31) / 32, L = (uint32_t)large.size();
+    const uint64_t n = c->n;
+    TK_TRY(ensure(c, c->fps_slot_of_seg, sizeof(uint32_t) * S));
+    TK_TRY(ensure(c, c->fps_words, sizeof(uint32_t) * n_words));
+    TK_TRY(ensure(c, c->offsets, sizeof(uint32_t) * (size_t)(n_words + 1)));
+    TK_TRY(ensure(c, c->fps_leaf_lo, sizeof(float4) * nl));
+    TK_TRY(ensure(c, c->fps_leaf_hi, sizeof(float4) * nl));
+    TK_TRY(ensure(c, c->fps_leaf_first, sizeof(uint32_t) * nl));
+    TK_TRY(ensure(c, c->fps_leaf_key, sizeof(uint64_t) * nl));
+    TK_TRY(ensure(c, c->fps_D, sizeof(float) * n));
+    TK_TRY(ensure(c, c->fps_pos_of, sizeof(uint32_t) * n));
+    TK_TRY(ensure(c, c->fps_best, sizeof(uint64_t) * 3 * (size_t)L));
+    TK_CUDA(c, cudaMemcpyAsync(c->fps_slot_of_seg.p, slot_of_seg.data(), sizeof(uint32_t) * S, cudaMemcpyHostToDevice, st));
+    const uint32_t* seg_of = c->segmented ? c->seg_of.as<uint32_t>() : nullptr;
+    uint32_t* words = c->fps_words.as<uint32_t>();
+    fps::leaf_flag_kernel<<<blocks_for(nl, fps::INIT_THREADS), fps::INIT_THREADS, 0, st>>>(
+        c->leaf_start.as<uint32_t>(), nl, seg_of, c->fps_slot_of_seg.as<uint32_t>(), words);
+    TK_CUDA(c, cudaGetLastError());
+    TK_TRY(popc_scan(c, words, n_words, c->offsets.as<uint32_t>(), &launches));  // compact leaf count -> sc[SC_TOTAL]
+    fps::leaf_init_kernel<<<blocks_for((uint64_t)nl * WARP, fps::INIT_THREADS), fps::INIT_THREADS, 0, st>>>(
+        c->pts.as<float4>(), c->leaf_start.as<uint32_t>(), nl, seg_of, c->fps_slot_of_seg.as<uint32_t>(), words,
+        c->offsets.as<uint32_t>(), c->fps_leaf_lo.as<float4>(), c->fps_leaf_hi.as<float4>(), c->fps_leaf_first.as<uint32_t>(),
+        c->fps_leaf_key.as<uint64_t>(), c->fps_D.as<float>(), c->fps_pos_of.as<uint32_t>());
+    fps::slot_init_kernel<<<blocks_for(L, fps::INIT_THREADS), fps::INIT_THREADS, 0, st>>>(d_large, L, c->fps_best.as<uint64_t>(),
+                                                                                          d_idx, d_dist);
+    TK_CUDA(c, cudaGetLastError());
+    launches += 3;
+    fps::GridParams P;
+    P.pts = c->pts.as<float4>();
+    P.leaf_lo = c->fps_leaf_lo.as<float4>();
+    P.leaf_hi = c->fps_leaf_hi.as<float4>();
+    P.leaf_first = c->fps_leaf_first.as<uint32_t>();
+    P.leaf_key = c->fps_leaf_key.as<uint64_t>();
+    P.D = c->fps_D.as<float>();
+    P.pos_of = c->fps_pos_of.as<uint32_t>();
+    P.segs = d_large;
+    P.n_slots = L;
+    P.max_m = large_max_m;
+    P.n_leaves = sc + SC_TOTAL;
+    P.best = c->fps_best.as<uint64_t>();
+    P.idx_out = d_idx;
+    P.dist_out = d_dist;
+    P.squared = c->squared;
+    P.counters = counters;
+    void (*kernel)(const fps::GridParams) = c->counters ? fps::fps_grid_kernel<true> : fps::fps_grid_kernel<false>;
+    int per_sm = 0;
+    TK_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, fps::GRID_THREADS, 0));
+    if (per_sm < 1) return fail(c, TKNN_ECUDA, "tknn_fps: the grid-tier kernel cannot be resident on an SM");
+    // every block must be resident for the grid barrier: at most what the occupancy calculator allows, and two blocks per
+    // SM at most, since a barrier over more blocks costs more than their extra warps hide
+    const unsigned grid_blocks = (unsigned)(std::min(per_sm, 2) * c->sm_count);
+    void* args[] = {&P};
+    TK_CUDA(c, cudaEventRecord(ev[6], st));
+    TK_CUDA(c, cudaLaunchCooperativeKernel((const void*)kernel, dim3(grid_blocks), dim3(fps::GRID_THREADS), args, 0, st));
+    TK_CUDA(c, cudaEventRecord(ev[7], st));
+    ++launches;
+  }
+  TK_CUDA(c, cudaEventRecord(ev[5], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
+
+  if (!idx_dev && total) TK_CUDA(c, cudaMemcpyAsync(idx_out, d_idx, sizeof(int32_t) * total, cudaMemcpyDeviceToHost, st));
+  if (dist_out && !dist_dev && total) TK_CUDA(c, cudaMemcpyAsync(dist_out, d_dist, sizeof(float) * total, cudaMemcpyDeviceToHost, st));
+  TK_CUDA(c, cudaStreamSynchronize(st));
+  c->stats.d2h_bytes = (idx_dev ? 0 : sizeof(int32_t) * total) + (dist_out && !dist_dev ? sizeof(float) * total : 0);
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
+  c->stats.n_queries = total;
+  c->stats.rounds = 2;
+  c->stats.round_queries[0] = small_samples;
+  c->stats.round_queries[1] = large_samples;
+  c->stats.kernel_launches = (uint32_t)launches;
+  TK_TRY(finish_round_stats(c));
+  TK_TRY(collect_counters(c));
   return TKNN_OK;
 }
 

@@ -68,6 +68,7 @@ class TrueKNN:
         self._own_stream = True  # until set_stream() hands over a caller stream
         self.n = 0
         self.n_segments = 1  # clouds of the last build (batch_size of query(batch=...) / radius_query(batch=...))
+        self._offsets = None  # the cloud offsets of a segmented build (numpy or a tensor), None for a plain build
         self._like = None
         for k, v in options.items():
             self.set_option(k, v)
@@ -181,11 +182,13 @@ class TrueKNN:
                 raise ValueError("batch_size needs a batch")
             self._check(self._L.tknn_build(self._h, self._in(points), int(points.shape[0]), int(dim), stride))
             self.n_segments = 1
+            self._offsets = None
         else:
             offsets = batch_to_offsets(batch, int(points.shape[0]), batch_size)
             self._check(self._L.tknn_build_segments(self._h, self._in(points), int(points.shape[0]), int(dim), stride,
                                                     self._in(offsets), int(offsets.shape[0]) - 1))
             self.n_segments = int(offsets.shape[0]) - 1
+            self._offsets = offsets
         self.n = int(points.shape[0])
         self._like = points
         return self
@@ -290,6 +293,54 @@ class TrueKNN:
         c = C.c_uint64(0)
         self._check(self._L.tknn_dbscan(self._h, C.c_float(eps), int(min_pts), _ptr(labels), _ptr(core), C.byref(c)))
         return labels, core, int(c.value)
+
+    def cloud_sizes(self) -> np.ndarray:
+        """Points per cloud of the last build (int64 numpy; [n] for a plain build)."""
+        if self._offsets is None:
+            return np.array([self.n], np.int64)
+        off = self._offsets.cpu().numpy() if _is_tensor(self._offsets) else self._offsets
+        return np.diff(off.astype(np.int64))
+
+    def fps(self, num_samples=None, ratio: float | None = None, start=None, with_dist: bool = False, out=None):
+        """Exact farthest point sampling of every cloud of the last build (tknn_fps; torch_cluster's fps selection rule).
+
+        Exactly one of num_samples (an int for a plain build, or one count per cloud) and ratio (in (0, 1]: cloud s gets
+        ceil(float32(n_s) * float32(ratio)) samples, fps_counts) is given.  start: None (the first point of every cloud)
+        or one global index per cloud.  Sample 0 of a cloud is its start; each next sample is the point farthest from the
+        samples so far (squared fp32 distance, ties to the lowest index).  Returns (idx [M] int32: global indices, cloud
+        by cloud; dist [M] float32 or None: the distance of each sample from the earlier ones when it was picked, FLT_MAX
+        for sample 0, d2 while squared_dist is set).  numpy outputs for numpy input, CUDA tensors for CUDA tensor input;
+        out = (idx, dist) supplies the arrays (dist may be None)."""
+        sizes = self.cloud_sizes()
+        if (num_samples is None) == (ratio is None):
+            raise ValueError("give exactly one of num_samples and ratio")
+        if ratio is not None:
+            counts = fps_counts(sizes, ratio)
+        else:
+            counts = np.atleast_1d(np.asarray(num_samples, dtype=np.int64))
+            if counts.shape != sizes.shape:
+                raise ValueError(f"num_samples: one count per cloud ({sizes.shape[0]}), got {counts.shape[0]}")
+        if (counts < 0).any():
+            raise ValueError("num_samples must be >= 0")
+        soff = np.concatenate([[0], np.cumsum(counts)]).astype(np.uint64)
+        total = int(soff[-1])
+        if start is not None and not _is_tensor(start):
+            start = np.ascontiguousarray(np.atleast_1d(start), dtype=np.int32)
+        if start is not None:
+            _check_dtype(start, np.int32, "start")
+            if int(start.shape[0]) != sizes.shape[0]:
+                raise ValueError(f"start: one index per cloud ({sizes.shape[0]}), got {int(start.shape[0])}")
+        if out is not None:
+            idx, dist = out
+        else:
+            idx = self._out(self._like, total, 1, np.int32).reshape(-1)
+            dist = self._out(self._like, total, 1, np.float32).reshape(-1) if with_dist else None
+        _check_dtype(idx, np.int32, "idx")
+        if dist is not None:
+            _check_dtype(dist, np.float32, "dist")
+        if total:  # an empty torch tensor has no address, and there is nothing to sample
+            self._check(self._L.tknn_fps(self._h, _ptr(soff), sizes.shape[0], self._in(start), _ptr(idx), _ptr(dist)))
+        return idx, dist
 
     def radius_search(self, radius: float, indices_only: bool = False, out=None):
         """Exact fixed-radius neighbour lists of every built point (closed ball, the point itself excluded).
@@ -680,6 +731,58 @@ def batch_to_offsets(batch, n: int, batch_size: int | None = None):
         raise ValueError(f"batch holds cloud id {int(b[-1])} >= batch_size = {batch_size}")
     counts = np.bincount(b, minlength=int(b[-1]) + 1 if batch_size is None else int(batch_size))
     return np.concatenate([[0], np.cumsum(counts)]).astype(np.uint64)
+
+
+def fps_counts(sizes, ratio: float) -> np.ndarray:
+    """Samples per cloud for a ratio, torch_cluster's rule: ceil(float32(n_s) * float32(ratio)), at most n_s, so an empty
+    cloud gets 0.  ratio must lie in (0, 1]."""
+    if not 0.0 < float(ratio) <= 1.0:
+        raise ValueError(f"ratio = {ratio} must lie in (0, 1]")
+    n = np.asarray(sizes, dtype=np.int64)
+    return np.minimum(np.ceil(n.astype(np.float32) * np.float32(ratio)).astype(np.int64), n)
+
+
+def fps_random_starts(offsets, like=None):
+    """One uniformly drawn start per cloud, as a global index, from the global RNG of `like`'s framework: torch.randint
+    on the tensor's device, numpy's global generator otherwise.  offsets: the n_clouds + 1 cloud offsets (numpy); an
+    empty cloud gets its offset (it has no samples).  Returns int32 on `like`'s device, or numpy."""
+    off = np.asarray(offsets, dtype=np.int64)
+    sizes = np.maximum(np.diff(off), 1)
+    if _is_tensor(like):
+        import torch
+
+        r = torch.randint(0, 2**62, (sizes.shape[0],), dtype=torch.int64, device=like.device)
+        base = torch.as_tensor(off[:-1], device=like.device)
+        return (base + r % torch.as_tensor(sizes, device=like.device)).to(torch.int32)
+    return (off[:-1] + np.random.randint(0, sizes)).astype(np.int32)
+
+
+def fps(src, batch=None, ratio: float = 0.5, random_start: bool = True, batch_size: int | None = None,
+        device: int | None = None):
+    """torch_cluster.fps(src, batch, ratio, random_start, batch_size) on the GPU, exact: farthest point sampling of every
+    cloud, ceil(n_s * ratio) samples each (fps_counts).  Returns int64 global indices, concatenated cloud by cloud, each
+    cloud's samples in the order they were picked.  random_start draws each cloud's first sample from the global RNG of
+    the input's framework (fps_random_starts); otherwise it is the cloud's first point.  numpy in, numpy out; a CUDA
+    tensor in, a tensor on its device out (device: the CUDA device for numpy input, default 0)."""
+    n = int(src.shape[0])
+    if n == 0:
+        fps_counts([0], ratio)  # the same argument check
+        if _is_tensor(src):
+            import torch
+
+            return torch.zeros((0,), dtype=torch.int64, device=src.device)
+        return np.zeros(0, np.int64)
+    dev = src.device.index if _is_tensor(src) else (device or 0)
+    with TrueKNN(dev) as t:
+        t.build(src, batch=batch, batch_size=batch_size)
+        sizes = t.cloud_sizes()
+        start = fps_random_starts(np.concatenate([[0], np.cumsum(sizes)]), src) if random_start else None
+        idx, _ = t.fps(ratio=ratio, start=start)
+    if _is_tensor(idx):
+        import torch
+
+        return idx.to(torch.int64)
+    return idx.astype(np.int64)
 
 
 def _edge_index(centre, neighbour, like):
