@@ -308,6 +308,32 @@ TKNN_API int tknn_radius_query_segments(tknn_ctx* ctx, const float* queries, uin
 TKNN_API int tknn_fps(tknn_ctx* ctx, const uint64_t* sample_offsets, uint64_t n_segments, const int32_t* start_ids,
                       int32_t* idx_out, float* dist_out);
 
+/* Exact k-nearest neighbours in feature space over a batch of clouds (torch_cluster's knn / knn_graph on features, as
+ * DGCNN's dynamic graphs use them).  x: n data rows, y: nq query rows, both row-major with their own pitch (stride >= f
+ * floats); only the first f columns are read.  y may alias x (the all-points form passes the same pointer twice).
+ * Distance rule, with d_j = fl(y_j - x_j): d2 = d_0 * d_0, then d2 = fmaf(d_j, d_j, d2) for j = 1 .. f - 1 in that
+ * order, in fp32.  For f = 3 this is the d2 rule above; for f = 2 it equals the 2-D path (z = 0).  fmaf(d, d, +0) has
+ * the bits of d * d, so the sum may start at +0.
+ * Segments: query segment s (rows [y_off[s], y_off[s + 1])) searches data segment s (rows [x_off[s], x_off[s + 1]))
+ * only.  Each offset array holds n_segments + 1 entries, host or device, that start at 0, never decrease and end at n
+ * (nq for y_off); empty segments are legal.  Both NULL: one segment, and n_segments must be 1; one NULL: TKNN_EINVAL.
+ * Row j holds the k points p of its data segment with index(p) != self_ids[j] and the smallest (d2, index), ordered
+ * ascending by that key (the key of make_key: +inf distances from overflow are ordered by index).  self_ids (may be
+ * NULL: nothing excluded): nq global data indices; -1 or an index outside the data segment excludes nothing.  Rows
+ * with fewer eligible points end in -1 / FLT_MAX.  dist_out (may be NULL: indices only) receives sqrtf(d2), or d2
+ * while TKNN_OPT_SQUARED_DIST is set.  idx_out / dist_out: nq * k entries.  Host or device arrays.
+ * The call needs no build and touches none: it works before tknn_build, and a search after it returns what it
+ * returned before.  No option selects its path: a tiled brute force on the CUDA cores (DESIGN.md §3.8), split over the
+ * data rows when the query tiles alone would leave the GPU idle, with a k-way merge of the splits.
+ * Errors (TKNN_EINVAL): f outside [1, 1024], a stride below f, k outside [1, min(n, TKNN_MAX_K)], n or nq >= 2^31, a
+ * non-finite value in the first f columns of x or y, malformed offsets, a NULL x, y or idx_out.  nq = 0 is a no-op.
+ * Statistics: n_queries, k, search_ms; rounds = 1 (the tile kernel) or 2 (tile kernel, then the merge of the splits),
+ * with round_ms / kernel_ms / round_queries per round; points_tested = the pair distances evaluated, sum_s nq_s * n_s. */
+TKNN_API int tknn_feature_knn(tknn_ctx* ctx, const float* x, uint64_t n, int f, int x_stride_floats,
+                              const uint64_t* x_seg_offsets, const float* y, uint64_t nq, int y_stride_floats,
+                              const uint64_t* y_seg_offsets, uint64_t n_segments, const int32_t* self_ids, int k,
+                              int32_t* idx_out, float* dist_out);
+
 /* Start-radius estimator alone (replaces samples/s01-trueknn/Util/random_sample.py:5-32). */
 TKNN_API int tknn_estimate_start_radius(tknn_ctx* ctx, int k, float* radius_out);
 

@@ -107,7 +107,7 @@ EXPORTS = [
     "tknn_multi_set_option", "tknn_multi_build", "tknn_multi_search", "tknn_multi_ranks", "tknn_multi_ctx",
     "tknn_multi_last_error", "tknn_multi_get_times", "tknn_measure_smem_bandwidth", "tknn_key_layout", "tknn_dbscan",
     "tknn_radius_search", "tknn_radius_query", "tknn_write_neighbour_lists", "tknn_build_segments",
-    "tknn_query_segments", "tknn_radius_query_segments", "tknn_fps",
+    "tknn_query_segments", "tknn_radius_query_segments", "tknn_fps", "tknn_feature_knn",
 ]
 
 _lib = None
@@ -142,6 +142,7 @@ def load() -> C.CDLL:
     L.tknn_range_count.argtypes = [vp, f32, vp]
     L.tknn_dbscan.argtypes = [vp, f32, C.c_int, vp, vp, C.POINTER(u64)]
     L.tknn_fps.argtypes = [vp, vp, u64, vp, vp, vp]
+    L.tknn_feature_knn.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, vp, u64, C.c_int, vp, u64, vp, C.c_int, vp, vp]
     L.tknn_radius_search.argtypes = [vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_radius_query.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_query_segments.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, vp, vp, C.c_int, f32, vp, vp]

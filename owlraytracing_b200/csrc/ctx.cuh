@@ -82,6 +82,10 @@ struct tknn_ctx {
   // tier's compact leaf records (box, first position, key), D by position, position by index and the key slots
   DevBuf fps_segs, fps_slot_of_seg, fps_words, fps_leaf_lo, fps_leaf_hi, fps_leaf_first, fps_leaf_key, fps_D, fps_pos_of,
       fps_best;
+  // tknn_feature_knn scratch (grow-only, features.cuh): staged host rows and self ids, the work list, the partial key
+  // lists of a split call and the distances the merge writes when the caller asked for indices only.  It touches no
+  // build state.
+  DevBuf fk_x, fk_y, fk_sid, fk_items, fk_partial, fk_dist;
   // cell grid over the sorted points (grid.cuh): runs per level-L cell and the table's frame; made by a plain build when
   // the cloud qualifies, and then round 1 of a dense kNN search with k <= 24 walks it instead of the LBVH
   int grid_mode = 0;        // TKNN_OPT_GRID: 0 = auto (occupancy decides), 1 = off, 2 = whenever the table is valid

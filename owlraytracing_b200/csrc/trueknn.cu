@@ -18,6 +18,7 @@
 #include "brute.cuh"
 #include "common.cuh"
 #include "ctx.cuh"
+#include "features.cuh"
 #include "fps.cuh"
 #include "grid.cuh"
 #include "lbvh.cuh"
@@ -912,7 +913,8 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp, &c->seg_off, &c->seg_of, &c->node_seg,
                     &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted, &c->grid_cells, &c->grid_frame, &c->fps_segs,
                     &c->fps_slot_of_seg, &c->fps_words, &c->fps_leaf_lo, &c->fps_leaf_hi, &c->fps_leaf_first,
-                    &c->fps_leaf_key, &c->fps_D, &c->fps_pos_of, &c->fps_best})
+                    &c->fps_leaf_key, &c->fps_D, &c->fps_pos_of, &c->fps_best, &c->fk_x, &c->fk_y, &c->fk_sid,
+                    &c->fk_items, &c->fk_partial, &c->fk_dist})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -1360,23 +1362,33 @@ int tknn_estimate_start_radius(tknn_ctx* c, int k, float* radius_out) {
 namespace {
 // Query offsets of the _segments calls (host or device): n_segments + 1 entries that start at 0, never decrease and end at
 // nq, with n_segments the segment count of the last build.  Device offsets cost one small read-back.
+// Reads n_segments + 1 offsets (host or device) into *off and checks that they start at 0, never decrease and end at
+// `total` (named `total_name` in the message); `side` names the offsets in the message.
+int read_offsets(tknn_ctx* c, const char* what, const char* side, const uint64_t* offsets, uint64_t n_segments,
+                 uint64_t total, const char* total_name, std::vector<uint64_t>* off_out) {
+  std::vector<uint64_t>& off = *off_out;
+  off.assign(n_segments + 1, 0);
+  if (is_device_ptr(offsets)) {
+    TK_CUDA(c, cudaMemcpyAsync(off.data(), offsets, off.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
+    TK_CUDA(c, cudaStreamSynchronize(c->stream));
+  } else {
+    std::memcpy(off.data(), offsets, off.size() * sizeof(uint64_t));
+  }
+  if (off[0] != 0) return fail(c, TKNN_EINVAL, "%s: %s offsets must start at 0", what, side);
+  if (off[n_segments] != total)
+    return fail(c, TKNN_EINVAL, "%s: %s offsets must end at %s = %llu", what, side, total_name, (unsigned long long)total);
+  for (uint64_t s = 0; s < n_segments; ++s)
+    if (off[s + 1] < off[s]) return fail(c, TKNN_EINVAL, "%s: %s offsets decrease at segment %llu", what, side, (unsigned long long)s);
+  return TKNN_OK;
+}
+
 int check_query_offsets(tknn_ctx* c, const char* what, const uint64_t* q_seg_offsets, uint64_t n_segments, uint64_t nq) {
   if (!q_seg_offsets) return fail(c, TKNN_EINVAL, "%s: null query segment offsets", what);
   if (n_segments != c->n_segments)
     return fail(c, TKNN_EINVAL, "%s: n_segments = %llu, the last build has %llu", what, (unsigned long long)n_segments,
                 (unsigned long long)c->n_segments);
-  std::vector<uint64_t> off(n_segments + 1);
-  if (is_device_ptr(q_seg_offsets)) {
-    TK_CUDA(c, cudaMemcpyAsync(off.data(), q_seg_offsets, off.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
-    TK_CUDA(c, cudaStreamSynchronize(c->stream));
-  } else {
-    std::memcpy(off.data(), q_seg_offsets, off.size() * sizeof(uint64_t));
-  }
-  if (off[0] != 0) return fail(c, TKNN_EINVAL, "%s: query segment offsets must start at 0", what);
-  if (off[n_segments] != nq) return fail(c, TKNN_EINVAL, "%s: query segment offsets must end at nq = %llu", what, (unsigned long long)nq);
-  for (uint64_t s = 0; s < n_segments; ++s)
-    if (off[s + 1] < off[s]) return fail(c, TKNN_EINVAL, "%s: query segment offsets decrease at segment %llu", what, (unsigned long long)s);
-  return TKNN_OK;
+  std::vector<uint64_t> off;
+  return read_offsets(c, what, "query segment", q_seg_offsets, n_segments, nq, "nq", &off);
 }
 
 // The query staging of tknn_query and tknn_radius_query: host inputs are copied to the device, the queries are sorted on
@@ -1977,6 +1989,200 @@ int tknn_fps(tknn_ctx* c, const uint64_t* sample_offsets, uint64_t n_segments, c
   c->stats.kernel_launches = (uint32_t)launches;
   TK_TRY(finish_round_stats(c));
   TK_TRY(collect_counters(c));
+  return TKNN_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+template <int QT>
+int launch_feature_knn(tknn_ctx* c, const feat::Params& P, uint32_t n_items) {
+  const size_t smem = feat::smem_bytes<QT>(P.k);
+  TK_CUDA(c, cudaFuncSetAttribute(feat::feature_knn_kernel<QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  feat::feature_knn_kernel<QT><<<n_items, QT * 4, smem, c->stream>>>(P);
+  TK_CUDA(c, cudaGetLastError());
+  return TKNN_OK;
+}
+
+// Partial key lists of a split call are bounded to this many bytes (splits x nq x k x 8 B)
+constexpr uint64_t FEATURE_PARTIAL_BYTES = 1ull << 29;
+
+}  // namespace
+
+extern "C" {
+
+int tknn_feature_knn(tknn_ctx* c, const float* x, uint64_t n, int f, int x_stride_floats, const uint64_t* x_seg_offsets,
+                     const float* y, uint64_t nq, int y_stride_floats, const uint64_t* y_seg_offsets, uint64_t n_segments,
+                     const int32_t* self_ids, int k, int32_t* idx_out, float* dist_out) {
+  TK_TRY(check_ctx(c));
+  const char* what = "tknn_feature_knn";
+  if (!x || !y || !idx_out) return fail(c, TKNN_EINVAL, "%s: null x, y or idx_out", what);
+  if (f < 1 || f > 1024) return fail(c, TKNN_EINVAL, "%s: f = %d outside [1, 1024]", what, f);
+  if (x_stride_floats < f || y_stride_floats < f)
+    return fail(c, TKNN_EINVAL, "%s: strides %d / %d below f = %d", what, x_stride_floats, y_stride_floats, f);
+  if (n >= (1ull << 31) || nq >= (1ull << 31)) return fail(c, TKNN_EINVAL, "%s: n and nq must be below 2^31", what);
+  if (k < 1 || k > TKNN_MAX_K || (uint64_t)k > n)
+    return fail(c, TKNN_EINVAL, "%s: k = %d outside [1, min(n = %llu, %d)]", what, k, (unsigned long long)n, TKNN_MAX_K);
+  if ((x_seg_offsets == nullptr) != (y_seg_offsets == nullptr))
+    return fail(c, TKNN_EINVAL, "%s: give both segment offset arrays or neither", what);
+  if (!x_seg_offsets && n_segments != 1)
+    return fail(c, TKNN_EINVAL, "%s: n_segments = %llu without offsets (must be 1)", what, (unsigned long long)n_segments);
+  if (n_segments < 1 || n_segments >= (1ull << 31))
+    return fail(c, TKNN_EINVAL, "%s: n_segments = %llu outside [1, 2^31 - 1]", what, (unsigned long long)n_segments);
+  ScopedDevice sd(c->device);
+  cudaStream_t st = c->stream;
+  std::vector<uint64_t> xo{0, n}, yo{0, nq};
+  if (x_seg_offsets) {
+    TK_TRY(read_offsets(c, what, "data segment", x_seg_offsets, n_segments, n, "n", &xo));
+    TK_TRY(read_offsets(c, what, "query segment", y_seg_offsets, n_segments, nq, "nq", &yo));
+  }
+  reset_search_stats(c);
+  c->stats.n_queries = nq;
+  c->stats.k = k;
+  if (nq == 0) return TKNN_OK;
+
+  // work list: (segment, tile of QT query rows, split of the segment's data rows); splits only when the tiles alone
+  // leave the GPU idle (few queries against big clouds), at least 4 data tiles each, the partial lists bounded
+  const int QT = feat::query_tile(k);
+  uint64_t tiles = 0, max_n = 0, pairs = 0;
+  for (uint64_t s = 0; s < n_segments; ++s) {
+    const uint64_t ns = xo[s + 1] - xo[s], ms = yo[s + 1] - yo[s];
+    tiles += (ms + QT - 1) / QT;
+    if (ms) max_n = std::max(max_n, ns);
+    pairs += ns * ms;
+  }
+  const uint64_t target = (uint64_t)c->sm_count * 2;
+  uint64_t splits = 1;
+  if (tiles < target) {
+    splits = (target + tiles - 1) / tiles;
+    splits = std::min<uint64_t>(splits, std::max<uint64_t>(1, max_n / (4 * feat::PT)));
+    splits = std::min<uint64_t>(splits, 256);
+    splits = std::min<uint64_t>(splits, std::max<uint64_t>(1, FEATURE_PARTIAL_BYTES / (nq * (uint64_t)k * sizeof(uint64_t))));
+  }
+  std::vector<feat::Item> items;
+  items.reserve(tiles * splits);
+  for (uint64_t s = 0; s < n_segments; ++s) {
+    const uint64_t ns = xo[s + 1] - xo[s];
+    const uint64_t chunk = ((ns + splits - 1) / splits + feat::PT - 1) / feat::PT * feat::PT;
+    for (uint64_t q0 = yo[s]; q0 < yo[s + 1]; q0 += QT)
+      for (uint64_t sp = 0; sp < splits; ++sp) {
+        const uint64_t a = std::min(xo[s] + sp * chunk, xo[s + 1]), b = std::min(a + chunk, xo[s + 1]);
+        items.push_back({(uint32_t)q0, (uint32_t)std::min<uint64_t>(QT, yo[s + 1] - q0), (uint32_t)a, (uint32_t)b,
+                         (uint32_t)sp, 0, 0, 0});
+      }
+  }
+
+  // inputs: host rows are staged (y aliasing x is staged once), device rows are read in place
+  const float* d_x = x;
+  const float* d_y = y;
+  const bool same = y == x && y_stride_floats == x_stride_floats && nq == n;
+  if (!is_device_ptr(x)) {
+    const size_t bytes = ((size_t)(n - 1) * x_stride_floats + f) * sizeof(float);
+    TK_TRY(ensure(c, c->fk_x, bytes));
+    TK_CUDA(c, cudaMemcpyAsync(c->fk_x.p, x, bytes, cudaMemcpyHostToDevice, st));
+    d_x = c->fk_x.as<float>();
+  }
+  if (same) {
+    d_y = d_x;
+  } else if (!is_device_ptr(y)) {
+    const size_t bytes = ((size_t)(nq - 1) * y_stride_floats + f) * sizeof(float);
+    TK_TRY(ensure(c, c->fk_y, bytes));
+    TK_CUDA(c, cudaMemcpyAsync(c->fk_y.p, y, bytes, cudaMemcpyHostToDevice, st));
+    d_y = c->fk_y.as<float>();
+  }
+  const int32_t* d_sid = self_ids;
+  if (self_ids && !is_device_ptr(self_ids)) {
+    TK_TRY(ensure(c, c->fk_sid, nq * sizeof(int32_t)));
+    TK_CUDA(c, cudaMemcpyAsync(c->fk_sid.p, self_ids, nq * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    d_sid = c->fk_sid.as<int32_t>();
+  }
+  TK_TRY(ensure(c, c->fk_items, items.size() * sizeof(feat::Item)));
+  TK_CUDA(c, cudaMemcpyAsync(c->fk_items.p, items.data(), items.size() * sizeof(feat::Item), cudaMemcpyHostToDevice, st));
+  const size_t out_elems = (size_t)nq * k;
+  const bool idx_dev = is_device_ptr(idx_out), dist_dev = dist_out && is_device_ptr(dist_out);
+  if (!idx_dev) TK_TRY(ensure(c, c->stage_idx, out_elems * sizeof(int32_t)));
+  if (dist_out && !dist_dev) TK_TRY(ensure(c, c->stage_dist, out_elems * sizeof(float)));
+  int32_t* d_idx = idx_dev ? idx_out : c->stage_idx.as<int32_t>();
+  float* d_dist = dist_out ? (dist_dev ? dist_out : c->stage_dist.as<float>()) : nullptr;
+  if (splits > 1) {
+    TK_TRY(ensure(c, c->fk_partial, splits * out_elems * sizeof(uint64_t)));
+    if (!d_dist) {  // the merge writes distances unconditionally
+      TK_TRY(ensure(c, c->fk_dist, out_elems * sizeof(float)));
+    }
+  }
+  for (size_t i = c->round_ev.size(); i < 8; ++i) {
+    cudaEvent_t e;
+    TK_CUDA(c, cudaEventCreate(&e));
+    c->round_ev.push_back(e);
+  }
+  cudaEvent_t* ev = c->round_ev.data();  // round r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its kernel
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  int launches = 0;
+  TK_CUDA(c, cudaEventRecord(c->ev[0], st));
+  TK_CUDA(c, cudaEventRecord(ev[0], st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), st));
+  {
+    const unsigned blocks = (unsigned)std::min<uint64_t>((uint64_t)c->sm_count * 8, std::max<uint64_t>(1, (n * f + 255) / 256));
+    feat::finite_kernel<<<blocks, 256, 0, st>>>(d_x, n, f, x_stride_floats, sc + SC_QBAD);
+    ++launches;
+    if (!same) {
+      const unsigned qblocks = (unsigned)std::min<uint64_t>((uint64_t)c->sm_count * 8, std::max<uint64_t>(1, (nq * f + 255) / 256));
+      feat::finite_kernel<<<qblocks, 256, 0, st>>>(d_y, nq, f, y_stride_floats, sc + SC_QBAD);
+      ++launches;
+    }
+    TK_CUDA(c, cudaGetLastError());
+  }
+  feat::Params P;
+  P.x = d_x;
+  P.y = d_y;
+  P.sid = d_sid;
+  P.items = c->fk_items.as<feat::Item>();
+  P.f = f;
+  P.x_stride = x_stride_floats;
+  P.y_stride = y_stride_floats;
+  P.k = k;
+  P.squared = c->squared;
+  P.nq = (uint32_t)nq;
+  P.idx_out = d_idx;
+  P.dist_out = d_dist;
+  P.partial = splits > 1 ? c->fk_partial.as<uint64_t>() : nullptr;
+  TK_CUDA(c, cudaEventRecord(ev[2], st));
+  if (QT == 64) TK_TRY(launch_feature_knn<64>(c, P, (uint32_t)items.size()));
+  else TK_TRY(launch_feature_knn<32>(c, P, (uint32_t)items.size()));
+  ++launches;
+  TK_CUDA(c, cudaEventRecord(ev[3], st));
+  TK_CUDA(c, cudaEventRecord(ev[1], st));
+  if (splits > 1) {
+    float* m_dist = d_dist ? d_dist : c->fk_dist.as<float>();
+    const size_t smem = (size_t)k * 32 * sizeof(uint64_t);
+    TK_CUDA(c, cudaEventRecord(ev[4], st));
+    TK_CUDA(c, cudaEventRecord(ev[6], st));
+    TK_CUDA(c, cudaFuncSetAttribute(brute::merge_keys_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    brute::merge_keys_kernel<<<(unsigned)((nq + 31) / 32), 32, smem, st>>>(c->fk_partial.as<uint64_t>(), (int)splits,
+                                                                          (uint32_t)nq, k, nullptr, c->squared, d_idx, m_dist);
+    TK_CUDA(c, cudaGetLastError());
+    ++launches;
+    TK_CUDA(c, cudaEventRecord(ev[7], st));
+    TK_CUDA(c, cudaEventRecord(ev[5], st));
+  }
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
+  if (!idx_dev) TK_CUDA(c, cudaMemcpyAsync(idx_out, d_idx, out_elems * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  if (dist_out && !dist_dev) TK_CUDA(c, cudaMemcpyAsync(dist_out, d_dist, out_elems * sizeof(float), cudaMemcpyDeviceToHost, st));
+  TK_CUDA(c, cudaEventRecord(c->ev[3], st));
+  TK_CUDA(c, cudaStreamSynchronize(st));
+  c->stats.d2h_bytes = (idx_dev ? 0 : out_elems * sizeof(int32_t)) + (dist_out && !dist_dev ? out_elems * sizeof(float) : 0);
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.d2h_ms, c->ev[2], c->ev[3]));
+  c->stats.rounds = splits > 1 ? 2 : 1;
+  c->stats.round_queries[0] = nq;
+  if (splits > 1) c->stats.round_queries[1] = nq;
+  c->stats.points_tested = pairs;
+  c->stats.kernel_launches = (uint32_t)(launches + (c->mailbox_h ? 1 : 0));  // + the error-flag fetch below
+  TK_TRY(finish_round_stats(c));
+  uint32_t e[2] = {0, 0};
+  TK_TRY(fetch_words(c, sc + SC_ERROR, 2, nullptr, 0, e));
+  if (e[1]) return fail(c, TKNN_EINVAL, "%s: non-finite value in the first %d columns of x or y", what, f);
   return TKNN_OK;
 }
 

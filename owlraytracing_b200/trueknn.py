@@ -161,7 +161,8 @@ class TrueKNN:
 
     # ---- the path ----
     def build(self, points, dim: int | None = None, batch=None, batch_size: int | None = None):
-        """Build the LBVH over `points` ([n, 2|3] float32; extra columns are skipped through the stride).
+        """Build the LBVH over `points` ([n, 2|3] float32; extra columns are skipped through the stride, so columns
+        beyond the third are ignored: feature_knn() searches over all columns).
 
         batch (optional, torch_cluster's convention): one non-decreasing, non-negative integer cloud id per point, numpy
         or a CUDA tensor.  Each cloud then is searched on its own: search(), estimate_start_radius(), range_count() and
@@ -340,6 +341,46 @@ class TrueKNN:
             _check_dtype(dist, np.float32, "dist")
         if total:  # an empty torch tensor has no address, and there is nothing to sample
             self._check(self._L.tknn_fps(self._h, _ptr(soff), sizes.shape[0], self._in(start), _ptr(idx), _ptr(dist)))
+        return idx, dist
+
+    def feature_knn(self, x, y, k: int, batch_x=None, batch_y=None, self_ids=None, indices_only: bool = False):
+        """Exact k nearest rows of x for every row of y in feature space (tknn_feature_knn): all f = x.shape[1] columns
+        count, d2 = fmaf chain over the columns in order (include/trueknn.h).  Needs no build and leaves the last build
+        untouched.  batch_x / batch_y (optional, torch_cluster's convention): cloud ids of the rows; the rows of y in
+        cloud c search the rows of x in cloud c only (batch_size = max over both + 1; a missing one is all zeros).
+        self_ids (optional): per row of y, a global index into x to exclude (-1 or outside its cloud: none).  Returns
+        (idx [nq, k] int32, dist [nq, k] float32 or None when indices_only); rows ascend by (d2, index) and end in -1 /
+        FLT_MAX when the cloud has fewer eligible rows; dist is d2 while squared_dist is set.  numpy outputs for numpy
+        input, CUDA tensors (on x's device) for CUDA tensor input.  float32 only."""
+        if not _is_tensor(x):
+            x = np.ascontiguousarray(x, dtype=np.float32)
+        if not _is_tensor(y):
+            y = np.ascontiguousarray(y, dtype=np.float32)
+        _check_dtype(x, np.float32, "x")
+        _check_dtype(y, np.float32, "y")
+        if x.ndim != 2 or y.ndim != 2:
+            raise ValueError("x and y must be [rows, f]")
+        n, f, nq = int(x.shape[0]), int(x.shape[1]), int(y.shape[0])
+        if int(y.shape[1]) != f:
+            raise ValueError(f"x has {f} columns, y has {int(y.shape[1])}")
+        if self_ids is not None and not _is_tensor(self_ids):
+            self_ids = np.ascontiguousarray(self_ids, dtype=np.int32)
+        if self_ids is not None:
+            _check_dtype(self_ids, np.int32, "self_ids")
+        x_off = y_off = None
+        n_seg = 1
+        if (batch_x is not None or batch_y is not None) and n and nq:
+            bx, by, size = _bipartite_setup(x, y, batch_x, batch_y)
+            x_off, y_off = batch_to_offsets(bx, n, size), batch_to_offsets(by, nq, size)
+            n_seg = size
+        idx = self._out(y, nq, k, np.int32)
+        dist = None if indices_only else self._out(y, nq, k, np.float32)
+        if nq == 0:  # an empty torch tensor has no address, and there is nothing to search
+            return idx, dist
+        y_ptr = self._in(x) if y is x else self._in(y)
+        self._check(self._L.tknn_feature_knn(self._h, self._in(x), n, f, f, self._in(x_off), y_ptr, nq, f, self._in(y_off),
+                                             n_seg, self._in(self_ids), int(k), _ptr(idx),
+                                             _ptr(dist) if dist is not None else None))
         return idx, dist
 
     def radius_search(self, radius: float, indices_only: bool = False, out=None):
@@ -800,7 +841,9 @@ def knn_graph(x, k: int, batch=None, device: int | None = None):
     Returns edge_index [2, E] int64 (row 0 the neighbour, row 1 the centre), edges ordered by centre and then by
     (distance, index); a cloud of at most k points gives each of its points fewer than k edges.  Differences from
     torch_cluster: no `loop` option (a point is never its own neighbour) and no truncation of any kind.  numpy in, numpy
-    out; a CUDA tensor in, a tensor on its device out (device: the CUDA device for numpy input, default 0)."""
+    out; a CUDA tensor in, a tensor on its device out (device: the CUDA device for numpy input, default 0).
+    Only the first 2 or 3 columns of x are positions: columns beyond the third are ignored (they are skipped through
+    the stride).  For neighbours over all columns (feature space, DGCNN) use feature_knn_graph()."""
     dev = x.device.index if _is_tensor(x) else (device or 0)
     with TrueKNN(dev) as t:
         idx, _ = t.build(x, batch=batch).search(int(k), indices_only=True)
@@ -871,7 +914,8 @@ def knn(x, y, k: int, batch_x=None, batch_y=None, device: int | None = None):
     batch_size = max(batch_x.max(), batch_y.max()) + 1; a cloud present in only one of x and y gives no edges.  k is
     clamped to len(x); an empty x or y gives [2, 0].  A point of y is not excluded from its own neighbours: there is no
     self exclusion, as in torch_cluster.  numpy in, numpy out; a CUDA tensor in, a tensor on its device out (device:
-    the CUDA device for numpy input, default 0)."""
+    the CUDA device for numpy input, default 0).  Only the first 2 or 3 columns of x and y are positions: columns beyond
+    the third are ignored.  For neighbours over all columns (feature space) use feature_knn()."""
     if int(x.shape[0]) == 0 or int(y.shape[0]) == 0:
         return _empty_edges(x)
     batch_x, batch_y, batch_size = _bipartite_setup(x, y, batch_x, batch_y)
@@ -892,6 +936,60 @@ def knn(x, y, k: int, batch_x=None, batch_y=None, device: int | None = None):
     flat = idx.reshape(-1)
     keep = flat >= 0
     return _edge_index(flat[keep], query[keep], idx)
+
+
+def _knn_edges(idx, k: int, query_row: int):
+    """Edges of [m, k] neighbour rows (-1 slots dropped): query_row 1 gives knn_graph's [neighbour, centre] rows, 0
+    gives knn()'s [query, neighbour] rows."""
+    m = int(idx.shape[0])
+    if _is_tensor(idx):
+        import torch
+
+        query = torch.arange(m, device=idx.device).repeat_interleave(int(k))
+    else:
+        query = np.repeat(np.arange(m), int(k))
+    flat = idx.reshape(-1)
+    keep = flat >= 0
+    if query_row == 1:
+        return _edge_index(query[keep], flat[keep], idx)
+    return _edge_index(flat[keep], query[keep], idx)
+
+
+def feature_knn_graph(x, k: int, batch=None, device: int | None = None):
+    """knn_graph() in feature space: the k nearest rows of every row of x ([n, F] float32, all F columns count) inside
+    its own cloud, exact (tknn_feature_knn with self_ids = arange(n)).  Returns edge_index [2, E] int64 (row 0 the
+    neighbour, row 1 the centre), edges ordered by centre and then by (d2, index); a point is never its own neighbour
+    and a cloud of at most k points gives each of its points fewer than k edges.  numpy in, numpy out; a CUDA tensor
+    in, a tensor on its device out (device: the CUDA device for numpy input, default 0)."""
+    n = int(x.shape[0])
+    if n == 0:
+        return _empty_edges(x)
+    k = int(k)
+    dev = x.device.index if _is_tensor(x) else (device or 0)
+    if _is_tensor(x):
+        import torch
+
+        self_ids = torch.arange(n, dtype=torch.int32, device=x.device)
+    else:
+        self_ids = np.arange(n, dtype=np.int32)
+    with TrueKNN(dev) as t:
+        idx, _ = t.feature_knn(x, x, k, batch_x=batch, batch_y=batch, self_ids=self_ids, indices_only=True)
+    return _knn_edges(idx, k, 1)
+
+
+def feature_knn(x, y, k: int, batch_x=None, batch_y=None, device: int | None = None):
+    """knn() in feature space: for every row of y, the k nearest rows of x in the same cloud over all F columns, exact
+    (tknn_feature_knn).  Returns [2, E] int64 with row 0 the index into y (the query) and row 1 the index into x,
+    edges ordered by query and then by (d2, index).  Batches as knn(); k is clamped to len(x); an empty x or y gives
+    [2, 0]; no self exclusion, so DynamicEdgeConv's knn(x, x, k, b, b) is feature_knn(x, x, k, b, b).  numpy in, numpy
+    out; a CUDA tensor in, a tensor on its device out (device: the CUDA device for numpy input, default 0)."""
+    if int(x.shape[0]) == 0 or int(y.shape[0]) == 0:
+        return _empty_edges(x)
+    k = min(int(k), int(x.shape[0]))
+    dev = x.device.index if _is_tensor(x) else (device or 0)
+    with TrueKNN(dev) as t:
+        idx, _ = t.feature_knn(x, y, k, batch_x=batch_x, batch_y=batch_y, indices_only=True)
+    return _knn_edges(idx, k, 0)
 
 
 def radius(x, y, r: float, batch_x=None, batch_y=None, max_num_neighbors: int | None = None, device: int | None = None):
