@@ -334,6 +334,49 @@ TKNN_API int tknn_feature_knn(tknn_ctx* ctx, const float* x, uint64_t n, int f, 
                               const uint64_t* y_seg_offsets, uint64_t n_segments, const int32_t* self_ids, int k,
                               int32_t* idx_out, float* dist_out);
 
+/* Exact voxel-grid clustering over a batch of clouds (torch_cluster's grid_cluster, PyG's voxel_grid; DESIGN.md §3.9).
+ * points: n rows of `stride_floats` floats (host or device), the first dim (2 or 3) columns are the position.  size,
+ * start, end: HOST arrays of dim floats; start / end may be NULL (the column min / max).  Raw voxel id of a point, in
+ * fp32 with IEEE rounding and int64 arithmetic, over its columns d = 0 .. D - 1:
+ *   c = 0; m = 1;  for each d:  c += (int64) fl(fl(p_d - start_d) / size_d) * m;  m *= (int64) fl(fl(end_d - start_d) / size_d) + 1
+ * with truncation toward zero, so a point up to one voxel below start lands in cell 0, one further below gives a
+ * negative term, and one beyond end aliases into the next row: all as torch_cluster computes them.
+ * Batches (seg_offsets, n_segments + 1 entries, host or device, validated as for tknn_build_segments; NULL: one cloud,
+ * n_segments must be 1): the rule runs over [position | cloud id] (D = dim + 1) with size 1 for the id column, which
+ * starts at 0 when start is given and at the first non-empty cloud's id otherwise, and ends at the last non-empty
+ * cloud's id (PyG's voxel_grid).  A single cloud gives the ids of the position columns alone.
+ * Consecutive ids: the rank of the raw id among the distinct raw ids, ascending as int64 (torch.unique(sorted=True,
+ * return_inverse=True)).  raw_out (int64, may be NULL) and cluster_out (int32, may be NULL): n entries by point, host
+ * or device.  *n_voxels_out: the number of distinct ids (0 for n = 0).  The clustering stays in the context for
+ * tknn_voxel_members / tknn_voxel_pool until the next tknn_voxel_grid or tknn_destroy; builds and searches neither
+ * need it nor touch it, and it touches no build state.
+ * Errors (TKNN_EINVAL): dim not 2 or 3, a stride below dim, n > 2^30 - 1 (the sort's limit), n_segments >= 2^24 (ids
+ * exact in fp32), malformed offsets, a NULL points, size or n_voxels_out, a non-finite coordinate, size, start or end,
+ * a size <= 0, a per-axis cell count or a product of counts outside int64, and a raw id outside int64 at a corner of the
+ * points' bounding box (points far outside a given [start, end]; every raw id lies between those of the corners). */
+TKNN_API int tknn_voxel_grid(tknn_ctx* ctx, const float* points, uint64_t n, int dim, int stride_floats,
+                             const uint64_t* seg_offsets, uint64_t n_segments, const float* size, const float* start,
+                             const float* end, int64_t* raw_out, int32_t* cluster_out, uint64_t* n_voxels_out);
+
+/* Members of the last tknn_voxel_grid's voxels, each output may be NULL, host or device: offsets_out (n_voxels + 1)
+ * CSR offsets into members_out (n point indices, voxel by voxel, ascending index inside a voxel), first_out (n_voxels)
+ * the lowest point index of each voxel (PyG's consecutive_cluster picks an arbitrary one), seg_out (n_voxels) the cloud
+ * of each voxel.  Before any tknn_voxel_grid: TKNN_ESTATE. */
+TKNN_API int tknn_voxel_members(tknn_ctx* ctx, uint64_t* offsets_out, int32_t* members_out, int32_t* first_out,
+                                int32_t* seg_out);
+
+#define TKNN_REDUCE_MEAN 0
+#define TKNN_REDUCE_MAX 1
+/* Pools the rows x (n x f, pitch stride_floats >= f, 1 <= f <= 1024, host or device) over the last clustering into
+ * out (n_voxels x f, host or device).  n must be the clustering's point count.  Members are taken in ascending index.
+ * TKNN_REDUCE_MEAN: the members are split into chunks of 32 consecutive members, each chunk summed in order from +0.0f,
+ * the chunk sums summed in chunk order from +0.0f, and mean = sum / (float)count, all round-to-nearest (a voxel of at
+ * most 32 points is the plain sequential sum).  TKNN_REDUCE_MAX: the largest value as a float, the lowest index among
+ * equal ones (so +0 / -0 ties keep the first), and a non-finite value anywhere in x's first f columns is TKNN_EINVAL.
+ * The result depends on the inputs only.  Any number of calls per clustering.  Before any tknn_voxel_grid: TKNN_ESTATE;
+ * another n, f or stride out of range, an unknown reduce or a NULL x or out (with n_voxels > 0): TKNN_EINVAL. */
+TKNN_API int tknn_voxel_pool(tknn_ctx* ctx, const float* x, uint64_t n, int f, int stride_floats, int reduce, float* out);
+
 /* Start-radius estimator alone (replaces samples/s01-trueknn/Util/random_sample.py:5-32). */
 TKNN_API int tknn_estimate_start_radius(tknn_ctx* ctx, int k, float* radius_out);
 

@@ -93,6 +93,7 @@ class DistStats(C.Structure):
 
 
 SHARD_QUERIES, PARTITION_POINTS = 1, 2
+REDUCE_MEAN, REDUCE_MAX = 0, 1
 UNIQUE_ID_BYTES = 128
 
 # every symbol include/trueknn.h declares (tests check the library exports all of them)
@@ -108,6 +109,7 @@ EXPORTS = [
     "tknn_multi_last_error", "tknn_multi_get_times", "tknn_measure_smem_bandwidth", "tknn_key_layout", "tknn_dbscan",
     "tknn_radius_search", "tknn_radius_query", "tknn_write_neighbour_lists", "tknn_build_segments",
     "tknn_query_segments", "tknn_radius_query_segments", "tknn_fps", "tknn_feature_knn",
+    "tknn_voxel_grid", "tknn_voxel_members", "tknn_voxel_pool",
 ]
 
 _lib = None
@@ -143,6 +145,9 @@ def load() -> C.CDLL:
     L.tknn_dbscan.argtypes = [vp, f32, C.c_int, vp, vp, C.POINTER(u64)]
     L.tknn_fps.argtypes = [vp, vp, u64, vp, vp, vp]
     L.tknn_feature_knn.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, vp, u64, C.c_int, vp, u64, vp, C.c_int, vp, vp]
+    L.tknn_voxel_grid.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, vp, vp, vp, vp, vp, C.POINTER(u64)]
+    L.tknn_voxel_members.argtypes = [vp, vp, vp, vp, vp]
+    L.tknn_voxel_pool.argtypes = [vp, vp, u64, C.c_int, C.c_int, C.c_int, vp]
     L.tknn_radius_search.argtypes = [vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_radius_query.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_query_segments.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, vp, vp, C.c_int, f32, vp, vp]

@@ -86,6 +86,15 @@ struct tknn_ctx {
   // lists of a split call and the distances the merge writes when the caller asked for indices only.  It touches no
   // build state.
   DevBuf fk_x, fk_y, fk_sid, fk_items, fk_partial, fk_dist;
+  // the clustering of the last tknn_voxel_grid (grow-only, voxel.cuh): staged rows and offsets, raw and dense ids by
+  // point, the sort buffers, head words and their scan, members by sorted position, per voxel the offsets, lowest index,
+  // cloud and long-voxel chunk offsets, the list of long voxels, the box / flag / count words, and the staging of host
+  // pool rows and outputs.
+  // Builds and searches never touch it.
+  DevBuf vx_pts, vx_seg_off, vx_raw, vx_cluster, vx_keys_a, vx_keys_b, vx_vals_a, vx_vals_b, vx_sort_tmp, vx_words,
+      vx_word_off, vx_members, vx_off, vx_first, vx_seg, vx_chunks, vx_chunk_off, vx_words_sc, vx_x, vx_out, vx_cs, vx_longs;
+  bool vx_valid = false;  // a clustering exists
+  uint64_t vx_n = 0, vx_nv = 0, vx_long_chunks = 0, vx_n_long = 0;
   // cell grid over the sorted points (grid.cuh): runs per level-L cell and the table's frame; made by a plain build when
   // the cloud qualifies, and then round 1 of a dense kNN search with k <= 24 walks it instead of the LBVH
   int grid_mode = 0;        // TKNN_OPT_GRID: 0 = auto (occupancy decides), 1 = off, 2 = whenever the table is valid

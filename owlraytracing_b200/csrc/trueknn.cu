@@ -25,6 +25,7 @@
 #include "radix_sort.cuh"
 #include "radius.cuh"
 #include "traverse.cuh"
+#include "voxel.cuh"
 
 using namespace tknn;
 
@@ -914,7 +915,10 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted, &c->grid_cells, &c->grid_frame, &c->fps_segs,
                     &c->fps_slot_of_seg, &c->fps_words, &c->fps_leaf_lo, &c->fps_leaf_hi, &c->fps_leaf_first,
                     &c->fps_leaf_key, &c->fps_D, &c->fps_pos_of, &c->fps_best, &c->fk_x, &c->fk_y, &c->fk_sid,
-                    &c->fk_items, &c->fk_partial, &c->fk_dist})
+                    &c->fk_items, &c->fk_partial, &c->fk_dist, &c->vx_pts, &c->vx_seg_off, &c->vx_raw,
+                    &c->vx_cluster, &c->vx_keys_a, &c->vx_keys_b, &c->vx_vals_a, &c->vx_vals_b, &c->vx_sort_tmp, &c->vx_words,
+                    &c->vx_word_off, &c->vx_members, &c->vx_off, &c->vx_first, &c->vx_seg, &c->vx_chunks, &c->vx_chunk_off,
+                    &c->vx_words_sc, &c->vx_x, &c->vx_out, &c->vx_cs, &c->vx_longs})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -2826,6 +2830,286 @@ int tknn_measure_smem_bandwidth(tknn_ctx* c, double* conflict_free_gbs, double* 
     if (mode == 1 && broadcast_gbs) *broadcast_gbs = best;
   }
   TK_CUDA(c, cudaGetLastError());
+  return TKNN_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// voxel-grid clustering and pooling (voxel.cuh, DESIGN.md §3.9)
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+constexpr double VOXEL_I64 = 9223372036854775808.0;  // 2^63
+constexpr uint64_t VOXEL_CS_FLOATS = 1ull << 22;     // chunk results of one pooling pass (16 MB)
+
+inline float voxel_unordered(uint32_t o) { uint32_t b = (o & 0x80000000u) ? (o & 0x7fffffffu) : ~o; float v; std::memcpy(&v, &b, 4); return v; }
+
+inline bool fits_i64(__int128 v) { return v >= -(__int128)VOXEL_I64 && v < (__int128)VOXEL_I64; }
+
+// (int64) q when q lies in int64's range (truncation toward zero), else false
+inline bool voxel_trunc(float q, int64_t* t) {
+  if (!(q >= -(float)VOXEL_I64 && q < (float)VOXEL_I64)) return false;  // also NaN
+  *t = (int64_t)q;
+  return true;
+}
+
+unsigned voxel_blocks(tknn_ctx* c, uint64_t work) {
+  return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((work + voxel::THREADS - 1) / voxel::THREADS, (uint64_t)c->sm_count * 16));
+}
+
+}  // namespace
+
+extern "C" {
+
+int tknn_voxel_grid(tknn_ctx* c, const float* points, uint64_t n, int dim, int stride_floats, const uint64_t* seg_offsets,
+                    uint64_t n_segments, const float* size, const float* start, const float* end, int64_t* raw_out,
+                    int32_t* cluster_out, uint64_t* n_voxels_out) {
+  TK_TRY(check_ctx(c));
+  const char* what = "tknn_voxel_grid";
+  if (!size || !n_voxels_out || (!points && n)) return fail(c, TKNN_EINVAL, "%s: null points, size or n_voxels_out", what);
+  if (dim != 2 && dim != 3) return fail(c, TKNN_EINVAL, "%s: dim = %d (must be 2 or 3)", what, dim);
+  if (stride_floats < dim) return fail(c, TKNN_EINVAL, "%s: stride %d below dim = %d", what, stride_floats, dim);
+  if (n > rsort::MAX_N) return fail(c, TKNN_EINVAL, "%s: n = %llu exceeds %llu", what, (unsigned long long)n, (unsigned long long)rsort::MAX_N);
+  if (!seg_offsets && n_segments != 1)
+    return fail(c, TKNN_EINVAL, "%s: n_segments = %llu without offsets (must be 1)", what, (unsigned long long)n_segments);
+  if (n_segments < 1 || n_segments >= (1ull << 24))
+    return fail(c, TKNN_EINVAL, "%s: n_segments = %llu outside [1, 2^24 - 1]", what, (unsigned long long)n_segments);
+  for (int d = 0; d < dim; ++d) {
+    if (!std::isfinite(size[d]) || !(size[d] > 0.f)) return fail(c, TKNN_EINVAL, "%s: size[%d] = %g must be finite and > 0", what, d, size[d]);
+    if ((start && !std::isfinite(start[d])) || (end && !std::isfinite(end[d])))
+      return fail(c, TKNN_EINVAL, "%s: non-finite start or end in column %d", what, d);
+  }
+  ScopedDevice sd(c->device);
+  cudaStream_t st = c->stream;
+  std::vector<uint64_t> off{0, n};
+  if (seg_offsets) TK_TRY(read_offsets(c, what, "segment", seg_offsets, n_segments, n, "n", &off));
+  c->vx_valid = false;  // the previous clustering is gone whatever happens below
+  c->vx_n = c->vx_nv = c->vx_long_chunks = c->vx_n_long = 0;
+  if (n == 0) {
+    c->vx_valid = true;
+    *n_voxels_out = 0;
+    return TKNN_OK;
+  }
+  const bool batched = seg_offsets != nullptr;
+  const float* d_pts = points;
+  if (!is_device_ptr(points)) {
+    const size_t bytes = ((size_t)(n - 1) * stride_floats + dim) * sizeof(float);
+    TK_TRY(ensure(c, c->vx_pts, bytes));
+    TK_CUDA(c, cudaMemcpyAsync(c->vx_pts.p, points, bytes, cudaMemcpyHostToDevice, st));
+    d_pts = c->vx_pts.as<float>();
+  }
+  if (batched) {
+    TK_TRY(ensure(c, c->vx_seg_off, off.size() * sizeof(uint64_t)));
+    TK_CUDA(c, cudaMemcpyAsync(c->vx_seg_off.p, off.data(), off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+  }
+
+  // 1. exact column box and the non-finite flag
+  TK_TRY(ensure(c, c->vx_words_sc, 16 * sizeof(uint32_t)));
+  uint32_t* w = c->vx_words_sc.as<uint32_t>();  // [0, 4) min, [4, 8) max, 8 flag, [10, 12) long chunks (u64), 12 long voxels
+  TK_CUDA(c, cudaMemsetAsync(w, 0xff, 4 * sizeof(uint32_t), st));
+  TK_CUDA(c, cudaMemsetAsync(w + 4, 0, 12 * sizeof(uint32_t), st));
+  voxel::box_kernel<<<voxel_blocks(c, n), voxel::THREADS, 0, st>>>(d_pts, n, dim, stride_floats, w, w + 8);
+  TK_CUDA(c, cudaGetLastError());
+  uint32_t box[9];
+  TK_TRY(fetch_words(c, w, 9, nullptr, 0, box));
+  if (box[8]) return fail(c, TKNN_EINVAL, "%s: non-finite coordinate", what);
+
+  // 2. per column start / size / multiplier and the bound [lo, hi] of every raw id (the ids of the box's corners)
+  voxel::RawParams P{};
+  P.p = d_pts;
+  P.n = n;
+  P.dim = dim;
+  P.stride = stride_floats;
+  P.seg_off = batched ? c->vx_seg_off.as<uint64_t>() : nullptr;
+  P.n_seg = (uint32_t)n_segments;
+  uint64_t s_first = 0, s_last = 0;
+  if (batched) {
+    while (off[s_first + 1] == 0) ++s_first;
+    s_last = n_segments - 1;
+    while (off[s_last] == n) --s_last;
+  }
+  const int cols = dim + (batched ? 1 : 0);
+  __int128 m = 1, lo = 0, hi = 0;
+  for (int d = 0; d < cols; ++d) {
+    const bool id = d == dim;
+    const float mn = id ? (float)s_first : voxel_unordered(box[d]), mx = id ? (float)s_last : voxel_unordered(box[4 + d]);
+    const float s0 = id ? (start ? 0.f : mn) : (start ? start[d] : mn);
+    const float e0 = id ? mx : (end ? end[d] : mx);
+    const float sz = id ? 1.f : size[d];
+    int64_t cnt, tlo, thi;
+    const float span = e0 - s0;  // IEEE single: the host evaluates the formula as the device does
+    if (!voxel_trunc(span / sz, &cnt)) return fail(c, TKNN_EINVAL, "%s: the cell count of column %d overflows int64", what, d);
+    const float qlo = (mn - s0) / sz, qhi = (mx - s0) / sz;
+    if (!voxel_trunc(qlo, &tlo) || !voxel_trunc(qhi, &thi))
+      return fail(c, TKNN_EINVAL, "%s: a cell index of column %d overflows int64 (points far outside [start, end])", what, d);
+    const __int128 a = (__int128)tlo * m, b = (__int128)thi * m;
+    lo += std::min(a, b);
+    hi += std::max(a, b);
+    if (!fits_i64(a) || !fits_i64(b) || !fits_i64(lo) || !fits_i64(hi))
+      return fail(c, TKNN_EINVAL, "%s: a raw voxel id overflows int64 (points far outside [start, end])", what);
+    P.start[d] = s0;
+    P.size[d] = sz;
+    P.mult[d] = (long long)m;
+    m *= (__int128)cnt + 1;
+    if (!fits_i64(m)) return fail(c, TKNN_EINVAL, "%s: the product of the cell counts overflows int64", what);
+  }
+  P.lo = (long long)lo;
+  const uint64_t range = (uint64_t)(int64_t)hi - (uint64_t)(int64_t)lo;
+  const int bits = range ? 64 - __builtin_clzll(range) : 0;
+  const bool packed = bits + voxel::IDX_BITS <= 64;
+  const int passes = (bits + 7) / 8;
+
+  // 3. raw ids and sort keys, the sort
+  TK_TRY(ensure(c, c->vx_raw, n * sizeof(int64_t)));
+  TK_TRY(ensure(c, c->vx_keys_a, n * sizeof(uint64_t)));
+  TK_TRY(ensure(c, c->vx_keys_b, n * sizeof(uint64_t)));
+  if (!packed) {
+    TK_TRY(ensure(c, c->vx_vals_a, n * sizeof(uint32_t)));
+    TK_TRY(ensure(c, c->vx_vals_b, n * sizeof(uint32_t)));
+  }
+  TK_TRY(ensure(c, c->vx_sort_tmp, rsort::temp_words(n) * sizeof(uint32_t)));
+  P.packed = packed;
+  P.raw = c->vx_raw.as<long long>();
+  P.keys = c->vx_keys_a.as<uint64_t>();
+  P.vals = packed ? nullptr : c->vx_vals_a.as<uint32_t>();
+  voxel::raw_kernel<<<blocks_for(n, voxel::THREADS), voxel::THREADS, 0, st>>>(P);
+  TK_CUDA(c, cudaGetLastError());
+  int launches = 0;
+  bool in_b = false;
+  if (passes > 0) {
+    if (packed)
+      launches += rsort::sort_keys(c->vx_keys_a.as<uint64_t>(), c->vx_keys_b.as<uint64_t>(), n, c->vx_sort_tmp.as<uint32_t>(),
+                                   c->sm_count, st, voxel::IDX_BITS, passes, &in_b);
+    else
+      launches += rsort::sort_pairs(c->vx_keys_a.as<uint64_t>(), c->vx_vals_a.as<uint32_t>(), c->vx_keys_b.as<uint64_t>(),
+                                    c->vx_vals_b.as<uint32_t>(), n, c->vx_sort_tmp.as<uint32_t>(), c->sm_count, st, passes,
+                                    &in_b);
+    TK_CUDA(c, cudaGetLastError());
+  }
+  const uint64_t* keys = in_b ? c->vx_keys_b.as<uint64_t>() : c->vx_keys_a.as<uint64_t>();
+  const uint32_t* vals = packed ? nullptr : (in_b ? c->vx_vals_b.as<uint32_t>() : c->vx_vals_a.as<uint32_t>());
+
+  // 4. heads, their ranks, labels, long-voxel chunk layout
+  const uint64_t nw = (n + 31) / 32;
+  TK_TRY(ensure(c, c->vx_words, nw * sizeof(uint32_t)));
+  TK_TRY(ensure(c, c->vx_word_off, nw * sizeof(uint32_t)));
+  TK_TRY(ensure(c, c->vx_members, n * sizeof(uint32_t)));
+  TK_TRY(ensure(c, c->vx_cluster, n * sizeof(int32_t)));
+  TK_TRY(ensure(c, c->vx_off, (n + 1) * sizeof(uint64_t)));
+  TK_TRY(ensure(c, c->vx_first, n * sizeof(int32_t)));
+  TK_TRY(ensure(c, c->vx_seg, n * sizeof(int32_t)));
+  TK_TRY(ensure(c, c->vx_chunks, n * sizeof(uint32_t)));
+  TK_TRY(ensure(c, c->vx_chunk_off, (n + 1) * sizeof(uint64_t)));
+  TK_TRY(ensure(c, c->vx_longs, (n / (voxel::LONG_VOXEL + 1) + 1) * sizeof(uint32_t)));
+  voxel::heads_kernel<<<blocks_for(n, voxel::THREADS), voxel::THREADS, 0, st>>>(keys, n, packed ? voxel::IDX_BITS : 0,
+                                                                                 c->vx_words.as<uint32_t>());
+  TK_CUDA(c, cudaGetLastError());
+  TK_TRY(popc_scan(c, c->vx_words.as<uint32_t>(), nw, c->vx_word_off.as<uint32_t>(), &launches));  // nv -> sc[SC_TOTAL]
+  voxel::LabelParams Lp{keys, vals, n, c->vx_words.as<uint32_t>(), c->vx_word_off.as<uint32_t>(), P.seg_off, P.n_seg,
+                        c->vx_members.as<uint32_t>(), c->vx_cluster.as<int32_t>(), c->vx_off.as<uint64_t>(),
+                        c->vx_first.as<int32_t>(), c->vx_seg.as<int32_t>()};
+  voxel::label_kernel<<<blocks_for(n, voxel::THREADS), voxel::THREADS, 0, st>>>(Lp);
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  voxel::long_chunks_kernel<<<blocks_for(n, voxel::THREADS), voxel::THREADS, 0, st>>>(c->vx_off.as<uint64_t>(), sc + SC_TOTAL,
+                                                                                      n, c->vx_chunks.as<uint32_t>(),
+                                                                                      c->vx_longs.as<uint32_t>(), w + 12);
+  TK_CUDA(c, cudaGetLastError());
+  TK_TRY(scan_counts(c, c->vx_chunks.as<uint32_t>(), n, c->vx_chunk_off.as<uint64_t>(), reinterpret_cast<uint64_t*>(w + 10),
+                     &launches));
+  if (raw_out) TK_CUDA(c, cudaMemcpyAsync(raw_out, c->vx_raw.p, n * sizeof(int64_t), cudaMemcpyDefault, st));
+  if (cluster_out) TK_CUDA(c, cudaMemcpyAsync(cluster_out, c->vx_cluster.p, n * sizeof(int32_t), cudaMemcpyDefault, st));
+  uint32_t h[4];
+  TK_TRY(fetch_words(c, w + 10, 3, sc + SC_TOTAL, 1, h));  // synchronises the stream
+  c->vx_long_chunks = (uint64_t)h[0] | ((uint64_t)h[1] << 32);
+  c->vx_n_long = h[2];
+  c->vx_nv = h[3];
+  c->vx_n = n;
+  c->vx_valid = true;
+  *n_voxels_out = c->vx_nv;
+  return TKNN_OK;
+}
+
+int tknn_voxel_members(tknn_ctx* c, uint64_t* offsets_out, int32_t* members_out, int32_t* first_out, int32_t* seg_out) {
+  TK_TRY(check_ctx(c));
+  if (!c->vx_valid) return fail(c, TKNN_ESTATE, "tknn_voxel_members before tknn_voxel_grid");
+  ScopedDevice sd(c->device);
+  cudaStream_t st = c->stream;
+  const uint64_t n = c->vx_n, nv = c->vx_nv;
+  const uint64_t zero = 0;
+  if (offsets_out)
+    TK_CUDA(c, cudaMemcpyAsync(offsets_out, n ? c->vx_off.p : (const void*)&zero, (nv + 1) * sizeof(uint64_t), cudaMemcpyDefault, st));
+  if (n) {
+    if (members_out) TK_CUDA(c, cudaMemcpyAsync(members_out, c->vx_members.p, n * sizeof(int32_t), cudaMemcpyDefault, st));
+    if (first_out) TK_CUDA(c, cudaMemcpyAsync(first_out, c->vx_first.p, nv * sizeof(int32_t), cudaMemcpyDefault, st));
+    if (seg_out) TK_CUDA(c, cudaMemcpyAsync(seg_out, c->vx_seg.p, nv * sizeof(int32_t), cudaMemcpyDefault, st));
+  }
+  TK_CUDA(c, cudaStreamSynchronize(st));
+  return TKNN_OK;
+}
+
+int tknn_voxel_pool(tknn_ctx* c, const float* x, uint64_t n, int f, int stride_floats, int reduce, float* out) {
+  TK_TRY(check_ctx(c));
+  const char* what = "tknn_voxel_pool";
+  if (!c->vx_valid) return fail(c, TKNN_ESTATE, "%s before tknn_voxel_grid", what);
+  if (n != c->vx_n)
+    return fail(c, TKNN_EINVAL, "%s: n = %llu, the clustering has %llu points", what, (unsigned long long)n, (unsigned long long)c->vx_n);
+  if (f < 1 || f > 1024) return fail(c, TKNN_EINVAL, "%s: f = %d outside [1, 1024]", what, f);
+  if (stride_floats < f) return fail(c, TKNN_EINVAL, "%s: stride %d below f = %d", what, stride_floats, f);
+  if (reduce != TKNN_REDUCE_MEAN && reduce != TKNN_REDUCE_MAX) return fail(c, TKNN_EINVAL, "%s: unknown reduce %d", what, reduce);
+  const uint64_t nv = c->vx_nv;
+  if (nv == 0) return TKNN_OK;
+  if (!x || !out) return fail(c, TKNN_EINVAL, "%s: null x or out", what);
+  ScopedDevice sd(c->device);
+  cudaStream_t st = c->stream;
+  const float* d_x = x;
+  if (!is_device_ptr(x)) {
+    const size_t bytes = ((size_t)(n - 1) * stride_floats + f) * sizeof(float);
+    TK_TRY(ensure(c, c->vx_x, bytes));
+    TK_CUDA(c, cudaMemcpyAsync(c->vx_x.p, x, bytes, cudaMemcpyHostToDevice, st));
+    d_x = c->vx_x.as<float>();
+  }
+  const bool out_dev = is_device_ptr(out);
+  const size_t out_bytes = nv * (size_t)f * sizeof(float);
+  if (!out_dev) TK_TRY(ensure(c, c->vx_out, out_bytes));
+  float* d_out = out_dev ? out : c->vx_out.as<float>();
+  uint32_t* w = c->vx_words_sc.as<uint32_t>();
+  const bool mx = reduce == TKNN_REDUCE_MAX;
+  if (mx) {
+    TK_CUDA(c, cudaMemsetAsync(w + 8, 0, sizeof(uint32_t), st));
+    feat::finite_kernel<<<voxel_blocks(c, n * (uint64_t)f), 256, 0, st>>>(d_x, n, f, stride_floats, w + 8);
+    TK_CUDA(c, cudaGetLastError());
+  }
+  // columns in passes so that the chunk results of long voxels stay bounded
+  const uint64_t chunks = c->vx_long_chunks;
+  const int cb = chunks ? (int)std::min<uint64_t>((uint64_t)f, std::max<uint64_t>(1, VOXEL_CS_FLOATS / chunks)) : f;
+  if (chunks) TK_TRY(ensure(c, c->vx_cs, chunks * (uint64_t)cb * sizeof(float)));
+  voxel::PoolParams P{d_x, stride_floats, f, 0, cb, c->vx_members.as<uint32_t>(), c->vx_off.as<uint64_t>(),
+                      c->vx_chunk_off.as<uint64_t>(), nv, chunks, c->vx_cs.as<float>(), d_out};
+  for (int c0 = 0; c0 < f; c0 += cb) {
+    P.c0 = c0;
+    P.cb = std::min(cb, f - c0);
+    if (chunks) {
+      if (mx) voxel::chunk_kernel<true><<<voxel_blocks(c, chunks * P.cb), voxel::THREADS, 0, st>>>(P);
+      else voxel::chunk_kernel<false><<<voxel_blocks(c, chunks * P.cb), voxel::THREADS, 0, st>>>(P);
+    }
+    if (mx) voxel::voxel_kernel<true><<<voxel_blocks(c, nv * P.cb), voxel::THREADS, 0, st>>>(P);
+    else voxel::voxel_kernel<false><<<voxel_blocks(c, nv * P.cb), voxel::THREADS, 0, st>>>(P);
+    if (c->vx_n_long) {
+      const unsigned fb = voxel_blocks(c, c->vx_n_long * P.cb * 32);
+      if (mx) voxel::fold_kernel<true><<<fb, voxel::THREADS, 0, st>>>(P, c->vx_longs.as<uint32_t>(), c->vx_n_long);
+      else voxel::fold_kernel<false><<<fb, voxel::THREADS, 0, st>>>(P, c->vx_longs.as<uint32_t>(), c->vx_n_long);
+    }
+    TK_CUDA(c, cudaGetLastError());
+  }
+  if (!out_dev) TK_CUDA(c, cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, st));
+  if (mx) {
+    uint32_t bad = 0;
+    TK_TRY(fetch_words(c, w + 8, 1, nullptr, 0, &bad));
+    if (bad) return fail(c, TKNN_EINVAL, "%s: non-finite value in the first %d columns of x", what, f);
+  } else {
+    TK_CUDA(c, cudaStreamSynchronize(st));
+  }
   return TKNN_OK;
 }
 

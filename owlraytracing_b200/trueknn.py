@@ -383,6 +383,78 @@ class TrueKNN:
                                              _ptr(dist) if dist is not None else None))
         return idx, dist
 
+    def voxel_grid(self, points, size, start=None, end=None, batch=None, batch_size: int | None = None):
+        """Exact voxel-grid clustering of `points` ([n, >= 2] float32, the first 2 or 3 columns are the position;
+        tknn_voxel_grid).  size: a scalar or one value per axis; start / end (optional): the same, by default the column
+        min / max.  Raw id: torch_cluster's grid rule, c = sum_d (int64) fl(fl(p_d - start_d) / size_d) * m_d with m_d
+        the product of the cell counts (int64) fl(fl(end_e - start_e) / size_e) + 1 of the earlier axes, truncation
+        toward zero, evaluated in fp32 as written.  batch (optional, torch_cluster's convention) adds the cloud id as a
+        last column of size 1, as PyG's voxel_grid does; batch_size pads trailing empty clouds.  Returns (raw [n] int64,
+        cluster [n] int32: the rank of the raw id among the distinct ones, n_voxels).  numpy outputs for numpy input,
+        CUDA tensors for CUDA tensor input.  The clustering stays in the context for voxel_members() and voxel_pool()
+        until the next voxel_grid(); builds and searches do not touch it.  Unlike torch_cluster, ids that leave int64
+        are rejected (TrueKNNError, TKNN_EINVAL) instead of wrapping."""
+        points, dim, size, start, end = _voxel_args(points, size, start, end)
+        n = int(points.shape[0])
+        raw = _empty_like_rows(points, n, np.int64)
+        cluster = _empty_like_rows(points, n, np.int32)
+        self._settle_outputs(raw)
+        offsets, n_seg = None, 1
+        if batch is not None:
+            offsets = batch_to_offsets(batch, n, batch_size)
+            n_seg = int(offsets.shape[0]) - 1
+        nv = C.c_uint64()
+        self._check(self._L.tknn_voxel_grid(self._h, self._in(points) if n else None, n, dim, int(points.shape[1]),
+                                            self._in(offsets), n_seg, _ptr(size), _ptr(start), _ptr(end),
+                                            _ptr(raw) if n else None, _ptr(cluster) if n else None, C.byref(nv)))
+        self._vx_like = points
+        self._vx_n = n
+        self._vx_nv = int(nv.value)
+        return raw, cluster, self._vx_nv
+
+    def voxel_members(self):
+        """Members of the last voxel_grid()'s voxels (tknn_voxel_members): (offsets [nv + 1] CSR offsets, uint64 numpy or
+        int64 tensor; members [n] int32 point indices voxel by voxel, ascending inside a voxel; first [nv] int32 the
+        lowest point index of each voxel (PyG's consecutive_cluster returns an arbitrary member); seg [nv] int32 the
+        cloud of each voxel)."""
+        like = getattr(self, "_vx_like", None)
+        if like is None:
+            raise TrueKNNError(_lib.ESTATE, "voxel_members before voxel_grid")
+        n, nv = self._vx_n, self._vx_nv
+        offsets = _empty_like_rows(like, nv + 1, np.uint64)
+        members = _empty_like_rows(like, n, np.int32)
+        first = _empty_like_rows(like, nv, np.int32)
+        seg = _empty_like_rows(like, nv, np.int32)
+        self._settle_outputs(offsets)
+        self._check(self._L.tknn_voxel_members(self._h, _ptr(offsets), _ptr(members) if n else None,
+                                               _ptr(first) if nv else None, _ptr(seg) if nv else None))
+        return offsets, members, first, seg
+
+    def voxel_pool(self, x, reduce: str = "mean"):
+        """Pools the rows of x ([n] or [n, f] float32, 1 <= f <= 1024, n the clustering's point count) over the last
+        voxel_grid() (tknn_voxel_pool).  Returns [n_voxels, f] float32.  reduce="mean": members in ascending index in
+        chunks of 32, each chunk summed from +0 in order, the chunk sums summed in order, divided by the count, all in
+        fp32 (no atomics, so the result is the same on every run); reduce="max": the first maximum in index order, and
+        a non-finite value in x is TKNN_EINVAL.  Call it any number of times per clustering."""
+        if reduce not in ("mean", "max"):
+            raise ValueError(f"reduce must be 'mean' or 'max', got {reduce!r}")
+        if getattr(self, "_vx_like", None) is None:
+            raise TrueKNNError(_lib.ESTATE, "voxel_pool before voxel_grid")
+        if not _is_tensor(x):
+            x = np.ascontiguousarray(x, dtype=np.float32)
+        _check_dtype(x, np.float32, "x")
+        if x.ndim == 1:
+            x = x.reshape(-1, 1)
+        if x.ndim != 2:
+            raise ValueError("x must be [n] or [n, f]")
+        n, f = int(x.shape[0]), int(x.shape[1])
+        out = _empty_like_rows(x, (self._vx_nv, f), np.float32)
+        self._settle_outputs(out)
+        code = _lib.REDUCE_MAX if reduce == "max" else _lib.REDUCE_MEAN
+        self._check(self._L.tknn_voxel_pool(self._h, self._in(x) if n else None, n, f, f, code,
+                                            _ptr(out) if self._vx_nv else None))
+        return out
+
     def radius_search(self, radius: float, indices_only: bool = False, out=None):
         """Exact fixed-radius neighbour lists of every built point (closed ball, the point itself excluded).
 
@@ -824,6 +896,104 @@ def fps(src, batch=None, ratio: float = 0.5, random_start: bool = True, batch_si
 
         return idx.to(torch.int64)
     return idx.astype(np.int64)
+
+
+def _empty_like_rows(like, shape, np_dtype):
+    """An uninitialised array of `shape` beside `like`: a tensor on its device, or numpy."""
+    if _is_tensor(like):
+        import torch
+
+        dt = {np.int64: torch.int64, np.uint64: torch.int64, np.int32: torch.int32, np.float32: torch.float32}[np_dtype]
+        return torch.empty(shape, dtype=dt, device=like.device)
+    return np.empty(shape, np_dtype)
+
+
+def _voxel_args(points, size, start, end, all_columns=False):
+    """Host-side checks of voxel_grid(): (points, dim, size, start, end) with size / start / end as float32 numpy of
+    dim entries (scalars broadcast).  Raises ValueError for a shape, a non-finite value or a size <= 0.  all_columns:
+    every column of points is a coordinate (torch_cluster's and PyG's signatures), so more than 3 is an error rather
+    than columns skipped through the stride."""
+    if not _is_tensor(points):
+        points = np.ascontiguousarray(points, dtype=np.float32)
+    _check_dtype(points, np.float32, "points")
+    if points.ndim != 2 or int(points.shape[1]) < 2:
+        raise ValueError("points must be [n, >= 2] (2-D or 3-D positions)")
+    if all_columns and int(points.shape[1]) > 3:
+        raise ValueError(f"pos has {int(points.shape[1])} columns: only 2-D and 3-D positions are supported")
+    dim = min(int(points.shape[1]), 3)
+
+    def axes(v, name):
+        if v is None:
+            return None
+        if _is_tensor(v):
+            v = v.detach().cpu().numpy()
+        a = np.asarray(v, dtype=np.float32).reshape(-1)
+        if a.shape[0] == 1:
+            a = np.repeat(a, dim)
+        if a.shape[0] != dim:
+            raise ValueError(f"{name}: a scalar or {dim} values, got {a.shape[0]}")
+        if not np.isfinite(a).all():
+            raise ValueError(f"{name} must be finite")
+        return np.ascontiguousarray(a)
+
+    size = axes(size, "size")
+    if size is None or not (size > 0).all():
+        raise ValueError("size must be > 0 on every axis")
+    return points, dim, size, axes(start, "start"), axes(end, "end")
+
+
+def _device_of(a, device):
+    return a.device.index if _is_tensor(a) else (device or 0)
+
+
+def grid_cluster(pos, size, start=None, end=None, device: int | None = None):
+    """torch_cluster.grid_cluster(pos, size, start, end) on the GPU, exact: the raw voxel id of every point (int64), by
+    torch_cluster's rule in fp32 (TrueKNN.voxel_grid).  pos: [n, 2] or [n, 3] float32.  Differences from torch_cluster:
+    only 2-D and 3-D positions (more columns raise ValueError rather than give other ids), and ids that do not fit in
+    int64 (cell counts, their product, or points far outside [start, end]) raise TrueKNNError instead of overflowing
+    silently.
+    numpy in, numpy out; a CUDA tensor in, a tensor on its device out (device: the CUDA device for numpy input)."""
+    return voxel_grid(pos, size, None, start, end, device)
+
+
+def voxel_grid(pos, size, batch=None, start=None, end=None, device: int | None = None):
+    """PyG's voxel_grid(pos, size, batch, start, end) on the GPU, exact: grid_cluster over [pos | batch] with size 1 for
+    the cloud id column (which starts at 0 when start is given and ends at the largest cloud id).  Returns the raw int64
+    ids; torch.unique(raw, sorted=True, return_inverse=True)[1] is the `cluster` of grid_sampling().  Same differences
+    as grid_cluster()."""
+    _voxel_args(pos, size, start, end, all_columns=True)  # argument errors before any device is touched
+    with TrueKNN(_device_of(pos, device)) as t:
+        raw, _, _ = t.voxel_grid(pos, size, start, end, batch=batch)
+    return raw
+
+
+def grid_sampling(pos, size, x=None, batch=None, reduce: str = "mean", device: int | None = None):
+    """PyG's GridSampling(size) in one call: the voxel grid of voxel_grid(), then per voxel the mean position and x
+    pooled with `reduce` ("mean" or "max").  Returns (pos_mean [nv, D] float32, x_pooled [nv, F] float32 or None,
+    batch_out [nv] int64 or None: the cloud of each voxel, cluster [n] int64: the voxel of each point, PyG's
+    consecutive_cluster ids).  Voxels are ordered by raw id, as in PyG.  Differences from PyG: the sums run in a fixed
+    order without atomics, so every run gives the same bits; the position is always the mean (PyG pools it with
+    `reduce` too); x must be float32; the overflow cases of grid_cluster() are rejected."""
+    if reduce not in ("mean", "max"):
+        raise ValueError(f"reduce must be 'mean' or 'max', got {reduce!r}")
+    pos, _, _, _, _ = _voxel_args(pos, size, None, None, all_columns=True)
+    with TrueKNN(_device_of(pos, device)) as t:
+        _, cluster, _ = t.voxel_grid(pos, size, batch=batch)
+        pos_mean = t.voxel_pool(pos, "mean")
+        xp = t.voxel_pool(x, reduce) if x is not None else None
+        batch_out = None
+        if batch is not None:
+            _, _, _, seg = t.voxel_members()
+            batch_out = _int64(seg)
+    return pos_mean, xp, batch_out, _int64(cluster)
+
+
+def _int64(a):
+    if _is_tensor(a):
+        import torch
+
+        return a.to(torch.int64)
+    return a.astype(np.int64)
 
 
 def _edge_index(centre, neighbour, like):
