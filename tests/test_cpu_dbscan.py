@@ -28,11 +28,11 @@ def d2_matrix(x):
     return _fmaf(dz, dz, _fmaf(dy, dy, dx * dx))
 
 
-def dbscan_brute(x, eps, min_pts):
-    """The contract restated on the full d2 matrix (small clouds only)."""
+def dbscan_brute(x, eps, min_pts, d2=None):
+    """The contract restated on the full d2 matrix (small clouds only; d2: that matrix, when the caller has it)."""
     n = len(x)
     eps2 = np.float32(eps) * np.float32(eps)
-    ball = d2_matrix(x) <= eps2
+    ball = (d2_matrix(x) if d2 is None else d2) <= eps2
     core = ball.sum(1) >= min_pts
     ci = np.flatnonzero(core)
     labels = np.full(n, -1, np.int32)
