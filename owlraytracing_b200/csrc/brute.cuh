@@ -179,6 +179,15 @@ static __global__ void __launch_bounds__(256) gather_r2_kernel(const float* __re
 // global cubic grid, cell id = the top 3*bits bits of the Morton code).  A ball only touches the cells
 // between the cells of its two extreme corners — computed with the builder's own monotone quantiser, so
 // no point of the ball can lie in a cell outside that range — usually 1..8 of them.  mask bit s = rank s.
+//
+// The ball is the fp32 rule, not the real one: a point p must be reached when dist2(q, p) <= r2.  The fma chain only
+// adds non-negative terms, so RN(da * da) <= r2 on every axis; that rounding errs by 2^-24 relative, or by up to 2^-150
+// absolute where da * da is subnormal or underflows to 0, so da^2 <= r2 (1 + 2^-23) + 2^-150 and, since
+// sqrt(r2 + 2^-148) <= sqrt(r2) + 2^-74, |q - p| <= rho = fma(sqrt_ru(r2), 1.000001, 2^-74) per axis with room for the
+// rounding of the fma.  q -/+ rho rounds outward and the quantiser is monotone, so p's cell lies in [c0, c1].  Without
+// the absolute term a subnormal or zero r2 (a cloud at 1e-21 scale) misses remote points whose d2 underflows to it.
+// lim needs no such change: a box holding p is no farther from q than p on any axis, so the box's sum is the point's
+// chain up to reassociation, and its 1e-5 relative and 1e-30 absolute slack exceed that rounding, subnormal included.
 __device__ __forceinline__ uint32_t reach_mask_of(float qx, float qy, float qz, float r2, const float* __restrict__ box6,
                                                   const float* __restrict__ summ, int n_ranks, int bits, int self_rank) {
   const float lx = box6[0], ly = box6[1], lz = box6[2];
@@ -186,7 +195,7 @@ __device__ __forceinline__ uint32_t reach_mask_of(float qx, float qy, float qz, 
   const float scale = 2097152.0f / ext;  // identical to morton_kernel
   const int cells = 1 << bits, shift = 21 - bits;
   int c0[3] = {0, 0, 0}, c1[3] = {cells - 1, cells - 1, cells - 1};
-  const float rho = __fmul_rn(__fsqrt_ru(r2), 1.000001f);
+  const float rho = __fmaf_rn(__fsqrt_ru(r2), 1.000001f, 0x1p-74f);
   if (rho < 1e30f) {
     const float q[3] = {qx, qy, qz}, l[3] = {lx, ly, lz};
 #pragma unroll
