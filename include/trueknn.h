@@ -377,6 +377,46 @@ TKNN_API int tknn_voxel_members(tknn_ctx* ctx, uint64_t* offsets_out, int32_t* m
  * another n, f or stride out of range, an unknown reduce or a NULL x or out (with n_voxels > 0): TKNN_EINVAL. */
 TKNN_API int tknn_voxel_pool(tknn_ctx* ctx, const float* x, uint64_t n, int f, int stride_floats, int reduce, float* out);
 
+/* Exact k-NN interpolation (PyG's knn_interpolate: the feature propagation, or upsampling, of PointNet++; DESIGN.md
+ * §3.10).  idx / d2: the nq x k rows of tknn_query / tknn_query_segments with TKNN_OPT_SQUARED_DIST = 1 (squared
+ * distances); x: n feature rows of f columns with pitch x_stride_floats >= f.  For row i and its slots s = 0 .. k-1 in
+ * slot order, a slot with idx = -1 is skipped wherever it lies; for every other slot, in fp32 with round-to-nearest:
+ *   w[i,s]   = fl(1 / max(d2[i,s], (float)1e-16))            (a NaN d2 stays NaN, d2 = +inf gives w = 0)
+ *   den[i]   = sum_s w[i,s]                                   (from +0, in slot order)
+ *   num[i,c] = sum_s fl(x[idx[i,s], c] * w[i,s])              (each product rounded on its own, no FMA; from +0, in slot order)
+ *   out[i,c] = fl(num[i,c] / den[i])
+ * Since the slot order is PyG's edge order (rows ascending by (d2, index)), this is PyG's arithmetic on the same d2.
+ * A row without a filled slot gives 0 / 0 = NaN in every column, as in PyG; NaN in d2 or x propagates (which NaN, its
+ * sign and payload, is not part of the contract).
+ * out: nq x f, dense; weight_out (may be NULL): nq x k, w of every slot and +0 for skipped slots; den_out (may be NULL):
+ * nq entries.  These are what tknn_interpolate_backward takes.  Host or device arrays.
+ * The call needs no build and touches none: it works before tknn_build, and a search after it returns what it returned
+ * before.
+ * Errors (TKNN_EINVAL): k outside [1, TKNN_MAX_K], f < 1, a stride below f, n or nq >= 2^31, an idx entry outside {-1}
+ * and [0, n) (found on the device and reported after the call, whose outputs are then undefined), and a NULL idx, d2 or
+ * out, or a NULL x with n > 0, when nq > 0.  nq = 0 is a no-op.
+ * Statistics: n_queries, k, search_ms, d2h_ms; rounds = 1 with its round_ms / kernel_ms / round_queries (nq). */
+TKNN_API int tknn_interpolate(tknn_ctx* ctx, const int32_t* idx, const float* d2, uint64_t nq, int k, const float* x,
+                              uint64_t n, int f, int x_stride_floats, float* out, float* weight_out, float* den_out);
+
+/* Backward pass of tknn_interpolate with respect to x (PyG computes the weights without gradient, so there is none for
+ * the positions).  idx, weight and den: what tknn_interpolate took and returned for nq rows of k slots; grad_out: nq
+ * rows of f columns with pitch g_stride_floats >= f; grad_x: n x f, dense.  For data row j and column c:
+ *   grad_x[j,c] = sum over the edges e = i*k + s with idx[i,s] = j, in ascending e, from +0, of
+ *                 fl( fl(grad_out[i,c] / den[i]) * weight[i,s] )
+ * i.e. PyG's autograd chain (DivBackward, the gather of the scatter sum, MulBackward, index_add_ into zeros) evaluated
+ * sequentially in edge order.  A data row no edge references gets +0.  No float atomics: the result depends only on
+ * the inputs and is identical from call to call, on any stream and launch shape.  A data row that many queries
+ * reference is summed as one serial run (DESIGN.md §3.10 gives its cost).  Host or device arrays.
+ * Errors (TKNN_EINVAL): those of tknn_interpolate (with g_stride_floats for the stride), nq * k above 2^30 - 1 edges
+ * (the limit of the edge sort: 357 913 941 queries at k = 3), an idx entry outside {-1} and [0, n) (reported after the
+ * call), and a NULL idx, weight, den or grad_out, or a NULL grad_x with n > 0, when nq > 0.  nq = 0 fills grad_x with +0.
+ * Statistics: n_queries, k, search_ms, d2h_ms; rounds = 3 phases in round_ms: edge keys and counts, the sort, then the
+ * run offsets and the column sums; kernel_ms: the edge kernel, the whole sort, the column-sum kernel; round_queries =
+ * {nq, nq * k, n}. */
+TKNN_API int tknn_interpolate_backward(tknn_ctx* ctx, const int32_t* idx, const float* weight, const float* den, uint64_t nq,
+                                       int k, const float* grad_out, int g_stride_floats, uint64_t n, int f, float* grad_x);
+
 /* Start-radius estimator alone (replaces samples/s01-trueknn/Util/random_sample.py:5-32). */
 TKNN_API int tknn_estimate_start_radius(tknn_ctx* ctx, int k, float* radius_out);
 

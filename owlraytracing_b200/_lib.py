@@ -109,7 +109,7 @@ EXPORTS = [
     "tknn_multi_last_error", "tknn_multi_get_times", "tknn_measure_smem_bandwidth", "tknn_key_layout", "tknn_dbscan",
     "tknn_radius_search", "tknn_radius_query", "tknn_write_neighbour_lists", "tknn_build_segments",
     "tknn_query_segments", "tknn_radius_query_segments", "tknn_fps", "tknn_feature_knn",
-    "tknn_voxel_grid", "tknn_voxel_members", "tknn_voxel_pool",
+    "tknn_voxel_grid", "tknn_voxel_members", "tknn_voxel_pool", "tknn_interpolate", "tknn_interpolate_backward",
 ]
 
 _lib = None
@@ -148,6 +148,8 @@ def load() -> C.CDLL:
     L.tknn_voxel_grid.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, vp, vp, vp, vp, vp, C.POINTER(u64)]
     L.tknn_voxel_members.argtypes = [vp, vp, vp, vp, vp]
     L.tknn_voxel_pool.argtypes = [vp, vp, u64, C.c_int, C.c_int, C.c_int, vp]
+    L.tknn_interpolate.argtypes = [vp, vp, vp, u64, C.c_int, vp, u64, C.c_int, C.c_int, vp, vp, vp]
+    L.tknn_interpolate_backward.argtypes = [vp, vp, vp, vp, u64, C.c_int, vp, C.c_int, u64, C.c_int, vp]
     L.tknn_radius_search.argtypes = [vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_radius_query.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_query_segments.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, vp, vp, C.c_int, f32, vp, vp]

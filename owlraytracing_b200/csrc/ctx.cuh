@@ -95,6 +95,11 @@ struct tknn_ctx {
       vx_word_off, vx_members, vx_off, vx_first, vx_seg, vx_chunks, vx_chunk_off, vx_words_sc, vx_x, vx_out, vx_cs, vx_longs;
   bool vx_valid = false;  // a clustering exists
   uint64_t vx_n = 0, vx_nv = 0, vx_long_chunks = 0, vx_n_long = 0;
+  // tknn_interpolate / _backward scratch (grow-only unless keep_scratch == 0, interpolate.cuh): staged host inputs and
+  // outputs, and the backward's edge keys, values, sort buffers, per-row counts and run offsets.  It touches no build
+  // state.
+  DevBuf ip_idx, ip_w, ip_den, ip_x, ip_out, ip_wout, ip_dout, ip_keys_a, ip_keys_b, ip_vals_a, ip_vals_b, ip_sort_tmp,
+      ip_cnt, ip_off;
   // cell grid over the sorted points (grid.cuh): runs per level-L cell and the table's frame; made by a plain build when
   // the cloud qualifies, and then round 1 of a dense kNN search with k <= 24 walks it instead of the LBVH
   int grid_mode = 0;        // TKNN_OPT_GRID: 0 = auto (occupancy decides), 1 = off, 2 = whenever the table is valid

@@ -21,6 +21,7 @@
 #include "features.cuh"
 #include "fps.cuh"
 #include "grid.cuh"
+#include "interpolate.cuh"
 #include "lbvh.cuh"
 #include "radix_sort.cuh"
 #include "radius.cuh"
@@ -918,7 +919,9 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->fk_items, &c->fk_partial, &c->fk_dist, &c->vx_pts, &c->vx_seg_off, &c->vx_raw,
                     &c->vx_cluster, &c->vx_keys_a, &c->vx_keys_b, &c->vx_vals_a, &c->vx_vals_b, &c->vx_sort_tmp, &c->vx_words,
                     &c->vx_word_off, &c->vx_members, &c->vx_off, &c->vx_first, &c->vx_seg, &c->vx_chunks, &c->vx_chunk_off,
-                    &c->vx_words_sc, &c->vx_x, &c->vx_out, &c->vx_cs, &c->vx_longs})
+                    &c->vx_words_sc, &c->vx_x, &c->vx_out, &c->vx_cs, &c->vx_longs, &c->ip_idx, &c->ip_w, &c->ip_den,
+                    &c->ip_x, &c->ip_out, &c->ip_wout, &c->ip_dout, &c->ip_keys_a, &c->ip_keys_b, &c->ip_vals_a,
+                    &c->ip_vals_b, &c->ip_sort_tmp, &c->ip_cnt, &c->ip_off})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -3111,6 +3114,266 @@ int tknn_voxel_pool(tknn_ctx* c, const float* x, uint64_t n, int f, int stride_f
     TK_CUDA(c, cudaStreamSynchronize(st));
   }
   return TKNN_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// k-NN interpolation and its backward pass (interpolate.cuh, DESIGN.md §3.10)
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+unsigned interp_blocks(tknn_ctx* c, uint64_t threads) {
+  return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((threads + interp::THREADS - 1) / interp::THREADS,
+                                                            (uint64_t)c->sm_count * 16));
+}
+
+// a device pointer to `bytes` of the caller's input: the pointer itself, or a copy of host memory in `stage`
+int interp_in(tknn_ctx* c, const void* p, size_t bytes, DevBuf& stage, const void** d) {
+  if (is_device_ptr(p)) {
+    *d = p;
+    return TKNN_OK;
+  }
+  TK_TRY(ensure(c, stage, bytes));
+  TK_CUDA(c, cudaMemcpyAsync(stage.p, p, bytes, cudaMemcpyHostToDevice, c->stream));
+  *d = stage.p;
+  return TKNN_OK;
+}
+
+// the device buffer an output is written to: the caller's array, or `stage` (copied back by interp_out)
+int interp_out_buf(tknn_ctx* c, void* p, size_t bytes, DevBuf& stage, void** d) {
+  if (!p || is_device_ptr(p)) {
+    *d = p;
+    return TKNN_OK;
+  }
+  TK_TRY(ensure(c, stage, bytes));
+  *d = stage.p;
+  return TKNN_OK;
+}
+
+int interp_out(tknn_ctx* c, void* p, const void* d, size_t bytes) {
+  if (p && p != d) TK_CUDA(c, cudaMemcpyAsync(p, d, bytes, cudaMemcpyDeviceToHost, c->stream));
+  return TKNN_OK;
+}
+
+void interp_release(tknn_ctx* c) {
+  if (c->keep_scratch) return;
+  for (DevBuf* b : {&c->ip_idx, &c->ip_w, &c->ip_den, &c->ip_x, &c->ip_out, &c->ip_wout, &c->ip_dout, &c->ip_keys_a,
+                    &c->ip_keys_b, &c->ip_vals_a, &c->ip_vals_b, &c->ip_sort_tmp, &c->ip_cnt, &c->ip_off, &c->rl_sums})
+    release(*b);
+}
+
+int interp_events(tknn_ctx* c, size_t count) {
+  for (size_t i = c->round_ev.size(); i < count; ++i) {
+    cudaEvent_t e;
+    TK_CUDA(c, cudaEventCreate(&e));
+    c->round_ev.push_back(e);
+  }
+  return TKNN_OK;
+}
+
+int interpolate_core(tknn_ctx* c, const int32_t* idx, const float* d2, uint64_t nq, int k, const float* x, uint64_t n,
+                     int f, int x_stride, float* out, float* weight_out, float* den_out) {
+  const char* what = "tknn_interpolate";
+  cudaStream_t st = c->stream;
+  const size_t slots = (size_t)nq * k;
+  const void *d_idx, *d_d2, *d_x = nullptr;
+  TK_TRY(interp_in(c, idx, slots * sizeof(int32_t), c->ip_idx, &d_idx));
+  TK_TRY(interp_in(c, d2, slots * sizeof(float), c->ip_w, &d_d2));
+  if (n) TK_TRY(interp_in(c, x, ((size_t)(n - 1) * x_stride + f) * sizeof(float), c->ip_x, &d_x));
+  void *d_out, *d_w, *d_den;
+  TK_TRY(interp_out_buf(c, out, (size_t)nq * f * sizeof(float), c->ip_out, &d_out));
+  TK_TRY(interp_out_buf(c, weight_out, slots * sizeof(float), c->ip_wout, &d_w));
+  TK_TRY(interp_out_buf(c, den_out, nq * sizeof(float), c->ip_dout, &d_den));
+  TK_TRY(interp_events(c, 4));
+  cudaEvent_t* ev = c->round_ev.data();
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  TK_CUDA(c, cudaEventRecord(c->ev[0], st));
+  TK_CUDA(c, cudaEventRecord(ev[0], st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_QBAD, 0, sizeof(uint32_t), st));
+  interp::FwdParams P{static_cast<const int32_t*>(d_idx), static_cast<const float*>(d_d2), static_cast<const float*>(d_x),
+                      nq, (uint32_t)n, k, f, x_stride, static_cast<float*>(d_out), static_cast<float*>(d_w),
+                      static_cast<float*>(d_den), sc + SC_QBAD};
+  const int G = interp::group_of(f);
+  const unsigned blocks = interp_blocks(c, nq * (uint64_t)G);
+  TK_CUDA(c, cudaEventRecord(ev[2], st));
+  switch (G) {
+    case 4: interp::forward_kernel<4><<<blocks, interp::THREADS, 0, st>>>(P); break;
+    case 8: interp::forward_kernel<8><<<blocks, interp::THREADS, 0, st>>>(P); break;
+    case 16: interp::forward_kernel<16><<<blocks, interp::THREADS, 0, st>>>(P); break;
+    default: interp::forward_kernel<32><<<blocks, interp::THREADS, 0, st>>>(P); break;
+  }
+  TK_CUDA(c, cudaGetLastError());
+  TK_CUDA(c, cudaEventRecord(ev[3], st));
+  TK_CUDA(c, cudaEventRecord(ev[1], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
+  TK_TRY(interp_out(c, out, d_out, (size_t)nq * f * sizeof(float)));
+  TK_TRY(interp_out(c, weight_out, d_w, slots * sizeof(float)));
+  TK_TRY(interp_out(c, den_out, d_den, nq * sizeof(float)));
+  TK_CUDA(c, cudaEventRecord(c->ev[3], st));
+  uint32_t bad = 0;
+  TK_TRY(fetch_words(c, sc + SC_QBAD, 1, nullptr, 0, &bad));  // synchronises the stream
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.d2h_ms, c->ev[2], c->ev[3]));
+  c->stats.rounds = 1;
+  c->stats.round_queries[0] = nq;
+  c->stats.kernel_launches = 1 + (c->mailbox_h ? 1 : 0);
+  TK_TRY(finish_round_stats(c));
+  if (bad) return fail(c, TKNN_EINVAL, "%s: an idx entry lies outside {-1} and [0, n = %llu)", what, (unsigned long long)n);
+  return TKNN_OK;
+}
+
+int interpolate_backward_core(tknn_ctx* c, const int32_t* idx, const float* weight, const float* den, uint64_t nq, int k,
+                              const float* grad_out, int g_stride, uint64_t n, int f, float* grad_x) {
+  const char* what = "tknn_interpolate_backward";
+  cudaStream_t st = c->stream;
+  const uint64_t edges = nq * (uint64_t)k;
+  const void *d_idx, *d_w, *d_den, *d_g;
+  TK_TRY(interp_in(c, idx, edges * sizeof(int32_t), c->ip_idx, &d_idx));
+  TK_TRY(interp_in(c, weight, edges * sizeof(float), c->ip_w, &d_w));
+  TK_TRY(interp_in(c, den, nq * sizeof(float), c->ip_den, &d_den));
+  TK_TRY(interp_in(c, grad_out, ((size_t)(nq - 1) * g_stride + f) * sizeof(float), c->ip_x, &d_g));
+  void* d_gx = nullptr;
+  if (n) TK_TRY(interp_out_buf(c, grad_x, (size_t)n * f * sizeof(float), c->ip_out, &d_gx));
+  TK_TRY(ensure(c, c->ip_keys_a, edges * sizeof(uint64_t)));
+  TK_TRY(ensure(c, c->ip_keys_b, edges * sizeof(uint64_t)));
+  TK_TRY(ensure(c, c->ip_vals_a, edges * sizeof(uint32_t)));
+  TK_TRY(ensure(c, c->ip_vals_b, edges * sizeof(uint32_t)));
+  TK_TRY(ensure(c, c->ip_sort_tmp, rsort::temp_words(edges) * sizeof(uint32_t)));
+  TK_TRY(ensure(c, c->ip_cnt, n * sizeof(uint32_t)));
+  TK_TRY(ensure(c, c->ip_off, (n + 1) * sizeof(uint64_t)));
+  TK_TRY(interp_events(c, 12));
+  cudaEvent_t* ev = c->round_ev.data();  // phase r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its kernels
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  int launches = 0;
+  TK_CUDA(c, cudaEventRecord(c->ev[0], st));
+
+  // 1. edge keys and per-row counts
+  TK_CUDA(c, cudaEventRecord(ev[0], st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_QBAD, 0, sizeof(uint32_t), st));
+  if (n) TK_CUDA(c, cudaMemsetAsync(c->ip_cnt.p, 0, n * sizeof(uint32_t), st));
+  TK_CUDA(c, cudaEventRecord(ev[2], st));
+  interp::edge_kernel<<<interp_blocks(c, edges), interp::THREADS, 0, st>>>(
+      static_cast<const int32_t*>(d_idx), edges, (uint32_t)n, c->ip_keys_a.as<uint64_t>(), c->ip_vals_a.as<uint32_t>(),
+      c->ip_cnt.as<uint32_t>(), sc + SC_QBAD);
+  TK_CUDA(c, cudaGetLastError());
+  ++launches;
+  TK_CUDA(c, cudaEventRecord(ev[3], st));
+  TK_CUDA(c, cudaEventRecord(ev[1], st));
+
+  // 2. stable sort of the edges by data row: keys 0 .. n need bits(n) bits
+  const int passes = n ? (64 - __builtin_clzll(n) + 7) / 8 : 0;
+  bool in_b = false;
+  TK_CUDA(c, cudaEventRecord(ev[4], st));
+  TK_CUDA(c, cudaEventRecord(ev[6], st));
+  if (passes > 0) {
+    launches += rsort::sort_pairs(c->ip_keys_a.as<uint64_t>(), c->ip_vals_a.as<uint32_t>(), c->ip_keys_b.as<uint64_t>(),
+                                  c->ip_vals_b.as<uint32_t>(), edges, c->ip_sort_tmp.as<uint32_t>(), c->sm_count, st, passes,
+                                  &in_b);
+    TK_CUDA(c, cudaGetLastError());
+  }
+  TK_CUDA(c, cudaEventRecord(ev[7], st));
+  TK_CUDA(c, cudaEventRecord(ev[5], st));
+
+  // 3. run offsets, 4. column sums in edge order
+  TK_CUDA(c, cudaEventRecord(ev[8], st));
+  if (n) {
+    uint64_t* off = c->ip_off.as<uint64_t>();
+    TK_TRY(scan_counts(c, c->ip_cnt.as<uint32_t>(), n, off, off + n, &launches));
+    const int G = interp::group_of(f);
+    interp::BwdParams P{in_b ? c->ip_vals_b.as<uint32_t>() : c->ip_vals_a.as<uint32_t>(), off,
+                        static_cast<const float*>(d_w), static_cast<const float*>(d_den), static_cast<const float*>(d_g),
+                        (uint32_t)n, k, f, g_stride, (f + G - 1) / G, static_cast<float*>(d_gx)};
+    const unsigned blocks = interp_blocks(c, n * (uint64_t)P.blocks * G);
+    TK_CUDA(c, cudaEventRecord(ev[10], st));
+    switch (G) {
+      case 4: interp::colsum_kernel<4><<<blocks, interp::THREADS, 0, st>>>(P); break;
+      case 8: interp::colsum_kernel<8><<<blocks, interp::THREADS, 0, st>>>(P); break;
+      case 16: interp::colsum_kernel<16><<<blocks, interp::THREADS, 0, st>>>(P); break;
+      default: interp::colsum_kernel<32><<<blocks, interp::THREADS, 0, st>>>(P); break;
+    }
+    TK_CUDA(c, cudaGetLastError());
+    ++launches;
+    TK_CUDA(c, cudaEventRecord(ev[11], st));
+  } else {
+    TK_CUDA(c, cudaEventRecord(ev[10], st));
+    TK_CUDA(c, cudaEventRecord(ev[11], st));
+  }
+  TK_CUDA(c, cudaEventRecord(ev[9], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
+  if (n) TK_TRY(interp_out(c, grad_x, d_gx, (size_t)n * f * sizeof(float)));
+  TK_CUDA(c, cudaEventRecord(c->ev[3], st));
+  uint32_t bad = 0;
+  TK_TRY(fetch_words(c, sc + SC_QBAD, 1, nullptr, 0, &bad));  // synchronises the stream
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.d2h_ms, c->ev[2], c->ev[3]));
+  c->stats.rounds = 3;
+  c->stats.round_queries[0] = nq;
+  c->stats.round_queries[1] = edges;
+  c->stats.round_queries[2] = n;
+  c->stats.kernel_launches = (uint32_t)(launches + (c->mailbox_h ? 1 : 0));
+  TK_TRY(finish_round_stats(c));
+  if (bad) return fail(c, TKNN_EINVAL, "%s: an idx entry lies outside {-1} and [0, n = %llu)", what, (unsigned long long)n);
+  return TKNN_OK;
+}
+
+int interp_args(tknn_ctx* c, const char* what, uint64_t nq, int k, uint64_t n, int f, int stride, const char* stride_name) {
+  if (k < 1 || k > TKNN_MAX_K) return fail(c, TKNN_EINVAL, "%s: k = %d outside [1, %d]", what, k, TKNN_MAX_K);
+  if (f < 1) return fail(c, TKNN_EINVAL, "%s: f = %d below 1", what, f);
+  if (stride < f) return fail(c, TKNN_EINVAL, "%s: %s = %d below f = %d", what, stride_name, stride, f);
+  if (n >= (1ull << 31) || nq >= (1ull << 31)) return fail(c, TKNN_EINVAL, "%s: n and nq must be below 2^31", what);
+  return TKNN_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tknn_interpolate(tknn_ctx* c, const int32_t* idx, const float* d2, uint64_t nq, int k, const float* x, uint64_t n,
+                     int f, int x_stride_floats, float* out, float* weight_out, float* den_out) {
+  TK_TRY(check_ctx(c));
+  const char* what = "tknn_interpolate";
+  TK_TRY(interp_args(c, what, nq, k, n, f, x_stride_floats, "x_stride_floats"));
+  if (nq > 0 && (!idx || !d2 || !out || (n > 0 && !x)))
+    return fail(c, TKNN_EINVAL, "%s: null idx, d2, x or out", what);
+  ScopedDevice sd(c->device);
+  reset_search_stats(c);
+  c->stats.n_queries = nq;
+  c->stats.k = k;
+  if (nq == 0) return TKNN_OK;
+  const int rc = interpolate_core(c, idx, d2, nq, k, x, n, f, x_stride_floats, out, weight_out, den_out);
+  interp_release(c);
+  return rc;
+}
+
+int tknn_interpolate_backward(tknn_ctx* c, const int32_t* idx, const float* weight, const float* den, uint64_t nq, int k,
+                              const float* grad_out, int g_stride_floats, uint64_t n, int f, float* grad_x) {
+  TK_TRY(check_ctx(c));
+  const char* what = "tknn_interpolate_backward";
+  TK_TRY(interp_args(c, what, nq, k, n, f, g_stride_floats, "g_stride_floats"));
+  if (nq * (uint64_t)k > rsort::MAX_N)
+    return fail(c, TKNN_EINVAL, "%s: nq * k = %llu edges exceed the sort's %llu", what,
+                (unsigned long long)(nq * (uint64_t)k), (unsigned long long)rsort::MAX_N);
+  if (nq > 0 && (!idx || !weight || !den || !grad_out || (n > 0 && !grad_x)))
+    return fail(c, TKNN_EINVAL, "%s: null idx, weight, den, grad_out or grad_x", what);
+  ScopedDevice sd(c->device);
+  reset_search_stats(c);
+  c->stats.n_queries = nq;
+  c->stats.k = k;
+  if (nq == 0) {  // no edge: every row of grad_x is +0
+    if (n && grad_x) {
+      if (is_device_ptr(grad_x)) {
+        TK_CUDA(c, cudaMemsetAsync(grad_x, 0, (size_t)n * f * sizeof(float), c->stream));
+        TK_CUDA(c, cudaStreamSynchronize(c->stream));
+      } else {
+        std::memset(grad_x, 0, (size_t)n * f * sizeof(float));
+      }
+    }
+    return TKNN_OK;
+  }
+  const int rc = interpolate_backward_core(c, idx, weight, den, nq, k, grad_out, g_stride_floats, n, f, grad_x);
+  interp_release(c);
+  return rc;
 }
 
 }  // extern "C"

@@ -455,6 +455,53 @@ class TrueKNN:
                                             _ptr(out) if self._vx_nv else None))
         return out
 
+    def interpolate(self, idx, d2, x):
+        """k-NN interpolation of the rows of x ([n, f] float32) at nq query rows (tknn_interpolate): idx [nq, k] int32 and
+        d2 [nq, k] float32 are kNN rows with squared distances (query() with squared_dist=1), -1 slots skipped.  Per row,
+        w = 1 / max(d2, 1e-16), out = sum_s fl(x[idx_s] * w_s) / sum_s w_s, both sums in slot order from +0 in fp32, so
+        the result is PyG's knn_interpolate on the same neighbours, bit for bit on every run.  Returns (out [nq, f],
+        weight [nq, k] (+0 for skipped slots), den [nq]), the inputs of interpolate_backward().  Needs no build and
+        leaves the last build untouched.  numpy outputs for numpy x, CUDA tensors (on x's device) for a CUDA tensor."""
+        x = _rows_f32(x, "x")
+        idx, d2 = _rows_like(idx, np.int32, "idx"), _rows_like(d2, np.float32, "d2")
+        nq, k = int(idx.shape[0]), int(idx.shape[1])
+        if tuple(d2.shape) != (nq, k):
+            raise ValueError(f"d2 has shape {tuple(d2.shape)}, idx {(nq, k)}")
+        n, f = int(x.shape[0]), int(x.shape[1])
+        out = _empty_like_rows(x, (nq, f), np.float32)
+        weight = _empty_like_rows(x, (nq, k), np.float32)
+        den = _empty_like_rows(x, (nq,), np.float32)
+        if nq == 0:  # an empty torch tensor has no address, and there is nothing to compute
+            return out, weight, den
+        self._settle_outputs(out)
+        self._check(self._L.tknn_interpolate(self._h, self._in(idx), self._in(d2), nq, k, self._in(x) if n else None, n, f,
+                                             f, _ptr(out), _ptr(weight), _ptr(den)))
+        return out, weight, den
+
+    def interpolate_backward(self, idx, weight, den, grad_out, n: int):
+        """Gradient of interpolate()'s out with respect to x (tknn_interpolate_backward): grad_x [n, f] with
+        grad_x[j] = sum over the slots (i, s) with idx[i, s] = j, in ascending i * k + s, of fl(fl(grad_out[i] / den[i]) *
+        weight[i, s]), from +0 in fp32; +0 for a row no slot references.  No float atomics: the same bits on every run.
+        idx / weight / den: what interpolate() took and returned; grad_out: [nq, f] float32.  numpy outputs for numpy
+        grad_out, CUDA tensors for a CUDA tensor."""
+        g = _rows_f32(grad_out, "grad_out")
+        idx, weight = _rows_like(idx, np.int32, "idx"), _rows_like(weight, np.float32, "weight")
+        if not _is_tensor(den):
+            den = np.ascontiguousarray(den, dtype=np.float32)
+        _check_dtype(den, np.float32, "den")
+        nq, k, f, n = int(idx.shape[0]), int(idx.shape[1]), int(g.shape[1]), int(n)
+        if tuple(weight.shape) != (nq, k) or tuple(den.shape) != (nq,) or int(g.shape[0]) != nq:
+            raise ValueError(f"shapes idx {tuple(idx.shape)}, weight {tuple(weight.shape)}, den {tuple(den.shape)}, "
+                             f"grad_out {tuple(g.shape)} do not match")
+        grad_x = _empty_like_rows(g, (n, f), np.float32)
+        if nq == 0:  # no slot references a row
+            grad_x[:] = 0
+            return grad_x
+        self._settle_outputs(grad_x)
+        self._check(self._L.tknn_interpolate_backward(self._h, self._in(idx), self._in(weight), self._in(den), nq, k,
+                                                      self._in(g), f, n, f, _ptr(grad_x) if n else None))
+        return grad_x
+
     def radius_search(self, radius: float, indices_only: bool = False, out=None):
         """Exact fixed-radius neighbour lists of every built point (closed ball, the point itself excluded).
 
@@ -1160,6 +1207,112 @@ def feature_knn(x, y, k: int, batch_x=None, batch_y=None, device: int | None = N
     with TrueKNN(dev) as t:
         idx, _ = t.feature_knn(x, y, k, batch_x=batch_x, batch_y=batch_y, indices_only=True)
     return _knn_edges(idx, k, 0)
+
+
+def _rows_f32(a, name):
+    """A 2-D float32 array or tensor, C-contiguous (numpy float32 is not cast: a float64 x raises TypeError)."""
+    if not _is_tensor(a):
+        a = np.ascontiguousarray(a)
+    _check_dtype(a, np.float32, name)
+    if a.ndim != 2:
+        raise ValueError(f"{name} must be [rows, f]")
+    return a.contiguous() if _is_tensor(a) else a
+
+
+def _rows_like(a, np_dtype, name):
+    if not _is_tensor(a):
+        a = np.ascontiguousarray(a, dtype=np_dtype)
+    _check_dtype(a, np_dtype, name)
+    if a.ndim != 2:
+        raise ValueError(f"{name} must be [nq, k]")
+    return a.contiguous() if _is_tensor(a) else a
+
+
+def _positions(pos, name):
+    """pos as [rows, 2|3] float32: PyG's knn_interpolate measures distances over every column, so other widths raise."""
+    if not _is_tensor(pos):
+        pos = np.ascontiguousarray(pos, dtype=np.float32)
+    _check_dtype(pos, np.float32, name)
+    if pos.ndim != 2 or int(pos.shape[1]) not in (2, 3):
+        raise ValueError(f"{name} must be [n, 2] or [n, 3] (only 2-D and 3-D positions are supported), got "
+                         f"{tuple(pos.shape)}")
+    return pos
+
+
+_KnnInterpolate = None
+
+
+def _knn_interpolate_function():
+    """The torch.autograd.Function of knn_interpolate(), made on first use (importing the package needs no torch)."""
+    global _KnnInterpolate
+    if _KnnInterpolate is None:
+        import torch
+
+        class KnnInterpolate(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, x, idx, d2, t):
+                out, weight, den = t.interpolate(idx, d2, x)
+                ctx.save_for_backward(idx, weight, den)
+                ctx.n = int(x.shape[0])
+                return out
+
+            @staticmethod
+            def backward(ctx, grad_out):
+                idx, weight, den = ctx.saved_tensors
+                with TrueKNN(grad_out.device.index) as t:
+                    grad_x = t.interpolate_backward(idx, weight, den, grad_out.contiguous(), ctx.n)
+                return grad_x, None, None, None
+
+        _KnnInterpolate = KnnInterpolate
+    return _KnnInterpolate
+
+
+def knn_interpolate(x, pos_x, pos_y, batch_x=None, batch_y=None, k: int = 3, num_workers: int = 1,
+                    device: int | None = None):
+    """PyG's knn_interpolate(x, pos_x, pos_y, batch_x, batch_y, k) on the GPU, exact and deterministic: the feature
+    propagation (upsampling) step of PointNet++.  For every point of pos_y, its k nearest points of pos_x in the same
+    cloud (knn(), squared distances), then out = sum fl(x_j * w_j) / sum w_j with w_j = 1 / max(d2_j, 1e-16), each sum in
+    neighbour order from +0 in fp32 (TrueKNN.interpolate).  x: [n, f] float32 with n = len(pos_x); positions: [*, 2] or
+    [*, 3] float32 (other widths raise ValueError); batches as knn(); k is clamped to len(pos_x); num_workers is accepted
+    and ignored.  Returns [len(pos_y), f] float32; a query whose cloud has no data point gets NaN, as in PyG.
+    numpy in, numpy out (no autograd).  For a CUDA tensor x the result is differentiable with respect to x only, as in
+    PyG: the backward pass (TrueKNN.interpolate_backward) sums in edge order without atomics, so x.grad has the same bits
+    on every run; the positions get no gradient.  device: the CUDA device for numpy input (default 0)."""
+    del num_workers
+    x = _rows_f32(x, "x")
+    pos_x, pos_y = _positions(pos_x, "pos_x"), _positions(pos_y, "pos_y")
+    if int(pos_x.shape[1]) != int(pos_y.shape[1]):
+        raise ValueError(f"pos_x has {int(pos_x.shape[1])} columns, pos_y {int(pos_y.shape[1])}")
+    n, f, nq = int(x.shape[0]), int(x.shape[1]), int(pos_y.shape[0])
+    if int(pos_x.shape[0]) != n:
+        raise ValueError(f"x has {n} rows, pos_x {int(pos_x.shape[0])}")
+    if int(k) < 1:
+        raise ValueError(f"k = {k} must be >= 1")
+    tensor = _is_tensor(x)
+    if tensor:
+        import torch
+
+        if not x.is_cuda:
+            raise ValueError("x must be a CUDA tensor or a numpy array")
+        pos_x, pos_y = (torch.as_tensor(p, device=x.device) for p in (pos_x, pos_y))
+    if nq == 0:
+        return x[:0].clone() if tensor else np.zeros((0, f), np.float32)
+    if n == 0:  # PyG: no neighbour, 0 / 0
+        if tensor:
+            return x.new_full((nq, f), float("nan")) + x.sum() * 0  # still part of x's graph
+        return np.full((nq, f), np.nan, np.float32)
+    batch_x, batch_y, batch_size = _bipartite_setup(pos_x, pos_y, batch_x, batch_y)
+    k = min(int(k), n)
+    with TrueKNN(_device_of(x, device), squared_dist=1) as t:
+        if n == 1:  # a build needs two points; the feature-space search has the same d2 rule for 2 or 3 columns
+            idx, d2 = t.feature_knn(pos_x, pos_y, 1, batch_x=batch_x, batch_y=batch_y)
+        else:
+            t.build(pos_x, batch=batch_x, batch_size=batch_size)
+            idx, d2 = t.query(pos_y, k, batch=batch_y)
+        if not tensor:
+            out, _, _ = t.interpolate(idx, d2, x)
+            return out
+        return _knn_interpolate_function().apply(x, idx, d2, t)
 
 
 def radius(x, y, r: float, batch_x=None, batch_y=None, max_num_neighbors: int | None = None, device: int | None = None):
