@@ -91,7 +91,8 @@ enum {
                                   pairs, log2(n)/3 + 8 bits per axis, 24 B per point and pass (round 1's sort) */
   ,TKNN_OPT_SPARSE_DIVISOR = 9 /* rounds >= 2 with fewer than n/divisor active queries run the
                                   thread-per-query kernel (default 8; 0 = never)                  */
-  ,TKNN_OPT_GRID = 20           /* cell grid over the sorted points for round 1 of a dense kNN search with k <= 24 (same results):
+  ,TKNN_OPT_GRID = 20           /* cell grid over the sorted points for round 1 and the non-final sparse rounds of a dense kNN
+                                  search with k <= 24 (same results):
                                   0 (default) = auto: a plain build without coincident-point leaves makes the table, and uses it
                                   when no cell holds more than 64 points (uniform clouds); 1 = off (the LBVH only); 2 = whenever
                                   the table is valid, whatever its occupancy (tests, A/B)  */
@@ -139,14 +140,15 @@ typedef struct tknn_stats {
   uint64_t filter_violations;/* counting build: pairs the pre-filter rejected but the exact test accepts; must be 0 */
   uint64_t h2d_bytes, d2h_bytes; /* staging traffic of the last build / search */
   /* cell grid (TKNN_OPT_GRID) of the last build; with it, nodes_visited / warp_node_visits count the non-empty cells a
-   * round-1 group tested and warp_leaf_visits the cells it staged */
+   * round-1 group tested (a sparse round: every cell a query tested) and warp_leaf_visits the cells staged */
   int32_t grid_level;        /* 2^grid_level cells per axis; 0: no table was made                         */
   int32_t grid_selected;     /* 1: round 1 of dense kNN searches (k <= 24) walks the grid                  */
   uint32_t grid_max_cell;    /* points in the fullest cell                                                */
   uint32_t grid_split_cells; /* cells whose points were not one contiguous run of the sort (always 0)     */
   float grid_ms;             /* table build, included in build_ms                                         */
   uint32_t grid_reserved;
-  uint64_t grid_deferred;    /* counting build: round-1 groups whose cell range exceeded the cap, left to the LBVH rounds */
+  uint64_t grid_deferred;    /* counting build: round-1 groups and sparse-round queries whose cell range exceeded the cap,
+                              * left to the LBVH rounds */
 } tknn_stats;
 
 /* Replaces owlContextCreate + module/program/pipeline/SBT setup (hostCode.cpp:141-159,267-269).

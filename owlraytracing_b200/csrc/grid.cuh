@@ -332,5 +332,176 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
   }
 }
 
+// Sparse MODE_KNN round with k <= 24 on the grid: one thread per queue entry, with traverse_sparse_kernel's Params, k-list
+// layout (trav::sparse_smem: [slot][lane], sentinel slot), accept rule, emit and unresolved ballots.  The leftover queries of a
+// round are scattered, so a 32-query group shares no cells; each thread walks its own cells instead, and a cell's run is one
+// independent load where the LBVH walk is a chain of dependent node loads.  Never a final round: a query whose cell range is
+// too large (more than MAX_SPAN cells on an axis, more than TKNN_GRID_CAP cells, or a bound that is not finite) tests nothing
+// and stays unresolved, and the LBVH rounds after it finish it exactly.  The queries are built points (the all-points search),
+// so each lies in its own cell c = cell_of(q) (clamped to the top cell like the ranges): B[c] <= q <= B[c + 1].
+// Range: grid_knn_kernel's, for the thread's own bound (the same s, see there).
+// Visit order: Chebyshev rings around c (ring t = the cells whose largest |cell - c| over the axes is t), clipped to the range;
+// in a ring x, then y, then z, each cell's box term entering dist2's chain in dist2's order (x first), so the x and y partial
+// sums cull whole slabs and rows as conservatively as the cell's own distance.  A cell is staged when its box distance is
+// <= bound, like a wanted LBVH leaf.
+// Early exit.  Along an axis, gap(x) = axis_gap(q, B[x], B[x + 1]) is 0 at c and never decreases as |x - c| grows: B[] is
+// non-decreasing, so B[x] - q rises with x and q - B[x + 1] falls with x, and RN subtraction is monotone.  A cell of ring
+// t' >= t has some axis a with |x_a - c_a| = t' >= t, so its box distance fma(tz, tz, fma(ty, ty, tx * tx)) — rounded to
+// nearest and never below any one of its squared terms, all terms being >= 0 — is >= RN(gap_a(c_a +- t)^2) on the side of
+// that cell.  The smallest such term over the axes and sides that ring t reaches inside the range therefore bounds every
+// cell of ring t and beyond from below; once it exceeds the bound (which only shrinks), none of their points can pass
+// `d <= bound`, and the walk stops.
+// Counting build: counters[0] and [3] = cell box tests, [1] and [5] = staged points, [2] = inserts, [4] = cells staged,
+// [7] = queries left unresolved by the cap (every load is private to its thread: per-warp figures equal per-query ones).
+template <bool COUNT>
+static __global__ void __launch_bounds__(trav::SPARSE_THREADS, COUNT ? 1 : 8) grid_sparse_kernel(const trav::Params P, const GridParams G) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  constexpr int C = trav::SPARSE_CHUNK;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int k = P.k;
+  uint64_t* H = reinterpret_cast<uint64_t*>(smem) + 3 * 32 + (size_t)warp * (k + 1) * 32 + lane;
+  H[0] = 0;  // sentinel
+  unsigned long long c_cells = 0, c_staged = 0, c_tests = 0, c_ins = 0, c_defer = 0;
+
+  const uint64_t gi = (uint64_t)blockIdx.x * trav::SPARSE_THREADS + threadIdx.x;
+  const uint64_t n_active = P.n_active_dev ? min((uint64_t)__ldg(P.n_active_dev), P.n_active) : P.n_active;
+  const bool valid = gi < n_active;
+  uint64_t qpos = 0;
+  if (valid) qpos = P.queue ? (uint64_t)P.queue[gi] : P.q_begin + gi;
+  float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (valid) q = __ldg(&P.queries[qpos]);
+  const int row_id = __float_as_int(q.w);
+  int self = -1;
+  if (valid) self = P.self_ids ? P.self_ids[qpos] : (P.self_is_row ? row_id : -1);
+  float r2 = P.r2_dev ? __ldg(P.r2_dev) : P.r2;
+  if (valid && P.query_r2) r2 = fminf(r2, P.query_r2[qpos]);
+  float bound = r2;
+  int cnt = 0;
+
+  if (valid) {
+    const int level = G.level, sh = 21 - level;
+    const int per = (1 << level) + 1;
+    const float scale = __ldg(&G.frame[3]);
+    const float sb = sqrtf(bound);
+    int lo[3], hi[3], c[3];
+    bool defer = !(bound >= 0.0f && bound <= FLT_MAX);
+    uint32_t vol = 1;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      const float qa = a == 0 ? q.x : (a == 1 ? q.y : q.z);
+      const float org = __ldg(&G.frame[a]);
+      const uint32_t top = __ldg(reinterpret_cast<const uint32_t*>(G.frame) + 4 + a);
+      const float s = __fmaf_rn(sb, 1.0001f, __fmaf_rn(fabsf(qa), 0x1p-18f, 0x1p-74f));
+      const uint32_t l = cell_of(__fsub_rn(qa, s), org, scale, sh);
+      const uint32_t h = min(cell_of(__fadd_rn(qa, s), org, scale, sh), top);
+      const uint32_t w = h - l + 1;
+      if (w > (uint32_t)MAX_SPAN) defer = true;
+      vol *= min(w, 32u);
+      lo[a] = (int)l;
+      hi[a] = (int)h;
+      c[a] = (int)min(cell_of(qa, org, scale, sh), top);
+    }
+    if (vol > (uint32_t)TKNN_GRID_CAP) defer = true;
+
+    if (!defer) {
+      const float* Bx = G.frame + FRAME_WORDS;
+      const float* By = Bx + per;
+      const float* Bz = By + per;
+      const int rings = max(max(max(c[0] - lo[0], hi[0] - c[0]), max(c[1] - lo[1], hi[1] - c[1])),
+                            max(c[2] - lo[2], hi[2] - c[2]));
+#pragma unroll 1
+      for (int t = 0; t <= rings; ++t) {
+        if (t > 0) {  // the early exit (above): a lower bound for every cell of ring t and beyond
+          float lb = INFINITY;
+#pragma unroll
+          for (int a = 0; a < 3; ++a) {
+            const float* B = a == 0 ? Bx : (a == 1 ? By : Bz);
+            const float qa = a == 0 ? q.x : (a == 1 ? q.y : q.z);
+            if (c[a] - t >= lo[a]) {
+              const float g = axis_gap(qa, __ldg(&B[c[a] - t]), __ldg(&B[c[a] - t + 1]));
+              lb = fminf(lb, __fmul_rn(g, g));
+            }
+            if (c[a] + t <= hi[a]) {
+              const float g = axis_gap(qa, __ldg(&B[c[a] + t]), __ldg(&B[c[a] + t + 1]));
+              lb = fminf(lb, __fmul_rn(g, g));
+            }
+          }
+          if (lb > bound) break;
+        }
+        const int x1 = min(hi[0], c[0] + t), y0 = max(lo[1], c[1] - t), y1 = min(hi[1], c[1] + t);
+#pragma unroll 1
+        for (int x = max(lo[0], c[0] - t); x <= x1; ++x) {
+          const float tx = axis_gap(q.x, __ldg(&Bx[x]), __ldg(&Bx[x + 1]));
+          const float ax2 = __fmul_rn(tx, tx);
+          if (!(ax2 <= bound)) continue;
+          const bool xe = x == c[0] - t || x == c[0] + t;
+#pragma unroll 1
+          for (int y = y0; y <= y1; ++y) {
+            const float ty = axis_gap(q.y, __ldg(&By[y]), __ldg(&By[y + 1]));
+            const float ay2 = __fmaf_rn(ty, ty, ax2);
+            if (!(ay2 <= bound)) continue;
+            // on the ring's x or y faces the whole z range of the ring; inside them only its two z faces
+            const bool edge = xe || y == c[1] - t || y == c[1] + t;
+            const int zs = edge ? 1 : 2 * t;
+            const int z1 = min(hi[2], c[2] + t);
+#pragma unroll 1
+            for (int z = edge ? max(lo[2], c[2] - t) : c[2] - t; z <= z1; z += zs) {
+              if (z < lo[2]) continue;
+              const float tz = axis_gap(q.z, __ldg(&Bz[z]), __ldg(&Bz[z + 1]));
+              const float d = __fmaf_rn(tz, tz, ay2);
+              if (COUNT) c_cells += 1;
+              if (!(d <= bound)) continue;
+              const uint2 run = __ldg(&G.cells[((uint64_t)x << (2 * level)) | ((uint64_t)y << level) | (uint64_t)z]);
+              const int lcount = (int)(run.y - run.x);
+              if (lcount <= 0) continue;
+              if (COUNT) { c_staged += 1; c_tests += lcount; }
+              const float4* lp = P.pts + run.x;
+              // traverse_sparse_kernel's point loop: C independent loads in flight per step (the tail re-reads the last point)
+              for (int j = 0; j < lcount; j += C) {
+                float4 p[C];
+#pragma unroll
+                for (int u = 0; u < C; ++u) p[u] = __ldg(lp + min(j + u, lcount - 1));
+#pragma unroll
+                for (int u = 0; u < C; ++u) {
+                  const float dp = dist2(q.x, q.y, q.z, p[u].x, p[u].y, p[u].z);
+                  const int pid = __float_as_int(p[u].w);
+                  if (j + u < lcount && dp <= bound && pid != self) {
+                    const uint64_t key = make_key(dp, pid);
+                    if (cnt < k || key < trav::kl_worst(H, k, false)) {
+                      trav::kl_insert(H, cnt, k, key, false);
+                      if (cnt == k) bound = key_d2(trav::kl_worst(H, k, false));
+                      if (COUNT) c_ins += 1;
+                    }
+                  }
+                }
+              }
+            }
+          }
+        }
+      }
+    } else if (COUNT) {
+      c_defer = 1;
+    }
+  }
+
+  const bool resolved = valid && cnt == k;
+  const unsigned un = __ballot_sync(FULL_MASK, valid && !resolved);
+  if (lane == 0 && P.unresolved && (gi >> 5) < P.n_groups) P.unresolved[gi >> 5] = un;  // P.n_groups: the launch's capacity
+  if (resolved) {
+    const uint64_t row = P.row_mode == 0 ? (uint64_t)(uint32_t)row_id : (P.row_mode == 1 ? qpos - P.q_begin : gi);
+    if (P.row_mode && P.qid_out) P.qid_out[row] = row_id;
+    trav::kl_emit(H, cnt, k, false, P.squared != 0, P.idx_out + row * (uint64_t)k, P.dist_out + row * (uint64_t)k);
+  }
+  if (COUNT && P.counters) {
+    atomicAdd(&P.counters[0], c_cells);
+    atomicAdd(&P.counters[1], c_tests);
+    atomicAdd(&P.counters[2], c_ins);
+    atomicAdd(&P.counters[3], c_cells);
+    atomicAdd(&P.counters[4], c_staged);
+    atomicAdd(&P.counters[5], c_tests);
+    if (c_defer) atomicAdd(&P.counters[7], c_defer);
+  }
+}
+
 }  // namespace grid
 }  // namespace tknn

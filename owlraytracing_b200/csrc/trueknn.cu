@@ -202,6 +202,14 @@ int launch_traverse(tknn_ctx* c, const trav::Params& P) {
   return TKNN_OK;
 }
 
+grid::GridParams grid_params(const tknn_ctx* c) {
+  grid::GridParams G;
+  G.cells = c->grid_cells.as<uint2>();
+  G.frame = c->grid_frame.as<float>();
+  G.level = c->built_grid_level;
+  return G;
+}
+
 // dense kNN round (k <= 24, not final) on the cell grid of the current build (grid.cuh)
 int launch_grid(tknn_ctx* c, const trav::Params& P) {
   void (*kern)(const trav::Params, const grid::GridParams) = c->counters ? grid::grid_knn_kernel<true> : grid::grid_knn_kernel<false>;
@@ -216,12 +224,20 @@ int launch_grid(tknn_ctx* c, const trav::Params& P) {
   uint64_t grid = (uint64_t)c->sm_count * bps;
   const uint64_t need = ((uint64_t)P.n_groups + warps - 1) / warps;
   if (grid > need) grid = std::max<uint64_t>(1, need);
-  grid::GridParams G;
-  G.cells = c->grid_cells.as<uint2>();
-  G.frame = c->grid_frame.as<float>();
-  G.level = c->built_grid_level;
   TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<(unsigned)grid, warps * 32, smem, c->stream>>>(P, G);
+  kern<<<(unsigned)grid, warps * 32, smem, c->stream>>>(P, grid_params(c));
+  TK_CUDA(c, cudaGetLastError());
+  return TKNN_OK;
+}
+
+// sparse kNN round (k <= 24, not final) on the cell grid: one thread per query (grid.cuh: grid_sparse_kernel)
+int launch_grid_sparse(tknn_ctx* c, const trav::Params& P) {
+  const size_t smem = trav::sparse_smem(P.k);
+  const unsigned grid = (unsigned)((P.n_active + trav::SPARSE_THREADS - 1) / trav::SPARSE_THREADS);
+  void (*kern)(const trav::Params, const grid::GridParams) =
+      c->counters ? grid::grid_sparse_kernel<true> : grid::grid_sparse_kernel<false>;
+  TK_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<grid, trav::SPARSE_THREADS, smem, c->stream>>>(P, grid_params(c));
   TK_CUDA(c, cudaGetLastError());
   return TKNN_OK;
 }
@@ -375,13 +391,25 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
                                               active * (uint64_t)c->sparse_divisor <= n0));
     // one warp per query: small rounds; four times further for k > 24, where a private heap per THREAD is slow
     // (cfg3, 51 725 leftover queries: 3.6 ms on the thread-per-query kernel, profiles/r2_ab_opts.jsonl)
-    const bool tiny = c->warp_round_max > 0 &&
-                      active <= (uint64_t)c->warp_round_max * (job.k > trav::LIST_MAX_K ? 4u : 1u);
-    // the cell grid: round 1 only (its groups are 32 consecutive sorted queries, or a regular slice of them), never final
-    const bool on_grid = job.grid && c->grid_on && round == 0 && !last && job.k <= trav::LIST_MAX_K;
+    bool tiny = c->warp_round_max > 0 && active <= (uint64_t)c->warp_round_max * (job.k > trav::LIST_MAX_K ? 4u : 1u);
+    // the cell grid, never in a final round (a query it leaves unresolved, capped or underfilled, reaches an exact LBVH
+    // round): the dense round 1 (its groups are 32 consecutive sorted queries, or a regular slice of them) and the sparse
+    // rounds (one thread per query)
+    const bool grid_ok = job.grid && c->grid_on && !c->segmented && !last && job.k <= trav::LIST_MAX_K;
+    // A small sparse round still takes the grid when it holds more than three waves of the warp kernel's resident queries:
+    // the grid kernel's time stays near the length of one query's walk (cfg2, 3 K to 97 K leftovers: 0.15 - 0.17 ms), while
+    // the warp kernel's grows with its waves (0.08 ms at 3 K, 0.15 ms at 15 K, 0.24 ms at 30 K queries: the two cross near
+    // 17 K, about three of its waves; DESIGN.md §3.2a).
+    if (tiny && sparse && grid_ok) {
+      int bps = 0;
+      TK_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, trav::traverse_warp_kernel<false, 32>, trav::WQ_WARPS * 32,
+                                                              trav::warpq_smem(job.k)));
+      if (active > 3ull * (uint64_t)bps * trav::WQ_WARPS * (uint64_t)c->sm_count) tiny = false;
+    }
     if (tiny) TK_TRY(launch_traverse_warp(c, P));
+    else if (sparse && grid_ok) TK_TRY(launch_grid_sparse(c, P));
     else if (sparse) TK_TRY(launch_traverse_sparse_round(c, P));
-    else if (on_grid) TK_TRY(launch_grid(c, P));
+    else if (grid_ok && round == 0) TK_TRY(launch_grid(c, P));
     else TK_TRY(launch_traverse<trav::MODE_KNN>(c, P));
     if (timed) TK_CUDA(c, cudaEventRecord(c->round_ev[4 * round + 3], c->stream));
     ++launches;
