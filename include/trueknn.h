@@ -146,7 +146,8 @@ typedef struct tknn_stats {
   uint32_t grid_max_cell;    /* points in the fullest cell                                                */
   uint32_t grid_split_cells; /* cells whose points were not one contiguous run of the sort (always 0)     */
   float grid_ms;             /* table build, included in build_ms                                         */
-  uint32_t grid_reserved;
+  uint32_t grid_rounds;      /* last search: bit r set when round r (r < 32) ran a grid kernel, the dense grid_knn_kernel
+                              * (r = 0) or grid_sparse_kernel (r >= 1); ORed over the slices of a sliced search          */
   uint64_t grid_deferred;    /* counting build: round-1 groups and sparse-round queries whose cell range exceeded the cap,
                               * left to the LBVH rounds */
 } tknn_stats;

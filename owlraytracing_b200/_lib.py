@@ -64,7 +64,7 @@ class Stats(C.Structure):
         ("grid_max_cell", C.c_uint32),
         ("grid_split_cells", C.c_uint32),
         ("grid_ms", C.c_float),
-        ("grid_reserved", C.c_uint32),
+        ("grid_rounds", C.c_uint32),
         ("grid_deferred", C.c_uint64),
     ]
 

@@ -406,6 +406,8 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
                                                               trav::warpq_smem(job.k)));
       if (active > 3ull * (uint64_t)bps * trav::WQ_WARPS * (uint64_t)c->sm_count) tiny = false;
     }
+    // which rounds walked the grid (tknn_stats::grid_rounds), ORed over the slices of a sliced search
+    if (!tiny && grid_ok && (sparse || round == 0) && round < 32) c->stats.grid_rounds |= 1u << round;
     if (tiny) TK_TRY(launch_traverse_warp(c, P));
     else if (sparse && grid_ok) TK_TRY(launch_grid_sparse(c, P));
     else if (sparse) TK_TRY(launch_traverse_sparse_round(c, P));
@@ -681,6 +683,7 @@ void reset_search_stats(tknn_ctx* c) {
   s.kernel_launches = 0;
   s.nodes_visited = s.points_tested = s.heap_inserts = 0;
   s.warp_node_visits = s.warp_leaf_visits = s.warp_point_loads = s.filter_violations = 0;
+  s.grid_rounds = 0;
   s.grid_deferred = 0;
   s.d2h_bytes = 0;
   c->mailbox_launches = 0;

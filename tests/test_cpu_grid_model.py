@@ -38,13 +38,17 @@ def dist2(q, p):
 
 def key_frame(x):
     lo, hi = x.min(0), x.max(0)
-    ext = max(f32((hi - lo).max()), np.finfo(f32).tiny)
+    with np.errstate(over="ignore"):
+        ext = max(f32((hi - lo).max()), np.finfo(f32).tiny)
     return lo, hi, f32(f32(2097152.0) / ext)
 
 
 def cell(v, lo, scale, level):
-    t = ((np.asarray(v, f32) - lo).astype(f32) * scale).astype(f32)
-    return np.clip(t, f32(0), f32(2097151.0)).astype(np.uint32) >> np.uint32(21 - level)
+    """quantise21 >> (21 - level).  fmax / fmin as in CUDA: a frame of scale 0 (an extent that overflows) turns an overflowed
+    v - lo into inf * 0 = NaN, which fmaxf maps to cell 0 (np.clip would keep the NaN)."""
+    with np.errstate(over="ignore", invalid="ignore"):
+        t = ((np.asarray(v, f32) - lo).astype(f32) * scale).astype(f32)
+    return np.fmin(np.fmax(t, f32(0)), f32(2097151.0)).astype(np.uint32) >> np.uint32(21 - level)
 
 
 def _ordered(v):

@@ -3,8 +3,9 @@
 
 The clouds put the fp32 rule where it gets awkward: +inf distances (some pairs, every pair, across clusters, from a query
 outside the scene), an extent that overflows fp32 (curve-code scale 0), a normal cloud inside one curve cell beside an
-outlier, subnormal and zero d2, signed zeros, exact ties from coarse ulps.  The builder, the leaf cut, the cell grid,
-the query staging, the radius-list tiers, DBSCAN, both FPS tiers, segmented builds, feature kNN and every build option
+outlier, subnormal and zero d2, signed zeros, exact ties from coarse ulps.  The builder, the leaf cut, the cell grid's
+dense round (the grid cases route round 1 onto it and check tknn_stats::grid_rounds; test_gpu_grid_extreme.py covers both
+grid kernels on every cloud), the query staging, the radius-list tiers, DBSCAN, both FPS tiers, segmented builds, feature kNN and every build option
 run on them.  test_cpu_extreme_oracles.py checks the references themselves on the same clouds.
 """
 import os
@@ -92,8 +93,11 @@ def test_knn(name, k):
         qi, qd = squared_oracle(tree.query, E.xyz3(q), k)
     finally:
         tree.close()
-    for grid in (0, 2):  # 2: the cell grid of round 1 whenever its table is valid (k <= 24)
-        with TrueKNN(0, grid=grid) as t:
+    # grid = 2: the cell grid whenever its table is valid; warp_round_max = 0 keeps round 1 of these small clouds off the
+    # warp-per-query kernel, so that it runs on grid_knn_kernel (k <= 24)
+    for opts in ({"grid": 0}, {"grid": 2, "warp_round_max": 0}):
+        grid = opts["grid"]
+        with TrueKNN(0, **opts) as t:
             t.build(x)
             for squared in (1, 0):
                 t.set_option("squared_dist", squared)
@@ -102,6 +106,10 @@ def test_knn(name, k):
                 i, d = t.search(k)
                 same(i, ri, what + " search idx")
                 same(d, form(rd), what + " search dist")
+                if grid == 2:
+                    st = t.stats()
+                    assert st["grid_level"] > 0, what
+                    assert st["grid_rounds"] & 1 if k <= 24 else st["grid_rounds"] == 0, f"{what}: {st['grid_rounds']:#x}"
                 i, d = t.query(q, k)
                 same(i, qi, what + " query idx")
                 same(d, form(qd), what + " query dist")
@@ -367,7 +375,10 @@ OPTION_CLOUDS = {"outlier_dups": lambda: outlier_with_duplicates(20_000), "offse
 def run_all(t, x, r, knn_only=False):
     t.set_option("squared_dist", 1)
     t.build(x)
-    out = {f"search k={k}": t.search(k) for k in (10, 25)}
+    out = {}
+    for k in (10, 25):
+        out[f"search k={k}"] = t.search(k)
+        out[f"grid_rounds k={k}"] = t.stats()["grid_rounds"]
     out["grid_level"] = t.stats()["grid_level"]
     if not knn_only:
         out["radius_search"] = t.radius_search(r)
@@ -399,11 +410,13 @@ def option_refs():
 def test_build_options_change_no_result(option_refs, name, opts):
     x, r, want, default = option_refs[name]
     knn_only = "grid" in opts
-    with TrueKNN(0, **opts) as t:
+    # grid = 2 with warp_round_max = 0: round 1 of these small clouds runs on the grid instead of one warp per query
+    extra = {"warp_round_max": 0} if "grid" in opts else {}
+    with TrueKNN(0, **opts, **extra) as t:
         got = run_all(t, x, r, knn_only)
         st = t.stats()
     for op, res in got.items():
-        if op == "grid_level":
+        if op == "grid_level" or op.startswith("grid_rounds"):
             continue
         for j, (g, d, w) in enumerate(zip(res, default[op], want[op])):
             if w is None or isinstance(w, int):
@@ -415,6 +428,9 @@ def test_build_options_change_no_result(option_refs, name, opts):
         assert st["filter_violations"] == 0
     if "grid" in opts and name == "offset_1e6":
         assert got["grid_level"] > 0, "the cell grid was built"
+    if "grid" in opts:  # outlier_dups has coincident-point leaves: no table, and the LBVH alone
+        assert got["grid_rounds k=10"] & 1 if got["grid_level"] > 0 else got["grid_rounds k=10"] == 0
+        assert got["grid_rounds k=25"] == 0
 
 
 # ---------------------------------------------------------------- two ranks on one device

@@ -203,6 +203,8 @@ def test_large_k(kind, mode):
 
 # ---------------------------------------------------------------- build options
 
+# {"grid": 2} builds the cell table on every rank, but covers no grid kernel: each rank's local search of about 7 000
+# queries runs one warp per query (below warp_round_max), and test_gpu_grid_extreme.py covers the kernels themselves
 OPTIONS = [{"squared_dist": 1}, {"grid": 2}, {"tie_pruning": 0}, {"tie_pruning": 1}, {"tie_pruning": 2},
            {"leaf_size": 4}, {"leaf_policy": 1}, {"curve": 1}, {"sort_mode": 1}, {"blocks_per_sm": 1},
            {"approx_filter": 1, "counters": 1}]
