@@ -62,7 +62,9 @@ enum {
   TKNN_OPT_SQUARED_DIST = 6,  /* 1: dist_out receives d2 instead of sqrtf(d2)                      */
   TKNN_OPT_RADIUS_QUANTILE = 7 /* start-radius estimator: per-mille quantile of the sampled k-th
                                   neighbour distance (default 990)                                */
-  ,TKNN_OPT_KEEP_SCRATCH = 8   /* 1 (default): keep the build scratch buffers for the next tknn_build    */
+  ,TKNN_OPT_KEEP_SCRATCH = 8   /* 1 (default): keep the grow-only scratch of builds, queries (tknn_query*,
+                                  tknn_radius_query*), radius lists and interpolation for the next call;
+                                  0: release it when each such call returns                              */
   ,TKNN_OPT_APPROX_FILTER = 10 /* 1: conservative 3-FMA pre-filter before the exact distance test
                                   (DESIGN.md §3.2; audited, -1 % time); 0 (default): exact test on every pair */
   ,TKNN_OPT_OUTPUT_CHUNKS = 11 /* tknn_search_shard with HOST outputs: number of Morton slices whose

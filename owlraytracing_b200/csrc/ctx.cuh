@@ -6,6 +6,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <initializer_list>
 #include <string>
 #include <vector>
 
@@ -37,14 +38,15 @@ struct tknn_ctx {
   float scene_box[6] = {0, 0, 0, 0, 0, 0};
   // search scratch (grown on demand, kept across searches)
   DevBuf queue_a, queue_b, unresolved, offsets, block_sums, scalars, stage_idx, stage_dist, sample;
-  // build scratch, kept across builds (grow-only) unless keep_scratch == 0
+  // build scratch, kept across builds (grow-only) unless keep_scratch == 0 (build_scratch)
   DevBuf b_in, b_keys_a, b_keys_b, b_vals_a, b_vals_b, b_sort_tmp, b_delta, b_ballots, b_leaf_key, b_child_info,
       b_parent_leaf, b_parent_node, b_arrive;
-  // tknn_query scratch (grow-only; the reference has no analogue — it only queries its own points)
+  // tknn_query / tknn_radius_query scratch (grow-only unless keep_scratch == 0: query_scratch; the reference has no
+  // analogue — it only queries its own points)
   DevBuf q_stage, q_keys_a, q_keys_b, q_vals_a, q_vals_b, q_sort_tmp, q_pts, q_sid_stage, q_sid_sorted, q_rad_stage,
       q_r2_sorted;
   // query sets of a segmented build (tknn_query_segments / tknn_radius_query_segments): the uploaded host offsets (u64,
-  // n_segments + 1), the segment of every query row and of every sorted query position (u32)
+  // n_segments + 1), the segment of every query row and of every sorted query position (u32); query scratch as above
   DevBuf q_seg_off, q_seg_row, q_seg_sorted;
   int keep_scratch = 1;
   int sparse_divisor = 8;
@@ -67,8 +69,9 @@ struct tknn_ctx {
   DevBuf chunk_queue;
   // tknn_dbscan scratch (grow-only): union-find parents, per-root smallest original index and cluster id per position
   DevBuf db_parent, db_min_idx, db_pos_label, db_bits, db_core_stage;
-  // tknn_radius_search / _query scratch (grow-only): counts and u64 offsets by position and by row, scan block sums, the
-  // mailbox words, self positions, the unsorted rows, the long-row list and the long-row sort buffers (radius.cuh)
+  // tknn_radius_search / _query scratch (grow-only unless keep_scratch == 0: radius_list_scratch): counts and u64
+  // offsets by position and by row, scan block sums, the mailbox words, self positions, the unsorted rows, the long-row
+  // list and the long-row sort buffers (radius.cuh)
   DevBuf rl_cnt_pos, rl_cnt_row, rl_off_pos, rl_off_row, rl_sums, rl_stats, rl_pos_of, rl_self_pos, rl_keys, rl_long_pos,
       rl_long_len, rl_boff, rl_ka, rl_kb, rl_kc, rl_va, rl_vb, rl_vc, rl_row_of, rl_sort_tmp;
   // segmented build (tknn_build_segments with n_segments > 1; a later tknn_build clears it): the offsets (u64,
@@ -95,9 +98,9 @@ struct tknn_ctx {
       vx_word_off, vx_members, vx_off, vx_first, vx_seg, vx_chunks, vx_chunk_off, vx_words_sc, vx_x, vx_out, vx_cs, vx_longs;
   bool vx_valid = false;  // a clustering exists
   uint64_t vx_n = 0, vx_nv = 0, vx_long_chunks = 0, vx_n_long = 0;
-  // tknn_interpolate / _backward scratch (grow-only unless keep_scratch == 0, interpolate.cuh): staged host inputs and
-  // outputs, and the backward's edge keys, values, sort buffers, per-row counts and run offsets.  It touches no build
-  // state.
+  // tknn_interpolate / _backward scratch (grow-only unless keep_scratch == 0: interp_scratch, interpolate.cuh): staged
+  // host inputs and outputs, and the backward's edge keys, values, sort buffers, per-row counts and run offsets.  It
+  // touches no build state.
   DevBuf ip_idx, ip_w, ip_den, ip_x, ip_out, ip_wout, ip_dout, ip_keys_a, ip_keys_b, ip_vals_a, ip_vals_b, ip_sort_tmp,
       ip_cnt, ip_off;
   // cell grid over the sorted points (grid.cuh): runs per level-L cell and the table's frame; made by a plain build when
@@ -158,6 +161,115 @@ enum { SC_GROUP_COUNTER = 0, SC_TOTAL = 1, SC_ERROR = 2, SC_QBAD = 3 /* non-fini
     int rc__ = (expr);               \
     if (rc__ != TKNN_OK) return rc__; \
   } while (0)
+
+// ---- caller arrays, which may be host or device memory ----
+
+// *d = a device copy of the caller's input p[0 .. count): p itself on the device, a copy of host memory in `stage`
+// (cudaMemcpyAsync on c->stream), nullptr for a null p.  T may be const.
+template <class T> int stage_in(tknn_ctx* c, T* p, size_t count, DevBuf& stage, T** d) {
+  if (!p || is_device_ptr(p)) {
+    *d = p;
+    return TKNN_OK;
+  }
+  TK_TRY(ensure(c, stage, count * sizeof(T)));
+  TK_CUDA(c, cudaMemcpyAsync(stage.p, p, count * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+  *d = stage.as<T>();
+  return TKNN_OK;
+}
+
+// Grows `stage` as stage_in would for a host p, so that the allocation can happen before a timed region.
+template <class T> int reserve_stage(tknn_ctx* c, const T* p, size_t count, DevBuf& stage) {
+  return p && !is_device_ptr(p) ? ensure(c, stage, count * sizeof(T)) : TKNN_OK;
+}
+
+// *d = where the device writes the caller's output p[0 .. count): p itself on the device, `stage` for host memory (copied
+// back by copy_back), nullptr for a null p.
+template <class T> int out_view(tknn_ctx* c, T* p, size_t count, DevBuf& stage, T** d) {
+  if (!p || is_device_ptr(p)) {
+    *d = p;
+    return TKNN_OK;
+  }
+  TK_TRY(ensure(c, stage, count * sizeof(T)));
+  *d = stage.as<T>();
+  return TKNN_OK;
+}
+
+// Copies d[0 .. count) back to the caller's p when out_view staged it (cudaMemcpyAsync on c->stream) and adds the bytes
+// copied to *d2h if given.
+template <class T> int copy_back(tknn_ctx* c, T* p, const T* d, size_t count, uint64_t* d2h = nullptr) {
+  if (!p || p == d || count == 0) return TKNN_OK;
+  TK_CUDA(c, cudaMemcpyAsync(p, d, count * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+  if (d2h) *d2h += count * sizeof(T);
+  return TKNN_OK;
+}
+
+// host[0 .. count) = p[0 .. count): a read-back on c->stream that waits for it, or a memcpy of host memory
+template <class T> int read_to_host(tknn_ctx* c, const T* p, size_t count, T* host) {
+  if (is_device_ptr(p)) {
+    TK_CUDA(c, cudaMemcpyAsync(host, p, count * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+    TK_CUDA(c, cudaStreamSynchronize(c->stream));
+  } else {
+    std::memcpy(host, p, count * sizeof(T));
+  }
+  return TKNN_OK;
+}
+
+// p[0 .. count) = 0: a memset on c->stream that waits for it, or a memset of host memory
+template <class T> int zero_fill(tknn_ctx* c, T* p, size_t count) {
+  if (is_device_ptr(p)) {
+    TK_CUDA(c, cudaMemsetAsync(p, 0, count * sizeof(T), c->stream));
+    TK_CUDA(c, cudaStreamSynchronize(c->stream));
+  } else {
+    std::memset(p, 0, count * sizeof(T));
+  }
+  return TKNN_OK;
+}
+
+// ---- scratch ----
+
+// Releases its buffers when it leaves scope: always for buffers local to one call (no context given), else unless the
+// context keeps its scratch (TKNN_OPT_KEEP_SCRATCH).
+class ScratchScope {
+ public:
+  explicit ScratchScope(std::initializer_list<DevBuf*> bufs, const tknn_ctx* c = nullptr) : c_(c), bufs_(bufs) {}
+  ScratchScope(const ScratchScope&) = delete;
+  ScratchScope& operator=(const ScratchScope&) = delete;
+  ~ScratchScope() {
+    if (c_ && c_->keep_scratch) return;
+    for (DevBuf* b : bufs_) release(*b);
+  }
+
+ private:
+  const tknn_ctx* c_;
+  std::vector<DevBuf*> bufs_;
+};
+
+// The scratch families that TKNN_OPT_KEEP_SCRATCH = 0 releases after each call
+inline ScratchScope build_scratch(tknn_ctx* c) {
+  return ScratchScope({&c->b_in, &c->b_keys_a, &c->b_keys_b, &c->b_vals_a, &c->b_vals_b, &c->b_sort_tmp, &c->b_delta,
+                       &c->b_ballots, &c->b_leaf_key, &c->b_child_info, &c->b_parent_leaf, &c->b_parent_node, &c->b_arrive},
+                      c);
+}
+inline ScratchScope query_scratch(tknn_ctx* c) {
+  return ScratchScope({&c->q_stage, &c->q_keys_a, &c->q_keys_b, &c->q_vals_a, &c->q_vals_b, &c->q_sort_tmp, &c->q_pts,
+                       &c->q_sid_stage, &c->q_sid_sorted, &c->q_rad_stage, &c->q_r2_sorted, &c->q_seg_off, &c->q_seg_row,
+                       &c->q_seg_sorted},
+                      c);
+}
+inline ScratchScope radius_list_scratch(tknn_ctx* c) {
+  return ScratchScope({&c->rl_cnt_pos, &c->rl_cnt_row, &c->rl_off_pos, &c->rl_off_row, &c->rl_sums, &c->rl_stats,
+                       &c->rl_pos_of, &c->rl_self_pos, &c->rl_keys, &c->rl_long_pos, &c->rl_long_len, &c->rl_boff,
+                       &c->rl_ka, &c->rl_kb, &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp},
+                      c);
+}
+inline ScratchScope interp_scratch(tknn_ctx* c) {  // rl_sums: the backward's run-offset scan
+  return ScratchScope({&c->ip_idx, &c->ip_w, &c->ip_den, &c->ip_x, &c->ip_out, &c->ip_wout, &c->ip_dout, &c->ip_keys_a,
+                       &c->ip_keys_b, &c->ip_vals_a, &c->ip_vals_b, &c->ip_sort_tmp, &c->ip_cnt, &c->ip_off, &c->rl_sums},
+                      c);
+}
+
+// grows c->round_ev to at least `count` events (the per-round / per-phase timers)
+int ensure_round_events(tknn_ctx* c, size_t count);
 
 // ---- internal entry points (trueknn.cu) used by the multi-GPU drivers (dist.cu) ----
 

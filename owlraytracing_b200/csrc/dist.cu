@@ -656,14 +656,10 @@ static int build_replicated(tknn_ctx* c, const float* xyz_local, uint64_t n_loca
   S->stats.n_global = n_total;
   TK_TRY(ensure(c, S->dense_local, std::max<uint64_t>(per, 1) * 3 * sizeof(float)));
   TK_TRY(ensure(c, S->full_xyz, per * cm->n * 3 * sizeof(float)));
-  const bool dev_in = is_device_ptr(xyz_local);
-  if (!dev_in && n_local) TK_TRY(ensure(c, c->b_in, n_local * (uint64_t)stride * sizeof(float)));
+  if (n_local) TK_TRY(reserve_stage(c, xyz_local, n_local * (uint64_t)stride, c->b_in));
   TK_TRY(mark(c, S, 0));
   const float* d_local = xyz_local;
-  if (!dev_in && n_local) {
-    TK_CUDA(c, cudaMemcpyAsync(c->b_in.p, xyz_local, n_local * (uint64_t)stride * sizeof(float), cudaMemcpyHostToDevice, st));
-    d_local = c->b_in.as<float>();
-  }
+  if (n_local) TK_TRY(stage_in(c, xyz_local, n_local * (uint64_t)stride, c->b_in, &d_local));
   TK_TRY(mark(c, S, 1));
   if (n_local) {
     dense_xyz_kernel<<<blocks_for(n_local, 256), 256, 0, st>>>(d_local, dim, stride, n_local, S->dense_local.as<float>());
@@ -677,7 +673,7 @@ static int build_replicated(tknn_ctx* c, const float* xyz_local, uint64_t n_loca
   S->stats.lbvh_ms = c->stats.build_ms;
   S->stats.build_total_ms = S->stats.h2d_ms + S->stats.allgather_ms + c->stats.build_ms;
   S->stats.bytes_sent_build = per * 3 * sizeof(float) * (uint64_t)(cm->n - 1);
-  c->stats.h2d_bytes = dev_in ? 0 : n_local * (uint64_t)stride * sizeof(float);
+  c->stats.h2d_bytes = d_local == xyz_local ? 0 : n_local * (uint64_t)stride * sizeof(float);
   c->stats.h2d_ms = S->stats.h2d_ms;
   S->partition_built = false;
   return TKNN_OK;
@@ -708,8 +704,7 @@ static int partition_build(tknn_ctx* c, const float* xyz_local, uint64_t n_local
 
   // ---- allocations whose size is known up front (cudaMalloc is a synchronous host call) ----
   const uint64_t nl = std::max<uint64_t>(n_local, 1);
-  const bool dev_in = is_device_ptr(xyz_local);
-  if (!dev_in) TK_TRY(ensure(c, c->b_in, nl * (uint64_t)stride * sizeof(float)));
+  TK_TRY(reserve_stage(c, xyz_local, nl * (uint64_t)stride, c->b_in));
   TK_TRY(ensure(c, c->b_keys_a, nl * sizeof(uint64_t)));
   TK_TRY(ensure(c, c->b_keys_b, nl * sizeof(uint64_t)));
   TK_TRY(ensure(c, c->b_vals_a, nl * sizeof(uint32_t)));
@@ -725,10 +720,7 @@ static int partition_build(tknn_ctx* c, const float* xyz_local, uint64_t n_local
 
   TK_TRY(mark(c, S, 0));
   const float* d_xyz = xyz_local;
-  if (!dev_in && n_local) {
-    TK_CUDA(c, cudaMemcpyAsync(c->b_in.p, xyz_local, n_local * (uint64_t)stride * sizeof(float), cudaMemcpyHostToDevice, st));
-    d_xyz = c->b_in.as<float>();
-  }
+  if (n_local) TK_TRY(stage_in(c, xyz_local, n_local * (uint64_t)stride, c->b_in, &d_xyz));
   TK_TRY(mark(c, S, 1));
 
   // ---- global box + global point count ----
@@ -919,14 +911,12 @@ static int partition_search(tknn_ctx* c, int k, float start_radius, int32_t* gid
     if (any) return fail(c, TKNN_EINVAL, "k = %d: a rank owns no more than k points (this rank: %llu) — use fewer ranks", k,
                          (unsigned long long)m);
   }
-  const bool gid_dev = is_device_ptr(gid_out), idx_dev = is_device_ptr(idx_out), dist_dev = is_device_ptr(dist_out);
-  int32_t* d_gid = gid_out;
-  int32_t* d_idx = idx_out;
-  float* d_d2 = dist_out;
+  int32_t *d_gid = nullptr, *d_idx = nullptr;
+  float* d_d2 = nullptr;
   const size_t elems = (size_t)m * k;
-  if (!gid_dev) { TK_TRY(ensure(c, S->out_gid, m * sizeof(int32_t))); d_gid = S->out_gid.as<int32_t>(); }
-  if (!idx_dev) { TK_TRY(ensure(c, S->out_idx, elems * sizeof(int32_t))); d_idx = S->out_idx.as<int32_t>(); }
-  if (!dist_dev) { TK_TRY(ensure(c, S->out_d2, elems * sizeof(float))); d_d2 = S->out_d2.as<float>(); }
+  TK_TRY(out_view(c, gid_out, m, S->out_gid, &d_gid));
+  TK_TRY(out_view(c, idx_out, elems, S->out_idx, &d_idx));
+  TK_TRY(out_view(c, dist_out, elems, S->out_d2, &d_d2));
   TK_TRY(ensure(c, S->mask, m * sizeof(uint32_t)));
   uint32_t* d_counts = S->small.as<uint32_t>() + 2112;
   uint32_t* d_cursor = S->small.as<uint32_t>() + 2144;
@@ -1020,9 +1010,9 @@ static int partition_search(tknn_ctx* c, int k, float start_radius, int32_t* gid
   }
   TK_TRY(mark(c, S, 17));
   uint64_t d2h = 0;
-  if (!gid_dev) { TK_CUDA(c, cudaMemcpyAsync(gid_out, d_gid, m * sizeof(int32_t), cudaMemcpyDeviceToHost, st)); d2h += m * 4; }
-  if (!idx_dev) { TK_CUDA(c, cudaMemcpyAsync(idx_out, d_idx, elems * sizeof(int32_t), cudaMemcpyDeviceToHost, st)); d2h += elems * 4; }
-  if (!dist_dev) { TK_CUDA(c, cudaMemcpyAsync(dist_out, d_d2, elems * sizeof(float), cudaMemcpyDeviceToHost, st)); d2h += elems * 4; }
+  TK_TRY(copy_back(c, gid_out, d_gid, m, &d2h));
+  TK_TRY(copy_back(c, idx_out, d_idx, elems, &d2h));
+  TK_TRY(copy_back(c, dist_out, d_d2, elems, &d2h));
   TK_TRY(mark(c, S, 18));
   TK_CUDA(c, cudaStreamSynchronize(st));
   *n_out = m;

@@ -70,6 +70,15 @@ bool is_device_ptr(const void* p) {
   return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
 }
 
+int ensure_round_events(tknn_ctx* c, size_t count) {
+  while (c->round_ev.size() < count) {
+    cudaEvent_t e;
+    TK_CUDA(c, cudaEventCreate(&e));
+    c->round_ev.push_back(e);
+  }
+  return TKNN_OK;
+}
+
 }  // namespace host
 }  // namespace tknn
 
@@ -351,14 +360,6 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
     P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
     set_segments(c, P, job.seg_of);
   };
-  auto round_events = [&](int r) -> int {
-    while ((int)c->round_ev.size() < 4 * (r + 1)) {
-      cudaEvent_t a;
-      TK_CUDA(c, cudaEventCreate(&a));
-      c->round_ev.push_back(a);
-    }
-    return TKNN_OK;
-  };
   // {unresolved count, radius} in one read-back: the one host decision of a round (hostCode.cpp:310-330)
   auto read_back = [&](uint32_t* count) -> int {
     struct { uint32_t total; float r; } h = {0, 0.f};
@@ -379,7 +380,7 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
     if (!radius_known) P.r2_dev = job.r_dev + 1;
     const bool timed = job.record_stats && round < TKNN_MAX_ROUNDS;
     if (timed) {
-      TK_TRY(round_events(round));
+      TK_TRY(ensure_round_events(c, 4 * (round + 1)));
       TK_CUDA(c, cudaEventRecord(c->round_ev[4 * round], c->stream));
       c->stats.round_queries[round] = active;
     }
@@ -436,7 +437,7 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
         F.n_active_dev = sc + SC_TOTAL;
         const bool timed2 = job.record_stats && round + 1 < TKNN_MAX_ROUNDS;
         if (timed2) {
-          TK_TRY(round_events(round + 1));
+          TK_TRY(ensure_round_events(c, 4 * (round + 2)));
           TK_CUDA(c, cudaEventRecord(c->round_ev[4 * (round + 1)], c->stream));
           TK_CUDA(c, cudaEventRecord(c->round_ev[4 * (round + 1) + 2], c->stream));
         }
@@ -603,6 +604,22 @@ int hilbert_levels(uint64_t n, int bits, int forced = 0) {
 }
 
 int check_ctx(tknn_ctx* c) { return c ? TKNN_OK : TKNN_EINVAL; }
+
+// Reads n_segments + 1 offsets (host or device: one small read-back) into *off and checks that they start at 0, never
+// decrease and end at `total` (named `total_name` in the message; a null total_name: they may end anywhere); `side`
+// names the offsets in the message.
+int read_offsets(tknn_ctx* c, const char* what, const char* side, const uint64_t* offsets, uint64_t n_segments,
+                 uint64_t total, const char* total_name, std::vector<uint64_t>* off_out) {
+  std::vector<uint64_t>& off = *off_out;
+  off.assign(n_segments + 1, 0);
+  TK_TRY(read_to_host(c, offsets, off.size(), off.data()));
+  if (off[0] != 0) return fail(c, TKNN_EINVAL, "%s: %s offsets must start at 0", what, side);
+  if (total_name && off[n_segments] != total)
+    return fail(c, TKNN_EINVAL, "%s: %s offsets must end at %s = %llu", what, side, total_name, (unsigned long long)total);
+  for (uint64_t s = 0; s < n_segments; ++s)
+    if (off[s + 1] < off[s]) return fail(c, TKNN_EINVAL, "%s: %s offsets decrease at segment %llu", what, side, (unsigned long long)s);
+  return TKNN_OK;
+}
 
 // the calls that do not restrict their neighbours to a segment yet refuse a segmented build rather than ignore it
 int refuse_segmented(tknn_ctx* c, const char* what) {
@@ -1063,20 +1080,10 @@ int tknn_build_segments(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int 
   if (n_segments < 1 || n_segments > (uint64_t)INT32_MAX)
     return fail(c, TKNN_EINVAL, "n_segments = %llu outside [1, 2^31 - 1]", (unsigned long long)n_segments);
   ScopedDevice sd(c->device);
-  std::vector<uint64_t> off(n_segments + 1);
-  if (is_device_ptr(seg_offsets)) {
-    TK_CUDA(c, cudaMemcpyAsync(off.data(), seg_offsets, off.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
-    TK_CUDA(c, cudaStreamSynchronize(c->stream));
-  } else {
-    std::memcpy(off.data(), seg_offsets, off.size() * sizeof(uint64_t));
-  }
-  if (off[0] != 0) return fail(c, TKNN_EINVAL, "segment offsets must start at 0");
-  if (off[n_segments] != n) return fail(c, TKNN_EINVAL, "segment offsets must end at n = %llu", (unsigned long long)n);
+  std::vector<uint64_t> off;
+  TK_TRY(read_offsets(c, "tknn_build_segments", "segment", seg_offsets, n_segments, n, "n", &off));
   uint64_t max_segment = 0;
-  for (uint64_t s = 0; s < n_segments; ++s) {
-    if (off[s + 1] < off[s]) return fail(c, TKNN_EINVAL, "segment offsets decrease at segment %llu", (unsigned long long)s);
-    max_segment = std::max(max_segment, off[s + 1] - off[s]);
-  }
+  for (uint64_t s = 0; s < n_segments; ++s) max_segment = std::max(max_segment, off[s + 1] - off[s]);
   if (n_segments == 1) return tknn_build(c, xyz, n, dim, stride_floats);  // one segment: an ordinary build
   tknn_internal_dist_invalidate(c);
   c->n = 0;  // the offsets of the previous build are overwritten: it is gone whatever happens below
@@ -1151,63 +1158,48 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
   int launches = 0;
 
   // ---- stage the input ----
-  DevBuf &in_stage = c->b_in, &keys_a = c->b_keys_a, &keys_b = c->b_keys_b, &vals_a = c->b_vals_a, &vals_b = c->b_vals_b,
-         &sort_tmp = c->b_sort_tmp, &delta = c->b_delta, &ballots = c->b_ballots, &leaf_key = c->b_leaf_key,
-         &child_info = c->b_child_info, &parent_leaf = c->b_parent_leaf, &parent_node = c->b_parent_node, &arrive = c->b_arrive;
-  auto cleanup = [&]() {
-    if (c->keep_scratch) return;
-    for (DevBuf* b : {&in_stage, &keys_a, &keys_b, &vals_a, &vals_b, &sort_tmp, &delta, &ballots, &leaf_key, &child_info,
-                      &parent_leaf, &parent_node, &arrive})
-      release(*b);
-  };
+  DevBuf &keys_a = c->b_keys_a, &keys_b = c->b_keys_b, &vals_a = c->b_vals_a, &vals_b = c->b_vals_b,
+         &sort_tmp = c->b_sort_tmp, &ballots = c->b_ballots, &leaf_key = c->b_leaf_key, &child_info = c->b_child_info,
+         &parent_leaf = c->b_parent_leaf, &parent_node = c->b_parent_node, &arrive = c->b_arrive;
+  ScratchScope scratch = build_scratch(c);
   // size-only allocations happen before the timed region (cudaMalloc is a synchronous host call)
   {
     const uint64_t nw0 = (n + 31) / 32;
-    int rc0 = TKNN_OK;
-    if (!is_device_ptr(xyz)) rc0 = ensure(c, in_stage, (size_t)n * stride_floats * sizeof(float));
-    if (rc0 == TKNN_OK) rc0 = ensure(c, keys_a, n * sizeof(uint64_t));
-    if (rc0 == TKNN_OK) rc0 = ensure(c, keys_b, n * sizeof(uint64_t));
-    if (rc0 == TKNN_OK) rc0 = ensure(c, vals_a, n * sizeof(uint32_t));
-    if (rc0 == TKNN_OK) rc0 = ensure(c, vals_b, n * sizeof(uint32_t));
-    if (rc0 == TKNN_OK) rc0 = ensure(c, sort_tmp, rsort::temp_words(n) * sizeof(uint32_t));
-    if (rc0 == TKNN_OK) rc0 = ensure(c, ballots, nw0 * sizeof(uint32_t));
-    if (rc0 == TKNN_OK) rc0 = ensure(c, c->offsets, (nw0 + 1) * sizeof(uint32_t));
-    if (rc0 == TKNN_OK) rc0 = ensure(c, c->block_sums, sizeof(uint32_t) * (size_t)(nw0 / lbvh::SCAN_CHUNK + 2));
-    if (rc0 == TKNN_OK) rc0 = ensure(c, c->pts, n * sizeof(float4));
-    if (rc0 == TKNN_OK && seg) rc0 = ensure(c, c->seg_of, n * sizeof(uint32_t));
-    if (rc0 != TKNN_OK) { cleanup(); return rc0; }
+    TK_TRY(reserve_stage(c, xyz, (size_t)n * stride_floats, c->b_in));
+    TK_TRY(ensure(c, keys_a, n * sizeof(uint64_t)));
+    TK_TRY(ensure(c, keys_b, n * sizeof(uint64_t)));
+    TK_TRY(ensure(c, vals_a, n * sizeof(uint32_t)));
+    TK_TRY(ensure(c, vals_b, n * sizeof(uint32_t)));
+    TK_TRY(ensure(c, sort_tmp, rsort::temp_words(n) * sizeof(uint32_t)));
+    TK_TRY(ensure(c, ballots, nw0 * sizeof(uint32_t)));
+    TK_TRY(ensure(c, c->offsets, (nw0 + 1) * sizeof(uint32_t)));
+    TK_TRY(ensure(c, c->block_sums, sizeof(uint32_t) * (size_t)(nw0 / lbvh::SCAN_CHUNK + 2)));
+    TK_TRY(ensure(c, c->pts, n * sizeof(float4)));
+    if (seg) TK_TRY(ensure(c, c->seg_of, n * sizeof(uint32_t)));
   }
-#define TK_B(expr) do { int rc_ = (expr); if (rc_ != TKNN_OK) { cleanup(); return rc_; } } while (0)
-#define TK_BC(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { cudaGetLastError(); cleanup(); \
-    return fail(c, e_ == cudaErrorMemoryAllocation ? TKNN_ENOMEM : TKNN_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_)); } } while (0)
 
-  TK_BC(cudaEventRecord(c->ev[0], st));
-  const float* d_xyz = xyz;
-  if (!is_device_ptr(xyz)) {
-    const size_t bytes = (size_t)n * stride_floats * sizeof(float);
-    TK_B(ensure(c, in_stage, bytes));
-    TK_BC(cudaMemcpyAsync(in_stage.p, xyz, bytes, cudaMemcpyHostToDevice, st));
-    d_xyz = in_stage.as<float>();
-    S.h2d_bytes = bytes;
-  }
-  TK_BC(cudaEventRecord(c->ev[1], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[0], st));
+  const float* d_xyz = nullptr;
+  TK_TRY(stage_in(c, xyz, (size_t)n * stride_floats, c->b_in, &d_xyz));
+  if (d_xyz != xyz) S.h2d_bytes = (size_t)n * stride_floats * sizeof(float);
+  TK_CUDA(c, cudaEventRecord(c->ev[1], st));
 
   // ---- scene bounds ----
   uint32_t* sc = c->scalars.as<uint32_t>();
   const uint32_t binit[8] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u, 0u, 0u};
-  TK_BC(cudaMemcpyAsync(sc + SC_BOUNDS, binit, sizeof(binit), cudaMemcpyHostToDevice, st));
+  TK_CUDA(c, cudaMemcpyAsync(sc + SC_BOUNDS, binit, sizeof(binit), cudaMemcpyHostToDevice, st));
   {
     const unsigned nb = (unsigned)std::min<uint64_t>((uint64_t)c->sm_count * 8, blocks_for(n, lbvh::THREADS));
     lbvh::bounds_kernel<<<nb, lbvh::THREADS, 0, st>>>(d_xyz, n, dim, stride_floats, sc + SC_BOUNDS);
     ++launches;
   }
-  TK_BC(cudaEventRecord(c->ev[2], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
 
   // ---- Morton codes ----
-  TK_B(ensure(c, keys_a, n * sizeof(uint64_t)));
-  TK_B(ensure(c, keys_b, n * sizeof(uint64_t)));
-  TK_B(ensure(c, vals_a, n * sizeof(uint32_t)));
-  TK_B(ensure(c, vals_b, n * sizeof(uint32_t)));
+  TK_TRY(ensure(c, keys_a, n * sizeof(uint64_t)));
+  TK_TRY(ensure(c, keys_b, n * sizeof(uint64_t)));
+  TK_TRY(ensure(c, vals_a, n * sizeof(uint32_t)));
+  TK_TRY(ensure(c, vals_b, n * sizeof(uint32_t)));
   int mbits = 0, idx_bits = 0, seg_bits = 0;
   if (seg) segment_key_layout(c, n, n_segments, max_segment, &mbits, &idx_bits, &seg_bits);
   else choose_key_layout(c, n, &mbits, &idx_bits);
@@ -1222,10 +1214,10 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
     ++launches;
   }
   const int sort_passes = (3 * mbits + seg_bits + 7) / 8;
-  TK_BC(cudaEventRecord(c->ev[3], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[3], st));
 
   // ---- onesweep radix sort ----
-  TK_B(ensure(c, sort_tmp, rsort::temp_words(n) * sizeof(uint32_t)));
+  TK_TRY(ensure(c, sort_tmp, rsort::temp_words(n) * sizeof(uint32_t)));
   bool sorted_in_b = false;
   if (idx_bits > 0)
     launches += rsort::sort_keys(keys_a.as<uint64_t>(), keys_b.as<uint64_t>(), n, sort_tmp.as<uint32_t>(), c->sm_count, st, idx_bits,
@@ -1235,13 +1227,13 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
                                   sort_tmp.as<uint32_t>(), c->sm_count, st, sort_passes, &sorted_in_b);
   const uint64_t* skeys = sorted_in_b ? keys_b.as<uint64_t>() : keys_a.as<uint64_t>();
   const uint32_t* svals = idx_bits > 0 ? nullptr : (sorted_in_b ? vals_b.as<uint32_t>() : vals_a.as<uint32_t>());
-  TK_BC(cudaGetLastError());
-  TK_BC(cudaEventRecord(c->ev[4], st));
+  TK_CUDA(c, cudaGetLastError());
+  TK_CUDA(c, cudaEventRecord(c->ev[4], st));
 
   // ---- leaf cut + point gather ----
   const uint64_t nw = (n + 31) / 32;
-  TK_B(ensure(c, ballots, nw * sizeof(uint32_t)));
-  TK_B(ensure(c, c->offsets, (nw + 1) * sizeof(uint32_t)));
+  TK_TRY(ensure(c, ballots, nw * sizeof(uint32_t)));
+  TK_TRY(ensure(c, c->offsets, (nw + 1) * sizeof(uint32_t)));
   const uint64_t force_split = (n <= (uint64_t)c->leaf_size) ? n / 2 : 0;
   lbvh::leaf_flag_kernel<<<blocks_for(nw * 32, lbvh::THREADS), lbvh::THREADS, 0, st>>>(
       skeys, n, c->leaf_size, c->leaf_policy, force_split, ballots.as<uint32_t>());
@@ -1251,44 +1243,44 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
                                                                                               ballots.as<uint32_t>());
     launches += 1;
   }
-  TK_B(popc_scan(c, ballots.as<uint32_t>(), nw, c->offsets.as<uint32_t>(), &launches));
+  TK_TRY(popc_scan(c, ballots.as<uint32_t>(), nw, c->offsets.as<uint32_t>(), &launches));
   uint32_t mb[2] = {0, 0};
-  TK_B(fetch_words(c, sc + SC_TOTAL, 1, sc + SC_BOUNDS + 6, 1, mb));  // the leaf count sizes every later launch
+  TK_TRY(fetch_words(c, sc + SC_TOTAL, 1, sc + SC_BOUNDS + 6, 1, mb));  // the leaf count sizes every later launch
   const uint32_t m = mb[0];
   const uint32_t bad[1] = {mb[1]};
-  if (bad[0]) { cleanup(); return fail(c, TKNN_EINVAL, "non-finite coordinate in the input points"); }
-  if (m < 2) { cleanup(); return fail(c, TKNN_ECUDA, "internal: leaf cut produced %u leaves", m); }
-  TK_B(ensure(c, c->leaf_start, (size_t)(m + 1) * sizeof(uint32_t)));
-  TK_B(ensure(c, leaf_key, (size_t)m * sizeof(uint64_t)));
-  TK_B(ensure(c, c->pts, n * sizeof(float4)));
+  if (bad[0]) return fail(c, TKNN_EINVAL, "non-finite coordinate in the input points");
+  if (m < 2) return fail(c, TKNN_ECUDA, "internal: leaf cut produced %u leaves", m);
+  TK_TRY(ensure(c, c->leaf_start, (size_t)(m + 1) * sizeof(uint32_t)));
+  TK_TRY(ensure(c, leaf_key, (size_t)m * sizeof(uint64_t)));
+  TK_TRY(ensure(c, c->pts, n * sizeof(float4)));
   lbvh::leaf_emit_kernel<<<blocks_for(n, lbvh::THREADS), lbvh::THREADS, 0, st>>>(
       ballots.as<uint32_t>(), c->offsets.as<uint32_t>(), skeys, n, m, c->leaf_start.as<uint32_t>(),
       leaf_key.as<uint64_t>());
   lbvh::gather_points_kernel<<<blocks_for(n, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_xyz, dim, stride_floats, svals, skeys, idx_bits,
                                                                                    n, ids_in_w ? 1 : 0, c->pts.as<float4>());
   launches += 2;
-  TK_BC(cudaEventRecord(c->ev[5], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[5], st));
 
   // ---- Karras hierarchy ----
-  TK_B(ensure(c, c->nodes, (size_t)(m - 1) * sizeof(Node)));
-  TK_B(ensure(c, c->node_min_idx, (size_t)(m - 1) * 2 * sizeof(int)));
-  TK_B(ensure(c, child_info, (size_t)(m - 1) * sizeof(int4)));
-  TK_B(ensure(c, parent_leaf, (size_t)m * sizeof(int32_t)));
-  TK_B(ensure(c, parent_node, (size_t)m * sizeof(int32_t)));
-  TK_B(ensure(c, arrive, (size_t)m * sizeof(uint32_t)));
-  TK_BC(cudaMemsetAsync(arrive.p, 0, (size_t)m * sizeof(uint32_t), st));
-  TK_BC(cudaMemsetAsync(sc + SC_DUPLEAF, 0, sizeof(uint32_t), st));
+  TK_TRY(ensure(c, c->nodes, (size_t)(m - 1) * sizeof(Node)));
+  TK_TRY(ensure(c, c->node_min_idx, (size_t)(m - 1) * 2 * sizeof(int)));
+  TK_TRY(ensure(c, child_info, (size_t)(m - 1) * sizeof(int4)));
+  TK_TRY(ensure(c, parent_leaf, (size_t)m * sizeof(int32_t)));
+  TK_TRY(ensure(c, parent_node, (size_t)m * sizeof(int32_t)));
+  TK_TRY(ensure(c, arrive, (size_t)m * sizeof(uint32_t)));
+  TK_CUDA(c, cudaMemsetAsync(arrive.p, 0, (size_t)m * sizeof(uint32_t), st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_DUPLEAF, 0, sizeof(uint32_t), st));
   lbvh::karras_kernel<<<blocks_for(m - 1, lbvh::THREADS), lbvh::THREADS, 0, st>>>(
       leaf_key.as<uint64_t>(), c->leaf_start.as<uint32_t>(), m, child_info.as<int4>(), parent_leaf.as<int32_t>(),
       parent_node.as<int32_t>());
   ++launches;
   if (seg) {
-    TK_B(ensure(c, c->node_seg, (size_t)(m - 1) * sizeof(int4)));
+    TK_TRY(ensure(c, c->node_seg, (size_t)(m - 1) * sizeof(int4)));
     lbvh::node_segments_kernel<<<blocks_for(m - 1, lbvh::THREADS), lbvh::THREADS, 0, st>>>(
         leaf_key.as<uint64_t>(), c->leaf_start.as<uint32_t>(), m, c->seg_of.as<uint32_t>(), c->node_seg.as<int4>());
     ++launches;
   }
-  TK_BC(cudaEventRecord(c->ev[6], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[6], st));
 
   // ---- bottom-up refit ----
   lbvh::refit_kernel<<<blocks_for(m, lbvh::THREADS), lbvh::THREADS, 0, st>>>(
@@ -1296,15 +1288,12 @@ int tknn::host::build_core(tknn_ctx* c, const float* xyz, uint64_t n, int dim, i
       parent_node.as<int32_t>(), arrive.as<uint32_t>(), c->nodes.as<Node>(), c->node_min_idx.as<int>(), sc + SC_DUPLEAF,
       (uint32_t)std::max(2, std::min(8, c->leaf_size)), reinterpret_cast<float*>(sc + SC_SCENE));
   ++launches;
-  TK_BC(cudaGetLastError());
-  TK_BC(cudaEventRecord(c->ev[7], st));
+  TK_CUDA(c, cudaGetLastError());
+  TK_CUDA(c, cudaEventRecord(c->ev[7], st));
   uint32_t tail[7] = {0, 0, 0, 0, 0, 0, 0};
-  TK_B(fetch_words(c, sc + SC_SCENE, 6, sc + SC_DUPLEAF, 1, tail));
+  TK_TRY(fetch_words(c, sc + SC_SCENE, 6, sc + SC_DUPLEAF, 1, tail));
   std::memcpy(c->scene_box, tail, 6 * sizeof(float));
   const uint32_t dupleaf = tail[6];
-  cleanup();
-#undef TK_B
-#undef TK_BC
 
   // ---- cell grid: plain builds without coincident-point leaves (those take the tie-pruning LBVH kernel) ----
   TK_CUDA(c, cudaEventRecord(c->ev[8], st));
@@ -1400,26 +1389,6 @@ int tknn_estimate_start_radius(tknn_ctx* c, int k, float* radius_out) {
 namespace {
 // Query offsets of the _segments calls (host or device): n_segments + 1 entries that start at 0, never decrease and end at
 // nq, with n_segments the segment count of the last build.  Device offsets cost one small read-back.
-// Reads n_segments + 1 offsets (host or device) into *off and checks that they start at 0, never decrease and end at
-// `total` (named `total_name` in the message); `side` names the offsets in the message.
-int read_offsets(tknn_ctx* c, const char* what, const char* side, const uint64_t* offsets, uint64_t n_segments,
-                 uint64_t total, const char* total_name, std::vector<uint64_t>* off_out) {
-  std::vector<uint64_t>& off = *off_out;
-  off.assign(n_segments + 1, 0);
-  if (is_device_ptr(offsets)) {
-    TK_CUDA(c, cudaMemcpyAsync(off.data(), offsets, off.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
-    TK_CUDA(c, cudaStreamSynchronize(c->stream));
-  } else {
-    std::memcpy(off.data(), offsets, off.size() * sizeof(uint64_t));
-  }
-  if (off[0] != 0) return fail(c, TKNN_EINVAL, "%s: %s offsets must start at 0", what, side);
-  if (off[n_segments] != total)
-    return fail(c, TKNN_EINVAL, "%s: %s offsets must end at %s = %llu", what, side, total_name, (unsigned long long)total);
-  for (uint64_t s = 0; s < n_segments; ++s)
-    if (off[s + 1] < off[s]) return fail(c, TKNN_EINVAL, "%s: %s offsets decrease at segment %llu", what, side, (unsigned long long)s);
-  return TKNN_OK;
-}
-
 int check_query_offsets(tknn_ctx* c, const char* what, const uint64_t* q_seg_offsets, uint64_t n_segments, uint64_t nq) {
   if (!q_seg_offsets) return fail(c, TKNN_EINVAL, "%s: null query segment offsets", what);
   if (n_segments != c->n_segments)
@@ -1440,41 +1409,22 @@ int stage_queries(tknn_ctx* c, const float* queries, uint64_t nq, int dim, int s
                   const uint64_t* q_seg_offsets = nullptr, uint64_t n_segments = 0, const uint32_t** seg_sorted_out = nullptr) {
   cudaStream_t st = c->stream;
   uint32_t* sc = c->scalars.as<uint32_t>();
-  DevBuf &q_stage = c->q_stage, &keys_a = c->q_keys_a, &keys_b = c->q_keys_b, &vals_a = c->q_vals_a, &vals_b = c->q_vals_b,
-         &sort_tmp = c->q_sort_tmp, &qpts = c->q_pts, &sid_stage = c->q_sid_stage, &sid_sorted = c->q_sid_sorted,
-         &rad_stage = c->q_rad_stage, &r2_sorted = c->q_r2_sorted;
+  DevBuf &keys_a = c->q_keys_a, &keys_b = c->q_keys_b, &vals_a = c->q_vals_a, &vals_b = c->q_vals_b,
+         &sort_tmp = c->q_sort_tmp, &qpts = c->q_pts, &sid_sorted = c->q_sid_sorted, &r2_sorted = c->q_r2_sorted;
   *sid_sorted_out = nullptr;
   *r2_sorted_out = nullptr;
   if (seg_sorted_out) *seg_sorted_out = nullptr;
-  const float* d_q = queries;
-  if (!is_device_ptr(queries)) {
-    const size_t bytes = (size_t)nq * stride_floats * sizeof(float);
-    TK_TRY(ensure(c, q_stage, bytes));
-    TK_CUDA(c, cudaMemcpyAsync(q_stage.p, queries, bytes, cudaMemcpyHostToDevice, st));
-    d_q = q_stage.as<float>();
-  }
-  const int32_t* d_sid = self_ids;
-  if (self_ids && !is_device_ptr(self_ids)) {
-    TK_TRY(ensure(c, sid_stage, nq * sizeof(int32_t)));
-    TK_CUDA(c, cudaMemcpyAsync(sid_stage.p, self_ids, nq * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    d_sid = sid_stage.as<int32_t>();
-  }
-  const float* d_rad = init_radius2;
-  if (init_radius2 && !is_device_ptr(init_radius2)) {
-    TK_TRY(ensure(c, rad_stage, nq * sizeof(float)));
-    TK_CUDA(c, cudaMemcpyAsync(rad_stage.p, init_radius2, nq * sizeof(float), cudaMemcpyHostToDevice, st));
-    d_rad = rad_stage.as<float>();
-  }
+  const float *d_q = nullptr, *d_rad = nullptr;
+  const int32_t* d_sid = nullptr;
+  TK_TRY(stage_in(c, queries, (size_t)nq * stride_floats, c->q_stage, &d_q));
+  TK_TRY(stage_in(c, self_ids, nq, c->q_sid_stage, &d_sid));
+  TK_TRY(stage_in(c, init_radius2, nq, c->q_rad_stage, &d_rad));
   const bool seg = q_seg_offsets != nullptr;
-  const uint64_t* d_qoff = q_seg_offsets;
+  const uint64_t* d_qoff = nullptr;
   if (seg) {
     TK_TRY(ensure(c, c->q_seg_row, nq * sizeof(uint32_t)));
     TK_TRY(ensure(c, c->q_seg_sorted, nq * sizeof(uint32_t)));
-    if (!is_device_ptr(q_seg_offsets)) {
-      TK_TRY(ensure(c, c->q_seg_off, (n_segments + 1) * sizeof(uint64_t)));
-      TK_CUDA(c, cudaMemcpyAsync(c->q_seg_off.p, q_seg_offsets, (n_segments + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-      d_qoff = c->q_seg_off.as<uint64_t>();
-    }
+    TK_TRY(stage_in(c, q_seg_offsets, n_segments + 1, c->q_seg_off, &d_qoff));
   }
   // Morton-sort the queries on the DATA's grid so that groups of 32 are spatially coherent
   TK_TRY(ensure(c, keys_a, nq * sizeof(uint64_t)));
@@ -1550,51 +1500,38 @@ int query_core(tknn_ctx* c, const char* what, const float* queries, uint64_t nq,
   uint32_t* sc = c->scalars.as<uint32_t>();
 
   // scratch lives in the context (grow-only): a call allocates nothing once the buffers have reached their size
-  DevBuf &q_stage = c->q_stage, &keys_a = c->q_keys_a, &keys_b = c->q_keys_b, &vals_a = c->q_vals_a, &vals_b = c->q_vals_b,
-         &sort_tmp = c->q_sort_tmp, &qpts = c->q_pts, &sid_stage = c->q_sid_stage, &sid_sorted = c->q_sid_sorted,
-         &rad_stage = c->q_rad_stage, &r2_sorted = c->q_r2_sorted;
-  auto cleanup = [&]() {
-    if (c->keep_scratch) return;
-    for (DevBuf* b : {&q_stage, &keys_a, &keys_b, &vals_a, &vals_b, &sort_tmp, &qpts, &sid_stage, &sid_sorted, &rad_stage,
-                      &r2_sorted, &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted})
-      release(*b);
-  };
-#define TK_B(expr) do { int rc_ = (expr); if (rc_ != TKNN_OK) { cleanup(); return rc_; } } while (0)
-#define TK_BC(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { cudaGetLastError(); cleanup(); \
-    return fail(c, e_ == cudaErrorMemoryAllocation ? TKNN_ENOMEM : TKNN_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_)); } } while (0)
-
-  TK_BC(cudaEventRecord(c->ev[0], st));
+  ScratchScope scratch = query_scratch(c);
+  TK_CUDA(c, cudaEventRecord(c->ev[0], st));
   int launches = 0;
   const int32_t* d_sid_sorted = nullptr;
   const float* d_r2_sorted = nullptr;
   const uint32_t* d_seg_sorted = nullptr;
-  TK_B(stage_queries(c, queries, nq, dim, stride_floats, self_ids, init_radius2, &d_sid_sorted, &d_r2_sorted, &launches,
-                     q_seg_offsets, n_segments, &d_seg_sorted));
+  TK_TRY(stage_queries(c, queries, nq, dim, stride_floats, self_ids, init_radius2, &d_sid_sorted, &d_r2_sorted, &launches,
+                       q_seg_offsets, n_segments, &d_seg_sorted));
 
-  const bool idx_dev = is_device_ptr(idx_out), dist_dev = is_device_ptr(dist_out);
-  int32_t* d_idx = idx_out;
-  float* d_dist = dist_out;
+  int32_t* d_idx = nullptr;
+  float* d_dist = nullptr;
   const size_t out_elems = (size_t)nq * k;
-  if (!idx_dev) { TK_B(ensure(c, c->stage_idx, out_elems * sizeof(int32_t))); d_idx = c->stage_idx.as<int32_t>(); }
-  if (!dist_dev) { TK_B(ensure(c, c->stage_dist, out_elems * sizeof(float))); d_dist = c->stage_dist.as<float>(); }
+  TK_TRY(out_view(c, idx_out, out_elems, c->stage_idx, &d_idx));
+  TK_TRY(out_view(c, dist_out, out_elems, c->stage_dist, &d_dist));
 
-  TK_BC(cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
   float r0 = start_radius;
   // a query set can hold fewer than k reachable neighbours only through self exclusion / radius caps
   const bool may_underfill = (uint64_t)k > c->n - (self_ids ? 1 : 0);
   bool estimated = false;
   if (!(r0 > 0.0f)) {
     if (init_radius2 || may_underfill) r0 = INFINITY;
-    else { TK_B(estimate_radius_device(c, qpts.as<float4>(), 0, nq, d_sid_sorted, 0, d_seg_sorted, k, &launches)); estimated = true; }
+    else { TK_TRY(estimate_radius_device(c, c->q_pts.as<float4>(), 0, nq, d_sid_sorted, 0, d_seg_sorted, k, &launches)); estimated = true; }
   }
-  TK_BC(cudaEventRecord(c->ev[1], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[1], st));
   c->stats.start_radius = r0;
   Job job;
   if (estimated) {
     job.r_dev = reinterpret_cast<const float*>(sc + SC_QUANTILE);
     job.r_host = &c->stats.start_radius;
   }
-  job.queries = qpts.as<float4>();
+  job.queries = c->q_pts.as<float4>();
   job.self_ids = d_sid_sorted;
   job.query_r2 = d_r2_sorted;
   job.seg_of = d_seg_sorted;
@@ -1607,15 +1544,12 @@ int query_core(tknn_ctx* c, const char* what, const float* queries, uint64_t nq,
   job.squared = c->squared;
   job.idx_out = d_idx;
   job.dist_out = d_dist;
-  TK_B(run_rounds(c, job, &launches));
-  TK_BC(cudaEventRecord(c->ev[2], st));
-  if (!idx_dev) { TK_BC(cudaMemcpyAsync(idx_out, d_idx, out_elems * sizeof(int32_t), cudaMemcpyDeviceToHost, st)); c->stats.d2h_bytes += out_elems * 4; }
-  if (!dist_dev) { TK_BC(cudaMemcpyAsync(dist_out, d_dist, out_elems * sizeof(float), cudaMemcpyDeviceToHost, st)); c->stats.d2h_bytes += out_elems * 4; }
-  TK_BC(cudaEventRecord(c->ev[3], st));
-  TK_BC(cudaStreamSynchronize(st));
-  cleanup();
-#undef TK_B
-#undef TK_BC
+  TK_TRY(run_rounds(c, job, &launches));
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
+  TK_TRY(copy_back(c, idx_out, d_idx, out_elems, &c->stats.d2h_bytes));
+  TK_TRY(copy_back(c, dist_out, d_dist, out_elems, &c->stats.d2h_bytes));
+  TK_CUDA(c, cudaEventRecord(c->ev[3], st));
+  TK_CUDA(c, cudaStreamSynchronize(st));
   TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
   TK_CUDA(c, cudaEventElapsedTime(&c->stats.d2h_ms, c->ev[2], c->ev[3]));
   c->stats.kernel_launches = (uint32_t)(launches + c->mailbox_launches + (c->mailbox_h ? 1 : 0));  // + the error-flag fetch below
@@ -1657,9 +1591,8 @@ int tknn_range_count(tknn_ctx* c, float radius, uint32_t* count_out) {
   reset_search_stats(c);
   c->stats.n_queries = c->n;
   uint32_t* sc = c->scalars.as<uint32_t>();
-  const bool dev = is_device_ptr(count_out);
-  uint32_t* d_out = count_out;
-  if (!dev) { TK_TRY(ensure(c, c->stage_idx, c->n * sizeof(uint32_t))); d_out = c->stage_idx.as<uint32_t>(); }
+  uint32_t* d_out = nullptr;
+  TK_TRY(out_view(c, count_out, c->n, c->stage_idx, &d_out));
   trav::Params P;
   std::memset(&P, 0, sizeof(P));
   P.nodes = c->nodes.as<Node>();
@@ -1683,10 +1616,7 @@ int tknn_range_count(tknn_ctx* c, float radius, uint32_t* count_out) {
   TK_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
   TK_TRY(launch_traverse<trav::MODE_RANGE_COUNT>(c, P));
   TK_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  if (!dev) {
-    TK_CUDA(c, cudaMemcpyAsync(count_out, d_out, c->n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-    c->stats.d2h_bytes = c->n * sizeof(uint32_t);
-  }
+  TK_TRY(copy_back(c, count_out, d_out, c->n, &c->stats.d2h_bytes));
   TK_CUDA(c, cudaStreamSynchronize(c->stream));
   TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
   c->stats.rounds = 1;
@@ -1714,7 +1644,6 @@ int tknn_dbscan(tknn_ctx* c, float eps, int min_pts, int32_t* label_out, uint8_t
   const uint32_t n_groups = (uint32_t)((n + 31) / 32);
   cudaStream_t st = c->stream;
   uint32_t* sc = c->scalars.as<uint32_t>();
-  const bool label_dev = is_device_ptr(label_out), core_dev = core_out && is_device_ptr(core_out);
   TK_TRY(ensure(c, c->unresolved, sizeof(uint32_t) * (size_t)(n_groups + 1)));
   TK_TRY(ensure(c, c->offsets, sizeof(uint32_t) * (size_t)(n_groups + 1)));
   TK_TRY(ensure(c, c->queue_a, sizeof(uint32_t) * n));
@@ -1723,10 +1652,10 @@ int tknn_dbscan(tknn_ctx* c, float eps, int min_pts, int32_t* label_out, uint8_t
   TK_TRY(ensure(c, c->db_min_idx, sizeof(int) * n));
   TK_TRY(ensure(c, c->db_pos_label, sizeof(int32_t) * n));
   TK_TRY(ensure(c, c->db_bits, sizeof(uint32_t) * (size_t)n_groups));
-  if (!label_dev) TK_TRY(ensure(c, c->stage_idx, sizeof(int32_t) * n));
-  if (core_out && !core_dev) TK_TRY(ensure(c, c->db_core_stage, n));
-  int32_t* d_label = label_dev ? label_out : c->stage_idx.as<int32_t>();
-  uint8_t* d_core = core_out ? (core_dev ? core_out : c->db_core_stage.as<uint8_t>()) : nullptr;
+  int32_t* d_label = nullptr;
+  uint8_t* d_core = nullptr;
+  TK_TRY(out_view(c, label_out, n, c->stage_idx, &d_label));
+  TK_TRY(out_view(c, core_out, n, c->db_core_stage, &d_core));
   uint32_t* core_words = c->unresolved.as<uint32_t>();
   uint32_t* core_q = c->queue_a.as<uint32_t>();
   uint32_t* other_q = c->queue_b.as<uint32_t>();
@@ -1735,11 +1664,7 @@ int tknn_dbscan(tknn_ctx* c, float eps, int min_pts, int32_t* label_out, uint8_t
   int32_t* pos_label = c->db_pos_label.as<int32_t>();
   uint32_t* cluster_bits = c->db_bits.as<uint32_t>();
   int launches = 0;
-  for (size_t i = c->round_ev.size(); i < 16; ++i) {
-    cudaEvent_t e;
-    TK_CUDA(c, cudaEventCreate(&e));
-    c->round_ev.push_back(e);
-  }
+  TK_TRY(ensure_round_events(c, 16));
   cudaEvent_t* ev = c->round_ev.data();  // phase r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its traversal kernel
 
   trav::Params P;
@@ -1818,9 +1743,8 @@ int tknn_dbscan(tknn_ctx* c, float eps, int min_pts, int32_t* label_out, uint8_t
   TK_CUDA(c, cudaEventRecord(c->ev[2], st));
   launches += 3 /* traversals */ + 4 /* split, flatten, mark, label */;
 
-  if (!label_dev) TK_CUDA(c, cudaMemcpyAsync(label_out, d_label, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, st));
-  if (core_out && !core_dev) TK_CUDA(c, cudaMemcpyAsync(core_out, d_core, n, cudaMemcpyDeviceToHost, st));
-  c->stats.d2h_bytes = (label_dev ? 0 : sizeof(int32_t) * n) + (core_out && !core_dev ? n : 0);
+  TK_TRY(copy_back(c, label_out, d_label, n, &c->stats.d2h_bytes));
+  TK_TRY(copy_back(c, core_out, d_core, n, &c->stats.d2h_bytes));
   uint32_t rb[3] = {0, 0, 0};  // core points, other points, clusters
   TK_TRY(fetch_words(c, sc + SC_DBSCAN, 2, sc + SC_TOTAL, 1, rb));  // synchronises the stream
   TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
@@ -1857,24 +1781,15 @@ int tknn_fps(tknn_ctx* c, const uint64_t* sample_offsets, uint64_t n_segments, c
   cudaStream_t st = c->stream;
   const uint64_t S = n_segments;
   const std::vector<uint64_t> off = c->segmented ? c->seg_off_host : std::vector<uint64_t>{0, c->n};
-  std::vector<uint64_t> soff(S + 1);
+  std::vector<uint64_t> soff;  // the sample total is free
+  TK_TRY(read_offsets(c, "tknn_fps", "sample", sample_offsets, S, 0, nullptr, &soff));
   std::vector<int32_t> starts(S);
-  if (is_device_ptr(sample_offsets))
-    TK_CUDA(c, cudaMemcpyAsync(soff.data(), sample_offsets, soff.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-  else
-    std::memcpy(soff.data(), sample_offsets, soff.size() * sizeof(uint64_t));
-  if (start_ids && is_device_ptr(start_ids))
-    TK_CUDA(c, cudaMemcpyAsync(starts.data(), start_ids, starts.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  else if (start_ids)
-    std::memcpy(starts.data(), start_ids, starts.size() * sizeof(int32_t));
-  TK_CUDA(c, cudaStreamSynchronize(st));
-  if (soff[0] != 0) return fail(c, TKNN_EINVAL, "tknn_fps: sample offsets must start at 0");
+  if (start_ids) TK_TRY(read_to_host(c, start_ids, S, starts.data()));
   std::vector<fps::Seg> small, large;
   std::vector<uint32_t> slot_of_seg;
   uint32_t small_max = 0, large_max_m = 0;
   uint64_t small_samples = 0, large_samples = 0;
   for (uint64_t s = 0; s < S; ++s) {
-    if (soff[s + 1] < soff[s]) return fail(c, TKNN_EINVAL, "tknn_fps: sample offsets decrease at segment %llu", (unsigned long long)s);
     const uint64_t ns = off[s + 1] - off[s], m = soff[s + 1] - soff[s];
     if (m > ns)
       return fail(c, TKNN_EINVAL, "tknn_fps: %llu samples of segment %llu, which has %llu points", (unsigned long long)m,
@@ -1909,11 +1824,10 @@ int tknn_fps(tknn_ctx* c, const uint64_t* sample_offsets, uint64_t n_segments, c
   }
 
   reset_search_stats(c);
-  const bool idx_dev = is_device_ptr(idx_out), dist_dev = dist_out && is_device_ptr(dist_out);
-  if (!idx_dev) TK_TRY(ensure(c, c->stage_idx, sizeof(int32_t) * std::max<uint64_t>(total, 1)));
-  if (dist_out && !dist_dev) TK_TRY(ensure(c, c->stage_dist, sizeof(float) * std::max<uint64_t>(total, 1)));
-  int32_t* d_idx = idx_dev ? idx_out : c->stage_idx.as<int32_t>();
-  float* d_dist = dist_out ? (dist_dev ? dist_out : c->stage_dist.as<float>()) : nullptr;
+  int32_t* d_idx = nullptr;
+  float* d_dist = nullptr;
+  TK_TRY(out_view(c, idx_out, std::max<uint64_t>(total, 1), c->stage_idx, &d_idx));
+  TK_TRY(out_view(c, dist_out, std::max<uint64_t>(total, 1), c->stage_dist, &d_dist));
   TK_TRY(ensure(c, c->fps_segs, sizeof(fps::Seg) * (small.size() + large.size())));
   fps::Seg* d_small = c->fps_segs.as<fps::Seg>();
   fps::Seg* d_large = d_small + small.size();
@@ -1921,11 +1835,7 @@ int tknn_fps(tknn_ctx* c, const uint64_t* sample_offsets, uint64_t n_segments, c
     TK_CUDA(c, cudaMemcpyAsync(d_small, small.data(), sizeof(fps::Seg) * small.size(), cudaMemcpyHostToDevice, st));
   if (!large.empty())
     TK_CUDA(c, cudaMemcpyAsync(d_large, large.data(), sizeof(fps::Seg) * large.size(), cudaMemcpyHostToDevice, st));
-  for (size_t i = c->round_ev.size(); i < 8; ++i) {
-    cudaEvent_t e;
-    TK_CUDA(c, cudaEventCreate(&e));
-    c->round_ev.push_back(e);
-  }
+  TK_TRY(ensure_round_events(c, 8));
   cudaEvent_t* ev = c->round_ev.data();  // tier r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its sampling kernel
   uint32_t* sc = c->scalars.as<uint32_t>();
   unsigned long long* counters = reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS);
@@ -2015,10 +1925,9 @@ int tknn_fps(tknn_ctx* c, const uint64_t* sample_offsets, uint64_t n_segments, c
   TK_CUDA(c, cudaEventRecord(ev[5], st));
   TK_CUDA(c, cudaEventRecord(c->ev[2], st));
 
-  if (!idx_dev && total) TK_CUDA(c, cudaMemcpyAsync(idx_out, d_idx, sizeof(int32_t) * total, cudaMemcpyDeviceToHost, st));
-  if (dist_out && !dist_dev && total) TK_CUDA(c, cudaMemcpyAsync(dist_out, d_dist, sizeof(float) * total, cudaMemcpyDeviceToHost, st));
+  TK_TRY(copy_back(c, idx_out, d_idx, total, &c->stats.d2h_bytes));
+  TK_TRY(copy_back(c, dist_out, d_dist, total, &c->stats.d2h_bytes));
   TK_CUDA(c, cudaStreamSynchronize(st));
-  c->stats.d2h_bytes = (idx_dev ? 0 : sizeof(int32_t) * total) + (dist_out && !dist_dev ? sizeof(float) * total : 0);
   TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
   c->stats.n_queries = total;
   c->stats.rounds = 2;
@@ -2112,48 +2021,27 @@ int tknn_feature_knn(tknn_ctx* c, const float* x, uint64_t n, int f, int x_strid
   }
 
   // inputs: host rows are staged (y aliasing x is staged once), device rows are read in place
-  const float* d_x = x;
-  const float* d_y = y;
+  const float *d_x = nullptr, *d_y = nullptr;
+  const int32_t* d_sid = nullptr;
   const bool same = y == x && y_stride_floats == x_stride_floats && nq == n;
-  if (!is_device_ptr(x)) {
-    const size_t bytes = ((size_t)(n - 1) * x_stride_floats + f) * sizeof(float);
-    TK_TRY(ensure(c, c->fk_x, bytes));
-    TK_CUDA(c, cudaMemcpyAsync(c->fk_x.p, x, bytes, cudaMemcpyHostToDevice, st));
-    d_x = c->fk_x.as<float>();
-  }
-  if (same) {
-    d_y = d_x;
-  } else if (!is_device_ptr(y)) {
-    const size_t bytes = ((size_t)(nq - 1) * y_stride_floats + f) * sizeof(float);
-    TK_TRY(ensure(c, c->fk_y, bytes));
-    TK_CUDA(c, cudaMemcpyAsync(c->fk_y.p, y, bytes, cudaMemcpyHostToDevice, st));
-    d_y = c->fk_y.as<float>();
-  }
-  const int32_t* d_sid = self_ids;
-  if (self_ids && !is_device_ptr(self_ids)) {
-    TK_TRY(ensure(c, c->fk_sid, nq * sizeof(int32_t)));
-    TK_CUDA(c, cudaMemcpyAsync(c->fk_sid.p, self_ids, nq * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    d_sid = c->fk_sid.as<int32_t>();
-  }
+  TK_TRY(stage_in(c, x, (size_t)(n - 1) * x_stride_floats + f, c->fk_x, &d_x));
+  if (same) d_y = d_x;
+  else TK_TRY(stage_in(c, y, (size_t)(nq - 1) * y_stride_floats + f, c->fk_y, &d_y));
+  TK_TRY(stage_in(c, self_ids, nq, c->fk_sid, &d_sid));
   TK_TRY(ensure(c, c->fk_items, items.size() * sizeof(feat::Item)));
   TK_CUDA(c, cudaMemcpyAsync(c->fk_items.p, items.data(), items.size() * sizeof(feat::Item), cudaMemcpyHostToDevice, st));
   const size_t out_elems = (size_t)nq * k;
-  const bool idx_dev = is_device_ptr(idx_out), dist_dev = dist_out && is_device_ptr(dist_out);
-  if (!idx_dev) TK_TRY(ensure(c, c->stage_idx, out_elems * sizeof(int32_t)));
-  if (dist_out && !dist_dev) TK_TRY(ensure(c, c->stage_dist, out_elems * sizeof(float)));
-  int32_t* d_idx = idx_dev ? idx_out : c->stage_idx.as<int32_t>();
-  float* d_dist = dist_out ? (dist_dev ? dist_out : c->stage_dist.as<float>()) : nullptr;
+  int32_t* d_idx = nullptr;
+  float* d_dist = nullptr;
+  TK_TRY(out_view(c, idx_out, out_elems, c->stage_idx, &d_idx));
+  TK_TRY(out_view(c, dist_out, out_elems, c->stage_dist, &d_dist));
   if (splits > 1) {
     TK_TRY(ensure(c, c->fk_partial, splits * out_elems * sizeof(uint64_t)));
     if (!d_dist) {  // the merge writes distances unconditionally
       TK_TRY(ensure(c, c->fk_dist, out_elems * sizeof(float)));
     }
   }
-  for (size_t i = c->round_ev.size(); i < 8; ++i) {
-    cudaEvent_t e;
-    TK_CUDA(c, cudaEventCreate(&e));
-    c->round_ev.push_back(e);
-  }
+  TK_TRY(ensure_round_events(c, 8));
   cudaEvent_t* ev = c->round_ev.data();  // round r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its kernel
   uint32_t* sc = c->scalars.as<uint32_t>();
   int launches = 0;
@@ -2205,11 +2093,10 @@ int tknn_feature_knn(tknn_ctx* c, const float* x, uint64_t n, int f, int x_strid
     TK_CUDA(c, cudaEventRecord(ev[5], st));
   }
   TK_CUDA(c, cudaEventRecord(c->ev[2], st));
-  if (!idx_dev) TK_CUDA(c, cudaMemcpyAsync(idx_out, d_idx, out_elems * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  if (dist_out && !dist_dev) TK_CUDA(c, cudaMemcpyAsync(dist_out, d_dist, out_elems * sizeof(float), cudaMemcpyDeviceToHost, st));
+  TK_TRY(copy_back(c, idx_out, d_idx, out_elems, &c->stats.d2h_bytes));
+  TK_TRY(copy_back(c, dist_out, d_dist, out_elems, &c->stats.d2h_bytes));
   TK_CUDA(c, cudaEventRecord(c->ev[3], st));
   TK_CUDA(c, cudaStreamSynchronize(st));
-  c->stats.d2h_bytes = (idx_dev ? 0 : out_elems * sizeof(int32_t)) + (dist_out && !dist_dev ? out_elems * sizeof(float) : 0);
   TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
   TK_CUDA(c, cudaEventElapsedTime(&c->stats.d2h_ms, c->ev[2], c->ev[3]));
   c->stats.rounds = splits > 1 ? 2 : 1;
@@ -2255,41 +2142,27 @@ int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* sel
   uint32_t* sc = c->scalars.as<uint32_t>();
   const uint64_t n = c->n;
   const bool fill_rows = idx_out != nullptr;
-  const bool off_dev = is_device_ptr(offsets_out);
-  auto cleanup = [&]() {
-    if (c->keep_scratch) return;
-    for (DevBuf* b : {&c->rl_cnt_pos, &c->rl_cnt_row, &c->rl_off_pos, &c->rl_off_row, &c->rl_sums, &c->rl_stats, &c->rl_pos_of,
-                      &c->rl_self_pos, &c->rl_keys, &c->rl_long_pos, &c->rl_long_len, &c->rl_boff, &c->rl_ka, &c->rl_kb,
-                      &c->rl_kc, &c->rl_va, &c->rl_vb, &c->rl_vc, &c->rl_row_of, &c->rl_sort_tmp})
-      release(*b);
-  };
-#define TK_R(expr) do { int rc_ = (expr); if (rc_ != TKNN_OK) { cleanup(); return rc_; } } while (0)
-#define TK_RC(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { cudaGetLastError(); cleanup(); \
-    return fail(c, e_ == cudaErrorMemoryAllocation ? TKNN_ENOMEM : TKNN_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_)); } } while (0)
-  for (size_t i = c->round_ev.size(); i < 12; ++i) {
-    cudaEvent_t e;
-    TK_RC(cudaEventCreate(&e));
-    c->round_ev.push_back(e);
-  }
+  ScratchScope scratch = radius_list_scratch(c);
+  TK_TRY(ensure_round_events(c, 12));
   cudaEvent_t* ev = c->round_ev.data();  // phase r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its kernels
 
-  TK_R(ensure(c, c->rl_cnt_pos, sizeof(uint32_t) * nq));
-  TK_R(ensure(c, c->rl_cnt_row, sizeof(uint32_t) * nq));
-  TK_R(ensure(c, c->rl_off_pos, sizeof(uint64_t) * (nq + 1)));
-  if (!off_dev) TK_R(ensure(c, c->rl_off_row, sizeof(uint64_t) * (nq + 1)));
-  TK_R(ensure(c, c->rl_stats, sizeof(uint64_t) * 4));
-  TK_R(ensure(c, c->rl_long_pos, sizeof(uint32_t) * nq));
-  TK_R(ensure(c, c->rl_long_len, sizeof(uint32_t) * nq));
+  TK_TRY(ensure(c, c->rl_cnt_pos, sizeof(uint32_t) * nq));
+  TK_TRY(ensure(c, c->rl_cnt_row, sizeof(uint32_t) * nq));
+  TK_TRY(ensure(c, c->rl_off_pos, sizeof(uint64_t) * (nq + 1)));
+  uint64_t* off_row = nullptr;
+  TK_TRY(out_view(c, offsets_out, nq + 1, c->rl_off_row, &off_row));
+  TK_TRY(ensure(c, c->rl_stats, sizeof(uint64_t) * 4));
+  TK_TRY(ensure(c, c->rl_long_pos, sizeof(uint32_t) * nq));
+  TK_TRY(ensure(c, c->rl_long_len, sizeof(uint32_t) * nq));
   uint32_t* cnt_pos = c->rl_cnt_pos.as<uint32_t>();
   uint32_t* cnt_row = c->rl_cnt_row.as<uint32_t>();
   uint64_t* off_pos = c->rl_off_pos.as<uint64_t>();
-  uint64_t* off_row = off_dev ? offsets_out : c->rl_off_row.as<uint64_t>();
   uint64_t* rstats = c->rl_stats.as<uint64_t>();  // row total, position total, long rows, long-row entries
   uint32_t* long_pos = c->rl_long_pos.as<uint32_t>();
   const int32_t* self_pos = nullptr;
   if (self_sorted) {
-    TK_R(ensure(c, c->rl_pos_of, sizeof(int32_t) * n));
-    TK_R(ensure(c, c->rl_self_pos, sizeof(int32_t) * nq));
+    TK_TRY(ensure(c, c->rl_pos_of, sizeof(int32_t) * n));
+    TK_TRY(ensure(c, c->rl_self_pos, sizeof(int32_t) * nq));
     self_pos = c->rl_self_pos.as<int32_t>();
   }
 
@@ -2311,90 +2184,86 @@ int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* sel
   P.group_counter = sc + SC_GROUP_COUNTER;
   P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
   set_segments(c, P, seg_of);
-  TK_RC(cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
 
   // 1. count (minus self, by position and by row), both scans, the long-row list; one read-back
-  TK_RC(cudaEventRecord(ev[0], st));
+  TK_CUDA(c, cudaEventRecord(ev[0], st));
   if (self_sorted) {
     radius::inverse_kernel<<<blocks_for(n, 256), 256, 0, st>>>(P.pts, n, c->rl_pos_of.as<int32_t>());
     radius::self_pos_kernel<<<blocks_for(nq, 256), 256, 0, st>>>(self_sorted, nq, c->rl_pos_of.as<int32_t>(), n,
                                                                  c->rl_self_pos.as<int32_t>());
-    TK_RC(cudaGetLastError());
+    TK_CUDA(c, cudaGetLastError());
     launches += 2;
   }
-  TK_RC(cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), st));
   P.count_out = cnt_pos;
   P.count_row = cnt_row;
-  TK_RC(cudaEventRecord(ev[2], st));
-  TK_R(launch_traverse<trav::MODE_RANGE_LIST_COUNT>(c, P));
-  TK_RC(cudaEventRecord(ev[3], st));
-  TK_R(scan_counts(c, cnt_row, nq, off_row, rstats, &launches));
-  TK_R(scan_counts(c, cnt_pos, nq, off_pos, rstats + 1, &launches));
-  TK_RC(cudaMemsetAsync(rstats + 2, 0, 2 * sizeof(uint64_t), st));
+  TK_CUDA(c, cudaEventRecord(ev[2], st));
+  TK_TRY(launch_traverse<trav::MODE_RANGE_LIST_COUNT>(c, P));
+  TK_CUDA(c, cudaEventRecord(ev[3], st));
+  TK_TRY(scan_counts(c, cnt_row, nq, off_row, rstats, &launches));
+  TK_TRY(scan_counts(c, cnt_pos, nq, off_pos, rstats + 1, &launches));
+  TK_CUDA(c, cudaMemsetAsync(rstats + 2, 0, 2 * sizeof(uint64_t), st));
   radius::long_rows_kernel<<<blocks_for(nq, 256), 256, 0, st>>>(cnt_pos, nq, long_pos, c->rl_long_len.as<uint32_t>(),
                                                                  reinterpret_cast<unsigned long long*>(rstats + 2));
-  TK_RC(cudaGetLastError());
+  TK_CUDA(c, cudaGetLastError());
   launches += 2;  // the traversal, long_rows_kernel
-  TK_RC(cudaEventRecord(ev[1], st));
+  TK_CUDA(c, cudaEventRecord(ev[1], st));
   uint64_t rb[4] = {0, 0, 0, 0};
-  TK_R(fetch_words(c, reinterpret_cast<const uint32_t*>(rstats), 8, nullptr, 0, reinterpret_cast<uint32_t*>(rb)));
+  TK_TRY(fetch_words(c, reinterpret_cast<const uint32_t*>(rstats), 8, nullptr, 0, reinterpret_cast<uint32_t*>(rb)));
   const uint64_t total = rb[0], n_long = rb[2];
-  if (rb[1] != total) { cleanup(); return fail(c, TKNN_ECUDA, "internal: row and position totals differ"); }
+  if (rb[1] != total) return fail(c, TKNN_ECUDA, "internal: row and position totals differ");
   if (total_out) *total_out = total;
-  if (!off_dev) {
-    TK_RC(cudaMemcpyAsync(offsets_out, off_row, sizeof(uint64_t) * (nq + 1), cudaMemcpyDeviceToHost, st));
-    c->stats.d2h_bytes += sizeof(uint64_t) * (nq + 1);
-  }
+  TK_TRY(copy_back(c, offsets_out, off_row, nq + 1, &c->stats.d2h_bytes));
   const bool write_rows = fill_rows && capacity >= total;
 
   // 2. fill: the unsorted rows in position order
-  TK_RC(cudaEventRecord(ev[4], st));
-  TK_RC(cudaEventRecord(ev[6], st));
-  const bool idx_dev = write_rows && is_device_ptr(idx_out), dist_dev = write_rows && dist_out && is_device_ptr(dist_out);
-  int32_t* d_idx = idx_out;
-  float* d_dist = dist_out;
+  TK_CUDA(c, cudaEventRecord(ev[4], st));
+  TK_CUDA(c, cudaEventRecord(ev[6], st));
+  int32_t* d_idx = nullptr;
+  float* d_dist = nullptr;
   if (write_rows && total) {
-    TK_R(ensure(c, c->rl_keys, sizeof(uint64_t) * total));
-    if (!idx_dev) { TK_R(ensure(c, c->stage_idx, sizeof(int32_t) * total)); d_idx = c->stage_idx.as<int32_t>(); }
-    if (dist_out && !dist_dev) { TK_R(ensure(c, c->stage_dist, sizeof(float) * total)); d_dist = c->stage_dist.as<float>(); }
-    TK_RC(cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), st));
+    TK_TRY(ensure(c, c->rl_keys, sizeof(uint64_t) * total));
+    TK_TRY(out_view(c, idx_out, total, c->stage_idx, &d_idx));
+    TK_TRY(out_view(c, dist_out, total, c->stage_dist, &d_dist));
+    TK_CUDA(c, cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), st));
     P.list_off = off_pos;
     P.list_keys = c->rl_keys.as<uint64_t>();
-    TK_R(launch_traverse<trav::MODE_RANGE_LIST>(c, P));
+    TK_TRY(launch_traverse<trav::MODE_RANGE_LIST>(c, P));
     ++launches;
   }
-  TK_RC(cudaEventRecord(ev[7], st));
-  TK_RC(cudaEventRecord(ev[5], st));
+  TK_CUDA(c, cudaEventRecord(ev[7], st));
+  TK_CUDA(c, cudaEventRecord(ev[5], st));
 
   // 3. order: short rows one warp each in shared memory, long rows by the radix sort in batches
-  TK_RC(cudaEventRecord(ev[8], st));
-  TK_RC(cudaEventRecord(ev[10], st));
+  TK_CUDA(c, cudaEventRecord(ev[8], st));
+  TK_CUDA(c, cudaEventRecord(ev[10], st));
   if (write_rows && total) {
     const uint64_t* keys = c->rl_keys.as<uint64_t>();
     radius::sort_rows_warp_kernel<<<blocks_for(nq, radius::SORT_WARPS), radius::SORT_WARPS * 32, 0, st>>>(
         keys, off_pos, cnt_pos, qpts, nq, off_row, c->squared, d_idx, d_dist);
-    TK_RC(cudaGetLastError());
+    TK_CUDA(c, cudaGetLastError());
     ++launches;
     if (n_long) {
       // the long rows in position order (the list was appended in any order), their lengths and global prefix
       std::vector<uint32_t> hpos(n_long), hlen(n_long), lp(n_long);
       std::vector<uint64_t> order(n_long), boff(n_long + 1);
-      TK_RC(cudaMemcpyAsync(hpos.data(), long_pos, sizeof(uint32_t) * n_long, cudaMemcpyDeviceToHost, st));
-      TK_RC(cudaMemcpyAsync(hlen.data(), c->rl_long_len.p, sizeof(uint32_t) * n_long, cudaMemcpyDeviceToHost, st));
-      TK_RC(cudaStreamSynchronize(st));
+      TK_CUDA(c, cudaMemcpyAsync(hpos.data(), long_pos, sizeof(uint32_t) * n_long, cudaMemcpyDeviceToHost, st));
+      TK_CUDA(c, cudaMemcpyAsync(hlen.data(), c->rl_long_len.p, sizeof(uint32_t) * n_long, cudaMemcpyDeviceToHost, st));
+      TK_CUDA(c, cudaStreamSynchronize(st));
       for (uint64_t r = 0; r < n_long; ++r) order[r] = r;
       std::sort(order.begin(), order.end(), [&](uint64_t a, uint64_t b) { return hpos[a] < hpos[b]; });
       boff[0] = 0;
       for (uint64_t r = 0; r < n_long; ++r) {
         lp[r] = hpos[order[r]];
         const uint64_t len = hlen[order[r]];
-        if (len > rsort::MAX_N) { cleanup(); return fail(c, TKNN_EINVAL, "a row of %llu entries exceeds the sort's limit",
-                                                         (unsigned long long)len); }
+        if (len > rsort::MAX_N)
+          return fail(c, TKNN_EINVAL, "a row of %llu entries exceeds the sort's limit", (unsigned long long)len);
         boff[r + 1] = boff[r] + len;
       }
-      TK_R(ensure(c, c->rl_boff, sizeof(uint64_t) * (n_long + 1)));
-      TK_RC(cudaMemcpyAsync(long_pos, lp.data(), sizeof(uint32_t) * n_long, cudaMemcpyHostToDevice, st));
-      TK_RC(cudaMemcpyAsync(c->rl_boff.p, boff.data(), sizeof(uint64_t) * (n_long + 1), cudaMemcpyHostToDevice, st));
+      TK_TRY(ensure(c, c->rl_boff, sizeof(uint64_t) * (n_long + 1)));
+      TK_CUDA(c, cudaMemcpyAsync(long_pos, lp.data(), sizeof(uint32_t) * n_long, cudaMemcpyHostToDevice, st));
+      TK_CUDA(c, cudaMemcpyAsync(c->rl_boff.p, boff.data(), sizeof(uint64_t) * (n_long + 1), cudaMemcpyHostToDevice, st));
       uint64_t batch_max = 0;  // entries of the largest batch
       std::vector<uint64_t> firsts;
       for (uint64_t r = 0; r < n_long;) {
@@ -2405,14 +2274,14 @@ int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* sel
         r = e;
       }
       firsts.push_back(n_long);
-      TK_R(ensure(c, c->rl_ka, sizeof(uint64_t) * batch_max));
-      TK_R(ensure(c, c->rl_kb, sizeof(uint64_t) * batch_max));
-      TK_R(ensure(c, c->rl_kc, sizeof(uint64_t) * batch_max));
-      TK_R(ensure(c, c->rl_va, sizeof(uint32_t) * batch_max));
-      TK_R(ensure(c, c->rl_vb, sizeof(uint32_t) * batch_max));
-      TK_R(ensure(c, c->rl_vc, sizeof(uint32_t) * batch_max));
-      TK_R(ensure(c, c->rl_row_of, sizeof(uint32_t) * batch_max));
-      TK_R(ensure(c, c->rl_sort_tmp, sizeof(uint32_t) * rsort::temp_words(batch_max)));
+      TK_TRY(ensure(c, c->rl_ka, sizeof(uint64_t) * batch_max));
+      TK_TRY(ensure(c, c->rl_kb, sizeof(uint64_t) * batch_max));
+      TK_TRY(ensure(c, c->rl_kc, sizeof(uint64_t) * batch_max));
+      TK_TRY(ensure(c, c->rl_va, sizeof(uint32_t) * batch_max));
+      TK_TRY(ensure(c, c->rl_vb, sizeof(uint32_t) * batch_max));
+      TK_TRY(ensure(c, c->rl_vc, sizeof(uint32_t) * batch_max));
+      TK_TRY(ensure(c, c->rl_row_of, sizeof(uint32_t) * batch_max));
+      TK_TRY(ensure(c, c->rl_sort_tmp, sizeof(uint32_t) * rsort::temp_words(batch_max)));
       uint64_t *ka = c->rl_ka.as<uint64_t>(), *kb = c->rl_kb.as<uint64_t>(), *kc = c->rl_kc.as<uint64_t>();
       uint32_t *va = c->rl_va.as<uint32_t>(), *vb = c->rl_vb.as<uint32_t>(), *vc = c->rl_vc.as<uint32_t>();
       uint32_t* row_of = c->rl_row_of.as<uint32_t>();
@@ -2424,7 +2293,7 @@ int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* sel
         // by key (all 64 bits: 8 passes, so the result is back in ka / va) ...
         bool in_b = false;
         launches += 1 + rsort::sort_pairs(ka, va, kb, vb, e, c->rl_sort_tmp.as<uint32_t>(), c->sm_count, st, rsort::PASSES, &in_b);
-        if (in_b) { cleanup(); return fail(c, TKNN_ECUDA, "internal: odd key-sort pass count"); }
+        if (in_b) return fail(c, TKNN_ECUDA, "internal: odd key-sort pass count");
         // ... then stably by the row's rank in the batch
         radius::long_rowkey_kernel<<<blocks_for(e, 256), 256, 0, st>>>(va, row_of, e, kb, vb);
         const int row_bits = rows > 1 ? 32 - __builtin_clz(rows - 1) : 1;
@@ -2432,28 +2301,19 @@ int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* sel
                                           (row_bits + 7) / 8, &in_b);
         radius::long_emit_kernel<<<blocks_for(e, 256), 256, 0, st>>>(ka, in_b ? kc : kb, in_b ? vc : vb, e, long_pos, d_boff,
                                                                      first, qpts, off_row, c->squared, d_idx, d_dist);
-        TK_RC(cudaGetLastError());
+        TK_CUDA(c, cudaGetLastError());
         ++launches;
       }
     }
   }
-  TK_RC(cudaEventRecord(ev[11], st));
-  TK_RC(cudaEventRecord(ev[9], st));
-  TK_RC(cudaEventRecord(c->ev[2], st));
+  TK_CUDA(c, cudaEventRecord(ev[11], st));
+  TK_CUDA(c, cudaEventRecord(ev[9], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
   if (write_rows && total) {
-    if (!idx_dev) {
-      TK_RC(cudaMemcpyAsync(idx_out, d_idx, sizeof(int32_t) * total, cudaMemcpyDeviceToHost, st));
-      c->stats.d2h_bytes += sizeof(int32_t) * total;
-    }
-    if (dist_out && !dist_dev) {
-      TK_RC(cudaMemcpyAsync(dist_out, d_dist, sizeof(float) * total, cudaMemcpyDeviceToHost, st));
-      c->stats.d2h_bytes += sizeof(float) * total;
-    }
+    TK_TRY(copy_back(c, idx_out, d_idx, total, &c->stats.d2h_bytes));
+    TK_TRY(copy_back(c, dist_out, d_dist, total, &c->stats.d2h_bytes));
   }
-  TK_RC(cudaStreamSynchronize(st));
-  cleanup();
-#undef TK_R
-#undef TK_RC
+  TK_CUDA(c, cudaStreamSynchronize(st));
   TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
   c->stats.n_queries = nq;
   c->stats.rounds = 3;
@@ -2496,29 +2356,18 @@ int radius_query_core(tknn_ctx* c, const char* what, const float* queries, uint6
   reset_search_stats(c);
   if (nq == 0) {
     if (total_out) *total_out = 0;
-    if (is_device_ptr(offsets_out)) {
-      TK_CUDA(c, cudaMemsetAsync(offsets_out, 0, sizeof(uint64_t), c->stream));
-      TK_CUDA(c, cudaStreamSynchronize(c->stream));
-    } else {
-      offsets_out[0] = 0;
-    }
-    return TKNN_OK;
+    return zero_fill(c, offsets_out, 1);
   }
   TK_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  ScratchScope scratch = query_scratch(c);
   int launches = 0;
   const int32_t* d_sid_sorted = nullptr;
   const float* d_r2_sorted = nullptr;
   const uint32_t* d_seg_sorted = nullptr;
-  int rc = stage_queries(c, queries, nq, dim, stride_floats, self_ids, nullptr, &d_sid_sorted, &d_r2_sorted, &launches,
-                         q_seg_offsets, n_segments, &d_seg_sorted);
-  if (rc == TKNN_OK)
-    rc = radius_core(c, c->q_pts.as<float4>(), nq, d_sid_sorted, 0, d_seg_sorted, radius, offsets_out, idx_out, dist_out,
+  TK_TRY(stage_queries(c, queries, nq, dim, stride_floats, self_ids, nullptr, &d_sid_sorted, &d_r2_sorted, &launches,
+                       q_seg_offsets, n_segments, &d_seg_sorted));
+  return radius_core(c, c->q_pts.as<float4>(), nq, d_sid_sorted, 0, d_seg_sorted, radius, offsets_out, idx_out, dist_out,
                      capacity, total_out, launches);
-  if (!c->keep_scratch)
-    for (DevBuf* b : {&c->q_stage, &c->q_keys_a, &c->q_keys_b, &c->q_vals_a, &c->q_vals_b, &c->q_sort_tmp, &c->q_pts,
-                      &c->q_sid_stage, &c->q_sid_sorted, &c->q_seg_off, &c->q_seg_row, &c->q_seg_sorted})
-      release(*b);
-  return rc;
 }
 
 }  // namespace
@@ -2568,12 +2417,7 @@ int tknn_brute_force(tknn_ctx* c, const int32_t* query_ids, uint64_t nq, int k, 
   ScopedDevice sd(c->device);
   cudaStream_t st = c->stream;
   std::vector<int32_t> ids(nq);
-  if (is_device_ptr(query_ids)) {
-    TK_CUDA(c, cudaMemcpyAsync(ids.data(), query_ids, nq * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    TK_CUDA(c, cudaStreamSynchronize(st));
-  } else {
-    std::memcpy(ids.data(), query_ids, nq * sizeof(int32_t));
-  }
+  TK_TRY(read_to_host(c, query_ids, nq, ids.data()));
   std::vector<uint32_t> perm(nq);
   for (uint32_t i = 0; i < nq; ++i) perm[i] = i;
   std::sort(perm.begin(), perm.end(), [&](uint32_t a, uint32_t b) { return ids[a] < ids[b]; });
@@ -2584,29 +2428,22 @@ int tknn_brute_force(tknn_ctx* c, const int32_t* query_ids, uint64_t nq, int k, 
     if (i && sorted[i] == sorted[i - 1]) return fail(c, TKNN_EINVAL, "duplicate query id %d", sorted[i]);
   }
   DevBuf d_ids, d_perm, qpts, o_idx, o_dist;
-  auto cleanup = [&]() { for (DevBuf* b : {&d_ids, &d_perm, &qpts, &o_idx, &o_dist}) release(*b); };
-#define TK_B(expr) do { int rc_ = (expr); if (rc_ != TKNN_OK) { cleanup(); return rc_; } } while (0)
-#define TK_BC(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { cudaGetLastError(); cleanup(); \
-    return fail(c, e_ == cudaErrorMemoryAllocation ? TKNN_ENOMEM : TKNN_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_)); } } while (0)
-  TK_B(ensure(c, d_ids, nq * sizeof(int32_t)));
-  TK_B(ensure(c, d_perm, nq * sizeof(uint32_t)));
-  TK_B(ensure(c, qpts, nq * sizeof(float4)));
-  TK_BC(cudaMemcpyAsync(d_ids.p, sorted.data(), nq * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  TK_BC(cudaMemcpyAsync(d_perm.p, perm.data(), nq * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-  const bool idx_dev = is_device_ptr(idx_out), dist_dev = is_device_ptr(dist_out);
-  int32_t* d_idx = idx_out;
-  float* d_dist = dist_out;
-  if (!idx_dev) { TK_B(ensure(c, o_idx, nq * k * sizeof(int32_t))); d_idx = o_idx.as<int32_t>(); }
-  if (!dist_dev) { TK_B(ensure(c, o_dist, nq * k * sizeof(float))); d_dist = o_dist.as<float>(); }
+  ScratchScope scratch({&d_ids, &d_perm, &qpts, &o_idx, &o_dist});
+  TK_TRY(ensure(c, d_ids, nq * sizeof(int32_t)));
+  TK_TRY(ensure(c, d_perm, nq * sizeof(uint32_t)));
+  TK_TRY(ensure(c, qpts, nq * sizeof(float4)));
+  TK_CUDA(c, cudaMemcpyAsync(d_ids.p, sorted.data(), nq * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  TK_CUDA(c, cudaMemcpyAsync(d_perm.p, perm.data(), nq * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  int32_t* d_idx = nullptr;
+  float* d_dist = nullptr;
+  TK_TRY(out_view(c, idx_out, nq * k, o_idx, &d_idx));
+  TK_TRY(out_view(c, dist_out, nq * k, o_dist, &d_dist));
   brute::lookup_queries_kernel<<<blocks_for(c->n, 256), 256, 0, st>>>(c->pts.as<float4>(), c->n, d_ids.as<int32_t>(),
                                                                        (uint32_t)nq, qpts.as<float4>());
-  TK_B(brute_core(c, qpts.as<float4>(), nq, k, d_perm.as<uint32_t>(), d_idx, d_dist, 0));
-  if (!idx_dev) TK_BC(cudaMemcpyAsync(idx_out, d_idx, nq * k * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  if (!dist_dev) TK_BC(cudaMemcpyAsync(dist_out, d_dist, nq * k * sizeof(float), cudaMemcpyDeviceToHost, st));
-  TK_BC(cudaStreamSynchronize(st));
-  cleanup();
-#undef TK_B
-#undef TK_BC
+  TK_TRY(brute_core(c, qpts.as<float4>(), nq, k, d_perm.as<uint32_t>(), d_idx, d_dist, 0));
+  TK_TRY(copy_back(c, idx_out, d_idx, nq * k));
+  TK_TRY(copy_back(c, dist_out, d_dist, nq * k));
+  TK_CUDA(c, cudaStreamSynchronize(st));
   return TKNN_OK;
 }
 
@@ -2622,8 +2459,8 @@ int tknn::host::brute_core(tknn_ctx* c, const float4* d_qpts, uint64_t nq, int k
   int splits = (int)std::max<uint64_t>(1, std::min<uint64_t>(256, ((uint64_t)c->sm_count * 64 + groups - 1) / groups));
   splits = (int)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)splits, (c->n + 1023) / 1024));
   DevBuf partial;
-  int rc = ensure(c, partial, (size_t)splits * nq * k * sizeof(uint64_t));
-  if (rc != TKNN_OK) return rc;
+  ScratchScope scratch({&partial});
+  TK_TRY(ensure(c, partial, (size_t)splits * nq * k * sizeof(uint64_t)));
   const size_t smem = 32 * sizeof(float4) + (size_t)k * 32 * sizeof(uint64_t);
   cudaError_t e = cudaFuncSetAttribute(brute::brute_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(brute::merge_keys_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -2634,8 +2471,7 @@ int tknn::host::brute_core(tknn_ctx* c, const float4* d_qpts, uint64_t nq, int k
                                                                  d_idx, d_dist);
     e = cudaGetLastError();
   }
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // `partial` is released below
-  release(partial);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // `partial` is released on return
   if (e != cudaSuccess) { cudaGetLastError(); return fail(c, TKNN_ECUDA, "brute force: %s", cudaGetErrorString(e)); }
   return TKNN_OK;
 }
@@ -2673,28 +2509,21 @@ int tknn_sort_pairs(tknn_ctx* c, uint64_t* keys, uint32_t* values, uint64_t n) {
   if (n > rsort::MAX_N) return fail(c, TKNN_EINVAL, "n too large");
   ScopedDevice sd(c->device);
   cudaStream_t st = c->stream;
-  const bool kd = is_device_ptr(keys), vd = !values || is_device_ptr(values);  // values == nullptr: keys only
   DevBuf ka, kb, va, vb, tmp;
-  auto cleanup = [&]() { for (DevBuf* b : {&ka, &kb, &va, &vb, &tmp}) release(*b); };
-#define TK_B(expr) do { int rc_ = (expr); if (rc_ != TKNN_OK) { cleanup(); return rc_; } } while (0)
-#define TK_BC(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { cudaGetLastError(); cleanup(); \
-    return fail(c, e_ == cudaErrorMemoryAllocation ? TKNN_ENOMEM : TKNN_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_)); } } while (0)
-  uint64_t* dk = keys;
-  uint32_t* dv = values;
-  if (!kd) { TK_B(ensure(c, ka, n * sizeof(uint64_t))); dk = ka.as<uint64_t>(); TK_BC(cudaMemcpyAsync(dk, keys, n * 8, cudaMemcpyHostToDevice, st)); }
-  if (!vd) { TK_B(ensure(c, va, n * sizeof(uint32_t))); dv = va.as<uint32_t>(); TK_BC(cudaMemcpyAsync(dv, values, n * 4, cudaMemcpyHostToDevice, st)); }
-  TK_B(ensure(c, kb, n * sizeof(uint64_t)));
-  if (values) TK_B(ensure(c, vb, n * sizeof(uint32_t)));
-  TK_B(ensure(c, tmp, rsort::temp_words(n) * sizeof(uint32_t)));
+  ScratchScope scratch({&ka, &kb, &va, &vb, &tmp});
+  uint64_t* dk = nullptr;
+  uint32_t* dv = nullptr;  // values == nullptr: keys only
+  TK_TRY(stage_in(c, keys, n, ka, &dk));
+  TK_TRY(stage_in(c, values, n, va, &dv));
+  TK_TRY(ensure(c, kb, n * sizeof(uint64_t)));
+  if (values) TK_TRY(ensure(c, vb, n * sizeof(uint32_t)));
+  TK_TRY(ensure(c, tmp, rsort::temp_words(n) * sizeof(uint32_t)));
   if (values) rsort::sort_pairs(dk, dv, kb.as<uint64_t>(), vb.as<uint32_t>(), n, tmp.as<uint32_t>(), c->sm_count, st);
   else rsort::sort_keys(dk, kb.as<uint64_t>(), n, tmp.as<uint32_t>(), c->sm_count, st, 0, rsort::PASSES);
-  TK_BC(cudaGetLastError());
-  if (!kd) TK_BC(cudaMemcpyAsync(keys, dk, n * 8, cudaMemcpyDeviceToHost, st));
-  if (!vd) TK_BC(cudaMemcpyAsync(values, dv, n * 4, cudaMemcpyDeviceToHost, st));
-  TK_BC(cudaStreamSynchronize(st));
-  cleanup();
-#undef TK_B
-#undef TK_BC
+  TK_CUDA(c, cudaGetLastError());
+  TK_TRY(copy_back(c, keys, dk, n));
+  TK_TRY(copy_back(c, values, dv, n));
+  TK_CUDA(c, cudaStreamSynchronize(st));
   return TKNN_OK;
 }
 
@@ -2722,40 +2551,24 @@ int tknn_morton_codes(tknn_ctx* c, const float* xyz, uint64_t n, int dim, int st
   ScopedDevice sd(c->device);
   cudaStream_t st = c->stream;
   float hbox[6];
-  if (is_device_ptr(box6)) {
-    TK_CUDA(c, cudaMemcpyAsync(hbox, box6, sizeof(hbox), cudaMemcpyDeviceToHost, st));
-    TK_CUDA(c, cudaStreamSynchronize(st));
-  } else {
-    std::memcpy(hbox, box6, sizeof(hbox));
-  }
+  TK_TRY(read_to_host(c, box6, 6, hbox));
   // same order-preserving encoding the builder's bounds kernel produces
   auto enc = [](float f) { uint32_t b; std::memcpy(&b, &f, 4); return (b & 0x80000000u) ? ~b : (b | 0x80000000u); };
   uint32_t ob[8] = {enc(hbox[0]), enc(hbox[1]), enc(hbox[2]), enc(hbox[3]), enc(hbox[4]), enc(hbox[5]), 0u, 0u};
   DevBuf in, keys, vals, dob;
-  auto cleanup = [&]() { for (DevBuf* b : {&in, &keys, &vals, &dob}) release(*b); };
-#define TK_B(expr) do { int rc_ = (expr); if (rc_ != TKNN_OK) { cleanup(); return rc_; } } while (0)
-#define TK_BC(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { cudaGetLastError(); cleanup(); \
-    return fail(c, e_ == cudaErrorMemoryAllocation ? TKNN_ENOMEM : TKNN_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_)); } } while (0)
-  const float* d_xyz = xyz;
-  if (!is_device_ptr(xyz)) {
-    TK_B(ensure(c, in, (size_t)n * stride_floats * sizeof(float)));
-    TK_BC(cudaMemcpyAsync(in.p, xyz, (size_t)n * stride_floats * sizeof(float), cudaMemcpyHostToDevice, st));
-    d_xyz = in.as<float>();
-  }
-  const bool out_dev = is_device_ptr(codes_out);
-  uint64_t* d_keys = codes_out;
-  if (!out_dev) { TK_B(ensure(c, keys, n * sizeof(uint64_t))); d_keys = keys.as<uint64_t>(); }
-  TK_B(ensure(c, vals, n * sizeof(uint32_t)));
-  TK_B(ensure(c, dob, sizeof(ob)));
-  TK_BC(cudaMemcpyAsync(dob.p, ob, sizeof(ob), cudaMemcpyHostToDevice, st));
+  ScratchScope scratch({&in, &keys, &vals, &dob});
+  const float* d_xyz = nullptr;
+  uint64_t* d_keys = nullptr;
+  TK_TRY(stage_in(c, xyz, (size_t)n * stride_floats, in, &d_xyz));
+  TK_TRY(out_view(c, codes_out, n, keys, &d_keys));
+  TK_TRY(ensure(c, vals, n * sizeof(uint32_t)));
+  TK_TRY(ensure(c, dob, sizeof(ob)));
+  TK_CUDA(c, cudaMemcpyAsync(dob.p, ob, sizeof(ob), cudaMemcpyHostToDevice, st));
   lbvh::morton_kernel<<<blocks_for(n, lbvh::THREADS), lbvh::THREADS, 0, st>>>(d_xyz, n, dim, stride_floats, dob.as<uint32_t>(), 21,
                                                                              0, 0, d_keys, vals.as<uint32_t>());
-  TK_BC(cudaGetLastError());
-  if (!out_dev) TK_BC(cudaMemcpyAsync(codes_out, d_keys, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-  TK_BC(cudaStreamSynchronize(st));
-  cleanup();
-#undef TK_B
-#undef TK_BC
+  TK_CUDA(c, cudaGetLastError());
+  TK_TRY(copy_back(c, codes_out, d_keys, n));
+  TK_CUDA(c, cudaStreamSynchronize(st));
   return TKNN_OK;
 }
 
@@ -2782,19 +2595,14 @@ int tknn_generate_uniform(tknn_ctx* c, uint64_t seed, uint64_t first, uint64_t n
   if (n == 0) return TKNN_OK;
   if (!xyz_out) return fail(c, TKNN_EINVAL, "null output array");
   ScopedDevice sd(c->device);
-  const bool dev = is_device_ptr(xyz_out);
   DevBuf tmp;
-  float* d = xyz_out;
-  if (!dev) {
-    int rc = ensure(c, tmp, 3 * n * sizeof(float));
-    if (rc != TKNN_OK) return rc;
-    d = tmp.as<float>();
-  }
+  ScratchScope scratch({&tmp});
+  float* d = nullptr;
+  TK_TRY(out_view(c, xyz_out, 3 * n, tmp, &d));
   brute::generate_uniform_kernel<<<blocks_for(3 * n, 256), 256, 0, c->stream>>>(seed, first, n, d);
   cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess && !dev) e = cudaMemcpyAsync(xyz_out, d, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
+  if (e == cudaSuccess && d != xyz_out) e = cudaMemcpyAsync(xyz_out, d, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  release(tmp);
   if (e != cudaSuccess) return fail(c, TKNN_ECUDA, "generate_uniform: %s", cudaGetErrorString(e));
   return TKNN_OK;
 }
@@ -2806,9 +2614,9 @@ int tknn_measure_bandwidth(tknn_ctx* c, double* l2_gbs, double* hbm_gbs, int* sm
   if (l2_bytes) *l2_bytes = c->l2_bytes;
   cudaStream_t st = c->stream;
   DevBuf buf;
+  ScratchScope scratch({&buf});
   const size_t big = (size_t)2 << 30;  // HBM-sized: 2 GiB >> L2
-  int rc = ensure(c, buf, big);
-  if (rc != TKNN_OK) return rc;
+  TK_TRY(ensure(c, buf, big));
   cudaError_t e = cudaMemsetAsync(buf.p, 1, big, st);
   uint32_t* sink = c->scalars.as<uint32_t>() + SC_WORDS - 1;
   const unsigned grid = (unsigned)c->sm_count * 16;
@@ -2833,7 +2641,6 @@ int tknn_measure_bandwidth(tknn_ctx* c, double* l2_gbs, double* hbm_gbs, int* sm
     run(big, 1, hbm_gbs);
     e = cudaGetLastError();
   }
-  release(buf);
   if (e != cudaSuccess) return fail(c, TKNN_ECUDA, "measure_bandwidth: %s", cudaGetErrorString(e));
   return TKNN_OK;
 }
@@ -2926,13 +2733,8 @@ int tknn_voxel_grid(tknn_ctx* c, const float* points, uint64_t n, int dim, int s
     return TKNN_OK;
   }
   const bool batched = seg_offsets != nullptr;
-  const float* d_pts = points;
-  if (!is_device_ptr(points)) {
-    const size_t bytes = ((size_t)(n - 1) * stride_floats + dim) * sizeof(float);
-    TK_TRY(ensure(c, c->vx_pts, bytes));
-    TK_CUDA(c, cudaMemcpyAsync(c->vx_pts.p, points, bytes, cudaMemcpyHostToDevice, st));
-    d_pts = c->vx_pts.as<float>();
-  }
+  const float* d_pts = nullptr;
+  TK_TRY(stage_in(c, points, (size_t)(n - 1) * stride_floats + dim, c->vx_pts, &d_pts));
   if (batched) {
     TK_TRY(ensure(c, c->vx_seg_off, off.size() * sizeof(uint64_t)));
     TK_CUDA(c, cudaMemcpyAsync(c->vx_seg_off.p, off.data(), off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
@@ -3096,17 +2898,10 @@ int tknn_voxel_pool(tknn_ctx* c, const float* x, uint64_t n, int f, int stride_f
   if (!x || !out) return fail(c, TKNN_EINVAL, "%s: null x or out", what);
   ScopedDevice sd(c->device);
   cudaStream_t st = c->stream;
-  const float* d_x = x;
-  if (!is_device_ptr(x)) {
-    const size_t bytes = ((size_t)(n - 1) * stride_floats + f) * sizeof(float);
-    TK_TRY(ensure(c, c->vx_x, bytes));
-    TK_CUDA(c, cudaMemcpyAsync(c->vx_x.p, x, bytes, cudaMemcpyHostToDevice, st));
-    d_x = c->vx_x.as<float>();
-  }
-  const bool out_dev = is_device_ptr(out);
-  const size_t out_bytes = nv * (size_t)f * sizeof(float);
-  if (!out_dev) TK_TRY(ensure(c, c->vx_out, out_bytes));
-  float* d_out = out_dev ? out : c->vx_out.as<float>();
+  const float* d_x = nullptr;
+  float* d_out = nullptr;
+  TK_TRY(stage_in(c, x, (size_t)(n - 1) * stride_floats + f, c->vx_x, &d_x));
+  TK_TRY(out_view(c, out, nv * (size_t)f, c->vx_out, &d_out));
   uint32_t* w = c->vx_words_sc.as<uint32_t>();
   const bool mx = reduce == TKNN_REDUCE_MAX;
   if (mx) {
@@ -3136,7 +2931,7 @@ int tknn_voxel_pool(tknn_ctx* c, const float* x, uint64_t n, int f, int stride_f
     }
     TK_CUDA(c, cudaGetLastError());
   }
-  if (!out_dev) TK_CUDA(c, cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, st));
+  TK_TRY(copy_back(c, out, d_out, nv * (size_t)f));
   if (mx) {
     uint32_t bad = 0;
     TK_TRY(fetch_words(c, w + 8, 1, nullptr, 0, &bad));
@@ -3159,72 +2954,28 @@ unsigned interp_blocks(tknn_ctx* c, uint64_t threads) {
                                                             (uint64_t)c->sm_count * 16));
 }
 
-// a device pointer to `bytes` of the caller's input: the pointer itself, or a copy of host memory in `stage`
-int interp_in(tknn_ctx* c, const void* p, size_t bytes, DevBuf& stage, const void** d) {
-  if (is_device_ptr(p)) {
-    *d = p;
-    return TKNN_OK;
-  }
-  TK_TRY(ensure(c, stage, bytes));
-  TK_CUDA(c, cudaMemcpyAsync(stage.p, p, bytes, cudaMemcpyHostToDevice, c->stream));
-  *d = stage.p;
-  return TKNN_OK;
-}
-
-// the device buffer an output is written to: the caller's array, or `stage` (copied back by interp_out)
-int interp_out_buf(tknn_ctx* c, void* p, size_t bytes, DevBuf& stage, void** d) {
-  if (!p || is_device_ptr(p)) {
-    *d = p;
-    return TKNN_OK;
-  }
-  TK_TRY(ensure(c, stage, bytes));
-  *d = stage.p;
-  return TKNN_OK;
-}
-
-int interp_out(tknn_ctx* c, void* p, const void* d, size_t bytes) {
-  if (p && p != d) TK_CUDA(c, cudaMemcpyAsync(p, d, bytes, cudaMemcpyDeviceToHost, c->stream));
-  return TKNN_OK;
-}
-
-void interp_release(tknn_ctx* c) {
-  if (c->keep_scratch) return;
-  for (DevBuf* b : {&c->ip_idx, &c->ip_w, &c->ip_den, &c->ip_x, &c->ip_out, &c->ip_wout, &c->ip_dout, &c->ip_keys_a,
-                    &c->ip_keys_b, &c->ip_vals_a, &c->ip_vals_b, &c->ip_sort_tmp, &c->ip_cnt, &c->ip_off, &c->rl_sums})
-    release(*b);
-}
-
-int interp_events(tknn_ctx* c, size_t count) {
-  for (size_t i = c->round_ev.size(); i < count; ++i) {
-    cudaEvent_t e;
-    TK_CUDA(c, cudaEventCreate(&e));
-    c->round_ev.push_back(e);
-  }
-  return TKNN_OK;
-}
-
 int interpolate_core(tknn_ctx* c, const int32_t* idx, const float* d2, uint64_t nq, int k, const float* x, uint64_t n,
                      int f, int x_stride, float* out, float* weight_out, float* den_out) {
   const char* what = "tknn_interpolate";
   cudaStream_t st = c->stream;
   const size_t slots = (size_t)nq * k;
-  const void *d_idx, *d_d2, *d_x = nullptr;
-  TK_TRY(interp_in(c, idx, slots * sizeof(int32_t), c->ip_idx, &d_idx));
-  TK_TRY(interp_in(c, d2, slots * sizeof(float), c->ip_w, &d_d2));
-  if (n) TK_TRY(interp_in(c, x, ((size_t)(n - 1) * x_stride + f) * sizeof(float), c->ip_x, &d_x));
-  void *d_out, *d_w, *d_den;
-  TK_TRY(interp_out_buf(c, out, (size_t)nq * f * sizeof(float), c->ip_out, &d_out));
-  TK_TRY(interp_out_buf(c, weight_out, slots * sizeof(float), c->ip_wout, &d_w));
-  TK_TRY(interp_out_buf(c, den_out, nq * sizeof(float), c->ip_dout, &d_den));
-  TK_TRY(interp_events(c, 4));
+  ScratchScope scratch = interp_scratch(c);
+  const int32_t* d_idx = nullptr;
+  const float *d_d2 = nullptr, *d_x = nullptr;
+  TK_TRY(stage_in(c, idx, slots, c->ip_idx, &d_idx));
+  TK_TRY(stage_in(c, d2, slots, c->ip_w, &d_d2));
+  if (n) TK_TRY(stage_in(c, x, (size_t)(n - 1) * x_stride + f, c->ip_x, &d_x));
+  float *d_out = nullptr, *d_w = nullptr, *d_den = nullptr;
+  TK_TRY(out_view(c, out, (size_t)nq * f, c->ip_out, &d_out));
+  TK_TRY(out_view(c, weight_out, slots, c->ip_wout, &d_w));
+  TK_TRY(out_view(c, den_out, nq, c->ip_dout, &d_den));
+  TK_TRY(ensure_round_events(c, 4));
   cudaEvent_t* ev = c->round_ev.data();
   uint32_t* sc = c->scalars.as<uint32_t>();
   TK_CUDA(c, cudaEventRecord(c->ev[0], st));
   TK_CUDA(c, cudaEventRecord(ev[0], st));
   TK_CUDA(c, cudaMemsetAsync(sc + SC_QBAD, 0, sizeof(uint32_t), st));
-  interp::FwdParams P{static_cast<const int32_t*>(d_idx), static_cast<const float*>(d_d2), static_cast<const float*>(d_x),
-                      nq, (uint32_t)n, k, f, x_stride, static_cast<float*>(d_out), static_cast<float*>(d_w),
-                      static_cast<float*>(d_den), sc + SC_QBAD};
+  interp::FwdParams P{d_idx, d_d2, d_x, nq, (uint32_t)n, k, f, x_stride, d_out, d_w, d_den, sc + SC_QBAD};
   const int G = interp::group_of(f);
   const unsigned blocks = interp_blocks(c, nq * (uint64_t)G);
   TK_CUDA(c, cudaEventRecord(ev[2], st));
@@ -3238,9 +2989,9 @@ int interpolate_core(tknn_ctx* c, const int32_t* idx, const float* d2, uint64_t 
   TK_CUDA(c, cudaEventRecord(ev[3], st));
   TK_CUDA(c, cudaEventRecord(ev[1], st));
   TK_CUDA(c, cudaEventRecord(c->ev[2], st));
-  TK_TRY(interp_out(c, out, d_out, (size_t)nq * f * sizeof(float)));
-  TK_TRY(interp_out(c, weight_out, d_w, slots * sizeof(float)));
-  TK_TRY(interp_out(c, den_out, d_den, nq * sizeof(float)));
+  TK_TRY(copy_back(c, out, d_out, (size_t)nq * f));
+  TK_TRY(copy_back(c, weight_out, d_w, slots));
+  TK_TRY(copy_back(c, den_out, d_den, nq));
   TK_CUDA(c, cudaEventRecord(c->ev[3], st));
   uint32_t bad = 0;
   TK_TRY(fetch_words(c, sc + SC_QBAD, 1, nullptr, 0, &bad));  // synchronises the stream
@@ -3259,13 +3010,15 @@ int interpolate_backward_core(tknn_ctx* c, const int32_t* idx, const float* weig
   const char* what = "tknn_interpolate_backward";
   cudaStream_t st = c->stream;
   const uint64_t edges = nq * (uint64_t)k;
-  const void *d_idx, *d_w, *d_den, *d_g;
-  TK_TRY(interp_in(c, idx, edges * sizeof(int32_t), c->ip_idx, &d_idx));
-  TK_TRY(interp_in(c, weight, edges * sizeof(float), c->ip_w, &d_w));
-  TK_TRY(interp_in(c, den, nq * sizeof(float), c->ip_den, &d_den));
-  TK_TRY(interp_in(c, grad_out, ((size_t)(nq - 1) * g_stride + f) * sizeof(float), c->ip_x, &d_g));
-  void* d_gx = nullptr;
-  if (n) TK_TRY(interp_out_buf(c, grad_x, (size_t)n * f * sizeof(float), c->ip_out, &d_gx));
+  ScratchScope scratch = interp_scratch(c);
+  const int32_t* d_idx = nullptr;
+  const float *d_w = nullptr, *d_den = nullptr, *d_g = nullptr;
+  TK_TRY(stage_in(c, idx, edges, c->ip_idx, &d_idx));
+  TK_TRY(stage_in(c, weight, edges, c->ip_w, &d_w));
+  TK_TRY(stage_in(c, den, nq, c->ip_den, &d_den));
+  TK_TRY(stage_in(c, grad_out, (size_t)(nq - 1) * g_stride + f, c->ip_x, &d_g));
+  float* d_gx = nullptr;
+  if (n) TK_TRY(out_view(c, grad_x, (size_t)n * f, c->ip_out, &d_gx));
   TK_TRY(ensure(c, c->ip_keys_a, edges * sizeof(uint64_t)));
   TK_TRY(ensure(c, c->ip_keys_b, edges * sizeof(uint64_t)));
   TK_TRY(ensure(c, c->ip_vals_a, edges * sizeof(uint32_t)));
@@ -3273,7 +3026,7 @@ int interpolate_backward_core(tknn_ctx* c, const int32_t* idx, const float* weig
   TK_TRY(ensure(c, c->ip_sort_tmp, rsort::temp_words(edges) * sizeof(uint32_t)));
   TK_TRY(ensure(c, c->ip_cnt, n * sizeof(uint32_t)));
   TK_TRY(ensure(c, c->ip_off, (n + 1) * sizeof(uint64_t)));
-  TK_TRY(interp_events(c, 12));
+  TK_TRY(ensure_round_events(c, 12));
   cudaEvent_t* ev = c->round_ev.data();  // phase r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its kernels
   uint32_t* sc = c->scalars.as<uint32_t>();
   int launches = 0;
@@ -3285,7 +3038,7 @@ int interpolate_backward_core(tknn_ctx* c, const int32_t* idx, const float* weig
   if (n) TK_CUDA(c, cudaMemsetAsync(c->ip_cnt.p, 0, n * sizeof(uint32_t), st));
   TK_CUDA(c, cudaEventRecord(ev[2], st));
   interp::edge_kernel<<<interp_blocks(c, edges), interp::THREADS, 0, st>>>(
-      static_cast<const int32_t*>(d_idx), edges, (uint32_t)n, c->ip_keys_a.as<uint64_t>(), c->ip_vals_a.as<uint32_t>(),
+      d_idx, edges, (uint32_t)n, c->ip_keys_a.as<uint64_t>(), c->ip_vals_a.as<uint32_t>(),
       c->ip_cnt.as<uint32_t>(), sc + SC_QBAD);
   TK_CUDA(c, cudaGetLastError());
   ++launches;
@@ -3312,9 +3065,8 @@ int interpolate_backward_core(tknn_ctx* c, const int32_t* idx, const float* weig
     uint64_t* off = c->ip_off.as<uint64_t>();
     TK_TRY(scan_counts(c, c->ip_cnt.as<uint32_t>(), n, off, off + n, &launches));
     const int G = interp::group_of(f);
-    interp::BwdParams P{in_b ? c->ip_vals_b.as<uint32_t>() : c->ip_vals_a.as<uint32_t>(), off,
-                        static_cast<const float*>(d_w), static_cast<const float*>(d_den), static_cast<const float*>(d_g),
-                        (uint32_t)n, k, f, g_stride, (f + G - 1) / G, static_cast<float*>(d_gx)};
+    interp::BwdParams P{in_b ? c->ip_vals_b.as<uint32_t>() : c->ip_vals_a.as<uint32_t>(), off, d_w, d_den, d_g,
+                        (uint32_t)n, k, f, g_stride, (f + G - 1) / G, d_gx};
     const unsigned blocks = interp_blocks(c, n * (uint64_t)P.blocks * G);
     TK_CUDA(c, cudaEventRecord(ev[10], st));
     switch (G) {
@@ -3332,7 +3084,7 @@ int interpolate_backward_core(tknn_ctx* c, const int32_t* idx, const float* weig
   }
   TK_CUDA(c, cudaEventRecord(ev[9], st));
   TK_CUDA(c, cudaEventRecord(c->ev[2], st));
-  if (n) TK_TRY(interp_out(c, grad_x, d_gx, (size_t)n * f * sizeof(float)));
+  if (n) TK_TRY(copy_back(c, grad_x, d_gx, (size_t)n * f));
   TK_CUDA(c, cudaEventRecord(c->ev[3], st));
   uint32_t bad = 0;
   TK_TRY(fetch_words(c, sc + SC_QBAD, 1, nullptr, 0, &bad));  // synchronises the stream
@@ -3372,9 +3124,7 @@ int tknn_interpolate(tknn_ctx* c, const int32_t* idx, const float* d2, uint64_t 
   c->stats.n_queries = nq;
   c->stats.k = k;
   if (nq == 0) return TKNN_OK;
-  const int rc = interpolate_core(c, idx, d2, nq, k, x, n, f, x_stride_floats, out, weight_out, den_out);
-  interp_release(c);
-  return rc;
+  return interpolate_core(c, idx, d2, nq, k, x, n, f, x_stride_floats, out, weight_out, den_out);
 }
 
 int tknn_interpolate_backward(tknn_ctx* c, const int32_t* idx, const float* weight, const float* den, uint64_t nq, int k,
@@ -3392,19 +3142,10 @@ int tknn_interpolate_backward(tknn_ctx* c, const int32_t* idx, const float* weig
   c->stats.n_queries = nq;
   c->stats.k = k;
   if (nq == 0) {  // no edge: every row of grad_x is +0
-    if (n && grad_x) {
-      if (is_device_ptr(grad_x)) {
-        TK_CUDA(c, cudaMemsetAsync(grad_x, 0, (size_t)n * f * sizeof(float), c->stream));
-        TK_CUDA(c, cudaStreamSynchronize(c->stream));
-      } else {
-        std::memset(grad_x, 0, (size_t)n * f * sizeof(float));
-      }
-    }
+    if (n && grad_x) TK_TRY(zero_fill(c, grad_x, (size_t)n * f));
     return TKNN_OK;
   }
-  const int rc = interpolate_backward_core(c, idx, weight, den, nq, k, grad_out, g_stride_floats, n, f, grad_x);
-  interp_release(c);
-  return rc;
+  return interpolate_backward_core(c, idx, weight, den, nq, k, grad_out, g_stride_floats, n, f, grad_x);
 }
 
 }  // extern "C"
