@@ -28,9 +28,9 @@ def _is_tensor(a) -> bool:
     return hasattr(a, "data_ptr") and hasattr(a, "is_cuda")
 
 
-def _ptr(a):
-    """Raw address of a numpy array or torch tensor (None -> NULL)."""
-    if a is None:
+def _ptr(a, null_if_empty: bool = False):
+    """Raw address of a numpy array or torch tensor (None -> NULL; with null_if_empty, an array without rows too)."""
+    if a is None or (null_if_empty and a.shape[0] == 0):
         return None
     if _is_tensor(a):
         if not a.is_contiguous():
@@ -41,16 +41,78 @@ def _ptr(a):
     return C.c_void_p(a.ctypes.data)
 
 
+def _torch_dtype(np_dtype):
+    """The tensor dtype of an array the library reads or writes as np_dtype: uint32 and uint64 arrays travel as int32 and
+    int64 tensors."""
+    import torch
+
+    return {np.float32: torch.float32, np.int32: torch.int32, np.uint32: torch.int32, np.int64: torch.int64,
+            np.uint64: torch.int64, np.uint8: torch.uint8}[np_dtype]
+
+
 def _check_dtype(a, np_dtype, name):
+    """TypeError naming `name` unless `a` (None passes) holds np_dtype, or its tensor dtype (torch.uint32 for uint32 too)."""
+    if a is None:
+        return
     if _is_tensor(a):
         import torch
 
-        want = {np.float32: torch.float32, np.int32: torch.int32, np.uint32: torch.int32, np.uint64: torch.int64,
-                np.uint8: torch.uint8}[np_dtype]
+        want = _torch_dtype(np_dtype)
         if a.dtype != want and not (np_dtype is np.uint32 and a.dtype == torch.uint32):
             raise TypeError(f"{name}: expected {want}, got {a.dtype}")
     elif a.dtype != np_dtype:
         raise TypeError(f"{name}: expected {np.dtype(np_dtype)}, got {a.dtype}")
+
+
+def _arg(a, np_dtype, name, ndim: int | None = None, cast: bool = True, copy: bool = False):
+    """An input array (None passes) ready for _ptr: anything numpy takes becomes a C-contiguous array, cast to np_dtype
+    unless cast is False (then another dtype raises); a tensor is passed in place, or as a contiguous copy when copy is
+    set (otherwise _ptr refuses a non-contiguous one).  TypeError for another dtype, ValueError for another rank."""
+    if a is None:
+        return None
+    if _is_tensor(a):
+        a = a.contiguous() if copy else a
+    else:
+        a = np.ascontiguousarray(a, dtype=np_dtype if cast else None)
+    _check_dtype(a, np_dtype, name)
+    if ndim is not None and a.ndim != ndim:
+        raise ValueError(f"{name} must be {ndim}-D, got shape {tuple(a.shape)}")
+    return a
+
+
+def _points(a, name, dim: int | None = None):
+    """Positions [n, stride] float32 as the LBVH calls take them: (array, n, dim, stride), dim = min(stride, 3) unless
+    given, so columns beyond the third are skipped through the stride."""
+    a = _arg(a, np.float32, name, ndim=2)
+    stride = int(a.shape[1])
+    return a, int(a.shape[0]), min(stride, 3) if dim is None else int(dim), stride
+
+
+def _empty_like_rows(like, shape, np_dtype):
+    """An uninitialised array of `shape` beside `like`: a tensor on its device, or numpy."""
+    if _is_tensor(like):
+        import torch
+
+        return torch.empty(shape, dtype=_torch_dtype(np_dtype), device=like.device)
+    return np.empty(shape, np_dtype)
+
+
+def _zeros_like_rows(like, shape, np_dtype):
+    """_empty_like_rows, filled with zeros."""
+    if _is_tensor(like):
+        import torch
+
+        return torch.zeros(shape, dtype=_torch_dtype(np_dtype), device=like.device)
+    return np.zeros(shape, np_dtype)
+
+
+def _arange_like(like, n: int, np_dtype=np.int64):
+    """0 .. n - 1 beside `like`: a tensor on its device, or numpy."""
+    if _is_tensor(like):
+        import torch
+
+        return torch.arange(n, dtype=_torch_dtype(np_dtype), device=like.device)
+    return np.arange(n, dtype=np_dtype)
 
 
 class TrueKNN:
@@ -64,14 +126,18 @@ class TrueKNN:
             raise TrueKNNError(rc, f"tknn_create(device={device}) failed — a CUDA sm_100 device is required, "
                                    "there is no CPU fallback")
         self._h = h
+        self._init_state(device)
+        for k, v in options.items():
+            self.set_option(k, v)
+
+    def _init_state(self, device: int):
         self.device = int(device)
         self._own_stream = True  # until set_stream() hands over a caller stream
         self.n = 0
         self.n_segments = 1  # clouds of the last build (batch_size of query(batch=...) / radius_query(batch=...))
         self._offsets = None  # the cloud offsets of a segmented build (numpy or a tensor), None for a plain build
-        self._like = None
-        for k, v in options.items():
-            self.set_option(k, v)
+        self._like = None  # the last build's points: outputs of searches on it follow their kind and device
+        self._vx_like = None  # the points of the last voxel_grid(), None before the first
 
     # ---- plumbing ----
     def _check(self, rc: int):
@@ -127,37 +193,31 @@ class TrueKNN:
             handle = cuda_stream
         self._check(self._L.tknn_set_stream(self._h, C.c_void_p(handle)))
 
-    def _in(self, a):
-        """Pointer of an INPUT array.  While the context runs on its own stream, a CUDA tensor produced by
-        torch on another stream must be complete before the library reads it: settle torch's current stream."""
-        if a is not None and _is_tensor(a) and a.is_cuda and self._own_stream:
+    def _settle(self, a):
+        """While the context runs on its OWN stream, nothing orders torch's current stream before the library's work:
+        a CUDA tensor torch produced there must be complete before the library reads it, and the caching allocator may
+        hand back, as an output, a block that a kernel still pending there uses.  Settle torch's stream (nothing to do
+        when the context was given torch's stream with set_stream)."""
+        if self._own_stream and _is_tensor(a) and a.is_cuda:
             import torch
 
             torch.cuda.current_stream(a.device).synchronize()
-        return _ptr(a)
+
+    def _in(self, a, null_if_empty: bool = False):
+        """Pointer of an INPUT array (see _settle)."""
+        self._settle(a)
+        return _ptr(a, null_if_empty)
+
+    def _empty(self, like, shape, np_dtype):
+        """An OUTPUT array of `shape` beside `like` (a tensor on its device, or numpy), settled (see _settle)."""
+        out = _empty_like_rows(like, shape, np_dtype)
+        self._settle(out)
+        return out
 
     def stats(self) -> dict:
         s = Stats()
         self._check(self._L.tknn_get_stats(self._h, C.byref(s)))
         return s.as_dict()
-
-    def _out(self, like, rows, k, dtype):
-        if _is_tensor(like):
-            import torch
-
-            out = torch.empty((rows, k), dtype={np.int32: torch.int32, np.float32: torch.float32}[dtype], device=like.device)
-            self._settle_outputs(out)
-            return out
-        return np.empty((rows, k), dtype)
-
-    def _settle_outputs(self, t):
-        """The caching allocator may hand back a block that a kernel still pending on torch's current stream uses.
-        While the context runs on its OWN stream nothing orders that kernel before the engine's writes: settle torch's
-        stream first (a no-op cost when the context was given torch's stream with set_stream)."""
-        if self._own_stream and _is_tensor(t) and t.is_cuda:
-            import torch
-
-            torch.cuda.current_stream(t.device).synchronize()
 
     # ---- the path ----
     def build(self, points, dim: int | None = None, batch=None, batch_size: int | None = None):
@@ -170,27 +230,20 @@ class TrueKNN:
         batch): the number of clouds, for trailing clouds without points.  A separate query set of a batch takes
         query(..., batch=) / radius_query(..., batch=); without a batch they, search_shard(), dbscan() and brute_force()
         raise TrueKNNError (TKNN_ESTATE) on such a build."""
-        if not _is_tensor(points):
-            points = np.ascontiguousarray(points, dtype=np.float32)
-        _check_dtype(points, np.float32, "points")
-        if points.ndim != 2:
-            raise ValueError("points must be [n, >=dim]")
-        stride = int(points.shape[1])
-        if dim is None:
-            dim = min(stride, 3)
+        points, n, dim, stride = _points(points, "points", dim)
         if batch is None:
             if batch_size is not None:
                 raise ValueError("batch_size needs a batch")
-            self._check(self._L.tknn_build(self._h, self._in(points), int(points.shape[0]), int(dim), stride))
+            self._check(self._L.tknn_build(self._h, self._in(points), n, dim, stride))
             self.n_segments = 1
             self._offsets = None
         else:
-            offsets = batch_to_offsets(batch, int(points.shape[0]), batch_size)
-            self._check(self._L.tknn_build_segments(self._h, self._in(points), int(points.shape[0]), int(dim), stride,
-                                                    self._in(offsets), int(offsets.shape[0]) - 1))
+            offsets = batch_to_offsets(batch, n, batch_size)
+            self._check(self._L.tknn_build_segments(self._h, self._in(points), n, dim, stride, self._in(offsets),
+                                                    int(offsets.shape[0]) - 1))
             self.n_segments = int(offsets.shape[0]) - 1
             self._offsets = offsets
-        self.n = int(points.shape[0])
+        self.n = n
         self._like = points
         return self
 
@@ -198,14 +251,13 @@ class TrueKNN:
         """All-points kNN. Returns (idx [n,k] int32, dist [n,k] float32), rows in build order.
         indices_only (or out = (idx, None)): dist_out = NULL — no distances are returned or copied."""
         if out is None:
-            idx = self._out(self._like, self.n, k, np.int32)
-            dist = None if indices_only else self._out(self._like, self.n, k, np.float32)
+            idx = self._empty(self._like, (self.n, k), np.int32)
+            dist = None if indices_only else self._empty(self._like, (self.n, k), np.float32)
         else:
             idx, dist = out
         _check_dtype(idx, np.int32, "idx_out")
-        if dist is not None:
-            _check_dtype(dist, np.float32, "dist_out")
-        self._check(self._L.tknn_search(self._h, int(k), C.c_float(start_radius), _ptr(idx), _ptr(dist) if dist is not None else None))
+        _check_dtype(dist, np.float32, "dist_out")
+        self._check(self._L.tknn_search(self._h, int(k), C.c_float(start_radius), _ptr(idx), _ptr(dist)))
         return idx, dist
 
     def shard_capacity(self, n_shards: int) -> int:
@@ -215,14 +267,9 @@ class TrueKNN:
         """Query-sharded search: returns (qid [m], idx [m,k], dist [m,k]) for this shard's Morton slice."""
         cap = self.shard_capacity(n_shards)
         if out is None:
-            if _is_tensor(self._like):
-                import torch
-
-                qid = torch.empty((cap,), dtype=torch.int32, device=self._like.device)
-            else:
-                qid = np.empty((cap,), np.int32)
-            idx = self._out(self._like, cap, k, np.int32)
-            dist = self._out(self._like, cap, k, np.float32)
+            qid = self._empty(self._like, (cap,), np.int32)
+            idx = self._empty(self._like, (cap, k), np.int32)
+            dist = self._empty(self._like, (cap, k), np.float32)
         else:
             qid, idx, dist = out
         m = C.c_uint64(0)
@@ -237,36 +284,25 @@ class TrueKNN:
         init_radius2: optional per-query cap on the squared distance (closed; negative = none).
         batch (after build(batch=...)): the cloud id of every query, as build()'s; the queries of cloud c search the points
         of cloud c only (tknn_query_segments), and a query whose cloud has too few points ends in -1 / FLT_MAX."""
-        if not _is_tensor(queries):
-            queries = np.ascontiguousarray(queries, dtype=np.float32)
-        _check_dtype(queries, np.float32, "queries")
-        nq, stride = int(queries.shape[0]), int(queries.shape[1])
-        if dim is None:
-            dim = min(stride, 3)
-        if self_ids is not None and not _is_tensor(self_ids):
-            self_ids = np.ascontiguousarray(self_ids, dtype=np.int32)
-        if init_radius2 is not None and not _is_tensor(init_radius2):
-            init_radius2 = np.ascontiguousarray(init_radius2, dtype=np.float32)
-        idx = self._out(queries, nq, k, np.int32)
-        dist = self._out(queries, nq, k, np.float32)
+        queries, nq, dim, stride = _points(queries, "queries", dim)
+        self_ids = _arg(self_ids, np.int32, "self_ids")
+        init_radius2 = _arg(init_radius2, np.float32, "init_radius2")
+        idx = self._empty(queries, (nq, k), np.int32)
+        dist = self._empty(queries, (nq, k), np.float32)
         if batch is None:
-            self._check(self._L.tknn_query(self._h, self._in(queries), nq, int(dim), stride, self._in(self_ids), self._in(init_radius2), int(k),
-                                           C.c_float(start_radius), _ptr(idx), _ptr(dist)))
+            self._check(self._L.tknn_query(self._h, self._in(queries), nq, dim, stride, self._in(self_ids),
+                                           self._in(init_radius2), int(k), C.c_float(start_radius), _ptr(idx), _ptr(dist)))
         else:
             offsets = batch_to_offsets(batch, nq, self.n_segments)
-            self._check(self._L.tknn_query_segments(self._h, self._in(queries), nq, int(dim), stride, self._in(offsets),
+            self._check(self._L.tknn_query_segments(self._h, self._in(queries), nq, dim, stride, self._in(offsets),
                                                     int(offsets.shape[0]) - 1, self._in(self_ids), self._in(init_radius2),
                                                     int(k), C.c_float(start_radius), _ptr(idx), _ptr(dist)))
         return idx, dist
 
     def range_count(self, radius: float):
-        """Neighbours within the closed ball of `radius` for every point (DBSCAN core-point test; see dbscan())."""
-        if _is_tensor(self._like):
-            import torch
-
-            out = torch.empty((self.n,), dtype=torch.int32, device=self._like.device)
-        else:
-            out = np.empty((self.n,), np.uint32)
+        """Neighbours within the closed ball of `radius` for every point (DBSCAN core-point test; see dbscan()): uint32
+        numpy, or an int32 tensor for a build from a tensor."""
+        out = self._empty(self._like, (self.n,), np.uint32)
         self._check(self._L.tknn_range_count(self._h, C.c_float(radius), _ptr(out)))
         return out
 
@@ -279,18 +315,11 @@ class TrueKNN:
         tensors for CUDA tensor input; out = (labels, core) supplies the arrays (core may be None)."""
         if out is not None:
             labels, core = out
-        elif _is_tensor(self._like):
-            import torch
-
-            labels = torch.empty((self.n,), dtype=torch.int32, device=self._like.device)
-            core = torch.empty((self.n,), dtype=torch.uint8, device=self._like.device) if with_core else None
-            self._settle_outputs(labels)
         else:
-            labels = np.empty((self.n,), np.int32)
-            core = np.empty((self.n,), np.uint8) if with_core else None
+            labels = self._empty(self._like, (self.n,), np.int32)
+            core = self._empty(self._like, (self.n,), np.uint8) if with_core else None
         _check_dtype(labels, np.int32, "labels")
-        if core is not None:
-            _check_dtype(core, np.uint8, "core")
+        _check_dtype(core, np.uint8, "core")
         c = C.c_uint64(0)
         self._check(self._L.tknn_dbscan(self._h, C.c_float(eps), int(min_pts), _ptr(labels), _ptr(core), C.byref(c)))
         return labels, core, int(c.value)
@@ -325,20 +354,16 @@ class TrueKNN:
             raise ValueError("num_samples must be >= 0")
         soff = np.concatenate([[0], np.cumsum(counts)]).astype(np.uint64)
         total = int(soff[-1])
-        if start is not None and not _is_tensor(start):
-            start = np.ascontiguousarray(np.atleast_1d(start), dtype=np.int32)
-        if start is not None:
-            _check_dtype(start, np.int32, "start")
-            if int(start.shape[0]) != sizes.shape[0]:
-                raise ValueError(f"start: one index per cloud ({sizes.shape[0]}), got {int(start.shape[0])}")
+        start = _arg(start, np.int32, "start")  # a scalar becomes [1]
+        if start is not None and int(start.shape[0]) != sizes.shape[0]:
+            raise ValueError(f"start: one index per cloud ({sizes.shape[0]}), got {int(start.shape[0])}")
         if out is not None:
             idx, dist = out
         else:
-            idx = self._out(self._like, total, 1, np.int32).reshape(-1)
-            dist = self._out(self._like, total, 1, np.float32).reshape(-1) if with_dist else None
+            idx = self._empty(self._like, (total,), np.int32)
+            dist = self._empty(self._like, (total,), np.float32) if with_dist else None
         _check_dtype(idx, np.int32, "idx")
-        if dist is not None:
-            _check_dtype(dist, np.float32, "dist")
+        _check_dtype(dist, np.float32, "dist")
         if total:  # an empty torch tensor has no address, and there is nothing to sample
             self._check(self._L.tknn_fps(self._h, _ptr(soff), sizes.shape[0], self._in(start), _ptr(idx), _ptr(dist)))
         return idx, dist
@@ -352,35 +377,25 @@ class TrueKNN:
         (idx [nq, k] int32, dist [nq, k] float32 or None when indices_only); rows ascend by (d2, index) and end in -1 /
         FLT_MAX when the cloud has fewer eligible rows; dist is d2 while squared_dist is set.  numpy outputs for numpy
         input, CUDA tensors (on x's device) for CUDA tensor input.  float32 only."""
-        if not _is_tensor(x):
-            x = np.ascontiguousarray(x, dtype=np.float32)
-        if not _is_tensor(y):
-            y = np.ascontiguousarray(y, dtype=np.float32)
-        _check_dtype(x, np.float32, "x")
-        _check_dtype(y, np.float32, "y")
+        x, y = _arg(x, np.float32, "x"), _arg(y, np.float32, "y")
         if x.ndim != 2 or y.ndim != 2:
             raise ValueError("x and y must be [rows, f]")
         n, f, nq = int(x.shape[0]), int(x.shape[1]), int(y.shape[0])
         if int(y.shape[1]) != f:
             raise ValueError(f"x has {f} columns, y has {int(y.shape[1])}")
-        if self_ids is not None and not _is_tensor(self_ids):
-            self_ids = np.ascontiguousarray(self_ids, dtype=np.int32)
-        if self_ids is not None:
-            _check_dtype(self_ids, np.int32, "self_ids")
+        self_ids = _arg(self_ids, np.int32, "self_ids")
         x_off = y_off = None
         n_seg = 1
         if (batch_x is not None or batch_y is not None) and n and nq:
             bx, by, size = _bipartite_setup(x, y, batch_x, batch_y)
             x_off, y_off = batch_to_offsets(bx, n, size), batch_to_offsets(by, nq, size)
             n_seg = size
-        idx = self._out(y, nq, k, np.int32)
-        dist = None if indices_only else self._out(y, nq, k, np.float32)
+        idx = self._empty(y, (nq, k), np.int32)
+        dist = None if indices_only else self._empty(y, (nq, k), np.float32)
         if nq == 0:  # an empty torch tensor has no address, and there is nothing to search
             return idx, dist
-        y_ptr = self._in(x) if y is x else self._in(y)
-        self._check(self._L.tknn_feature_knn(self._h, self._in(x), n, f, f, self._in(x_off), y_ptr, nq, f, self._in(y_off),
-                                             n_seg, self._in(self_ids), int(k), _ptr(idx),
-                                             _ptr(dist) if dist is not None else None))
+        self._check(self._L.tknn_feature_knn(self._h, self._in(x), n, f, f, self._in(x_off), self._in(y), nq, f,
+                                             self._in(y_off), n_seg, self._in(self_ids), int(k), _ptr(idx), _ptr(dist)))
         return idx, dist
 
     def voxel_grid(self, points, size, start=None, end=None, batch=None, batch_size: int | None = None):
@@ -396,17 +411,17 @@ class TrueKNN:
         are rejected (TrueKNNError, TKNN_EINVAL) instead of wrapping."""
         points, dim, size, start, end = _voxel_args(points, size, start, end)
         n = int(points.shape[0])
-        raw = _empty_like_rows(points, n, np.int64)
-        cluster = _empty_like_rows(points, n, np.int32)
-        self._settle_outputs(raw)
+        raw = self._empty(points, (n,), np.int64)
+        cluster = self._empty(points, (n,), np.int32)
         offsets, n_seg = None, 1
         if batch is not None:
             offsets = batch_to_offsets(batch, n, batch_size)
             n_seg = int(offsets.shape[0]) - 1
         nv = C.c_uint64()
-        self._check(self._L.tknn_voxel_grid(self._h, self._in(points) if n else None, n, dim, int(points.shape[1]),
+        self._check(self._L.tknn_voxel_grid(self._h, self._in(points, null_if_empty=True), n, dim, int(points.shape[1]),
                                             self._in(offsets), n_seg, _ptr(size), _ptr(start), _ptr(end),
-                                            _ptr(raw) if n else None, _ptr(cluster) if n else None, C.byref(nv)))
+                                            _ptr(raw, null_if_empty=True), _ptr(cluster, null_if_empty=True),
+                                            C.byref(nv)))
         self._vx_like = points
         self._vx_n = n
         self._vx_nv = int(nv.value)
@@ -417,17 +432,16 @@ class TrueKNN:
         int64 tensor; members [n] int32 point indices voxel by voxel, ascending inside a voxel; first [nv] int32 the
         lowest point index of each voxel (PyG's consecutive_cluster returns an arbitrary member); seg [nv] int32 the
         cloud of each voxel)."""
-        like = getattr(self, "_vx_like", None)
+        like = self._vx_like
         if like is None:
             raise TrueKNNError(_lib.ESTATE, "voxel_members before voxel_grid")
         n, nv = self._vx_n, self._vx_nv
-        offsets = _empty_like_rows(like, nv + 1, np.uint64)
-        members = _empty_like_rows(like, n, np.int32)
-        first = _empty_like_rows(like, nv, np.int32)
-        seg = _empty_like_rows(like, nv, np.int32)
-        self._settle_outputs(offsets)
-        self._check(self._L.tknn_voxel_members(self._h, _ptr(offsets), _ptr(members) if n else None,
-                                               _ptr(first) if nv else None, _ptr(seg) if nv else None))
+        offsets = self._empty(like, (nv + 1,), np.uint64)
+        members = self._empty(like, (n,), np.int32)
+        first = self._empty(like, (nv,), np.int32)
+        seg = self._empty(like, (nv,), np.int32)
+        self._check(self._L.tknn_voxel_members(self._h, _ptr(offsets), _ptr(members, null_if_empty=True),
+                                               _ptr(first, null_if_empty=True), _ptr(seg, null_if_empty=True)))
         return offsets, members, first, seg
 
     def voxel_pool(self, x, reduce: str = "mean"):
@@ -438,21 +452,18 @@ class TrueKNN:
         a non-finite value in x is TKNN_EINVAL.  Call it any number of times per clustering."""
         if reduce not in ("mean", "max"):
             raise ValueError(f"reduce must be 'mean' or 'max', got {reduce!r}")
-        if getattr(self, "_vx_like", None) is None:
+        if self._vx_like is None:
             raise TrueKNNError(_lib.ESTATE, "voxel_pool before voxel_grid")
-        if not _is_tensor(x):
-            x = np.ascontiguousarray(x, dtype=np.float32)
-        _check_dtype(x, np.float32, "x")
+        x = _arg(x, np.float32, "x")
         if x.ndim == 1:
             x = x.reshape(-1, 1)
         if x.ndim != 2:
             raise ValueError("x must be [n] or [n, f]")
         n, f = int(x.shape[0]), int(x.shape[1])
-        out = _empty_like_rows(x, (self._vx_nv, f), np.float32)
-        self._settle_outputs(out)
+        out = self._empty(x, (self._vx_nv, f), np.float32)
         code = _lib.REDUCE_MAX if reduce == "max" else _lib.REDUCE_MEAN
-        self._check(self._L.tknn_voxel_pool(self._h, self._in(x) if n else None, n, f, f, code,
-                                            _ptr(out) if self._vx_nv else None))
+        self._check(self._L.tknn_voxel_pool(self._h, self._in(x, null_if_empty=True), n, f, f, code,
+                                            _ptr(out, null_if_empty=True)))
         return out
 
     def interpolate(self, idx, d2, x):
@@ -462,20 +473,20 @@ class TrueKNN:
         the result is PyG's knn_interpolate on the same neighbours, bit for bit on every run.  Returns (out [nq, f],
         weight [nq, k] (+0 for skipped slots), den [nq]), the inputs of interpolate_backward().  Needs no build and
         leaves the last build untouched.  numpy outputs for numpy x, CUDA tensors (on x's device) for a CUDA tensor."""
-        x = _rows_f32(x, "x")
-        idx, d2 = _rows_like(idx, np.int32, "idx"), _rows_like(d2, np.float32, "d2")
+        x = _arg(x, np.float32, "x", ndim=2, cast=False, copy=True)
+        idx = _arg(idx, np.int32, "idx", ndim=2, copy=True)
+        d2 = _arg(d2, np.float32, "d2", ndim=2, copy=True)
         nq, k = int(idx.shape[0]), int(idx.shape[1])
         if tuple(d2.shape) != (nq, k):
             raise ValueError(f"d2 has shape {tuple(d2.shape)}, idx {(nq, k)}")
         n, f = int(x.shape[0]), int(x.shape[1])
-        out = _empty_like_rows(x, (nq, f), np.float32)
-        weight = _empty_like_rows(x, (nq, k), np.float32)
-        den = _empty_like_rows(x, (nq,), np.float32)
+        out = self._empty(x, (nq, f), np.float32)
+        weight = self._empty(x, (nq, k), np.float32)
+        den = self._empty(x, (nq,), np.float32)
         if nq == 0:  # an empty torch tensor has no address, and there is nothing to compute
             return out, weight, den
-        self._settle_outputs(out)
-        self._check(self._L.tknn_interpolate(self._h, self._in(idx), self._in(d2), nq, k, self._in(x) if n else None, n, f,
-                                             f, _ptr(out), _ptr(weight), _ptr(den)))
+        self._check(self._L.tknn_interpolate(self._h, self._in(idx), self._in(d2), nq, k, self._in(x, null_if_empty=True),
+                                             n, f, f, _ptr(out), _ptr(weight), _ptr(den)))
         return out, weight, den
 
     def interpolate_backward(self, idx, weight, den, grad_out, n: int):
@@ -484,22 +495,20 @@ class TrueKNN:
         weight[i, s]), from +0 in fp32; +0 for a row no slot references.  No float atomics: the same bits on every run.
         idx / weight / den: what interpolate() took and returned; grad_out: [nq, f] float32.  numpy outputs for numpy
         grad_out, CUDA tensors for a CUDA tensor."""
-        g = _rows_f32(grad_out, "grad_out")
-        idx, weight = _rows_like(idx, np.int32, "idx"), _rows_like(weight, np.float32, "weight")
-        if not _is_tensor(den):
-            den = np.ascontiguousarray(den, dtype=np.float32)
-        _check_dtype(den, np.float32, "den")
+        g = _arg(grad_out, np.float32, "grad_out", ndim=2, cast=False, copy=True)
+        idx = _arg(idx, np.int32, "idx", ndim=2, copy=True)
+        weight = _arg(weight, np.float32, "weight", ndim=2, copy=True)
+        den = _arg(den, np.float32, "den")
         nq, k, f, n = int(idx.shape[0]), int(idx.shape[1]), int(g.shape[1]), int(n)
         if tuple(weight.shape) != (nq, k) or tuple(den.shape) != (nq,) or int(g.shape[0]) != nq:
             raise ValueError(f"shapes idx {tuple(idx.shape)}, weight {tuple(weight.shape)}, den {tuple(den.shape)}, "
                              f"grad_out {tuple(g.shape)} do not match")
-        grad_x = _empty_like_rows(g, (n, f), np.float32)
+        grad_x = self._empty(g, (n, f), np.float32)
         if nq == 0:  # no slot references a row
             grad_x[:] = 0
             return grad_x
-        self._settle_outputs(grad_x)
         self._check(self._L.tknn_interpolate_backward(self._h, self._in(idx), self._in(weight), self._in(den), nq, k,
-                                                      self._in(g), f, n, f, _ptr(grad_x) if n else None))
+                                                      self._in(g), f, n, f, _ptr(grad_x, null_if_empty=True)))
         return grad_x
 
     def radius_search(self, radius: float, indices_only: bool = False, out=None):
@@ -523,16 +532,8 @@ class TrueKNN:
         none) names the data index each query excludes.  Returns (offsets, idx, dist) as radius_search().
         batch (after build(batch=...)): the cloud id of every query; the ball of a query holds points of its own cloud
         only (tknn_radius_query_segments)."""
-        if not _is_tensor(queries):
-            queries = np.ascontiguousarray(queries, dtype=np.float32)
-        _check_dtype(queries, np.float32, "queries")
-        nq, stride = int(queries.shape[0]), int(queries.shape[1])
-        if dim is None:
-            dim = min(stride, 3)
-        if self_ids is not None and not _is_tensor(self_ids):
-            self_ids = np.ascontiguousarray(self_ids, dtype=np.int32)
-        if self_ids is not None:
-            _check_dtype(self_ids, np.int32, "self_ids")
+        queries, nq, dim, stride = _points(queries, "queries", dim)
+        self_ids = _arg(self_ids, np.int32, "self_ids")
         q_ptr, sid_ptr = self._in(queries), self._in(self_ids)
         if batch is not None:
             q_off = batch_to_offsets(batch, nq, self.n_segments)
@@ -540,31 +541,20 @@ class TrueKNN:
 
         def call(off, idx, dist, cap, total):
             if batch is not None:
-                return self._L.tknn_radius_query_segments(self._h, q_ptr, nq, int(dim), stride, off_ptr, n_seg, sid_ptr,
+                return self._L.tknn_radius_query_segments(self._h, q_ptr, nq, dim, stride, off_ptr, n_seg, sid_ptr,
                                                           C.c_float(radius), _ptr(off), _ptr(idx), _ptr(dist), cap,
                                                           C.byref(total))
-            return self._L.tknn_radius_query(self._h, q_ptr, nq, int(dim), stride, sid_ptr, C.c_float(radius), _ptr(off),
+            return self._L.tknn_radius_query(self._h, q_ptr, nq, dim, stride, sid_ptr, C.c_float(radius), _ptr(off),
                                              _ptr(idx), _ptr(dist), cap, C.byref(total))
 
         return self._radius_lists(queries, nq, indices_only, out, call)
 
     def _radius_lists(self, like, nq: int, indices_only: bool, out, call):
-        def empty(m, dtype):
-            if _is_tensor(like):
-                import torch
-
-                t = torch.empty((m,), dtype={np.int64: torch.int64, np.int32: torch.int32, np.float32: torch.float32}[dtype],
-                                device=like.device)
-                self._settle_outputs(t)
-                return t
-            return np.empty((m,), dtype)
-
         total = C.c_uint64(0)
         if out is not None:
             offsets, idx, dist = out
             _check_dtype(idx, np.int32, "idx")
-            if dist is not None:
-                _check_dtype(dist, np.float32, "dist")
+            _check_dtype(dist, np.float32, "dist")
             if _is_tensor(offsets):
                 _check_dtype(offsets, np.uint64, "offsets")
             elif offsets.dtype not in (np.int64, np.uint64):
@@ -578,11 +568,11 @@ class TrueKNN:
             self._check(rc)
             t = int(total.value)
             return offsets, idx[:t], dist[:t] if dist is not None else None
-        offsets = empty(nq + 1, np.int64)
+        offsets = self._empty(like, (nq + 1,), np.int64)
         self._check(call(offsets, None, None, 0, total))
         t = int(total.value)
-        idx = empty(t, np.int32)
-        dist = None if indices_only else empty(t, np.float32)
+        idx = self._empty(like, (t,), np.int32)
+        dist = None if indices_only else self._empty(like, (t,), np.float32)
         if t:
             self._check(call(offsets, idx, dist, t, total))
         return offsets, idx, dist
@@ -594,19 +584,18 @@ class TrueKNN:
 
     def brute_force(self, query_ids, k: int):
         """Exact tiled brute force on the GPU for selected data indices (second oracle)."""
-        if not _is_tensor(query_ids):
-            query_ids = np.ascontiguousarray(query_ids, dtype=np.int32)
+        query_ids = _arg(query_ids, np.int32, "query_ids")
         nq = int(query_ids.shape[0])
-        idx = self._out(query_ids, nq, k, np.int32)
-        dist = self._out(query_ids, nq, k, np.float32)
+        idx = self._empty(query_ids, (nq, k), np.int32)
+        dist = self._empty(query_ids, (nq, k), np.float32)
         self._check(self._L.tknn_brute_force(self._h, self._in(query_ids), nq, int(k), _ptr(idx), _ptr(dist)))
         return idx, dist
 
     def merge_topk(self, idx_parts, d2_parts):
         """Merge [parts, nq, k] (idx, d2) device lists on (d2, index); returns (idx, dist=sqrt(d2))."""
         parts, nq, k = (int(x) for x in idx_parts.shape)
-        idx = self._out(idx_parts, nq, k, np.int32)
-        dist = self._out(idx_parts, nq, k, np.float32)
+        idx = self._empty(idx_parts, (nq, k), np.int32)
+        dist = self._empty(idx_parts, (nq, k), np.float32)
         self._check(self._L.tknn_merge_topk(self._h, self._in(idx_parts), self._in(d2_parts), parts, nq, k, _ptr(idx), _ptr(dist)))
         return idx, dist
 
@@ -644,14 +633,9 @@ class TrueKNN:
 
     def build_replicated(self, local_points, first: int, n_total: int, dim: int | None = None):
         """TKNN_SHARD_QUERIES build: this rank's contiguous slice in, the replicated LBVH out (one ncclAllGather)."""
-        if not _is_tensor(local_points):
-            local_points = np.ascontiguousarray(local_points, dtype=np.float32)
-        _check_dtype(local_points, np.float32, "local_points")
-        stride = int(local_points.shape[1])
-        if dim is None:
-            dim = min(stride, 3)
-        self._check(self._L.tknn_build_replicated(self._h, self._in(local_points), int(local_points.shape[0]), int(first),
-                                                  int(n_total), int(dim), stride))
+        local_points, n, dim, stride = _points(local_points, "local_points", dim)
+        self._check(self._L.tknn_build_replicated(self._h, self._in(local_points), n, int(first), int(n_total), dim,
+                                                  stride))
         self.n = int(n_total)
         self.n_segments = 1
         self._like = local_points
@@ -659,14 +643,8 @@ class TrueKNN:
 
     def partition_build(self, local_points, first_index: int, dim: int | None = None):
         """TKNN_PARTITION_POINTS build: rows of global indices first_index.. in, one Morton range of the cloud owned."""
-        if not _is_tensor(local_points):
-            local_points = np.ascontiguousarray(local_points, dtype=np.float32)
-        _check_dtype(local_points, np.float32, "local_points")
-        stride = int(local_points.shape[1])
-        if dim is None:
-            dim = min(stride, 3)
-        self._check(self._L.tknn_partition_build(self._h, self._in(local_points), int(local_points.shape[0]), int(first_index),
-                                                 int(dim), stride))
+        local_points, n, dim, stride = _points(local_points, "local_points", dim)
+        self._check(self._L.tknn_partition_build(self._h, self._in(local_points), n, int(first_index), dim, stride))
         self.n = int(self._L.tknn_partition_owned(self._h))
         self.n_segments = 1
         self._like = local_points
@@ -679,14 +657,9 @@ class TrueKNN:
         """Exact kNN of the owned points against the global cloud: (gid [m], idx [m,k] global ids, dist [m,k])."""
         m = self.partition_owned()
         if out is None:
-            if _is_tensor(self._like):
-                import torch
-
-                gid = torch.empty((m,), dtype=torch.int32, device=self._like.device)
-            else:
-                gid = np.empty((m,), np.int32)
-            idx = self._out(self._like, m, k, np.int32)
-            dist = self._out(self._like, m, k, np.float32)
+            gid = self._empty(self._like, (m,), np.int32)
+            idx = self._empty(self._like, (m, k), np.int32)
+            dist = self._empty(self._like, (m, k), np.float32)
         else:
             gid, idx, dist = out
         got = C.c_uint64(0)
@@ -705,7 +678,7 @@ class TrueKNN:
     # ---- introspection (tests / bench) ----
     def sort_pairs(self, keys, values=None):
         n = int(keys.shape[0])
-        self._check(self._L.tknn_sort_pairs(self._h, self._in(keys), self._in(values) if values is not None else None, n))
+        self._check(self._L.tknn_sort_pairs(self._h, self._in(keys), self._in(values), n))
         return keys, values
 
     def get_bvh(self):
@@ -719,20 +692,15 @@ class TrueKNN:
 
     def morton_codes(self, points, box6, dim: int | None = None):
         """63-bit Morton codes on the cubic grid over `box6` = (lo.xyz, hi.xyz); int64/uint64 [n]."""
-        if not _is_tensor(points):
-            points = np.ascontiguousarray(points, dtype=np.float32)
-        n, stride = int(points.shape[0]), int(points.shape[1])
-        if dim is None:
-            dim = min(stride, 3)
+        points, n, dim, stride = _points(points, "points", dim)
+        out = self._empty(points, (n,), np.uint64)
         if _is_tensor(points):
             import torch
 
-            out = torch.empty((n,), dtype=torch.int64, device=points.device)
             box = torch.as_tensor(box6, dtype=torch.float32).cpu().contiguous().numpy()
         else:
-            out = np.empty((n,), np.uint64)
             box = np.ascontiguousarray(box6, dtype=np.float32)
-        self._check(self._L.tknn_morton_codes(self._h, self._in(points), n, int(dim), stride, _ptr(box), _ptr(out)))
+        self._check(self._L.tknn_morton_codes(self._h, self._in(points), n, dim, stride, _ptr(box), _ptr(out)))
         return out
 
     def reach_mask(self, points, reach2, box6, summaries, self_rank: int, cell_bits: int = 3):
@@ -743,7 +711,7 @@ class TrueKNN:
         n_ranks = int(summaries.shape[0])
         box = torch.as_tensor(box6, dtype=torch.float32, device=points.device).contiguous()
         summ = summaries.contiguous()
-        out = torch.empty((n,), dtype=torch.int32, device=points.device)
+        out = self._empty(points, (n,), np.int32)
         self._check(self._L.tknn_reach_mask(self._h, self._in(points), n, stride, self._in(reach2.contiguous()), self._in(box),
                                             self._in(summ), n_ranks, int(cell_bits), int(self_rank), _ptr(out)))
         return out
@@ -768,8 +736,9 @@ class TrueKNN:
 class _RankView(TrueKNN):
     """A rank's context inside a MultiTrueKNN (owned by it): statistics and options only."""
 
-    def __init__(self, L, handle):  # noqa: D401 — no tknn_create here
-        self._L, self._h, self._own_stream, self.n, self._like = L, handle, True, 0, None
+    def __init__(self, L, handle, device: int):  # noqa: D401 — no tknn_create here
+        self._L, self._h = L, handle
+        self._init_state(device)
 
     def close(self):
         self._h = None
@@ -786,7 +755,8 @@ class MultiTrueKNN:
 
     def __init__(self, device_ids, mode: str = "shard", **options):
         self._L = _lib.load()
-        ids = (C.c_int * len(device_ids))(*[int(d) for d in device_ids])
+        self._device_ids = [int(d) for d in device_ids]  # rank r runs on device_ids[r]
+        ids = (C.c_int * len(device_ids))(*self._device_ids)
         h = C.c_void_p()
         rc = self._L.tknn_create_multi(ids, len(device_ids), self.MODES[mode], C.byref(h))
         if rc != _lib.OK:
@@ -807,7 +777,7 @@ class MultiTrueKNN:
         return int(self._L.tknn_multi_ranks(self._h))
 
     def rank(self, r: int) -> TrueKNN:
-        return _RankView(self._L, C.c_void_p(self._L.tknn_multi_ctx(self._h, int(r))))
+        return _RankView(self._L, C.c_void_p(self._L.tknn_multi_ctx(self._h, int(r))), self._device_ids[int(r)])
 
     def build(self, points, dim: int | None = None):
         points = np.ascontiguousarray(points, dtype=np.float32)
@@ -927,32 +897,13 @@ def fps(src, batch=None, ratio: float = 0.5, random_start: bool = True, batch_si
     n = int(src.shape[0])
     if n == 0:
         fps_counts([0], ratio)  # the same argument check
-        if _is_tensor(src):
-            import torch
-
-            return torch.zeros((0,), dtype=torch.int64, device=src.device)
-        return np.zeros(0, np.int64)
-    dev = src.device.index if _is_tensor(src) else (device or 0)
-    with TrueKNN(dev) as t:
+        return _zeros_like_rows(src, (0,), np.int64)
+    with TrueKNN(_device_of(src, device)) as t:
         t.build(src, batch=batch, batch_size=batch_size)
         sizes = t.cloud_sizes()
         start = fps_random_starts(np.concatenate([[0], np.cumsum(sizes)]), src) if random_start else None
         idx, _ = t.fps(ratio=ratio, start=start)
-    if _is_tensor(idx):
-        import torch
-
-        return idx.to(torch.int64)
-    return idx.astype(np.int64)
-
-
-def _empty_like_rows(like, shape, np_dtype):
-    """An uninitialised array of `shape` beside `like`: a tensor on its device, or numpy."""
-    if _is_tensor(like):
-        import torch
-
-        dt = {np.int64: torch.int64, np.uint64: torch.int64, np.int32: torch.int32, np.float32: torch.float32}[np_dtype]
-        return torch.empty(shape, dtype=dt, device=like.device)
-    return np.empty(shape, np_dtype)
+    return _int64(idx)
 
 
 def _voxel_args(points, size, start, end, all_columns=False):
@@ -960,9 +911,7 @@ def _voxel_args(points, size, start, end, all_columns=False):
     dim entries (scalars broadcast).  Raises ValueError for a shape, a non-finite value or a size <= 0.  all_columns:
     every column of points is a coordinate (torch_cluster's and PyG's signatures), so more than 3 is an error rather
     than columns skipped through the stride."""
-    if not _is_tensor(points):
-        points = np.ascontiguousarray(points, dtype=np.float32)
-    _check_dtype(points, np.float32, "points")
+    points = _arg(points, np.float32, "points")
     if points.ndim != 2 or int(points.shape[1]) < 2:
         raise ValueError("points must be [n, >= 2] (2-D or 3-D positions)")
     if all_columns and int(points.shape[1]) > 3:
@@ -1043,13 +992,39 @@ def _int64(a):
     return a.astype(np.int64)
 
 
-def _edge_index(centre, neighbour, like):
-    """[2, E] int64 in torch_cluster's source_to_target flow: row 0 the neighbour, row 1 the centre."""
-    if _is_tensor(like):
+def _edges(query, nbr, query_row: int):
+    """[2, E] int64 with the query (centre) ids in row query_row and their neighbours in the other: query_row 1 is
+    torch_cluster's source_to_target flow of knn_graph / radius_graph, 0 the [y index, x index] rows of knn / radius."""
+    rows = (nbr, query) if query_row == 1 else (query, nbr)
+    if _is_tensor(query):
         import torch
 
-        return torch.stack([neighbour.to(torch.int64), centre.to(torch.int64)])
-    return np.stack([neighbour.astype(np.int64), centre.astype(np.int64)])
+        return torch.stack([_int64(r) for r in rows])
+    return np.stack([_int64(r) for r in rows])
+
+
+def _repeat_rows(like, m: int, counts):
+    """The row id of every entry of m rows holding `counts` entries each (an int, or one count per row)."""
+    rows = _arange_like(like, m)
+    return rows.repeat_interleave(counts) if _is_tensor(rows) else np.repeat(rows, counts)
+
+
+def _knn_edges(idx, k: int, query_row: int):
+    """Edges of [m, k] neighbour rows, -1 slots dropped."""
+    query = _repeat_rows(idx, int(idx.shape[0]), int(k))
+    flat = idx.reshape(-1)
+    keep = flat >= 0
+    return _edges(query[keep], flat[keep], query_row)
+
+
+def _csr_edges(offsets, idx, query_row: int, max_num_neighbors: int | None = None):
+    """Edges of CSR neighbour rows (radius_search / radius_query); max_num_neighbors keeps the first entries of a row."""
+    off = _int64(offsets)
+    query = _repeat_rows(idx, int(offsets.shape[0]) - 1, off[1:] - off[:-1])
+    if max_num_neighbors is not None:
+        keep = _arange_like(idx, int(idx.shape[0])) - off[query] < int(max_num_neighbors)
+        idx, query = idx[keep], query[keep]
+    return _edges(query, idx, query_row)
 
 
 def knn_graph(x, k: int, batch=None, device: int | None = None):
@@ -1061,21 +1036,9 @@ def knn_graph(x, k: int, batch=None, device: int | None = None):
     out; a CUDA tensor in, a tensor on its device out (device: the CUDA device for numpy input, default 0).
     Only the first 2 or 3 columns of x are positions: columns beyond the third are ignored (they are skipped through
     the stride).  For neighbours over all columns (feature space, DGCNN) use feature_knn_graph()."""
-    dev = x.device.index if _is_tensor(x) else (device or 0)
-    with TrueKNN(dev) as t:
+    with TrueKNN(_device_of(x, device)) as t:
         idx, _ = t.build(x, batch=batch).search(int(k), indices_only=True)
-    n = int(idx.shape[0])
-    if _is_tensor(idx):
-        import torch
-
-        centre = torch.arange(n, device=idx.device).repeat_interleave(int(k))
-        flat = idx.reshape(-1)
-        keep = flat >= 0
-        return _edge_index(centre[keep], flat[keep], idx)
-    centre = np.repeat(np.arange(n), int(k))
-    flat = idx.reshape(-1)
-    keep = flat >= 0
-    return _edge_index(centre[keep], flat[keep], idx)
+    return _knn_edges(idx, k, 1)
 
 
 def radius_graph(x, r: float, batch=None, device: int | None = None):
@@ -1083,18 +1046,9 @@ def radius_graph(x, r: float, batch=None, device: int | None = None):
     cloud.  Returns edge_index [2, E] int64 (row 0 the neighbour, row 1 the centre), edges ordered by centre and then by
     (distance, index).  Differences from torch_cluster: no `loop` option (a point is never its own neighbour) and no
     max_num_neighbors truncation: every neighbour in the ball is returned."""
-    dev = x.device.index if _is_tensor(x) else (device or 0)
-    with TrueKNN(dev) as t:
+    with TrueKNN(_device_of(x, device)) as t:
         offsets, idx, _ = t.build(x, batch=batch).radius_search(float(r), indices_only=True)
-    n = int(offsets.shape[0]) - 1
-    if _is_tensor(idx):
-        import torch
-
-        counts = (offsets[1:] - offsets[:-1]).to(torch.int64)
-        centre = torch.arange(n, device=idx.device).repeat_interleave(counts)
-        return _edge_index(centre, idx, idx)
-    counts = np.diff(offsets.astype(np.int64))
-    return _edge_index(np.repeat(np.arange(n), counts), idx, idx)
+    return _csr_edges(offsets, idx, 1)
 
 
 def _bipartite_setup(x, y, batch_x, batch_y):
@@ -1102,26 +1056,10 @@ def _bipartite_setup(x, y, batch_x, batch_y):
     with zeros; batch_size = max(batch_x.max(), batch_y.max()) + 1."""
     if batch_x is None and batch_y is None:
         return None, None, None
-
-    def zeros_like_rows(a):
-        if _is_tensor(a):
-            import torch
-
-            return torch.zeros((int(a.shape[0]),), dtype=torch.int64, device=a.device)
-        return np.zeros(int(a.shape[0]), np.int64)
-
-    batch_x = zeros_like_rows(x) if batch_x is None else batch_x
-    batch_y = zeros_like_rows(y) if batch_y is None else batch_y
+    batch_x = _zeros_like_rows(x, (int(x.shape[0]),), np.int64) if batch_x is None else batch_x
+    batch_y = _zeros_like_rows(y, (int(y.shape[0]),), np.int64) if batch_y is None else batch_y
     top = max(int(b.max().item()) if _is_tensor(b) else int(np.max(b)) for b in (batch_x, batch_y))
     return batch_x, batch_y, top + 1
-
-
-def _empty_edges(like):
-    if _is_tensor(like):
-        import torch
-
-        return torch.zeros((2, 0), dtype=torch.int64, device=like.device)
-    return np.zeros((2, 0), np.int64)
 
 
 def knn(x, y, k: int, batch_x=None, batch_y=None, device: int | None = None):
@@ -1134,42 +1072,13 @@ def knn(x, y, k: int, batch_x=None, batch_y=None, device: int | None = None):
     the CUDA device for numpy input, default 0).  Only the first 2 or 3 columns of x and y are positions: columns beyond
     the third are ignored.  For neighbours over all columns (feature space) use feature_knn()."""
     if int(x.shape[0]) == 0 or int(y.shape[0]) == 0:
-        return _empty_edges(x)
+        return _zeros_like_rows(x, (2, 0), np.int64)
     batch_x, batch_y, batch_size = _bipartite_setup(x, y, batch_x, batch_y)
     k = min(int(k), int(x.shape[0]))
-    dev = x.device.index if _is_tensor(x) else (device or 0)
-    with TrueKNN(dev) as t:
+    with TrueKNN(_device_of(x, device)) as t:
         t.build(x, batch=batch_x, batch_size=batch_size)
         idx, _ = t.query(y, k, batch=batch_y)
-    m = int(idx.shape[0])
-    if _is_tensor(idx):
-        import torch
-
-        query = torch.arange(m, device=idx.device).repeat_interleave(k)
-        flat = idx.reshape(-1)
-        keep = flat >= 0
-        return _edge_index(flat[keep], query[keep], idx)
-    query = np.repeat(np.arange(m), k)
-    flat = idx.reshape(-1)
-    keep = flat >= 0
-    return _edge_index(flat[keep], query[keep], idx)
-
-
-def _knn_edges(idx, k: int, query_row: int):
-    """Edges of [m, k] neighbour rows (-1 slots dropped): query_row 1 gives knn_graph's [neighbour, centre] rows, 0
-    gives knn()'s [query, neighbour] rows."""
-    m = int(idx.shape[0])
-    if _is_tensor(idx):
-        import torch
-
-        query = torch.arange(m, device=idx.device).repeat_interleave(int(k))
-    else:
-        query = np.repeat(np.arange(m), int(k))
-    flat = idx.reshape(-1)
-    keep = flat >= 0
-    if query_row == 1:
-        return _edge_index(query[keep], flat[keep], idx)
-    return _edge_index(flat[keep], query[keep], idx)
+    return _knn_edges(idx, k, 0)
 
 
 def feature_knn_graph(x, k: int, batch=None, device: int | None = None):
@@ -1180,16 +1089,10 @@ def feature_knn_graph(x, k: int, batch=None, device: int | None = None):
     in, a tensor on its device out (device: the CUDA device for numpy input, default 0)."""
     n = int(x.shape[0])
     if n == 0:
-        return _empty_edges(x)
+        return _zeros_like_rows(x, (2, 0), np.int64)
     k = int(k)
-    dev = x.device.index if _is_tensor(x) else (device or 0)
-    if _is_tensor(x):
-        import torch
-
-        self_ids = torch.arange(n, dtype=torch.int32, device=x.device)
-    else:
-        self_ids = np.arange(n, dtype=np.int32)
-    with TrueKNN(dev) as t:
+    self_ids = _arange_like(x, n, np.int32)
+    with TrueKNN(_device_of(x, device)) as t:
         idx, _ = t.feature_knn(x, x, k, batch_x=batch, batch_y=batch, self_ids=self_ids, indices_only=True)
     return _knn_edges(idx, k, 1)
 
@@ -1201,38 +1104,16 @@ def feature_knn(x, y, k: int, batch_x=None, batch_y=None, device: int | None = N
     [2, 0]; no self exclusion, so DynamicEdgeConv's knn(x, x, k, b, b) is feature_knn(x, x, k, b, b).  numpy in, numpy
     out; a CUDA tensor in, a tensor on its device out (device: the CUDA device for numpy input, default 0)."""
     if int(x.shape[0]) == 0 or int(y.shape[0]) == 0:
-        return _empty_edges(x)
+        return _zeros_like_rows(x, (2, 0), np.int64)
     k = min(int(k), int(x.shape[0]))
-    dev = x.device.index if _is_tensor(x) else (device or 0)
-    with TrueKNN(dev) as t:
+    with TrueKNN(_device_of(x, device)) as t:
         idx, _ = t.feature_knn(x, y, k, batch_x=batch_x, batch_y=batch_y, indices_only=True)
     return _knn_edges(idx, k, 0)
 
 
-def _rows_f32(a, name):
-    """A 2-D float32 array or tensor, C-contiguous (numpy float32 is not cast: a float64 x raises TypeError)."""
-    if not _is_tensor(a):
-        a = np.ascontiguousarray(a)
-    _check_dtype(a, np.float32, name)
-    if a.ndim != 2:
-        raise ValueError(f"{name} must be [rows, f]")
-    return a.contiguous() if _is_tensor(a) else a
-
-
-def _rows_like(a, np_dtype, name):
-    if not _is_tensor(a):
-        a = np.ascontiguousarray(a, dtype=np_dtype)
-    _check_dtype(a, np_dtype, name)
-    if a.ndim != 2:
-        raise ValueError(f"{name} must be [nq, k]")
-    return a.contiguous() if _is_tensor(a) else a
-
-
 def _positions(pos, name):
     """pos as [rows, 2|3] float32: PyG's knn_interpolate measures distances over every column, so other widths raise."""
-    if not _is_tensor(pos):
-        pos = np.ascontiguousarray(pos, dtype=np.float32)
-    _check_dtype(pos, np.float32, name)
+    pos = _arg(pos, np.float32, name)
     if pos.ndim != 2 or int(pos.shape[1]) not in (2, 3):
         raise ValueError(f"{name} must be [n, 2] or [n, 3] (only 2-D and 3-D positions are supported), got "
                          f"{tuple(pos.shape)}")
@@ -1279,7 +1160,7 @@ def knn_interpolate(x, pos_x, pos_y, batch_x=None, batch_y=None, k: int = 3, num
     PyG: the backward pass (TrueKNN.interpolate_backward) sums in edge order without atomics, so x.grad has the same bits
     on every run; the positions get no gradient.  device: the CUDA device for numpy input (default 0)."""
     del num_workers
-    x = _rows_f32(x, "x")
+    x = _arg(x, np.float32, "x", ndim=2, cast=False, copy=True)
     pos_x, pos_y = _positions(pos_x, "pos_x"), _positions(pos_y, "pos_y")
     if int(pos_x.shape[1]) != int(pos_y.shape[1]):
         raise ValueError(f"pos_x has {int(pos_x.shape[1])} columns, pos_y {int(pos_y.shape[1])}")
@@ -1323,29 +1204,12 @@ def radius(x, y, r: float, batch_x=None, batch_y=None, max_num_neighbors: int | 
     keeps the first m entries of each sorted row, i.e. the m nearest.  This differs from torch_cluster, whose default
     is 32 and whose CUDA kernel keeps an unspecified m of the ball."""
     if int(x.shape[0]) == 0 or int(y.shape[0]) == 0:
-        return _empty_edges(x)
+        return _zeros_like_rows(x, (2, 0), np.int64)
     batch_x, batch_y, batch_size = _bipartite_setup(x, y, batch_x, batch_y)
-    dev = x.device.index if _is_tensor(x) else (device or 0)
-    with TrueKNN(dev) as t:
+    with TrueKNN(_device_of(x, device)) as t:
         t.build(x, batch=batch_x, batch_size=batch_size)
         offsets, idx, _ = t.radius_query(y, float(r), indices_only=True, batch=batch_y)
-    m = int(offsets.shape[0]) - 1
-    if _is_tensor(idx):
-        import torch
-
-        off = offsets.to(torch.int64)
-        counts = off[1:] - off[:-1]
-        query = torch.arange(m, device=idx.device).repeat_interleave(counts)
-        if max_num_neighbors is not None:
-            keep = torch.arange(int(idx.shape[0]), device=idx.device) - off[query] < int(max_num_neighbors)
-            idx, query = idx[keep], query[keep]
-        return _edge_index(idx, query, idx)
-    off = offsets.astype(np.int64)
-    query = np.repeat(np.arange(m), np.diff(off))
-    if max_num_neighbors is not None:
-        keep = np.arange(idx.shape[0]) - off[query] < int(max_num_neighbors)
-        idx, query = idx[keep], query[keep]
-    return _edge_index(idx, query, idx)
+    return _csr_edges(offsets, idx, 0, max_num_neighbors)
 
 
 def read_points(path: str, n: int, dim: int) -> np.ndarray:
