@@ -100,6 +100,9 @@ enum {
                                   the table is valid, whatever its occupancy (tests, A/B)  */
   ,TKNN_OPT_GRID_LEVEL = 21     /* cells per axis of the grid = 2^level: 0 (default) = floor(log2(n) / 3), else 1..8 (at most the
                                   key's code bits per axis) */
+  ,TKNN_OPT_GRID_RADIUS_QUANTILE = 22 /* start-radius estimator of a search whose round 1 walks the cell grid (a build that selected
+                                  the grid, k <= 24): per-mille quantile of the sampled k-th neighbour distance (default 990);
+                                  every other search uses TKNN_OPT_RADIUS_QUANTILE */
 };
 
 typedef struct tknn_ctx tknn_ctx;
@@ -152,6 +155,13 @@ typedef struct tknn_stats {
                               * (r = 0) or grid_sparse_kernel (r >= 1); ORed over the slices of a sliced search          */
   uint64_t grid_deferred;    /* counting build: round-1 groups and sparse-round queries whose cell range exceeded the cap,
                               * left to the LBVH rounds */
+  /* counting build, round 1 on the grid: clock64() cycles its warps spent per phase, summed over warps — range set-up,
+   * cell walk and votes, staging loads, filter, insert loop, emit — the insert loop's iterations per warp (the sum over
+   * its flushes of the largest survivor count of any lane) and round 1's inserts (grid_inserts / (32 x grid_insert_iters)
+   * is the loop's lane efficiency) */
+  uint64_t grid_phase_cycles[6];
+  uint64_t grid_insert_iters;
+  uint64_t grid_inserts;
 } tknn_stats;
 
 /* Replaces owlContextCreate + module/program/pipeline/SBT setup (hostCode.cpp:141-159,267-269).

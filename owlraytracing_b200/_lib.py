@@ -21,7 +21,7 @@ ERROR_NAMES = {0: "TKNN_OK", 1: "TKNN_EINVAL", 2: "TKNN_ENOMEM", 3: "TKNN_ECUDA"
 (OPT_LEAF_SIZE, OPT_COUNTERS, OPT_LEAF_POLICY, OPT_SAMPLE_GROUPS, OPT_BLOCKS_PER_SM, OPT_SQUARED_DIST, OPT_RADIUS_QUANTILE,
  OPT_KEEP_SCRATCH, OPT_SPARSE_DIVISOR, OPT_APPROX_FILTER, OPT_OUTPUT_CHUNKS, OPT_FILE_ORDER_CHUNKS, OPT_MORTON_BITS,
  OPT_TIE_PRUNING, OPT_WARP_ROUND_MAX, OPT_CURVE, OPT_SPECULATIVE_MAX, OPT_SPARSE_TEAM, OPT_SORT_MODE, OPT_GRID,
- OPT_GRID_LEVEL) = (1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17, 18, 19, 20, 21)
+ OPT_GRID_LEVEL, OPT_GRID_RADIUS_QUANTILE) = (1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17, 18, 19, 20, 21, 22)
 
 
 class Stats(C.Structure):
@@ -66,6 +66,9 @@ class Stats(C.Structure):
         ("grid_ms", C.c_float),
         ("grid_rounds", C.c_uint32),
         ("grid_deferred", C.c_uint64),
+        ("grid_phase_cycles", C.c_uint64 * 6),
+        ("grid_insert_iters", C.c_uint64),
+        ("grid_inserts", C.c_uint64),
     ]
 
     def as_dict(self) -> dict:
@@ -74,6 +77,8 @@ class Stats(C.Structure):
             v = getattr(self, name)
             if name in ("round_ms", "kernel_ms", "round_queries"):
                 v = list(v)[: max(0, int(self.rounds))]
+            elif name == "grid_phase_cycles":
+                v = list(v)
             d[name] = v
         return d
 

@@ -29,6 +29,7 @@ struct tknn_ctx {
   // options
   int leaf_size = 32, counters = 0, leaf_policy = 0, sample_groups = 128, blocks_per_sm = 0, squared = 0,
       radius_quantile = 990;
+  int grid_radius_quantile = 990;  // TKNN_OPT_GRID_RADIUS_QUANTILE: the estimator's quantile when round 1 walks the cell grid
   // BVH
   uint64_t n = 0;
   uint32_t n_leaves = 0;
@@ -142,9 +143,13 @@ inline unsigned blocks_for(uint64_t n, int threads) { return (unsigned)((n + thr
 
 // scalars layout (uint32 words unless noted)
 enum { SC_GROUP_COUNTER = 0, SC_TOTAL = 1, SC_ERROR = 2, SC_QBAD = 3 /* non-finite query coordinate */, SC_BOUNDS = 4 /* 7 words */, SC_SCENE = 12 /* 6 floats */,
-       SC_COUNTERS = 20 /* 8 x u64, 8-byte aligned */, SC_DUPLEAF = 40, SC_QUANTILE = 41 /* 2 floats: r, r * r */,
-       SC_DBSCAN = 43 /* core points, other points */,
-       SC_GRID = 45 /* largest cell, cells split into several runs */, SC_WORDS = 48 };
+       SC_DUPLEAF = 18, SC_QUANTILE = 19 /* 2 floats: r, r * r */, SC_DBSCAN = 21 /* core points, other points */,
+       SC_GRID = 23 /* largest cell, cells split into several runs */,
+       SC_COUNTERS = 26 /* N_COUNTERS x u64, 8-byte aligned */, SC_WORDS = 59 };
+// the counting kernels' counters: [0, 8) the tknn_stats counter fields, [8, 16) grid_knn_kernel's phase clocks, insert-loop
+// iterations and inserts (grid.cuh)
+constexpr int N_COUNTERS = 16;
+static_assert(SC_COUNTERS % 2 == 0 && SC_COUNTERS + 2 * N_COUNTERS < SC_WORDS, "scalars layout");
 
 #define TK_CUDA(c, expr)                                                                            \
   do {                                                                                              \

@@ -113,6 +113,15 @@ struct GridParams {
   int level;
 };
 
+// Phases of a round-1 group that the counting grid_knn_kernel times (counters[8 + phase]): range set-up (group fetch, query
+// load, cell range, boundaries and visit order), the slab / row / cell walk with its votes and row loads, the staging loads,
+// the filter of a flush, its insert loop, and the emit.
+enum { GRID_PHASE_SETUP = 0, GRID_PHASE_WALK, GRID_PHASE_STAGE, GRID_PHASE_FILTER, GRID_PHASE_INSERT, GRID_PHASE_EMIT,
+       GRID_PHASES };
+constexpr int GRID_PHASE_SLOT = 8;        // counters[GRID_PHASE_SLOT + phase]
+constexpr int GRID_INSERT_ITER_SLOT = 14; // counters[14]: insert-loop iterations per warp
+constexpr int GRID_INSERT_SLOT = 15;      // counters[15]: inserts of round 1 on the grid
+
 // per warp: the LBVH list kernel's layout (staging 64 points, stack area = the group's 3 x 32 cell boundaries, k-list,
 // SoA coordinates) + the visit order of the group's cells per axis (3 x 32 bytes) + its low cell and width per axis
 // (kept in shared memory: registers stay free for the loop nest)
@@ -138,12 +147,19 @@ __device__ __forceinline__ float axis_gap(float q, float lo, float hi) {
 // Per group: the integer cell range of the union of the lanes' boxes [q - s, q + s] (s >= sqrt(bound), see below), visited
 // x-slab, y-row, z-cell, each axis outward from the middle; a slab, row or cell is entered when ANY lane's box distance to it
 // is within that lane's current bound (warp vote).  The box term of each axis enters the chain in dist2's order (x first), so
-// the slab and row terms are partial sums of the cell's distance and cull as conservatively.  Wanted cells' runs are staged
-// into the 64-point area (NaN-padded), filtered into two masks by filter4 and inserted in one loop (the sibling-pair path of
-// the LBVH kernel) whenever TKNN_GRID_FLUSH points are staged.
+// the slab and row terms are partial sums of the cell's distance and cull as conservatively.  A row's cells are voted on
+// first, all against the bounds as they are at the row's start (a bound only shrinks, so a stale one culls less, never
+// wrongly); then the wanted cells' points are staged with one warp-wide gather, lane i loading the row's i-th wanted point
+// (a prefix sum over the cells' run lengths and a binary search in it), so a row waits for one load latency instead of one
+// per cell.  Staged points go into the 64-point area (NaN-padded), are filtered into two masks by filter4 and inserted in one
+// loop (the sibling-pair path of the LBVH kernel) whenever TKNN_GRID_FLUSH points are staged.  The k-lists keep the k
+// smallest (d2, index) keys whatever order the points arrive in, so the rows do not depend on the staging order.
 // Counting build: counters[0] = cell tests x active lanes (the nodes_visited field), [1] = staged points x active lanes,
 // [2] = inserts, [3] = cell tests per warp, [4] = cells staged per warp, [5] = points staged per warp, [7] = groups left
-// unresolved by the cap.
+// unresolved by the cap; [8 .. 13] = clock64() cycles per warp spent in each GRID_PHASE_* phase (every cycle of a group,
+// from fetching it to its emit, is charged to exactly one phase), [14] = insert-loop iterations per warp (the sum over
+// flushes of the largest survivor count of any lane: the trips the divergent loop takes), [15] = this kernel's inserts
+// ([2] also counts those of the rounds after it).
 template <bool COUNT>
 static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(const trav::Params P, const GridParams G) {
   extern __shared__ __align__(16) unsigned char smem[];
@@ -162,10 +178,21 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
   const int per = (1 << level) + 1;
 
   unsigned long long c_cells = 0, c_tests = 0, c_ins = 0, c_wcells = 0, c_wstaged = 0, c_wpts = 0, c_defer = 0;
+  // phase clocks: tick(ph) charges the cycles since the previous tick to phase ph
+  unsigned long long c_phase[GRID_PHASES] = {}, c_iters = 0;
+  long long t_mark = 0;
+  auto tick = [&](int ph) {
+    if (COUNT) {
+      const long long t = clock64();
+      c_phase[ph] += (unsigned long long)(t - t_mark);
+      t_mark = t;
+    }
+  };
   const float round_r2 = P.r2_dev ? __ldg(P.r2_dev) : P.r2;
   const uint64_t n_active = P.n_active_dev ? min((uint64_t)__ldg(P.n_active_dev), P.n_active) : P.n_active;
   const uint32_t n_groups = (uint32_t)((n_active + 31) / 32);
 
+  if (COUNT) t_mark = clock64();
   for (;;) {
     uint32_t group = 0;
     if (lane == 0) group = atomicAdd(P.group_counter, 1u);
@@ -221,12 +248,14 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
       if (vol > (uint32_t)TKNN_GRID_CAP) defer = true;
     }
     __syncwarp();
+    tick(GRID_PHASE_SETUP);
 
     if (!defer) {
 
       int fill = 0;  // points staged
       // filter the staged points against the bounds as they are now, then insert the survivors (one divergent loop)
       auto flush = [&]() {
+        tick(GRID_PHASE_STAGE);
         if (lane < 8 && fill + lane < NS) soa[fill + lane] = __int_as_float(0x7fc00000);  // NaN x: the padded tail never passes
         __syncwarp();
         if (COUNT) { c_tests += valid ? fill : 0; c_wpts += fill; }
@@ -240,6 +269,10 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
         for (int j0 = MAX_LEAF; j0 < fill; j0 += 8)
           mask_b |= (trav::filter4<NS>(soa, j0, qx2, qy2, qz2, bound) | (trav::filter4<NS>(soa, j0 + 4, qx2, qy2, qz2, bound) << 4))
                     << (j0 - MAX_LEAF);
+        if (COUNT) {
+          tick(GRID_PHASE_FILTER);
+          c_iters += __reduce_max_sync(FULL_MASK, (unsigned)(__popc(mask_a) + __popc(mask_b)));
+        }
         while (mask_a | mask_b) {
           int j;
           if (mask_a) { j = __ffs(mask_a) - 1; mask_a &= mask_a - 1u; }
@@ -250,6 +283,7 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
           if (pid != self && d <= bound) trav::list_take<S, COUNT>(H, cnt, k, bound, d, pid, c_ins);
         }
         __syncwarp();
+        tick(GRID_PHASE_INSERT);
         fill = 0;
       };
 
@@ -271,6 +305,8 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
           if (lane < wz)
             run = __ldg(&G.cells[((uint64_t)(rng[0] + ox) << (2 * level)) | ((uint64_t)(rng[1] + oy) << level) | (rng[2] + lane)]);
           const uint32_t full = __ballot_sync(FULL_MASK, run.y != run.x);
+          // the row's wanted cells first (votes against the bounds as they are now), then all their points in one gather
+          uint32_t want = 0;
 #pragma unroll 1
           for (int iz = 0; iz < wz; ++iz) {
             const int oz = ord[64 + iz];
@@ -278,30 +314,47 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
             const float tz = axis_gap(q.z, gb[64 + oz], gb[65 + oz]);
             const float d = __fmaf_rn(tz, tz, ay2);
             if (COUNT) { c_cells += valid ? 1 : 0; c_wcells += 1; }
-            if (!__any_sync(FULL_MASK, d <= bound)) continue;
-            uint32_t src = __shfl_sync(FULL_MASK, run.x, oz);
-            int rem = (int)(__shfl_sync(FULL_MASK, run.y, oz) - src);
-            if (COUNT) c_wstaged += 1;
-            while (rem > 0) {  // a run longer than the free space continues after a flush
-              const int take = min(rem, NS - fill);
-#pragma unroll
-              for (int h = 0; h < NS; h += 32) {
-                if (lane + h < take) {
-                  const float4 p = __ldg(&P.pts[(uint64_t)src + lane + h]);
-                  const int j = fill + lane + h;
-                  stage[j] = p;
-                  soa[j] = p.x; soa[NS + j] = p.y; soa[2 * NS + j] = p.z;
-                }
-              }
-              fill += take;
-              src += take;
-              rem -= take;
-              if (fill == NS) flush();
-            }
-            if (fill >= TKNN_GRID_FLUSH) flush();
+            if (__any_sync(FULL_MASK, d <= bound)) want |= 1u << oz;
           }
+          tick(GRID_PHASE_WALK);
+          if (!want) continue;
+          if (COUNT) c_wstaged += __popc(want);
+          // inclusive prefix over the lanes (cells in z order) of the wanted runs' lengths: the row's wanted points are
+          // numbered 0 .. total - 1 cell after cell, and point t lies in the first cell whose prefix exceeds t
+          uint32_t incl = ((want >> lane) & 1u) ? run.y - run.x : 0u;
+#pragma unroll
+          for (int s = 1; s < 32; s <<= 1) {
+            const uint32_t v = __shfl_up_sync(FULL_MASK, incl, s);
+            if (lane >= s) incl += v;
+          }
+          const uint32_t total = __shfl_sync(FULL_MASK, incl, 31);
+          for (uint32_t base = 0; base < total;) {  // a row longer than the free space continues after a flush
+            const int take = (int)min(total - base, (uint32_t)(NS - fill));
+#pragma unroll
+            for (int h = 0; h < NS; h += 32) {
+              if (h >= take) break;
+              const uint32_t t = base + (uint32_t)(lane + h);
+              int c = 0;
+#pragma unroll
+              for (int s = 16; s > 0; s >>= 1)
+                if (__shfl_sync(FULL_MASK, incl, c + s - 1) <= t) c += s;
+              const uint32_t src = __shfl_sync(FULL_MASK, run.y, c) - (__shfl_sync(FULL_MASK, incl, c) - t);
+              if (lane + h < take) {
+                const float4 p = __ldg(&P.pts[src]);
+                const int j = fill + lane + h;
+                stage[j] = p;
+                soa[j] = p.x; soa[NS + j] = p.y; soa[2 * NS + j] = p.z;
+              }
+            }
+            fill += take;
+            base += (uint32_t)take;
+            if (fill == NS) flush();
+          }
+          tick(GRID_PHASE_STAGE);
+          if (fill >= TKNN_GRID_FLUSH) flush();
         }
       }
+      tick(GRID_PHASE_WALK);
       if (fill > 0) flush();
     } else if (COUNT && lane == 0) {
       c_defer += 1;
@@ -317,17 +370,22 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
       trav::kl_emit<true, S>(H, cnt, k, false, P.squared != 0, P.idx_out + row * (uint64_t)k, P.dist_out + row * (uint64_t)k);
     }
     __syncwarp();
+    tick(GRID_PHASE_EMIT);
   }
 
   if (COUNT && P.counters) {
     atomicAdd(&P.counters[0], c_cells);
     atomicAdd(&P.counters[1], c_tests);
     atomicAdd(&P.counters[2], c_ins);
+    atomicAdd(&P.counters[GRID_INSERT_SLOT], c_ins);
     if (lane == 0) {
       atomicAdd(&P.counters[3], c_wcells);
       atomicAdd(&P.counters[4], c_wstaged);
       atomicAdd(&P.counters[5], c_wpts);
       if (c_defer) atomicAdd(&P.counters[7], c_defer);
+#pragma unroll
+      for (int ph = 0; ph < GRID_PHASES; ++ph) atomicAdd(&P.counters[GRID_PHASE_SLOT + ph], c_phase[ph]);
+      atomicAdd(&P.counters[GRID_INSERT_ITER_SLOT], c_iters);
     }
   }
 }

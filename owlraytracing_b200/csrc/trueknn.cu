@@ -489,10 +489,10 @@ int run_rounds(tknn_ctx* c, const Job& job, int* launches_io) {
 
 // Sampled k-th-neighbour distance -> start radius (role of Util/random_sample.py:5-32), entirely on the device: the
 // sample queue is generated by a kernel, the sampled queries run one unbounded final round (one warp per query), and a
-// one-block radix select leaves {r, r * r} at sc[SC_QUANTILE].  Nothing is copied and nothing waits: round 1 reads r2
-// from there (Job::r_dev).
+// one-block radix select leaves {r, r * r} at sc[SC_QUANTILE], r the quantile_pm per-mille quantile of the sampled k-th
+// neighbour distances.  Nothing is copied and nothing waits: round 1 reads r2 from there (Job::r_dev).
 int estimate_radius_device(tknn_ctx* c, const float4* queries, uint64_t q_begin, uint64_t nq, const int32_t* self_ids,
-                           int self_is_row, const uint32_t* seg_of, int k, int* launches) {
+                           int self_is_row, const uint32_t* seg_of, int k, int quantile_pm, int* launches) {
   // sample_groups runs of 32 consecutive sorted positions: neighbouring queries walk nearly the same nodes and leaves
   const uint64_t groups = (nq + 31) / 32;
   const uint64_t sg = std::min<uint64_t>((uint64_t)std::max(1, c->sample_groups), groups);
@@ -524,11 +524,12 @@ int estimate_radius_device(tknn_ctx* c, const float4* queries, uint64_t q_begin,
   int rc = run_rounds(c, job, launches);
   c->counters = saved;
   TK_TRY(rc);
-  const uint32_t pos = (uint32_t)((double)(m - 1) * std::min(1000, std::max(0, c->radius_quantile)) / 1000.0);
+  const int qpm = std::min(1000, std::max(0, quantile_pm));
+  const uint32_t pos = (uint32_t)((double)(m - 1) * qpm / 1000.0);
   // a segmented build leaves the rows of segments with at most k points unfilled: the quantile ignores them
   trav::radius_quantile_kernel<<<1, 1024, 0, c->stream>>>(dd, (uint32_t)m, k, pos,
                                                           reinterpret_cast<float*>(c->scalars.as<uint32_t>() + SC_QUANTILE),
-                                                          c->segmented ? std::min(1000, std::max(0, c->radius_quantile)) : -1);
+                                                          c->segmented ? qpm : -1);
   TK_CUDA(c, cudaGetLastError());
   if (launches) *launches += 2;
   return TKNN_OK;
@@ -665,7 +666,7 @@ int read_error_flag(tknn_ctx* c) {
 
 int collect_counters(tknn_ctx* c) {
   if (!c->counters) return TKNN_OK;
-  unsigned long long h[8];
+  unsigned long long h[N_COUNTERS];
   TK_CUDA(c, cudaMemcpyAsync(h, c->scalars.as<uint32_t>() + SC_COUNTERS, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
   TK_CUDA(c, cudaStreamSynchronize(c->stream));
   c->stats.nodes_visited = h[0];
@@ -676,6 +677,10 @@ int collect_counters(tknn_ctx* c) {
   c->stats.warp_point_loads = h[5];
   c->stats.filter_violations = h[6];
   c->stats.grid_deferred = h[7];
+  static_assert(grid::GRID_PHASES == 6 && grid::GRID_INSERT_SLOT < N_COUNTERS, "tknn_stats::grid_phase_cycles");
+  for (int p = 0; p < grid::GRID_PHASES; ++p) c->stats.grid_phase_cycles[p] = h[grid::GRID_PHASE_SLOT + p];
+  c->stats.grid_insert_iters = h[grid::GRID_INSERT_ITER_SLOT];
+  c->stats.grid_inserts = h[grid::GRID_INSERT_SLOT];
   return TKNN_OK;
 }
 
@@ -702,6 +707,8 @@ void reset_search_stats(tknn_ctx* c) {
   s.warp_node_visits = s.warp_leaf_visits = s.warp_point_loads = s.filter_violations = 0;
   s.grid_rounds = 0;
   s.grid_deferred = 0;
+  std::memset(s.grid_phase_cycles, 0, sizeof(s.grid_phase_cycles));
+  s.grid_insert_iters = s.grid_inserts = 0;
   s.d2h_bytes = 0;
   c->mailbox_launches = 0;
 }
@@ -743,13 +750,16 @@ int tknn::host::search_range(tknn_ctx* c, int k, float start_radius, uint64_t q_
   }
 
   TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), c->stream));
-  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), c->stream));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, N_COUNTERS * sizeof(unsigned long long), c->stream));
   TK_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
   int launches = 0;
   float r0 = start_radius;
   const bool estimated = nq > 0 && !(r0 > 0.0f);
+  // round 1 on the cell grid (run_rounds: grid_ok) has its own start-radius quantile (TKNN_OPT_GRID_RADIUS_QUANTILE)
+  const bool grid_round1 = c->grid_on && !c->segmented && k <= trav::LIST_MAX_K;
   if (estimated)
-    TK_TRY(estimate_radius_device(c, c->pts.as<float4>(), q_begin, nq, nullptr, 1, c->seg_of.as<uint32_t>(), k, &launches));
+    TK_TRY(estimate_radius_device(c, c->pts.as<float4>(), q_begin, nq, nullptr, 1, c->seg_of.as<uint32_t>(), k,
+                                  grid_round1 ? c->grid_radius_quantile : c->radius_quantile, &launches));
   TK_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   c->stats.start_radius = r0;
 
@@ -1064,6 +1074,10 @@ int tknn_set_option(tknn_ctx* c, int key, int64_t value) {
       if (value < 0 || value > 1000) return fail(c, TKNN_EINVAL, "radius quantile outside [0, 1000] per mille");
       c->radius_quantile = (int)value;
       return TKNN_OK;
+    case TKNN_OPT_GRID_RADIUS_QUANTILE:
+      if (value < 0 || value > 1000) return fail(c, TKNN_EINVAL, "grid radius quantile outside [0, 1000] per mille");
+      c->grid_radius_quantile = (int)value;
+      return TKNN_OK;
     default: return fail(c, TKNN_EINVAL, "unknown option %d", key);
   }
 }
@@ -1377,7 +1391,8 @@ int tknn_estimate_start_radius(tknn_ctx* c, int k, float* radius_out) {
                                                                      (unsigned long long)c->n);
   ScopedDevice sd(c->device);
   int launches = 0;
-  TK_TRY(estimate_radius_device(c, c->pts.as<float4>(), 0, c->n, nullptr, 1, c->seg_of.as<uint32_t>(), k, &launches));
+  TK_TRY(estimate_radius_device(c, c->pts.as<float4>(), 0, c->n, nullptr, 1, c->seg_of.as<uint32_t>(), k, c->radius_quantile,
+                                &launches));
   uint32_t rb = 0;
   TK_TRY(fetch_words(c, c->scalars.as<uint32_t>() + SC_QUANTILE, 1, nullptr, 0, &rb));
   std::memcpy(radius_out, &rb, sizeof(float));
@@ -1515,14 +1530,14 @@ int query_core(tknn_ctx* c, const char* what, const float* queries, uint64_t nq,
   TK_TRY(out_view(c, idx_out, out_elems, c->stage_idx, &d_idx));
   TK_TRY(out_view(c, dist_out, out_elems, c->stage_dist, &d_dist));
 
-  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, N_COUNTERS * sizeof(unsigned long long), st));
   float r0 = start_radius;
   // a query set can hold fewer than k reachable neighbours only through self exclusion / radius caps
   const bool may_underfill = (uint64_t)k > c->n - (self_ids ? 1 : 0);
   bool estimated = false;
   if (!(r0 > 0.0f)) {
     if (init_radius2 || may_underfill) r0 = INFINITY;
-    else { TK_TRY(estimate_radius_device(c, c->q_pts.as<float4>(), 0, nq, d_sid_sorted, 0, d_seg_sorted, k, &launches)); estimated = true; }
+    else { TK_TRY(estimate_radius_device(c, c->q_pts.as<float4>(), 0, nq, d_sid_sorted, 0, d_seg_sorted, k, c->radius_quantile, &launches)); estimated = true; }
   }
   TK_CUDA(c, cudaEventRecord(c->ev[1], st));
   c->stats.start_radius = r0;
@@ -1611,7 +1626,7 @@ int tknn_range_count(tknn_ctx* c, float radius, uint32_t* count_out) {
   P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
   set_segments(c, P, c->seg_of.as<uint32_t>());
   TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), c->stream));
-  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), c->stream));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, N_COUNTERS * sizeof(unsigned long long), c->stream));
   TK_CUDA(c, cudaMemsetAsync(sc + SC_GROUP_COUNTER, 0, sizeof(uint32_t), c->stream));
   TK_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
   TK_TRY(launch_traverse<trav::MODE_RANGE_COUNT>(c, P));
@@ -1683,7 +1698,7 @@ int tknn_dbscan(tknn_ctx* c, float eps, int min_pts, int32_t* label_out, uint8_t
   P.n_core_words = n_groups;
   const unsigned blocks = blocks_for(n, dbscan::THREADS);
   TK_CUDA(c, cudaMemsetAsync(sc + SC_ERROR, 0, 2 * sizeof(uint32_t), st));
-  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, N_COUNTERS * sizeof(unsigned long long), st));
   TK_CUDA(c, cudaEventRecord(c->ev[0], st));
 
   // 1. core test over every position, then the core / non-core queues
@@ -1840,7 +1855,7 @@ int tknn_fps(tknn_ctx* c, const uint64_t* sample_offsets, uint64_t n_segments, c
   uint32_t* sc = c->scalars.as<uint32_t>();
   unsigned long long* counters = reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS);
   int launches = 0;
-  TK_CUDA(c, cudaMemsetAsync(counters, 0, 8 * sizeof(unsigned long long), st));
+  TK_CUDA(c, cudaMemsetAsync(counters, 0, N_COUNTERS * sizeof(unsigned long long), st));
   TK_CUDA(c, cudaEventRecord(c->ev[0], st));
 
   // block tier: one CTA per segment, sized for the largest one (about BLOCK_TARGET_PER points per thread)
@@ -2184,7 +2199,7 @@ int radius_core(tknn_ctx* c, const float4* qpts, uint64_t nq, const int32_t* sel
   P.group_counter = sc + SC_GROUP_COUNTER;
   P.counters = c->counters ? reinterpret_cast<unsigned long long*>(sc + SC_COUNTERS) : nullptr;
   set_segments(c, P, seg_of);
-  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, 8 * sizeof(unsigned long long), st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_COUNTERS, 0, N_COUNTERS * sizeof(unsigned long long), st));
 
   // 1. count (minus self, by position and by row), both scans, the long-row list; one read-back
   TK_CUDA(c, cudaEventRecord(ev[0], st));

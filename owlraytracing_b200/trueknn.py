@@ -171,6 +171,7 @@ class TrueKNN:
         "tie_pruning": _lib.OPT_TIE_PRUNING, "warp_round_max": _lib.OPT_WARP_ROUND_MAX, "curve": _lib.OPT_CURVE,
         "speculative_max": _lib.OPT_SPECULATIVE_MAX, "sparse_team": _lib.OPT_SPARSE_TEAM, "sort_mode": _lib.OPT_SORT_MODE,
         "grid": _lib.OPT_GRID, "grid_level": _lib.OPT_GRID_LEVEL,
+        "grid_radius_quantile": _lib.OPT_GRID_RADIUS_QUANTILE,
     }
 
     def set_option(self, name: str, value: int):
