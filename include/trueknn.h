@@ -63,7 +63,8 @@ enum {
   TKNN_OPT_RADIUS_QUANTILE = 7 /* start-radius estimator: per-mille quantile of the sampled k-th
                                   neighbour distance (default 990)                                */
   ,TKNN_OPT_KEEP_SCRATCH = 8   /* 1 (default): keep the grow-only scratch of builds, queries (tknn_query*,
-                                  tknn_radius_query*), radius lists and interpolation for the next call;
+                                  tknn_radius_query*), radius lists, interpolation, tknn_knn_backward and
+                                  tknn_segment_reduce for the next call;
                                   0: release it when each such call returns                              */
   ,TKNN_OPT_APPROX_FILTER = 10 /* 1: conservative 3-FMA pre-filter before the exact distance test
                                   (DESIGN.md §3.2; audited, -1 % time); 0 (default): exact test on every pair */
@@ -382,6 +383,7 @@ TKNN_API int tknn_voxel_members(tknn_ctx* ctx, uint64_t* offsets_out, int32_t* m
 
 #define TKNN_REDUCE_MEAN 0
 #define TKNN_REDUCE_MAX 1
+#define TKNN_REDUCE_SUM 2 /* tknn_segment_reduce only */
 /* Pools the rows x (n x f, pitch stride_floats >= f, 1 <= f <= 1024, host or device) over the last clustering into
  * out (n_voxels x f, host or device).  n must be the clustering's point count.  Members are taken in ascending index.
  * TKNN_REDUCE_MEAN: the members are split into chunks of 32 consecutive members, each chunk summed in order from +0.0f,
@@ -431,6 +433,44 @@ TKNN_API int tknn_interpolate(tknn_ctx* ctx, const int32_t* idx, const float* d2
  * {nq, nq * k, n}. */
 TKNN_API int tknn_interpolate_backward(tknn_ctx* ctx, const int32_t* idx, const float* weight, const float* den, uint64_t nq,
                                        int k, const float* grad_out, int g_stride_floats, uint64_t n, int f, float* grad_x);
+
+/* Gradient of kNN squared distances with respect to both point sets (PyTorch3D's knn_points backward; the backward
+ * pass of the Chamfer distance, DESIGN.md §3.11).  queries: nq rows with pitch q_stride_floats, points: n rows with
+ * pitch p_stride_floats, dim 2 or 3 coordinate columns; idx and grad_d2: nq x k, dense, the rows of tknn_query /
+ * tknn_query_segments and the gradient of their squared distances.  A slot with idx = -1 is skipped (its grad_d2 is not
+ * read).  Every other slot (i, s) is an edge e = i*k + s with j = idx[i,s]; in fp32, every operation rounded on its own
+ * (round-to-nearest, no FMA), t = fl(2 * grad_d2[i,s]) and for each column c < dim:
+ *   term_q[e,c] = fl(t * fl(q[i,c] - p[j,c])),   term_p[e,c] = fl(t * fl(p[j,c] - q[i,c]))
+ *   grad_q[i,c] = the chunked sum of term_q over row i's edges in slot order
+ *   grad_p[j,c] = the chunked sum of term_p over the edges with idx = j in ascending e (+0 for a row no edge references)
+ * The chunked sum is the TKNN_REDUCE_MEAN rule of tknn_voxel_pool without the division: chunks of 32 consecutive terms,
+ * each summed in order from +0, then the chunk sums in chunk order from +0 (32 terms or fewer: the plain sequential
+ * sum).  This is PyTorch3D's 2 * grad * diff (the analytic gradient of d2, not the derivative of the rounded fma chain
+ * of the distance) in a fixed order: no float atomics, so the result depends only on the inputs, on any stream and
+ * launch shape.  grad_q_out: nq x dim, grad_p_out: n x dim, dense; either may be NULL and is then not computed (both
+ * NULL: a no-op).  Host or device arrays.  The call needs no build and touches none.
+ * Errors (TKNN_EINVAL): dim not 2 or 3, a stride below dim, k outside [1, TKNN_MAX_K], n or nq >= 2^31, nq * k above
+ * 2^30 - 1 edges (the edge sort's limit), an idx entry outside {-1} and [0, n) (found on the device and reported after
+ * the call, whose outputs are then undefined), and a NULL queries, idx or grad_d2, or a NULL points with n > 0, when
+ * nq > 0 and an output is requested.  nq = 0 fills grad_p_out with +0.
+ * Statistics: n_queries, k, search_ms, d2h_ms; rounds = 3 phases in round_ms: the terms (with grad_q) and the edge keys,
+ * the sort, then the run offsets and the chunked sums; kernel_ms likewise; round_queries = {nq, nq * k, n} ({nq, 0, 0}
+ * without grad_p_out). */
+TKNN_API int tknn_knn_backward(tknn_ctx* ctx, const float* queries, uint64_t nq, int q_stride_floats,
+                               const float* points, uint64_t n, int p_stride_floats, int dim,
+                               const int32_t* idx, int k, const float* grad_d2,
+                               float* grad_q_out, float* grad_p_out);
+
+/* Per-segment sum or mean of rows (the point and batch reductions of the Chamfer loss).  x: n rows of f columns with
+ * pitch stride_floats >= f, 1 <= f <= 1024; segment s is the rows [seg_offsets[s], seg_offsets[s + 1]) (n_segments + 1
+ * offsets, validated as for tknn_build_segments; NULL: one segment, n_segments must then be 1).  TKNN_REDUCE_SUM: the
+ * chunked sum of the segment's rows in index order (chunks of 32 consecutive rows, each summed from +0, then the chunk
+ * sums in order from +0); TKNN_REDUCE_MEAN: fl(sum / (float)count), tknn_voxel_pool's mean.  An empty segment gives +0
+ * for both.  out: n_segments x f, dense.  Host or device arrays.  Needs no build and touches none; no float atomics.
+ * Errors (TKNN_EINVAL): f outside [1, 1024], a stride below f, another reduce (TKNN_REDUCE_MAX included), n_segments
+ * outside [1, 2^31 - 1], malformed offsets, a NULL out, or a NULL x with n > 0. */
+TKNN_API int tknn_segment_reduce(tknn_ctx* ctx, const float* x, uint64_t n, int f, int stride_floats,
+                                 const uint64_t* seg_offsets, uint64_t n_segments, int reduce, float* out);
 
 /* Start-radius estimator alone (replaces samples/s01-trueknn/Util/random_sample.py:5-32). */
 TKNN_API int tknn_estimate_start_radius(tknn_ctx* ctx, int k, float* radius_out);

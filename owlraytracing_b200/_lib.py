@@ -98,7 +98,7 @@ class DistStats(C.Structure):
 
 
 SHARD_QUERIES, PARTITION_POINTS = 1, 2
-REDUCE_MEAN, REDUCE_MAX = 0, 1
+REDUCE_MEAN, REDUCE_MAX, REDUCE_SUM = 0, 1, 2
 UNIQUE_ID_BYTES = 128
 
 # every symbol include/trueknn.h declares (tests check the library exports all of them)
@@ -115,6 +115,7 @@ EXPORTS = [
     "tknn_radius_search", "tknn_radius_query", "tknn_write_neighbour_lists", "tknn_build_segments",
     "tknn_query_segments", "tknn_radius_query_segments", "tknn_fps", "tknn_feature_knn",
     "tknn_voxel_grid", "tknn_voxel_members", "tknn_voxel_pool", "tknn_interpolate", "tknn_interpolate_backward",
+    "tknn_knn_backward", "tknn_segment_reduce",
 ]
 
 _lib = None
@@ -155,6 +156,8 @@ def load() -> C.CDLL:
     L.tknn_voxel_pool.argtypes = [vp, vp, u64, C.c_int, C.c_int, C.c_int, vp]
     L.tknn_interpolate.argtypes = [vp, vp, vp, u64, C.c_int, vp, u64, C.c_int, C.c_int, vp, vp, vp]
     L.tknn_interpolate_backward.argtypes = [vp, vp, vp, vp, u64, C.c_int, vp, C.c_int, u64, C.c_int, vp]
+    L.tknn_knn_backward.argtypes = [vp, vp, u64, C.c_int, vp, u64, C.c_int, C.c_int, vp, C.c_int, vp, vp, vp]
+    L.tknn_segment_reduce.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, C.c_int, vp]
     L.tknn_radius_search.argtypes = [vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_radius_query.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_query_segments.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, vp, vp, C.c_int, f32, vp, vp]

@@ -104,6 +104,12 @@ struct tknn_ctx {
   // touches no build state.
   DevBuf ip_idx, ip_w, ip_den, ip_x, ip_out, ip_wout, ip_dout, ip_keys_a, ip_keys_b, ip_vals_a, ip_vals_b, ip_sort_tmp,
       ip_cnt, ip_off;
+  // tknn_knn_backward / tknn_segment_reduce scratch (grow-only unless keep_scratch == 0: knn_grad_scratch, knn_grad.cuh):
+  // staged host inputs and outputs, term_p, the edge keys, values, sort buffers, per-row counts and run offsets, and the
+  // chunk layout of the pooling (chunks per run, their scan, the long runs, the count words and the chunk results).  It
+  // touches no build state.
+  DevBuf kg_q, kg_p, kg_idx, kg_g, kg_gq, kg_gp, kg_terms, kg_keys_a, kg_keys_b, kg_vals_a, kg_vals_b, kg_sort_tmp,
+      kg_cnt, kg_off, kg_x, kg_seg_off, kg_out, kg_chunks, kg_chunk_off, kg_longs, kg_words, kg_cs;
   // cell grid over the sorted points (grid.cuh): runs per level-L cell and the table's frame; made by a plain build when
   // the cloud qualifies, and then round 1 of a dense kNN search with k <= 24 walks it instead of the LBVH
   int grid_mode = 0;        // TKNN_OPT_GRID: 0 = auto (occupancy decides), 1 = off, 2 = whenever the table is valid
@@ -270,6 +276,13 @@ inline ScratchScope radius_list_scratch(tknn_ctx* c) {
 inline ScratchScope interp_scratch(tknn_ctx* c) {  // rl_sums: the backward's run-offset scan
   return ScratchScope({&c->ip_idx, &c->ip_w, &c->ip_den, &c->ip_x, &c->ip_out, &c->ip_wout, &c->ip_dout, &c->ip_keys_a,
                        &c->ip_keys_b, &c->ip_vals_a, &c->ip_vals_b, &c->ip_sort_tmp, &c->ip_cnt, &c->ip_off, &c->rl_sums},
+                      c);
+}
+inline ScratchScope knn_grad_scratch(tknn_ctx* c) {  // rl_sums: the run-offset and chunk-offset scans
+  return ScratchScope({&c->kg_q, &c->kg_p, &c->kg_idx, &c->kg_g, &c->kg_gq, &c->kg_gp, &c->kg_terms, &c->kg_keys_a,
+                       &c->kg_keys_b, &c->kg_vals_a, &c->kg_vals_b, &c->kg_sort_tmp, &c->kg_cnt, &c->kg_off, &c->kg_x,
+                       &c->kg_seg_off, &c->kg_out, &c->kg_chunks, &c->kg_chunk_off, &c->kg_longs, &c->kg_words,
+                       &c->kg_cs, &c->rl_sums},
                       c);
 }
 

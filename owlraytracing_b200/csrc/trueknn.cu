@@ -22,6 +22,7 @@
 #include "fps.cuh"
 #include "grid.cuh"
 #include "interpolate.cuh"
+#include "knn_grad.cuh"
 #include "lbvh.cuh"
 #include "radix_sort.cuh"
 #include "radius.cuh"
@@ -979,7 +980,10 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->vx_word_off, &c->vx_members, &c->vx_off, &c->vx_first, &c->vx_seg, &c->vx_chunks, &c->vx_chunk_off,
                     &c->vx_words_sc, &c->vx_x, &c->vx_out, &c->vx_cs, &c->vx_longs, &c->ip_idx, &c->ip_w, &c->ip_den,
                     &c->ip_x, &c->ip_out, &c->ip_wout, &c->ip_dout, &c->ip_keys_a, &c->ip_keys_b, &c->ip_vals_a,
-                    &c->ip_vals_b, &c->ip_sort_tmp, &c->ip_cnt, &c->ip_off})
+                    &c->ip_vals_b, &c->ip_sort_tmp, &c->ip_cnt, &c->ip_off, &c->kg_q, &c->kg_p, &c->kg_idx, &c->kg_g,
+                    &c->kg_gq, &c->kg_gp, &c->kg_terms, &c->kg_keys_a, &c->kg_keys_b, &c->kg_vals_a, &c->kg_vals_b,
+                    &c->kg_sort_tmp, &c->kg_cnt, &c->kg_off, &c->kg_x, &c->kg_seg_off, &c->kg_out, &c->kg_chunks,
+                    &c->kg_chunk_off, &c->kg_longs, &c->kg_words, &c->kg_cs})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -2714,6 +2718,64 @@ unsigned voxel_blocks(tknn_ctx* c, uint64_t work) {
   return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((work + voxel::THREADS - 1) / voxel::THREADS, (uint64_t)c->sm_count * 16));
 }
 
+// The chunk layout of the pooling of voxel.cuh over the runs [vox_off[v], vox_off[v + 1]) of `members` entries in all,
+// v < *nv_dev <= bound (device words): chunks[v] and their scan chunk_off (bound + 1), the long runs listed in longs,
+// and in words[0, 2) the number of long-run chunks (u64), in words[2] the number of long runs.  Launches only: the
+// caller reads the words back.
+int pool_layout(tknn_ctx* c, const uint64_t* vox_off, const uint32_t* nv_dev, uint64_t bound, uint64_t members,
+                DevBuf& chunks, DevBuf& chunk_off, DevBuf& longs, uint32_t* words, int* launches) {
+  TK_TRY(ensure(c, chunks, bound * sizeof(uint32_t)));
+  TK_TRY(ensure(c, chunk_off, (bound + 1) * sizeof(uint64_t)));
+  TK_TRY(ensure(c, longs, (std::min(bound, members / (voxel::LONG_VOXEL + 1)) + 1) * sizeof(uint32_t)));
+  TK_CUDA(c, cudaMemsetAsync(words + 2, 0, sizeof(uint32_t), c->stream));
+  voxel::long_chunks_kernel<<<blocks_for(bound, voxel::THREADS), voxel::THREADS, 0, c->stream>>>(
+      vox_off, nv_dev, bound, chunks.as<uint32_t>(), longs.as<uint32_t>(), words + 2);
+  TK_CUDA(c, cudaGetLastError());
+  ++*launches;
+  return scan_counts(c, chunks.as<uint32_t>(), bound, chunk_off.as<uint64_t>(), reinterpret_cast<uint64_t*>(words),
+                     launches);
+}
+
+template <int R, bool IDENT>
+void launch_pool(tknn_ctx* c, const voxel::PoolParams& P, const uint32_t* longs, uint64_t n_long, int* launches) {
+  cudaStream_t st = c->stream;
+  if (P.n_chunks) {  // the chunks of a sum and of a mean are the same
+    voxel::chunk_kernel<R == voxel::R_MAX ? voxel::R_MAX : voxel::R_MEAN, IDENT>
+        <<<voxel_blocks(c, P.n_chunks * P.cb), voxel::THREADS, 0, st>>>(P);
+    ++*launches;
+  }
+  voxel::voxel_kernel<R, IDENT><<<voxel_blocks(c, P.nv * P.cb), voxel::THREADS, 0, st>>>(P);
+  ++*launches;
+  if (n_long) {
+    voxel::fold_kernel<R, IDENT><<<voxel_blocks(c, n_long * P.cb * 32), voxel::THREADS, 0, st>>>(P, longs, n_long);
+    ++*launches;
+  }
+}
+
+// The column passes of the pooling over a layout of pool_layout: P holds x, stride, f, members (nullptr: member j is
+// row j), vox_off, chunk_off, nv, n_chunks and out; the columns run in passes so that the chunk results in cs stay
+// bounded.  reduce: voxel::R_MEAN / R_MAX / R_SUM.
+int pool_columns(tknn_ctx* c, voxel::PoolParams P, int reduce, const uint32_t* longs, uint64_t n_long, DevBuf& cs,
+                 int* launches) {
+  const uint64_t chunks = P.n_chunks;
+  const int f = P.f;
+  const int cb = chunks ? (int)std::min<uint64_t>((uint64_t)f, std::max<uint64_t>(1, VOXEL_CS_FLOATS / chunks)) : f;
+  if (chunks) TK_TRY(ensure(c, cs, chunks * (uint64_t)cb * sizeof(float)));
+  P.cs = cs.as<float>();
+  const bool ident = P.members == nullptr;
+  for (int c0 = 0; c0 < f; c0 += cb) {
+    P.c0 = c0;
+    P.cb = std::min(cb, f - c0);
+    if (reduce == voxel::R_MAX) launch_pool<voxel::R_MAX, false>(c, P, longs, n_long, launches);
+    else if (reduce == voxel::R_MEAN && !ident) launch_pool<voxel::R_MEAN, false>(c, P, longs, n_long, launches);
+    else if (reduce == voxel::R_MEAN) launch_pool<voxel::R_MEAN, true>(c, P, longs, n_long, launches);
+    else if (!ident) launch_pool<voxel::R_SUM, false>(c, P, longs, n_long, launches);
+    else launch_pool<voxel::R_SUM, true>(c, P, longs, n_long, launches);
+    TK_CUDA(c, cudaGetLastError());
+  }
+  return TKNN_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -2850,9 +2912,6 @@ int tknn_voxel_grid(tknn_ctx* c, const float* points, uint64_t n, int dim, int s
   TK_TRY(ensure(c, c->vx_off, (n + 1) * sizeof(uint64_t)));
   TK_TRY(ensure(c, c->vx_first, n * sizeof(int32_t)));
   TK_TRY(ensure(c, c->vx_seg, n * sizeof(int32_t)));
-  TK_TRY(ensure(c, c->vx_chunks, n * sizeof(uint32_t)));
-  TK_TRY(ensure(c, c->vx_chunk_off, (n + 1) * sizeof(uint64_t)));
-  TK_TRY(ensure(c, c->vx_longs, (n / (voxel::LONG_VOXEL + 1) + 1) * sizeof(uint32_t)));
   voxel::heads_kernel<<<blocks_for(n, voxel::THREADS), voxel::THREADS, 0, st>>>(keys, n, packed ? voxel::IDX_BITS : 0,
                                                                                  c->vx_words.as<uint32_t>());
   TK_CUDA(c, cudaGetLastError());
@@ -2862,11 +2921,7 @@ int tknn_voxel_grid(tknn_ctx* c, const float* points, uint64_t n, int dim, int s
                         c->vx_first.as<int32_t>(), c->vx_seg.as<int32_t>()};
   voxel::label_kernel<<<blocks_for(n, voxel::THREADS), voxel::THREADS, 0, st>>>(Lp);
   uint32_t* sc = c->scalars.as<uint32_t>();
-  voxel::long_chunks_kernel<<<blocks_for(n, voxel::THREADS), voxel::THREADS, 0, st>>>(c->vx_off.as<uint64_t>(), sc + SC_TOTAL,
-                                                                                      n, c->vx_chunks.as<uint32_t>(),
-                                                                                      c->vx_longs.as<uint32_t>(), w + 12);
-  TK_CUDA(c, cudaGetLastError());
-  TK_TRY(scan_counts(c, c->vx_chunks.as<uint32_t>(), n, c->vx_chunk_off.as<uint64_t>(), reinterpret_cast<uint64_t*>(w + 10),
+  TK_TRY(pool_layout(c, c->vx_off.as<uint64_t>(), sc + SC_TOTAL, n, n, c->vx_chunks, c->vx_chunk_off, c->vx_longs, w + 10,
                      &launches));
   if (raw_out) TK_CUDA(c, cudaMemcpyAsync(raw_out, c->vx_raw.p, n * sizeof(int64_t), cudaMemcpyDefault, st));
   if (cluster_out) TK_CUDA(c, cudaMemcpyAsync(cluster_out, c->vx_cluster.p, n * sizeof(int32_t), cudaMemcpyDefault, st));
@@ -2924,28 +2979,11 @@ int tknn_voxel_pool(tknn_ctx* c, const float* x, uint64_t n, int f, int stride_f
     feat::finite_kernel<<<voxel_blocks(c, n * (uint64_t)f), 256, 0, st>>>(d_x, n, f, stride_floats, w + 8);
     TK_CUDA(c, cudaGetLastError());
   }
-  // columns in passes so that the chunk results of long voxels stay bounded
-  const uint64_t chunks = c->vx_long_chunks;
-  const int cb = chunks ? (int)std::min<uint64_t>((uint64_t)f, std::max<uint64_t>(1, VOXEL_CS_FLOATS / chunks)) : f;
-  if (chunks) TK_TRY(ensure(c, c->vx_cs, chunks * (uint64_t)cb * sizeof(float)));
-  voxel::PoolParams P{d_x, stride_floats, f, 0, cb, c->vx_members.as<uint32_t>(), c->vx_off.as<uint64_t>(),
-                      c->vx_chunk_off.as<uint64_t>(), nv, chunks, c->vx_cs.as<float>(), d_out};
-  for (int c0 = 0; c0 < f; c0 += cb) {
-    P.c0 = c0;
-    P.cb = std::min(cb, f - c0);
-    if (chunks) {
-      if (mx) voxel::chunk_kernel<true><<<voxel_blocks(c, chunks * P.cb), voxel::THREADS, 0, st>>>(P);
-      else voxel::chunk_kernel<false><<<voxel_blocks(c, chunks * P.cb), voxel::THREADS, 0, st>>>(P);
-    }
-    if (mx) voxel::voxel_kernel<true><<<voxel_blocks(c, nv * P.cb), voxel::THREADS, 0, st>>>(P);
-    else voxel::voxel_kernel<false><<<voxel_blocks(c, nv * P.cb), voxel::THREADS, 0, st>>>(P);
-    if (c->vx_n_long) {
-      const unsigned fb = voxel_blocks(c, c->vx_n_long * P.cb * 32);
-      if (mx) voxel::fold_kernel<true><<<fb, voxel::THREADS, 0, st>>>(P, c->vx_longs.as<uint32_t>(), c->vx_n_long);
-      else voxel::fold_kernel<false><<<fb, voxel::THREADS, 0, st>>>(P, c->vx_longs.as<uint32_t>(), c->vx_n_long);
-    }
-    TK_CUDA(c, cudaGetLastError());
-  }
+  voxel::PoolParams P{d_x, stride_floats, f, 0, f, c->vx_members.as<uint32_t>(), c->vx_off.as<uint64_t>(),
+                      c->vx_chunk_off.as<uint64_t>(), nv, c->vx_long_chunks, nullptr, d_out};
+  int launches = 0;
+  TK_TRY(pool_columns(c, P, mx ? voxel::R_MAX : voxel::R_MEAN, c->vx_longs.as<uint32_t>(), c->vx_n_long, c->vx_cs,
+                      &launches));
   TK_TRY(copy_back(c, out, d_out, nv * (size_t)f));
   if (mx) {
     uint32_t bad = 0;
@@ -3161,6 +3199,210 @@ int tknn_interpolate_backward(tknn_ctx* c, const int32_t* idx, const float* weig
     return TKNN_OK;
   }
   return interpolate_backward_core(c, idx, weight, den, nq, k, grad_out, g_stride_floats, n, f, grad_x);
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// gradients of kNN squared distances and segment reductions (knn_grad.cuh, voxel.cuh's pooling, DESIGN.md §3.11)
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+unsigned kgrad_blocks(tknn_ctx* c, uint64_t threads) {
+  return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((threads + kgrad::THREADS - 1) / kgrad::THREADS,
+                                                            (uint64_t)c->sm_count * 16));
+}
+
+// Uploads nv (< 2^32) to words[3] and lays out the chunks of the nv runs of vox_off (pool_layout); returns the chunk
+// totals through *long_chunks / *n_long.  `extra` (device word or nullptr) is read back in the same transfer.
+int kgrad_layout(tknn_ctx* c, const uint64_t* vox_off, uint64_t nv, uint64_t members, const uint32_t* extra,
+                 uint64_t* long_chunks, uint64_t* n_long, uint32_t* extra_out, int* launches) {
+  TK_TRY(ensure(c, c->kg_words, 4 * sizeof(uint32_t)));
+  uint32_t* w = c->kg_words.as<uint32_t>();  // [0, 2) long-run chunks (u64), 2 long runs, 3 nv
+  const uint32_t nv32 = (uint32_t)nv;
+  TK_CUDA(c, cudaMemcpyAsync(w + 3, &nv32, sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+  TK_TRY(pool_layout(c, vox_off, w + 3, nv, members, c->kg_chunks, c->kg_chunk_off, c->kg_longs, w, launches));
+  uint32_t h[4] = {0, 0, 0, 0};
+  TK_TRY(fetch_words(c, w, 3, extra, extra ? 1 : 0, h));  // synchronises the stream
+  *long_chunks = (uint64_t)h[0] | ((uint64_t)h[1] << 32);
+  *n_long = h[2];
+  if (extra_out) *extra_out = h[3];
+  return TKNN_OK;
+}
+
+template <int D>
+void launch_terms(tknn_ctx* c, const kgrad::Params& P) {
+  kgrad::terms_kernel<D><<<kgrad_blocks(c, P.nq), kgrad::THREADS, 0, c->stream>>>(P);
+}
+
+int knn_backward_core(tknn_ctx* c, const float* queries, uint64_t nq, int q_stride, const float* points, uint64_t n,
+                      int p_stride, int dim, const int32_t* idx, int k, const float* grad_d2, float* grad_q,
+                      float* grad_p) {
+  const char* what = "tknn_knn_backward";
+  cudaStream_t st = c->stream;
+  const uint64_t edges = nq * (uint64_t)k;
+  const bool want_p = grad_p && n > 0;
+  ScratchScope scratch = knn_grad_scratch(c);
+  const float *d_q = nullptr, *d_p = nullptr, *d_g = nullptr;
+  const int32_t* d_idx = nullptr;
+  TK_TRY(stage_in(c, queries, (size_t)(nq - 1) * q_stride + dim, c->kg_q, &d_q));
+  if (n) TK_TRY(stage_in(c, points, (size_t)(n - 1) * p_stride + dim, c->kg_p, &d_p));
+  TK_TRY(stage_in(c, idx, edges, c->kg_idx, &d_idx));
+  TK_TRY(stage_in(c, grad_d2, edges, c->kg_g, &d_g));
+  float *d_gq = nullptr, *d_gp = nullptr;
+  TK_TRY(out_view(c, grad_q, (size_t)nq * dim, c->kg_gq, &d_gq));
+  if (want_p) {
+    TK_TRY(out_view(c, grad_p, (size_t)n * dim, c->kg_gp, &d_gp));
+    TK_TRY(ensure(c, c->kg_terms, edges * dim * sizeof(float)));
+    TK_TRY(ensure(c, c->kg_keys_a, edges * sizeof(uint64_t)));
+    TK_TRY(ensure(c, c->kg_keys_b, edges * sizeof(uint64_t)));
+    TK_TRY(ensure(c, c->kg_vals_a, edges * sizeof(uint32_t)));
+    TK_TRY(ensure(c, c->kg_vals_b, edges * sizeof(uint32_t)));
+    TK_TRY(ensure(c, c->kg_sort_tmp, rsort::temp_words(edges) * sizeof(uint32_t)));
+    TK_TRY(ensure(c, c->kg_cnt, n * sizeof(uint32_t)));
+    TK_TRY(ensure(c, c->kg_off, (n + 1) * sizeof(uint64_t)));
+  }
+  TK_TRY(ensure_round_events(c, 12));
+  cudaEvent_t* ev = c->round_ev.data();  // phase r: [4r] start, [4r + 1] end, [4r + 2 / + 3] its kernels
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  int launches = 0;
+  TK_CUDA(c, cudaEventRecord(c->ev[0], st));
+
+  // 1. terms and grad_q; edge keys and per-row counts
+  TK_CUDA(c, cudaEventRecord(ev[0], st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_QBAD, 0, sizeof(uint32_t), st));
+  if (want_p) TK_CUDA(c, cudaMemsetAsync(c->kg_cnt.p, 0, n * sizeof(uint32_t), st));
+  TK_CUDA(c, cudaEventRecord(ev[2], st));
+  const kgrad::Params P{d_q, d_p, d_idx, d_g, nq, (uint32_t)n, k, q_stride, p_stride, d_gq,
+                        want_p ? c->kg_terms.as<float>() : nullptr, sc + SC_QBAD};
+  if (dim == 2) launch_terms<2>(c, P);
+  else launch_terms<3>(c, P);
+  TK_CUDA(c, cudaGetLastError());
+  ++launches;
+  if (want_p) {
+    interp::edge_kernel<<<interp_blocks(c, edges), interp::THREADS, 0, st>>>(
+        d_idx, edges, (uint32_t)n, c->kg_keys_a.as<uint64_t>(), c->kg_vals_a.as<uint32_t>(), c->kg_cnt.as<uint32_t>(),
+        sc + SC_QBAD);
+    TK_CUDA(c, cudaGetLastError());
+    ++launches;
+  }
+  TK_CUDA(c, cudaEventRecord(ev[3], st));
+  TK_CUDA(c, cudaEventRecord(ev[1], st));
+
+  // 2. stable sort of the edges by data row: keys 0 .. n need bits(n) bits
+  bool in_b = false;
+  TK_CUDA(c, cudaEventRecord(ev[4], st));
+  TK_CUDA(c, cudaEventRecord(ev[6], st));
+  if (want_p) {
+    const int passes = (64 - __builtin_clzll(n) + 7) / 8;
+    launches += rsort::sort_pairs(c->kg_keys_a.as<uint64_t>(), c->kg_vals_a.as<uint32_t>(), c->kg_keys_b.as<uint64_t>(),
+                                  c->kg_vals_b.as<uint32_t>(), edges, c->kg_sort_tmp.as<uint32_t>(), c->sm_count, st,
+                                  passes, &in_b);
+    TK_CUDA(c, cudaGetLastError());
+  }
+  TK_CUDA(c, cudaEventRecord(ev[7], st));
+  TK_CUDA(c, cudaEventRecord(ev[5], st));
+
+  // 3. run offsets, the chunk layout of the runs, the chunked sums of term_p
+  TK_CUDA(c, cudaEventRecord(ev[8], st));
+  TK_CUDA(c, cudaEventRecord(ev[10], st));
+  uint32_t bad = 0;
+  if (want_p) {
+    uint64_t* off = c->kg_off.as<uint64_t>();
+    TK_TRY(scan_counts(c, c->kg_cnt.as<uint32_t>(), n, off, off + n, &launches));
+    uint64_t long_chunks = 0, n_long = 0;
+    TK_TRY(kgrad_layout(c, off, n, edges, sc + SC_QBAD, &long_chunks, &n_long, &bad, &launches));
+    if (bad) return fail(c, TKNN_EINVAL, "%s: an idx entry lies outside {-1} and [0, n = %llu)", what, (unsigned long long)n);
+    const voxel::PoolParams Pp{c->kg_terms.as<float>(), dim, dim, 0, dim, in_b ? c->kg_vals_b.as<uint32_t>() : c->kg_vals_a.as<uint32_t>(),
+                               off, c->kg_chunk_off.as<uint64_t>(), n, long_chunks, nullptr, d_gp};
+    TK_TRY(pool_columns(c, Pp, voxel::R_SUM, c->kg_longs.as<uint32_t>(), n_long, c->kg_cs, &launches));
+  }
+  TK_CUDA(c, cudaEventRecord(ev[11], st));
+  TK_CUDA(c, cudaEventRecord(ev[9], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
+  TK_TRY(copy_back(c, grad_q, d_gq, (size_t)nq * dim));
+  if (want_p) TK_TRY(copy_back(c, grad_p, d_gp, (size_t)n * dim));
+  TK_CUDA(c, cudaEventRecord(c->ev[3], st));
+  TK_TRY(fetch_words(c, sc + SC_QBAD, 1, nullptr, 0, &bad));  // synchronises the stream
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.d2h_ms, c->ev[2], c->ev[3]));
+  c->stats.rounds = 3;
+  c->stats.round_queries[0] = nq;
+  c->stats.round_queries[1] = want_p ? edges : 0;
+  c->stats.round_queries[2] = want_p ? n : 0;
+  c->stats.kernel_launches = (uint32_t)(launches + c->mailbox_launches);
+  TK_TRY(finish_round_stats(c));
+  if (bad) return fail(c, TKNN_EINVAL, "%s: an idx entry lies outside {-1} and [0, n = %llu)", what, (unsigned long long)n);
+  return TKNN_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tknn_knn_backward(tknn_ctx* c, const float* queries, uint64_t nq, int q_stride_floats, const float* points, uint64_t n,
+                      int p_stride_floats, int dim, const int32_t* idx, int k, const float* grad_d2, float* grad_q_out,
+                      float* grad_p_out) {
+  TK_TRY(check_ctx(c));
+  const char* what = "tknn_knn_backward";
+  if (dim != 2 && dim != 3) return fail(c, TKNN_EINVAL, "%s: dim = %d (must be 2 or 3)", what, dim);
+  if (q_stride_floats < dim || p_stride_floats < dim)
+    return fail(c, TKNN_EINVAL, "%s: strides %d and %d must be at least dim = %d", what, q_stride_floats, p_stride_floats, dim);
+  if (k < 1 || k > TKNN_MAX_K) return fail(c, TKNN_EINVAL, "%s: k = %d outside [1, %d]", what, k, TKNN_MAX_K);
+  if (n >= (1ull << 31) || nq >= (1ull << 31)) return fail(c, TKNN_EINVAL, "%s: n and nq must be below 2^31", what);
+  if (nq * (uint64_t)k > rsort::MAX_N)
+    return fail(c, TKNN_EINVAL, "%s: nq * k = %llu edges exceed the sort's %llu", what,
+                (unsigned long long)(nq * (uint64_t)k), (unsigned long long)rsort::MAX_N);
+  if (!grad_q_out && !grad_p_out) return TKNN_OK;
+  if (nq > 0 && (!queries || !idx || !grad_d2 || (n > 0 && !points)))
+    return fail(c, TKNN_EINVAL, "%s: null queries, idx, grad_d2 or points", what);
+  ScopedDevice sd(c->device);
+  reset_search_stats(c);
+  c->stats.n_queries = nq;
+  c->stats.k = k;
+  if (nq == 0) {  // no edge: every row of grad_p is +0
+    if (n && grad_p_out) TK_TRY(zero_fill(c, grad_p_out, (size_t)n * dim));
+    return TKNN_OK;
+  }
+  return knn_backward_core(c, queries, nq, q_stride_floats, points, n, p_stride_floats, dim, idx, k, grad_d2, grad_q_out,
+                           grad_p_out);
+}
+
+int tknn_segment_reduce(tknn_ctx* c, const float* x, uint64_t n, int f, int stride_floats, const uint64_t* seg_offsets,
+                        uint64_t n_segments, int reduce, float* out) {
+  TK_TRY(check_ctx(c));
+  const char* what = "tknn_segment_reduce";
+  if (f < 1 || f > 1024) return fail(c, TKNN_EINVAL, "%s: f = %d outside [1, 1024]", what, f);
+  if (stride_floats < f) return fail(c, TKNN_EINVAL, "%s: stride %d below f = %d", what, stride_floats, f);
+  if (reduce != TKNN_REDUCE_SUM && reduce != TKNN_REDUCE_MEAN) return fail(c, TKNN_EINVAL, "%s: unknown reduce %d", what, reduce);
+  if (!seg_offsets && n_segments != 1)
+    return fail(c, TKNN_EINVAL, "%s: n_segments = %llu without offsets (must be 1)", what, (unsigned long long)n_segments);
+  if (n_segments < 1 || n_segments > (uint64_t)INT32_MAX)
+    return fail(c, TKNN_EINVAL, "%s: n_segments = %llu outside [1, 2^31 - 1]", what, (unsigned long long)n_segments);
+  if (!out || (n > 0 && !x)) return fail(c, TKNN_EINVAL, "%s: null x or out", what);
+  ScopedDevice sd(c->device);
+  cudaStream_t st = c->stream;
+  std::vector<uint64_t> off{0, n};
+  if (seg_offsets) TK_TRY(read_offsets(c, what, "segment", seg_offsets, n_segments, n, "n", &off));
+  if (n == 0) return zero_fill(c, out, (size_t)n_segments * f);  // every segment is empty
+  ScratchScope scratch = knn_grad_scratch(c);
+  const float* d_x = nullptr;
+  float* d_out = nullptr;
+  TK_TRY(stage_in(c, x, (size_t)(n - 1) * stride_floats + f, c->kg_x, &d_x));
+  TK_TRY(out_view(c, out, (size_t)n_segments * f, c->kg_out, &d_out));
+  TK_TRY(ensure(c, c->kg_seg_off, off.size() * sizeof(uint64_t)));
+  TK_CUDA(c, cudaMemcpyAsync(c->kg_seg_off.p, off.data(), off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+  const uint64_t* d_off = c->kg_seg_off.as<uint64_t>();
+  int launches = 0;
+  uint64_t long_chunks = 0, n_long = 0;
+  TK_TRY(kgrad_layout(c, d_off, n_segments, n, nullptr, &long_chunks, &n_long, nullptr, &launches));
+  const voxel::PoolParams P{d_x, stride_floats, f, 0, f, nullptr, d_off, c->kg_chunk_off.as<uint64_t>(), n_segments,
+                            long_chunks, nullptr, d_out};
+  TK_TRY(pool_columns(c, P, reduce == TKNN_REDUCE_SUM ? voxel::R_SUM : voxel::R_MEAN, c->kg_longs.as<uint32_t>(), n_long,
+                      c->kg_cs, &launches));
+  TK_TRY(copy_back(c, out, d_out, (size_t)n_segments * f));
+  TK_CUDA(c, cudaStreamSynchronize(st));
+  return TKNN_OK;
 }
 
 }  // extern "C"

@@ -8,8 +8,10 @@
 // (rsort), heads of equal keys are flagged, the existing popc scan ranks them, and label_kernel scatters the dense ids,
 // the CSR offsets, the lowest index of every voxel and its cloud.
 //
-// Pooling over members in ascending index: mean = chunked sum (chunks of 32 consecutive members, each summed from +0,
-// then the chunk sums in chunk order from +0) / count; max = the first maximum in index order.  Every (voxel, column)
+// Pooling over members in ascending index: sum = chunked sum (chunks of 32 consecutive members, each summed from +0,
+// then the chunk sums in chunk order from +0), mean = sum / count; max = the first maximum in index order.  The same
+// kernels pool any runs given as offsets over a member list (the sorted edges of tknn_knn_backward) or over the rows
+// themselves (IDENT: member j is row j, the segments of tknn_segment_reduce).  Every (voxel, column)
 // is one thread of voxel_kernel, column fastest, so a warp reads consecutive columns of a row (whole sectors once
 // f >= 8).  Voxels above LONG_VOXEL members first get their chunks reduced in parallel by chunk_kernel (one thread per
 // (chunk, column)); fold_kernel (one warp per (long voxel, column)) then folds the chunk results in order.  Every mapping performs the contract's
@@ -24,6 +26,7 @@ constexpr int THREADS = 256;
 constexpr int CHUNK = 32;        // members per chunk of the mean's two-level sum (part of the contract)
 constexpr uint32_t LONG_VOXEL = 256;  // voxels with more members reduce their chunks in parallel (chunk_kernel)
 constexpr int IDX_BITS = 31;     // packed sort keys: (raw - lo) << 31 | point index
+enum { R_MEAN = 0, R_MAX = 1, R_SUM = 2 };  // pooling reductions (TKNN_REDUCE_*)
 
 __device__ __forceinline__ uint32_t ordered(float v) {
   const uint32_t b = __float_as_uint(v);
@@ -187,19 +190,20 @@ struct PoolParams {
   float* out;                 // nv x f
 };
 
-template <bool MAX>
+template <bool MAX, bool IDENT>
 __device__ __forceinline__ float reduce_run(const PoolParams& P, uint64_t j0, uint64_t j1, int c) {
-  float a = MAX ? __ldg(P.x + (uint64_t)__ldg(P.members + j0) * P.stride + c) : 0.0f;
+  const auto row = [&](uint64_t j) -> uint64_t { return IDENT ? j : (uint64_t)__ldg(P.members + j); };
+  float a = MAX ? __ldg(P.x + row(j0) * P.stride + c) : 0.0f;
   for (uint64_t j = MAX ? j0 + 1 : j0; j < j1; ++j) {
-    const float v = __ldg(P.x + (uint64_t)__ldg(P.members + j) * P.stride + c);
+    const float v = __ldg(P.x + row(j) * P.stride + c);
     if (MAX) a = v > a ? v : a;  // strict: the lowest index keeps a tie
     else a = __fadd_rn(a, v);
   }
   return a;
 }
 
-// one thread per (long-voxel chunk, column): the chunk's sum from +0 (or its first maximum)
-template <bool MAX>
+// one thread per (long-voxel chunk, column): the chunk's sum from +0 (or its first maximum); R_SUM launches R_MEAN
+template <int R, bool IDENT = false>
 static __global__ void __launch_bounds__(THREADS) chunk_kernel(const PoolParams P) {
   const uint64_t total = P.n_chunks * (uint64_t)P.cb;
   for (uint64_t t = (uint64_t)blockIdx.x * THREADS + threadIdx.x; t < total; t += (uint64_t)gridDim.x * THREADS) {
@@ -212,13 +216,20 @@ static __global__ void __launch_bounds__(THREADS) chunk_kernel(const PoolParams 
     }
     const uint64_t j0 = __ldg(P.vox_off + a) + (g - __ldg(P.chunk_off + a)) * CHUNK;
     const uint64_t j1 = min(j0 + CHUNK, __ldg(P.vox_off + a + 1));
-    P.cs[t] = reduce_run<MAX>(P, j0, j1, c);
+    P.cs[t] = reduce_run<R == R_MAX, IDENT>(P, j0, j1, c);
   }
 }
 
+// the mean's division; an empty run (only segments have them) gives +0
+template <bool IDENT>
+__device__ __forceinline__ float mean_of(float sum, uint64_t count) {
+  return __fdiv_rn(sum, (float)(IDENT ? max(count, (uint64_t)1) : count));
+}
+
 // one thread per (short voxel, column): the members chunk by chunk (long voxels are left to fold_kernel)
-template <bool MAX>
+template <int R, bool IDENT = false>
 static __global__ void __launch_bounds__(THREADS) voxel_kernel(const PoolParams P) {
+  constexpr bool MAX = R == R_MAX;
   const uint64_t total = P.nv * (uint64_t)P.cb;
   for (uint64_t t = (uint64_t)blockIdx.x * THREADS + threadIdx.x; t < total; t += (uint64_t)gridDim.x * THREADS) {
     const uint64_t v = t / (uint64_t)P.cb;
@@ -227,21 +238,22 @@ static __global__ void __launch_bounds__(THREADS) voxel_kernel(const PoolParams 
     if (__ldg(P.chunk_off + v + 1) > __ldg(P.chunk_off + v)) continue;
     float a;
     if (MAX) {
-      a = reduce_run<true>(P, j0, j1, c);
+      a = reduce_run<true, IDENT>(P, j0, j1, c);
     } else {
       a = 0.0f;
-      for (uint64_t k = j0; k < j1; k += CHUNK) a = __fadd_rn(a, reduce_run<false>(P, k, min(k + CHUNK, j1), c));
+      for (uint64_t k = j0; k < j1; k += CHUNK) a = __fadd_rn(a, reduce_run<false, IDENT>(P, k, min(k + CHUNK, j1), c));
     }
-    if (!MAX) a = __fdiv_rn(a, (float)(j1 - j0));
+    if (R == R_MEAN) a = mean_of<IDENT>(a, j1 - j0);
     P.out[v * (uint64_t)P.f + c] = a;
   }
 }
 
 // one warp per (long voxel, column): the chunk results in chunk order.  The lanes load 32 consecutive chunk results at a
 // time and every lane folds them in order from the shuffles, so the serial chain is shuffles and adds, not loads.
-template <bool MAX>
+template <int R, bool IDENT = false>
 static __global__ void __launch_bounds__(THREADS) fold_kernel(const PoolParams P, const uint32_t* __restrict__ longs,
                                                               uint64_t n_long) {
+  constexpr bool MAX = R == R_MAX;
   const int lane = threadIdx.x & 31;
   const uint64_t total = n_long * (uint64_t)P.cb, warps = (uint64_t)gridDim.x * (THREADS / 32);
   for (uint64_t w = ((uint64_t)blockIdx.x * THREADS + threadIdx.x) >> 5; w < total; w += warps) {
@@ -264,7 +276,7 @@ static __global__ void __launch_bounds__(THREADS) fold_kernel(const PoolParams P
       }
     }
     if (lane == 0) {
-      if (!MAX) a = __fdiv_rn(a, (float)(__ldg(P.vox_off + v + 1) - __ldg(P.vox_off + v)));
+      if (R == R_MEAN) a = mean_of<IDENT>(a, __ldg(P.vox_off + v + 1) - __ldg(P.vox_off + v));
       P.out[(uint64_t)v * P.f + P.c0 + cc] = a;
     }
   }

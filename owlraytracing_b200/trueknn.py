@@ -512,6 +512,71 @@ class TrueKNN:
                                                       self._in(g), f, n, f, _ptr(grad_x, null_if_empty=True)))
         return grad_x
 
+    def knn_backward(self, queries, points, idx, grad_d2, need_queries: bool = True, need_points: bool = True):
+        """Gradient of kNN squared distances with respect to both point sets (tknn_knn_backward; PyTorch3D's knn_points
+        backward).  queries [nq, D] and points [n, D] float32 with D = 2 or 3; idx [nq, k] int32 and grad_d2 [nq, k]
+        float32: the kNN rows (-1 slots skipped) and the gradient of their d2.  Per edge (i, s) with j = idx[i, s],
+        t = fl(2 grad_d2[i, s]), term_q = fl(t fl(q_i - p_j)) and term_p = fl(t fl(p_j - q_i)); grad_q[i] sums row i's
+        terms in slot order and grad_p[j] the terms of the edges with idx = j in ascending i * k + s, both in chunks of 32
+        summed from +0 and then the chunk sums in order, all in fp32 without FMA or atomics: the same bits on every run.
+        Returns (grad_q [nq, D] or None unless need_queries, grad_p [n, D] or None unless need_points).  numpy outputs
+        for a numpy grad_d2, CUDA tensors (on its device) for a CUDA tensor."""
+        q, p = _positions(queries, "queries", copy=True), _positions(points, "points", copy=True)
+        dim = int(q.shape[1])
+        if int(p.shape[1]) != dim:
+            raise ValueError(f"queries have {dim} columns, points {int(p.shape[1])}")
+        idx = _arg(idx, np.int32, "idx", ndim=2, copy=True)
+        g = _arg(grad_d2, np.float32, "grad_d2", ndim=2, cast=False, copy=True)
+        nq, k, n = int(idx.shape[0]), int(idx.shape[1]), int(p.shape[0])
+        if tuple(g.shape) != (nq, k) or int(q.shape[0]) != nq:
+            raise ValueError(f"shapes queries {tuple(q.shape)}, idx {tuple(idx.shape)}, grad_d2 {tuple(g.shape)} do not "
+                             "match")
+        grad_q = self._empty(g, (nq, dim), np.float32) if need_queries else None
+        grad_p = self._empty(g, (n, dim), np.float32) if need_points else None
+        if nq == 0 or k == 0:  # no edge: grad_p is +0 (and grad_q has no rows, or no terms)
+            for a in (grad_q, grad_p):
+                if a is not None:
+                    a[:] = 0
+            return grad_q, grad_p
+        if grad_q is None and grad_p is None:
+            return None, None
+        self._check(self._L.tknn_knn_backward(self._h, self._in(q), nq, dim, self._in(p, null_if_empty=True), n, dim,
+                                              dim, self._in(idx), k, self._in(g), _ptr(grad_q),
+                                              _ptr(grad_p, null_if_empty=True)))
+        return grad_q, grad_p
+
+    def segment_reduce(self, x, batch=None, batch_size: int | None = None, reduce: str = "sum"):
+        """Per-cloud sum or mean of the rows of x ([n] or [n, f] float32, 1 <= f <= 1024; tknn_segment_reduce).  batch
+        (optional, torch_cluster's convention) and batch_size as in build(); without them x is one cloud.  "sum": the rows
+        in index order in chunks of 32, each chunk summed from +0 and then the chunk sums in order, in fp32 without
+        atomics; "mean": that sum / (float)count.  An empty cloud gives +0.  Returns [B] or [B, f] float32 as x is [n] or
+        [n, f].  numpy outputs for numpy x, CUDA tensors for a CUDA tensor."""
+        if reduce not in ("sum", "mean"):
+            raise ValueError(f"reduce must be 'sum' or 'mean', got {reduce!r}")
+        x = _arg(x, np.float32, "x", cast=False, copy=True)
+        if x.ndim not in (1, 2):
+            raise ValueError("x must be [n] or [n, f]")
+        n = int(x.shape[0])
+        if batch is None:
+            if batch_size is not None:
+                raise ValueError("batch_size needs a batch")
+            offsets = None
+        else:
+            offsets = batch_to_offsets(batch, n, batch_size)
+        return self._segment_reduce(x, offsets, reduce)
+
+    def _segment_reduce(self, x, offsets, reduce: str):
+        """segment_reduce() over cloud offsets (batch_to_offsets) or one cloud (None)."""
+        n_seg = 1 if offsets is None else int(offsets.shape[0]) - 1
+        rows = x.reshape(int(x.shape[0]), 1) if x.ndim == 1 else x
+        f = int(rows.shape[1])
+        out = self._empty(x, (n_seg, f), np.float32)
+        if n_seg:
+            code = _lib.REDUCE_SUM if reduce == "sum" else _lib.REDUCE_MEAN
+            self._check(self._L.tknn_segment_reduce(self._h, self._in(rows, null_if_empty=True), int(rows.shape[0]), f,
+                                                    f, self._in(offsets), n_seg, code, _ptr(out)))
+        return out.reshape(n_seg) if x.ndim == 1 else out
+
     def radius_search(self, radius: float, indices_only: bool = False, out=None):
         """Exact fixed-radius neighbour lists of every built point (closed ball, the point itself excluded).
 
@@ -1112,13 +1177,25 @@ def feature_knn(x, y, k: int, batch_x=None, batch_y=None, device: int | None = N
     return _knn_edges(idx, k, 0)
 
 
-def _positions(pos, name):
-    """pos as [rows, 2|3] float32: PyG's knn_interpolate measures distances over every column, so other widths raise."""
-    pos = _arg(pos, np.float32, name)
+def _positions(pos, name, copy: bool = False):
+    """pos as [rows, 2|3] float32: PyG's knn_interpolate measures distances over every column, so other widths raise.
+    copy: a non-contiguous tensor is copied (through autograd) rather than refused."""
+    pos = _arg(pos, np.float32, name, copy=copy)
     if pos.ndim != 2 or int(pos.shape[1]) not in (2, 3):
         raise ValueError(f"{name} must be [n, 2] or [n, 3] (only 2-D and 3-D positions are supported), got "
                          f"{tuple(pos.shape)}")
     return pos
+
+
+def _knn_rows(t, pos_x, pos_y, k: int, batch_x, batch_y):
+    """(idx [len(pos_y), k] int32, d2) on the squared_dist context t: for every point of pos_y its k <= len(pos_x) nearest
+    points of pos_x in the same cloud (batches as knn()).  One data point takes the feature-space search: a build needs
+    two, and the feature-space d2 rule is the same for 2 or 3 columns."""
+    batch_x, batch_y, batch_size = _bipartite_setup(pos_x, pos_y, batch_x, batch_y)
+    if int(pos_x.shape[0]) == 1:
+        return t.feature_knn(pos_x, pos_y, 1, batch_x=batch_x, batch_y=batch_y)
+    t.build(pos_x, batch=batch_x, batch_size=batch_size)
+    return t.query(pos_y, k, batch=batch_y)
 
 
 _KnnInterpolate = None
@@ -1183,18 +1260,186 @@ def knn_interpolate(x, pos_x, pos_y, batch_x=None, batch_y=None, k: int = 3, num
         if tensor:
             return x.new_full((nq, f), float("nan")) + x.sum() * 0  # still part of x's graph
         return np.full((nq, f), np.nan, np.float32)
-    batch_x, batch_y, batch_size = _bipartite_setup(pos_x, pos_y, batch_x, batch_y)
     k = min(int(k), n)
     with TrueKNN(_device_of(x, device), squared_dist=1) as t:
-        if n == 1:  # a build needs two points; the feature-space search has the same d2 rule for 2 or 3 columns
-            idx, d2 = t.feature_knn(pos_x, pos_y, 1, batch_x=batch_x, batch_y=batch_y)
-        else:
-            t.build(pos_x, batch=batch_x, batch_size=batch_size)
-            idx, d2 = t.query(pos_y, k, batch=batch_y)
+        idx, d2 = _knn_rows(t, pos_x, pos_y, k, batch_x, batch_y)
         if not tensor:
             out, _, _ = t.interpolate(idx, d2, x)
             return out
         return _knn_interpolate_function().apply(x, idx, d2, t)
+
+
+_KnnPoints = None
+_SegmentReduce = None
+
+
+def _knn_points_function():
+    """The torch.autograd.Function of knn_points(), made on first use: d2 is differentiable with respect to both point
+    sets, idx is not."""
+    global _KnnPoints
+    if _KnnPoints is None:
+        import torch
+
+        class KnnPoints(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, x, y, k, batch_x, batch_y, t):
+                idx, d2 = _knn_rows(t, x, y, k, batch_x, batch_y)
+                ctx.save_for_backward(x, y, idx)
+                idx64 = idx.to(torch.int64)
+                ctx.mark_non_differentiable(idx64)
+                return d2, idx64
+
+            @staticmethod
+            def backward(ctx, grad_d2, _grad_idx):
+                x, y, idx = ctx.saved_tensors
+                with TrueKNN(grad_d2.device.index) as t:
+                    grad_y, grad_x = t.knn_backward(y, x, idx, grad_d2.contiguous(), need_queries=ctx.needs_input_grad[1],
+                                                    need_points=ctx.needs_input_grad[0])
+                return grad_x, grad_y, None, None, None, None
+
+        _KnnPoints = KnnPoints
+    return _KnnPoints
+
+
+def _segment_reduce_function():
+    """The torch.autograd.Function of the Chamfer loss's reductions, made on first use.  Its backward is the gather
+    g[segment] (sum) or fl(g[segment] / (float)count) (mean) in plain torch, without atomics."""
+    global _SegmentReduce
+    if _SegmentReduce is None:
+        import torch
+
+        class SegmentReduce(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, v, offsets, reduce, t):
+                off = offsets.to(v.device)
+                counts = off[1:] - off[:-1]
+                ctx.save_for_backward(counts)
+                ctx.mean = reduce == "mean"
+                return t._segment_reduce(v, off, reduce)
+
+            @staticmethod
+            def backward(ctx, g):
+                (counts,) = ctx.saved_tensors
+                seg = torch.repeat_interleave(torch.arange(int(counts.shape[0]), device=g.device), counts)
+                out = g[seg]
+                if ctx.mean:
+                    out = out / counts.to(torch.float32)[seg]
+                return out, None, None, None
+
+        _SegmentReduce = SegmentReduce
+    return _SegmentReduce
+
+
+def knn_points(x, y, k: int, batch_x=None, batch_y=None, device: int | None = None):
+    """PyTorch3D's knn_points on PyG batch vectors, in this package's knn() orientation, exact: for every point of y, its
+    k nearest points of x in the same cloud by (d2, index) (tknn_query_segments with squared distances).  Returns
+    (d2 [len(y), k'] float32, idx [len(y), k'] int64) with k' = min(k, len(x)); rows of clouds with fewer than k' points
+    end in -1 / FLT_MAX.  Positions: [*, 2] or [*, 3] float32 (other widths raise ValueError); batches as knn().  For
+    CUDA tensors d2 is differentiable with respect to x and y: the backward pass (TrueKNN.knn_backward) is PyTorch3D's
+    2 * grad * diff summed in a fixed order without atomics, so x.grad and y.grad have the same bits on every run.
+    numpy in, numpy out (no autograd); device: the CUDA device for numpy input (default 0)."""
+    if int(k) < 1:
+        raise ValueError(f"k = {k} must be >= 1")
+    x, y = _positions(x, "x", copy=True), _positions(y, "y", copy=True)
+    if int(x.shape[1]) != int(y.shape[1]):
+        raise ValueError(f"x has {int(x.shape[1])} columns, y {int(y.shape[1])}")
+    tensor = _is_tensor(x)
+    if tensor:
+        if not x.is_cuda:
+            raise ValueError("x must be a CUDA tensor or a numpy array")
+        y = y.to(x.device)
+    with TrueKNN(_device_of(x, device), squared_dist=1) as t:
+        return _knn_points(t, x, y, k, batch_x, batch_y)
+
+
+def _knn_points(t, x, y, k: int, batch_x, batch_y):
+    """knn_points() on the squared_dist context t, x and y checked."""
+    n, nq = int(x.shape[0]), int(y.shape[0])
+    k = min(int(k), n)
+    if n == 0 or nq == 0:
+        d2, idx = _zeros_like_rows(y, (nq, k), np.float32), _zeros_like_rows(y, (nq, k), np.int64)
+        if _is_tensor(d2):
+            d2 = d2 + (x.sum() + y.sum()) * 0  # still part of the graph of x and y
+        return d2, idx
+    if _is_tensor(x):
+        return _knn_points_function().apply(x, y, k, batch_x, batch_y, t)
+    idx, d2 = _knn_rows(t, x, y, k, batch_x, batch_y)
+    return d2, _int64(idx)
+
+
+def _cloud_offsets(batch, n: int, size: int):
+    """batch_to_offsets(batch, n, size), or one cloud of all n points padded to `size` clouds when batch is None."""
+    if batch is not None:
+        return batch_to_offsets(batch, n, size)
+    off = np.full(size + 1, n, np.uint64)
+    off[0] = 0
+    return off
+
+
+def chamfer_distance(x, y, batch_x=None, batch_y=None, point_reduction: str | None = "mean",
+                     batch_reduction: str | None = "mean", single_directional: bool = False, device: int | None = None):
+    """PyTorch3D's chamfer_distance on PyG batch vectors, exact and deterministic.  a_i: the d2 from x_i to its nearest
+    point of y in x_i's cloud; b_j: the same for y_j and x (one k = 1 kNN search each, knn_points()).  Per cloud c,
+    X_c is the sum or mean of a over the x points of c (point_reduction "sum" / "mean", TrueKNN.segment_reduce) and Y_c
+    likewise; over the B = max(batch_x.max(), batch_y.max()) + 1 clouds, empty ones included, batch_reduction "sum" sums
+    X, "mean" gives fl(sum / B) and None keeps the [B] vector.  The result is fl(X + Y), or X alone when
+    single_directional.  point_reduction=None returns the per-point (a, b) (b is None when single_directional) and needs
+    batch_reduction=None.  Every sum runs in chunks of 32 in a fixed order without atomics, so the loss, x.grad and y.grad
+    have the same bits on every run.  A cloud with points in x and none in y, or (unless single_directional) in y and
+    none in x, raises ValueError: no nearest point is defined; a cloud empty on both sides contributes +0.
+    Positions: [*, 2] or [*, 3] float32.  CUDA tensors give a loss differentiable with respect to x and y; numpy gives
+    numpy float32 (no autograd).  device: the CUDA device for numpy input (default 0).  Not supported: PyTorch3D's
+    weights, norm=1, normals and point_reduction="max"."""
+    if point_reduction not in ("mean", "sum", None):
+        raise ValueError(f"point_reduction must be 'mean', 'sum' or None, got {point_reduction!r}")
+    if batch_reduction not in ("mean", "sum", None):
+        raise ValueError(f"batch_reduction must be 'mean', 'sum' or None, got {batch_reduction!r}")
+    if point_reduction is None and batch_reduction is not None:
+        raise ValueError("point_reduction=None needs batch_reduction=None")
+    x, y = _positions(x, "x", copy=True), _positions(y, "y", copy=True)
+    if int(x.shape[1]) != int(y.shape[1]):
+        raise ValueError(f"x has {int(x.shape[1])} columns, y {int(y.shape[1])}")
+    tensor = _is_tensor(x)
+    if tensor:
+        if not x.is_cuda:
+            raise ValueError("x must be a CUDA tensor or a numpy array")
+        y = y.to(x.device)
+    nx, ny = int(x.shape[0]), int(y.shape[0])
+    tops = [int(b.max().item()) if _is_tensor(b) else int(np.max(b))
+            for b, m in ((batch_x, nx), (batch_y, ny)) if b is not None and m]
+    size = max(tops) + 1 if tops else 1
+    ox, oy = _cloud_offsets(batch_x, nx, size), _cloud_offsets(batch_y, ny, size)
+    cx = np.diff(np.asarray(ox.cpu() if _is_tensor(ox) else ox, np.int64))
+    cy = np.diff(np.asarray(oy.cpu() if _is_tensor(oy) else oy, np.int64))
+    for c in np.nonzero((cx > 0) & (cy == 0))[0][:1]:
+        raise ValueError(f"cloud {int(c)} has points in x and none in y: no nearest point is defined")
+    if not single_directional:
+        for c in np.nonzero((cx == 0) & (cy > 0))[0][:1]:
+            raise ValueError(f"cloud {int(c)} has points in y and none in x: no nearest point is defined")
+    with TrueKNN(_device_of(x, device), squared_dist=1) as t:
+        a = _knn_points(t, y, x, 1, batch_y, batch_x)[0].reshape(-1)
+        b = None if single_directional else _knn_points(t, x, y, 1, batch_x, batch_y)[0].reshape(-1)
+        if point_reduction is None:
+            return a, b
+
+        def reduce(v, offsets, how):
+            if tensor:
+                import torch
+
+                off = offsets if _is_tensor(offsets) else torch.as_tensor(offsets.astype(np.int64))
+                return _segment_reduce_function().apply(v, off, how, t)
+            return t._segment_reduce(v, offsets, how)
+
+        one = np.array([0, size], np.uint64)
+        loss = None
+        for v, off in ((a, ox), (b, oy)):
+            if v is None:
+                continue
+            r = reduce(v, off, point_reduction)
+            if batch_reduction is not None:
+                r = reduce(r, one, batch_reduction).reshape(())
+            loss = r if loss is None else loss + r
+    return loss
 
 
 def radius(x, y, r: float, batch_x=None, batch_y=None, max_num_neighbors: int | None = None, device: int | None = None):
