@@ -26,9 +26,11 @@ constexpr int MAX_SPAN = 31;   // cells per axis a group may span (its 32 bounda
 #ifndef TKNN_GRID_CAP
 #define TKNN_GRID_CAP 1024     // cells a group may test; a larger range is left unresolved to the LBVH rounds
 #endif
+constexpr int STAGE = 128;     // points of a warp's staging area: four 32-bit survivor masks per lane
 #ifndef TKNN_GRID_FLUSH
-#define TKNN_GRID_FLUSH 64     // staged points that trigger the filter + insert pass (<= 64: the staging area)
+#define TKNN_GRID_FLUSH 128    // staged points that trigger the filter + insert pass (<= STAGE)
 #endif
+static_assert(TKNN_GRID_FLUSH >= 1 && TKNN_GRID_FLUSH <= STAGE, "TKNN_GRID_FLUSH must fit the staging area");
 // Selection: the grid serves a build only while its fullest cell holds at most this many points.  Uniform clouds stay far
 // below it (10 M points at level 7: 4.8 per cell on average, 23 at most); clustered clouds (LiDAR-like scans, duplicate
 // clusters) exceed it by orders of magnitude, and there cells as large as the leaves' boxes would gain nothing.
@@ -122,10 +124,14 @@ constexpr int GRID_PHASE_SLOT = 8;        // counters[GRID_PHASE_SLOT + phase]
 constexpr int GRID_INSERT_ITER_SLOT = 14; // counters[14]: insert-loop iterations per warp
 constexpr int GRID_INSERT_SLOT = 15;      // counters[15]: inserts of round 1 on the grid
 
-// per warp: the LBVH list kernel's layout (staging 64 points, stack area = the group's 3 x 32 cell boundaries, k-list,
-// SoA coordinates) + the visit order of the group's cells per axis (3 x 32 bytes) + its low cell and width per axis
-// (kept in shared memory: registers stay free for the loop nest)
-__host__ __device__ inline size_t smem_per_warp(int k) { return trav::smem_per_warp(k) + 128; }
+// per warp: the staging area as four arrays x[STAGE] | y[STAGE] | z[STAGE] | id[STAGE] (no float4 copy: the insert loop
+// reads its survivor from the arrays), the group's 3 x 32 cell boundaries, the 32 ascending k-lists (trav::klist_bytes),
+// the visit order of the group's cells per axis (3 x 32 bytes) and its low cell and width per axis (kept in shared memory:
+// registers stay free for the loop nest).  The staging area and the boundaries lie below the k-lists, so list_insert's
+// reads of up to three slots below a sentinel (768 B) stay inside the warp's own region.
+__host__ __device__ inline size_t smem_per_warp(int k) {
+  return 4 * STAGE * sizeof(float) + 3 * 32 * sizeof(float) + trav::klist_bytes(k) + 128;
+}
 
 // Visit order along one axis of w cells, outward from cell c: c, c + 1, c - 1, c + 2, ... and, once one side is used up,
 // the rest of the other side.  Near cells first, so the bounds tighten early.
@@ -151,8 +157,9 @@ __device__ __forceinline__ float axis_gap(float q, float lo, float hi) {
 // first, all against the bounds as they are at the row's start (a bound only shrinks, so a stale one culls less, never
 // wrongly); then the wanted cells' points are staged with one warp-wide gather, lane i loading the row's i-th wanted point
 // (a prefix sum over the cells' run lengths and a binary search in it), so a row waits for one load latency instead of one
-// per cell.  Staged points go into the 64-point area (NaN-padded), are filtered into two masks by filter4 and inserted in one
-// loop (the sibling-pair path of the LBVH kernel) whenever TKNN_GRID_FLUSH points are staged.  The k-lists keep the k
+// per cell.  Staged points go into the STAGE-point area (NaN-padded), are filtered into four masks by filter4 and inserted in
+// one loop whenever TKNN_GRID_FLUSH points are staged.  A flush costs the largest survivor count of any lane, and the survivors
+// sit on the few lanes near the staged cells, so a larger flush spreads them over more lanes per trip.  The k-lists keep the k
 // smallest (d2, index) keys whatever order the points arrive in, so the rows do not depend on the staging order.
 // Counting build: counters[0] = cell tests x active lanes (the nodes_visited field), [1] = staged points x active lanes,
 // [2] = inserts, [3] = cell tests per warp, [4] = cells staged per warp, [5] = points staged per warp, [7] = groups left
@@ -163,16 +170,15 @@ __device__ __forceinline__ float axis_gap(float q, float lo, float hi) {
 template <bool COUNT>
 static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(const trav::Params P, const GridParams G) {
   extern __shared__ __align__(16) unsigned char smem[];
-  constexpr int NS = trav::stage_pts(false);  // 64
+  constexpr int NS = STAGE;
   constexpr int S = trav::KLS;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int k = P.k;
   unsigned char* wbase = smem + (size_t)warp * smem_per_warp(k);
-  float4* stage = reinterpret_cast<float4*>(wbase);
-  float* gb = reinterpret_cast<float*>(wbase + NS * sizeof(float4));  // boundaries: x at [0, 32), y at [32, 64), z at [64, 96)
-  uint64_t* H = reinterpret_cast<uint64_t*>(wbase + NS * sizeof(float4) + STACK_DEPTH * sizeof(int)) + lane;
-  float* soa = reinterpret_cast<float*>(wbase + NS * sizeof(float4) + STACK_DEPTH * sizeof(int) + trav::klist_bytes(k));
-  uint8_t* ord = reinterpret_cast<uint8_t*>(soa + 3 * NS);  // visit order: x at [0, 32), y at [32, 64), z at [64, 96)
+  float* soa = reinterpret_cast<float*>(wbase);  // x at [0, NS), y at [NS, 2 NS), z at [2 NS, 3 NS), id bits at [3 NS, 4 NS)
+  float* gb = soa + 4 * NS;                      // boundaries: x at [0, 32), y at [32, 64), z at [64, 96)
+  uint64_t* H = reinterpret_cast<uint64_t*>(gb + 3 * 32) + lane;
+  uint8_t* ord = reinterpret_cast<uint8_t*>(gb + 3 * 32) + trav::klist_bytes(k);  // visit order: x at [0, 32), y at [32, 64), z at [64, 96)
   uint32_t* rng = reinterpret_cast<uint32_t*>(ord + 96);    // low cell per axis [0, 3), width per axis [3, 6)
   const int level = G.level, sh = 21 - level;
   const int per = (1 << level) + 1;
@@ -260,26 +266,27 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
         __syncwarp();
         if (COUNT) { c_tests += valid ? fill : 0; c_wpts += fill; }
         const float2 qx2 = make_float2(q.x, q.x), qy2 = make_float2(q.y, q.y), qz2 = make_float2(q.z, q.z);
-        uint32_t mask_a = 0, mask_b = 0;  // survivors among staged points 0..31 / 32..63
-        const int na = min(fill, MAX_LEAF);
+        uint32_t m[NS / 32];  // survivors among staged points 32 w .. 32 w + 31, in chunks of 8 at compile-time bit positions
+#pragma unroll
+        for (int w = 0; w < NS / 32; ++w) {
+          m[w] = 0;
+          const int end = min(fill, 32 * w + 32);
 #pragma unroll 1
-        for (int j0 = 0; j0 < na; j0 += 8)
-          mask_a |= (trav::filter4<NS>(soa, j0, qx2, qy2, qz2, bound) | (trav::filter4<NS>(soa, j0 + 4, qx2, qy2, qz2, bound) << 4)) << j0;
-#pragma unroll 1
-        for (int j0 = MAX_LEAF; j0 < fill; j0 += 8)
-          mask_b |= (trav::filter4<NS>(soa, j0, qx2, qy2, qz2, bound) | (trav::filter4<NS>(soa, j0 + 4, qx2, qy2, qz2, bound) << 4))
-                    << (j0 - MAX_LEAF);
+          for (int j0 = 32 * w; j0 < end; j0 += 8)
+            m[w] |= (trav::filter4<NS>(soa, j0, qx2, qy2, qz2, bound) | (trav::filter4<NS>(soa, j0 + 4, qx2, qy2, qz2, bound) << 4))
+                    << (j0 - 32 * w);
+        }
+        uint64_t mask_a = ((uint64_t)m[1] << 32) | m[0], mask_b = ((uint64_t)m[3] << 32) | m[2];  // points 0..63 / 64..127
         if (COUNT) {
           tick(GRID_PHASE_FILTER);
-          c_iters += __reduce_max_sync(FULL_MASK, (unsigned)(__popc(mask_a) + __popc(mask_b)));
+          c_iters += __reduce_max_sync(FULL_MASK, (unsigned)(__popcll(mask_a) + __popcll(mask_b)));
         }
         while (mask_a | mask_b) {
           int j;
-          if (mask_a) { j = __ffs(mask_a) - 1; mask_a &= mask_a - 1u; }
-          else { j = MAX_LEAF + __ffs(mask_b) - 1; mask_b &= mask_b - 1u; }
-          const float4 p = stage[j];
-          const float d = dist2(q.x, q.y, q.z, p.x, p.y, p.z);
-          const int pid = __float_as_int(p.w);
+          if (mask_a) { j = __ffsll(mask_a) - 1; mask_a &= mask_a - 1u; }
+          else { j = 64 + __ffsll(mask_b) - 1; mask_b &= mask_b - 1u; }
+          const float d = dist2(q.x, q.y, q.z, soa[j], soa[NS + j], soa[2 * NS + j]);
+          const int pid = __float_as_int(soa[3 * NS + j]);
           if (pid != self && d <= bound) trav::list_take<S, COUNT>(H, cnt, k, bound, d, pid, c_ins);
         }
         __syncwarp();
@@ -342,8 +349,7 @@ static __global__ void __launch_bounds__(256, COUNT ? 1 : 5) grid_knn_kernel(con
               if (lane + h < take) {
                 const float4 p = __ldg(&P.pts[src]);
                 const int j = fill + lane + h;
-                stage[j] = p;
-                soa[j] = p.x; soa[NS + j] = p.y; soa[2 * NS + j] = p.z;
+                soa[j] = p.x; soa[NS + j] = p.y; soa[2 * NS + j] = p.z; soa[3 * NS + j] = p.w;
               }
             }
             fill += take;

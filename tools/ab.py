@@ -1,7 +1,7 @@
 """A/B of library variants on one GPU: same workload, one subprocess per libtrueknn build (TKNN_LIB_PATH).
 
-    python tools/ab.py cfg2|cfg3|cfg4|cfg1 lib1.so lib2.so:curve=1 ...   (paths relative to owlraytracing_b200/lib/;
-                                                                        optional tknn_set_option settings after ':')
+    python tools/ab.py cfg2|cfg3|cfg4|cfg1[,k=K] lib1.so lib2.so:curve=1 ...   (paths relative to owlraytracing_b200/lib/;
+                                                                             optional tknn_set_option settings after ':')
 
 Per variant: best-of-5 search_ms through tknn_search_shard (compact rows, device outputs: the bench's timed call), the
 per-round kernel times, build phases, and a checksum of the result (all variants must agree; the first is compared
@@ -23,7 +23,9 @@ def child(which):
     sys.path.insert(0, ROOT)
     from owlraytracing_b200 import TrueKNN, datasets
 
+    which, _, kk = which.partition(",k=")  # "cfg2,k=16": the workload's cloud at another k
     n, k, cloud, seed = CFG[which]
+    k = int(kk) if kk else k
     opts = {kv.split("=")[0]: int(kv.split("=")[1]) for kv in os.environ.get("TKNN_AB_OPTS", "").split(",") if kv}
     t = TrueKNN(0, **opts)
     t.set_stream(torch.cuda.current_stream().cuda_stream)
@@ -55,7 +57,7 @@ def child(which):
     t.set_option("counters", 1)
     t.search_shard(k, 0, 1, out=out)
     c = t.stats()
-    print(json.dumps({"lib": os.path.basename(os.environ.get("TKNN_LIB_PATH", "default")), "opts": opts, "workload": which,
+    print(json.dumps({"lib": os.path.basename(os.environ.get("TKNN_LIB_PATH", "default")), "opts": opts, "workload": which, "k": k,
                       "search_ms": round(best["search_ms"], 4), "estimate_ms": round(best["estimate_ms"], 4),
                       "kernel_ms": [round(v, 4) for v in best["kernel_ms"]], "round_queries": best["round_queries"],
                       "qps_M": round(n / best["search_ms"] / 1e3, 1), "build_ms": round(b["build_ms"], 4),
