@@ -63,8 +63,8 @@ enum {
   TKNN_OPT_RADIUS_QUANTILE = 7 /* start-radius estimator: per-mille quantile of the sampled k-th
                                   neighbour distance (default 990)                                */
   ,TKNN_OPT_KEEP_SCRATCH = 8   /* 1 (default): keep the grow-only scratch of builds, queries (tknn_query*,
-                                  tknn_radius_query*), radius lists, interpolation, tknn_knn_backward and
-                                  tknn_segment_reduce for the next call;
+                                  tknn_radius_query*), radius lists, interpolation, tknn_knn_backward,
+                                  tknn_segment_reduce and tknn_local_frames for the next call;
                                   0: release it when each such call returns                              */
   ,TKNN_OPT_APPROX_FILTER = 10 /* 1: conservative 3-FMA pre-filter before the exact distance test
                                   (DESIGN.md §3.2; audited, -1 % time); 0 (default): exact test on every pair */
@@ -471,6 +471,50 @@ TKNN_API int tknn_knn_backward(tknn_ctx* ctx, const float* queries, uint64_t nq,
  * outside [1, 2^31 - 1], malformed offsets, a NULL out, or a NULL x with n > 0. */
 TKNN_API int tknn_segment_reduce(tknn_ctx* ctx, const float* x, uint64_t n, int f, int stride_floats,
                                  const uint64_t* seg_offsets, uint64_t n_segments, int reduce, float* out);
+
+/* Surface normals and local frames from the covariance of neighbourhoods (PyTorch3D's estimate_pointcloud_normals /
+ * estimate_pointcloud_local_coord_frames, Open3D's estimate_normals, PCL's NormalEstimation; DESIGN.md §3.12).
+ * points: n rows of 3-D positions with pitch stride_floats >= 3; idx: m rows of k indices into points, -1 for an empty
+ * slot.  For row i, S is its slots with idx != -1 in slot order and c = |S|.  In fp32, every operation rounded on its
+ * own (round-to-nearest; fl(a + b), fl(a * b), fl(a / b), fl(sqrt(a)), no FMA):
+ *   centroid    mean_d = fl(sum_S p[j,d] / (float)c)
+ *   covariance  e_sd = fl(p[j_s,d] - mean_d);  C_ab = fl(sum_S fl(e_sa * e_sb) / (float)c)  for ab in 00 01 02 11 12 22
+ *               (the mean over the neighbourhood, PyTorch3D's get_point_covariances)
+ * where each sum is the chunked sum of tknn_knn_backward: chunks of 32 terms in slot order, each summed from +0, then
+ * the chunk sums in order from +0 (result = fl(+0 + chunk 0), then fl(result + chunk 1), ...).
+ *   eigensolver cyclic Jacobi on A = C, starting from V = I.  A sweep rotates the pairs (p, q) = (0,1), (0,2), (1,2) in
+ *               that order; the solver stops before a sweep that starts with a01, a02 and a12 all +0 or -0, and after at
+ *               most 8 sweeps.  A pair with a_pq == 0 is skipped; otherwise, with r the third index:
+ *                 tau = fl(fl(a_qq - a_pp) / fl(2 * a_pq));  tt = fl(tau * tau)
+ *                 t   = fl(0.5 / tau) when tt = +inf, else fl(sg / fl(|tau| + fl(sqrt(fl(1 + tt)))))
+ *                       with sg = -1 for tau < 0 and +1 otherwise (tau = +-0 gives +1)
+ *                 c   = fl(1 / fl(sqrt(fl(1 + fl(t * t)))));  s = fl(t * c)
+ *                 then, all from the values before the rotation:
+ *                 a_pp = fl(a_pp - fl(t * a_pq));  a_qq = fl(a_qq + fl(t * a_pq));  a_pq = +0
+ *                 a_rp = fl(fl(c * a_rp) - fl(s * a_rq));  a_rq = fl(fl(s * a_rp) + fl(c * a_rq))
+ *                 for each row u of V:  V_up = fl(fl(c * V_up) - fl(s * V_uq));  V_uq = fl(fl(s * V_up) + fl(c * V_uq))
+ *               (Numerical Recipes' t and the plain (c, s) rotation; the matrix stays symmetric, a_qp = a_pq.)
+ *   ordering    w = (a00, a11, a22); compare-exchange (0,1), (1,2), (0,1), each exchanging when w_left > w_right (so
+ *               ties and NaN never exchange) and moving V's columns with their values.
+ *   disambiguate = 1 (PyTorch3D's rule, after Tombari et al.'s SHOT): the anchor a is the point of the row's first
+ *               valid slot (the point itself in the rows estimate_pointcloud_normals builds).  For v = column 0, then
+ *               v = column 2 of V: n_pos = #{s in S : fl(fl(fl(v0 * f0) + fl(v1 * f1)) + fl(v2 * f2)) > 0} with
+ *               f = fl(p[j_s] - a); v = -v when 2 * n_pos < c.  Then column 1 = n x z with n = column 0, z = column 2:
+ *               (fl(fl(n1 z2) - fl(n2 z1)), fl(fl(n2 z0) - fl(n0 z2)), fl(fl(n0 z1) - fl(n1 z0))), PyTorch3D's
+ *               y = cross(n, z).  The columns (2, 1, 0) then form a right-handed frame, SHOT's (x, y, z), so
+ *               det [n y z] = -1 as in PyTorch3D.  disambiguate = 0 leaves Jacobi's columns as they come out.
+ * Outputs: eigvals_out (m x 3, ascending w) and frames_out (m x 3 x 3, row-major: frames[i][u][j] = component u of
+ * eigenvector j, PyTorch3D's column convention; column 0 is the normal).  Either may be NULL (both NULL: a no-op).
+ * c = 0: every output of the row is NaN (which NaN is not part of the contract).  c = 1: a zero covariance, eigenvalues
+ * +0 and frame I (disambiguate = 1 then negates columns 0 and 2: no slot projects positively).  Coincident or collinear
+ * neighbourhoods follow from the rules above.  The result depends only on the inputs, on any stream and launch shape.
+ * Host or device arrays.  The call needs no build and touches none.
+ * Errors (TKNN_EINVAL): k outside [1, TKNN_MAX_K], a stride below 3, n or m >= 2^31, disambiguate not 0 or 1, and, when
+ * m > 0 and an output is requested, a NULL idx or a NULL points with n > 0, and an idx entry outside {-1} and [0, n)
+ * (found on the device and reported after the call, whose outputs are then undefined).  m = 0 is a no-op.
+ * Statistics: n_queries = m, k, search_ms, d2h_ms; rounds = 1 with its round_ms / kernel_ms / round_queries (m). */
+TKNN_API int tknn_local_frames(tknn_ctx* ctx, const float* points, uint64_t n, int stride_floats, const int32_t* idx,
+                               uint64_t m, int k, int disambiguate, float* eigvals_out, float* frames_out);
 
 /* Start-radius estimator alone (replaces samples/s01-trueknn/Util/random_sample.py:5-32). */
 TKNN_API int tknn_estimate_start_radius(tknn_ctx* ctx, int k, float* radius_out);

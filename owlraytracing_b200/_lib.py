@@ -115,7 +115,7 @@ EXPORTS = [
     "tknn_radius_search", "tknn_radius_query", "tknn_write_neighbour_lists", "tknn_build_segments",
     "tknn_query_segments", "tknn_radius_query_segments", "tknn_fps", "tknn_feature_knn",
     "tknn_voxel_grid", "tknn_voxel_members", "tknn_voxel_pool", "tknn_interpolate", "tknn_interpolate_backward",
-    "tknn_knn_backward", "tknn_segment_reduce",
+    "tknn_knn_backward", "tknn_segment_reduce", "tknn_local_frames",
 ]
 
 _lib = None
@@ -158,6 +158,7 @@ def load() -> C.CDLL:
     L.tknn_interpolate_backward.argtypes = [vp, vp, vp, vp, u64, C.c_int, vp, C.c_int, u64, C.c_int, vp]
     L.tknn_knn_backward.argtypes = [vp, vp, u64, C.c_int, vp, u64, C.c_int, C.c_int, vp, C.c_int, vp, vp, vp]
     L.tknn_segment_reduce.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, C.c_int, vp]
+    L.tknn_local_frames.argtypes = [vp, vp, u64, C.c_int, vp, u64, C.c_int, C.c_int, vp, vp]
     L.tknn_radius_search.argtypes = [vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_radius_query.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, f32, vp, vp, vp, u64, C.POINTER(u64)]
     L.tknn_query_segments.argtypes = [vp, vp, u64, C.c_int, C.c_int, vp, u64, vp, vp, C.c_int, f32, vp, vp]

@@ -110,6 +110,9 @@ struct tknn_ctx {
   // touches no build state.
   DevBuf kg_q, kg_p, kg_idx, kg_g, kg_gq, kg_gp, kg_terms, kg_keys_a, kg_keys_b, kg_vals_a, kg_vals_b, kg_sort_tmp,
       kg_cnt, kg_off, kg_x, kg_seg_off, kg_out, kg_chunks, kg_chunk_off, kg_longs, kg_words, kg_cs;
+  // tknn_local_frames scratch (grow-only unless keep_scratch == 0: frames_scratch, frames.cuh): staged host points and
+  // idx, and the outputs of host callers.  It touches no build state.
+  DevBuf lf_pts, lf_idx, lf_eig, lf_frames;
   // cell grid over the sorted points (grid.cuh): runs per level-L cell and the table's frame; made by a plain build when
   // the cloud qualifies, and then round 1 of a dense kNN search with k <= 24 walks it instead of the LBVH
   int grid_mode = 0;        // TKNN_OPT_GRID: 0 = auto (occupancy decides), 1 = off, 2 = whenever the table is valid
@@ -284,6 +287,9 @@ inline ScratchScope knn_grad_scratch(tknn_ctx* c) {  // rl_sums: the run-offset 
                        &c->kg_seg_off, &c->kg_out, &c->kg_chunks, &c->kg_chunk_off, &c->kg_longs, &c->kg_words,
                        &c->kg_cs, &c->rl_sums},
                       c);
+}
+inline ScratchScope frames_scratch(tknn_ctx* c) {
+  return ScratchScope({&c->lf_pts, &c->lf_idx, &c->lf_eig, &c->lf_frames}, c);
 }
 
 // grows c->round_ev to at least `count` events (the per-round / per-phase timers)

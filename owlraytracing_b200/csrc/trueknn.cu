@@ -20,6 +20,7 @@
 #include "ctx.cuh"
 #include "features.cuh"
 #include "fps.cuh"
+#include "frames.cuh"
 #include "grid.cuh"
 #include "interpolate.cuh"
 #include "knn_grad.cuh"
@@ -983,7 +984,8 @@ int tknn_destroy(tknn_ctx* c) {
                     &c->ip_vals_b, &c->ip_sort_tmp, &c->ip_cnt, &c->ip_off, &c->kg_q, &c->kg_p, &c->kg_idx, &c->kg_g,
                     &c->kg_gq, &c->kg_gp, &c->kg_terms, &c->kg_keys_a, &c->kg_keys_b, &c->kg_vals_a, &c->kg_vals_b,
                     &c->kg_sort_tmp, &c->kg_cnt, &c->kg_off, &c->kg_x, &c->kg_seg_off, &c->kg_out, &c->kg_chunks,
-                    &c->kg_chunk_off, &c->kg_longs, &c->kg_words, &c->kg_cs})
+                    &c->kg_chunk_off, &c->kg_longs, &c->kg_words, &c->kg_cs, &c->lf_pts, &c->lf_idx, &c->lf_eig,
+                    &c->lf_frames})
     release(*b);
   for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
   for (auto& ev : c->round_ev) cudaEventDestroy(ev);
@@ -3403,6 +3405,78 @@ int tknn_segment_reduce(tknn_ctx* c, const float* x, uint64_t n, int f, int stri
   TK_TRY(copy_back(c, out, d_out, (size_t)n_segments * f));
   TK_CUDA(c, cudaStreamSynchronize(st));
   return TKNN_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// surface normals and local frames (frames.cuh, DESIGN.md §3.12)
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+int local_frames_core(tknn_ctx* c, const float* points, uint64_t n, int stride, const int32_t* idx, uint64_t m, int k,
+                      int disambiguate, float* eigvals, float* frames_out) {
+  const char* what = "tknn_local_frames";
+  cudaStream_t st = c->stream;
+  ScratchScope scratch = frames_scratch(c);
+  const float* d_p = nullptr;
+  const int32_t* d_idx = nullptr;
+  if (n) TK_TRY(stage_in(c, points, (size_t)(n - 1) * stride + 3, c->lf_pts, &d_p));
+  TK_TRY(stage_in(c, idx, (size_t)m * k, c->lf_idx, &d_idx));
+  float *d_eig = nullptr, *d_frames = nullptr;
+  TK_TRY(out_view(c, eigvals, (size_t)m * 3, c->lf_eig, &d_eig));
+  TK_TRY(out_view(c, frames_out, (size_t)m * 9, c->lf_frames, &d_frames));
+  TK_TRY(ensure_round_events(c, 4));
+  cudaEvent_t* ev = c->round_ev.data();
+  uint32_t* sc = c->scalars.as<uint32_t>();
+  TK_CUDA(c, cudaEventRecord(c->ev[0], st));
+  TK_CUDA(c, cudaEventRecord(ev[0], st));
+  TK_CUDA(c, cudaMemsetAsync(sc + SC_QBAD, 0, sizeof(uint32_t), st));
+  const frames::Params P{d_p, d_idx, m, (uint32_t)n, k, stride, disambiguate, d_eig, d_frames, sc + SC_QBAD};
+  const unsigned blocks = (unsigned)std::max<uint64_t>(
+      1, std::min<uint64_t>((m + frames::THREADS - 1) / frames::THREADS, (uint64_t)c->sm_count * 16));
+  TK_CUDA(c, cudaEventRecord(ev[2], st));
+  frames::frames_kernel<<<blocks, frames::THREADS, 0, st>>>(P);
+  TK_CUDA(c, cudaGetLastError());
+  TK_CUDA(c, cudaEventRecord(ev[3], st));
+  TK_CUDA(c, cudaEventRecord(ev[1], st));
+  TK_CUDA(c, cudaEventRecord(c->ev[2], st));
+  TK_TRY(copy_back(c, eigvals, d_eig, (size_t)m * 3));
+  TK_TRY(copy_back(c, frames_out, d_frames, (size_t)m * 9));
+  TK_CUDA(c, cudaEventRecord(c->ev[3], st));
+  uint32_t bad = 0;
+  TK_TRY(fetch_words(c, sc + SC_QBAD, 1, nullptr, 0, &bad));  // synchronises the stream
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.search_ms, c->ev[0], c->ev[2]));
+  TK_CUDA(c, cudaEventElapsedTime(&c->stats.d2h_ms, c->ev[2], c->ev[3]));
+  c->stats.rounds = 1;
+  c->stats.round_queries[0] = m;
+  c->stats.kernel_launches = (uint32_t)(1 + c->mailbox_launches);
+  TK_TRY(finish_round_stats(c));
+  if (bad) return fail(c, TKNN_EINVAL, "%s: an idx entry lies outside {-1} and [0, n = %llu)", what, (unsigned long long)n);
+  return TKNN_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tknn_local_frames(tknn_ctx* c, const float* points, uint64_t n, int stride_floats, const int32_t* idx, uint64_t m,
+                      int k, int disambiguate, float* eigvals_out, float* frames_out) {
+  TK_TRY(check_ctx(c));
+  const char* what = "tknn_local_frames";
+  if (k < 1 || k > TKNN_MAX_K) return fail(c, TKNN_EINVAL, "%s: k = %d outside [1, %d]", what, k, TKNN_MAX_K);
+  if (stride_floats < 3) return fail(c, TKNN_EINVAL, "%s: stride %d below 3", what, stride_floats);
+  if (n >= (1ull << 31) || m >= (1ull << 31)) return fail(c, TKNN_EINVAL, "%s: n and m must be below 2^31", what);
+  if (disambiguate != 0 && disambiguate != 1)
+    return fail(c, TKNN_EINVAL, "%s: disambiguate = %d (must be 0 or 1)", what, disambiguate);
+  const bool work = m > 0 && (eigvals_out || frames_out);
+  if (work && (!idx || (n > 0 && !points))) return fail(c, TKNN_EINVAL, "%s: null idx or points", what);
+  ScopedDevice sd(c->device);
+  reset_search_stats(c);
+  c->stats.n_queries = m;
+  c->stats.k = k;
+  if (!work) return TKNN_OK;
+  return local_frames_core(c, points, n, stride_floats, idx, m, k, disambiguate, eigvals_out, frames_out);
 }
 
 }  // extern "C"

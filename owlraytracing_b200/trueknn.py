@@ -577,6 +577,29 @@ class TrueKNN:
                                                     f, self._in(offsets), n_seg, code, _ptr(out)))
         return out.reshape(n_seg) if x.ndim == 1 else out
 
+    def local_frames(self, points, idx, disambiguate: bool = False):
+        """Eigenvalues and eigenvectors of the covariance of every neighbourhood (tknn_local_frames, DESIGN.md §3.12).
+        points: [n, >= 3] float32, the first three columns are the position (more are skipped through the stride); idx:
+        [m, k] int32 rows of indices into points, -1 for an empty slot.  Per row, over its valid slots in slot order, in
+        fp32 without FMA: the centroid and the covariance (the mean over the neighbourhood) by chunked sums, cyclic Jacobi
+        (at most 8 sweeps) and the eigenvalues in ascending order.  disambiguate: PyTorch3D's sign rule for columns 0 and 2
+        (anchored at the point of the row's first valid slot), then column 1 = column 0 x column 2.  Returns (eigvals
+        [m, 3], frames [m, 3, 3]), frames[i, :, j] the j-th eigenvector (column 0: the normal); a row without a valid slot
+        is NaN.  The same bits on every run; no autograd.  Needs no build and leaves the last build untouched.  numpy
+        outputs for numpy points, CUDA tensors (on their device) for a CUDA tensor."""
+        points = _arg(points, np.float32, "points", ndim=2, copy=True)
+        if int(points.shape[1]) < 3:
+            raise ValueError(f"points must be [n, >= 3] (3-D positions), got {tuple(points.shape)}")
+        idx = _arg(idx, np.int32, "idx", ndim=2, copy=True)
+        n, stride, m, k = int(points.shape[0]), int(points.shape[1]), int(idx.shape[0]), int(idx.shape[1])
+        eig = self._empty(points, (m, 3), np.float32)
+        frames = self._empty(points, (m, 3, 3), np.float32)
+        if m == 0:  # an empty torch tensor has no address, and there is nothing to compute
+            return eig, frames
+        self._check(self._L.tknn_local_frames(self._h, self._in(points, null_if_empty=True), n, stride, self._in(idx), m,
+                                              k, int(bool(disambiguate)), _ptr(eig), _ptr(frames)))
+        return eig, frames
+
     def radius_search(self, radius: float, indices_only: bool = False, out=None):
         """Exact fixed-radius neighbour lists of every built point (closed ball, the point itself excluded).
 
@@ -1567,3 +1590,61 @@ def run_sample(argv: list[str], device: int = 0, neighbours_path: str | None = N
         write_neighbours(neighbours_path, idx, dist)
     return {"build_s": t1 - t0, "knn_s": t2 - t1, "total_s": total, "rounds": st["rounds"], "idx": idx, "dist": dist,
             "stats": st}
+
+
+def estimate_pointcloud_local_coord_frames(pos, neighborhood_size: int = 50, batch=None,
+                                           disambiguate_directions: bool = True, device: int | None = None):
+    """PyTorch3D's estimate_pointcloud_local_coord_frames on PyG batch vectors, exact and deterministic.  The
+    neighbourhood of a point is the point itself and its k - 1 nearest other points of its cloud (an exact kNN search,
+    ties by index), k = min(neighborhood_size, n); its covariance is the mean over the neighbourhood, and its
+    eigenvalues and eigenvectors come from a fixed cyclic Jacobi in fp32 (TrueKNN.local_frames, tknn_local_frames).
+    With disambiguate_directions, columns 0 and 2 follow PyTorch3D's sign rule (the side where most neighbours lie,
+    after Tombari et al.'s SHOT) and column 1 = column 0 x column 2, PyTorch3D's y = cross(n, z).
+    pos: [n, 3] float32, numpy or a CUDA tensor; batch (optional): cloud ids, as in knn_graph().  A cloud with fewer
+    than k points gives its rows -1 slots, which simply contribute nothing; an empty cloud has no rows.  Returns
+    (curvatures [n, 3] ascending, frames [n, 3, 3] with frames[i, :, j] the j-th eigenvector, column 0 the normal), of
+    pos's kind and device (device: the CUDA device for numpy input, default 0).  Every run gives the same bits.
+    The outputs carry no autograd: PyTorch3D differentiates through its eigensolver, and a deterministic backward of
+    the eigen-decomposition is not provided.  Raises ValueError for neighborhood_size < 1 or above 512 (after clamping
+    to n) and for positions that are not [n, 3]."""
+    pos = _arg(pos, np.float32, "pos", ndim=2, copy=True)
+    if int(pos.shape[1]) != 3:
+        raise ValueError(f"pos must be [n, 3] (3-D positions only), got {tuple(pos.shape)}")
+    if _is_tensor(pos) and not pos.is_cuda:
+        raise ValueError("pos must be a CUDA tensor or a numpy array")
+    if int(neighborhood_size) < 1:
+        raise ValueError(f"neighborhood_size = {neighborhood_size} must be >= 1")
+    n = int(pos.shape[0])
+    k = min(int(neighborhood_size), n)
+    if k > _lib.TKNN_MAX_K:
+        raise ValueError(f"neighborhood_size = {k} (after clamping to n) is above {_lib.TKNN_MAX_K}")
+    if batch is not None:
+        batch_to_offsets(batch, n)  # the same batch errors whatever k is
+    if n == 0:
+        return _zeros_like_rows(pos, (0, 3), np.float32), _zeros_like_rows(pos, (0, 3, 3), np.float32)
+    with TrueKNN(_device_of(pos, device)) as t:
+        own = _arange_like(pos, n, np.int32).reshape(n, 1)
+        if k == 1:
+            rows = own
+        else:
+            nbr, _ = t.build(pos, batch=batch).search(k - 1, indices_only=True)
+            if _is_tensor(nbr):
+                import torch
+
+                rows = torch.cat([own, nbr], 1)
+            else:
+                rows = np.concatenate([own, nbr], 1)
+        return t.local_frames(pos, rows, disambiguate=disambiguate_directions)
+
+
+def estimate_pointcloud_normals(pos, neighborhood_size: int = 50, batch=None, disambiguate_directions: bool = True,
+                                device: int | None = None):
+    """PyTorch3D's estimate_pointcloud_normals on PyG batch vectors: column 0 of
+    estimate_pointcloud_local_coord_frames(), the unit eigenvector of the smallest eigenvalue of each neighbourhood's
+    covariance.  Returns [n, 3] float32 of pos's kind; same arguments, rules and errors, no autograd.  The sign rule
+    points a normal to the side where most of its neighbours lie (inward on a convex surface).  To orient normals toward
+    a viewpoint instead (Open3D's and PCL's convention), flip them in torch:
+        normals = torch.where(((viewpoint - pos) * normals).sum(1, keepdim=True) < 0, -normals, normals)"""
+    _, frames = estimate_pointcloud_local_coord_frames(pos, neighborhood_size, batch, disambiguate_directions, device)
+    normals = frames[:, :, 0]
+    return normals.contiguous() if _is_tensor(normals) else np.ascontiguousarray(normals)
